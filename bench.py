@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the path-tracing hot path (BASELINE.json: Msamples/s and Mrays/s vs the host-CPU Embree path).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload dragon|cornell|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload dragon|cornell|...] [--dump-outputs DIR]
 
 Workload (config.workload): scenes/dragon.json, 1024 x 1024, PathTracer, startBounce 0, lastBounce 10 — the
 configuration the north-star target is quoted on (">= 100x the reference CPU Msamples/s on dragon.json on 1 B200").
@@ -228,6 +228,8 @@ def main():
     ap.add_argument("--paths-per-wave", type=int, default=0, help="override the library's wave size (paths resident per wave)")
     ap.add_argument("--bvh-builder", type=int, default=1, choices=[0, 1], help="1: device builder (default), 0: host binned-SAH builder")
     ap.add_argument("--lanes", type=int, default=0, help="part-waves traced side by side (ptc_set_option lanes); 0: the library's choice per wave")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the framebuffers the timed calls left (cumulative fp32 radiance sums) to DIR/<name>.npy")
     args = ap.parse_args()
     args.spp_per_step_given = args.spp_per_step is not None
     if args.spp_per_step is None:
@@ -310,6 +312,10 @@ def main():
     sampler.start()
     ms = timed(lambda i: step_device(i + args.warmup), args.steps)
     st = ctx.stats()
+    outputs = {}
+    if args.dump_outputs and rank == 0:
+        # the caller's radianceLookup after the last timed step: sums of every sample rendered so far (warm-up steps included)
+        outputs["radiance_device"] = (staging if distributed else local).view(height, width, 3).cpu().numpy()
     launches = int(st.kernel_launches)
     rays = int(st.closest_rays + st.shadow_rays)
     samples_total = float(n_pix) * total_spp * args.steps
@@ -373,6 +379,11 @@ def main():
     e2e_value = samples_total / (float(e2e_ms.item()) * 1e-3) * 1e-6
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        outputs["radiance_host"] = (pinned.numpy().reshape(height, width, 3) if distributed else host_accum).copy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, array in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), array)
 
     # ---- roofline of the dominant kernel (extend), rank 0 only: stage-timed pass, then counted pass (same seed)
     roofline, stages = None, None

@@ -7,7 +7,7 @@ import re
 import numpy as np
 import pytest
 
-from pathed_b200._binding import REPO_ROOT, PathedError, SceneFile, create_context, cuda_lib, host_lib
+from pathed_b200._binding import REPO_ROOT, PathedError, SceneFile, cuda_lib, host_lib
 
 
 def _declared(prefix):
@@ -24,15 +24,13 @@ def test_cuda_library_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback():
-    try:
-        import torch
-        has_gpu = torch.cuda.is_available()
-    except Exception:
-        has_gpu = False
-    if has_gpu:
-        pytest.skip("GPU present")
-    with pytest.raises(PathedError):
-        create_context(0)
+    # in a process of its own with an empty CUDA_VISIBLE_DEVICES, which hides every device, so it sees no GPU on a GPU machine as well
+    import subprocess
+    import sys
+    code = ("import sys\nsys.path.insert(0, %r)\nfrom pathed_b200._binding import PathedError, create_context\n"
+            "try:\n    create_context(0)\nexcept PathedError:\n    print('refused')\n" % REPO_ROOT)
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True)
+    assert r.returncode == 0 and r.stdout.strip() == "refused", r.stdout + r.stderr
 
 
 def test_product_does_not_link_the_oracle():

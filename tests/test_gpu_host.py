@@ -171,9 +171,15 @@ def test_multi_gpu_job_matches_single_gpu(tmp_path):
 
 
 REF_CUDA = os.path.join(REPO_ROOT, "oracle", "_ref", "pathed_ref_cuda")
+REF_CUDA_GOLDEN = os.path.join(REPO_ROOT, "tests", "golden", "reference_binding.json")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_CUDA), reason="oracle/_ref/pathed_ref_cuda is built where /root/reference is mounted (oracle/ref/build_ref.sh)")
+def image_digest(a):
+    """sha256 of an image's fp32 bytes: the comparisons below are bit for bit, so a digest stores as much as the image"""
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(a, np.float32).tobytes()).hexdigest()
+
+
 @pytest.mark.parametrize("scene,integrator,width,height", [
     ("scenes/cornell.json", "PathTracer", 48, 40), ("scenes/cornell-glass.json", "PathTracer", 48, 40), ("scenes/mis-pbrt.json", "PathTracer", 60, 40),
     ("scenes/teapot.json", "PathTracer", 64, 36), ("scenes/textured.json", "PathTracer", 48, 40), ("scenes/instanced.json", "PathTracer", 48, 36),
@@ -181,11 +187,22 @@ REF_CUDA = os.path.join(REPO_ROOT, "oracle", "_ref", "pathed_ref_cuda")
 def test_reference_tree_bound_to_the_cuda_library_renders_the_same_image(tmp_path, scene, integrator, width, height):
     """INTEGRATION.md as a binary: the UNMODIFIED reference (its Job, scene / OBJ parsers, Image, Integrator::run) linked against the
     Embree-API shim + libpathed_cuda (oracle/ref/cuda_main.cpp) and the repository's own host layer must feed the same geometry,
-    materials, lights and camera -- the final images are equal bit for bit (same Philox streams), and so are the checkpoint files"""
+    materials, lights and camera -- the final images are equal bit for bit (same Philox streams), and so are the checkpoint files.
+    The reference tree is not part of this repository, so tests/golden/reference_binding.json keeps the SHA-256 digests of what the
+    binding writes for these jobs (Image::m_raw, final.exr, auto-00004spp.exr); the repository's render and `pathed` are held to them
+    everywhere, and to the binary itself where oracle/_ref/pathed_ref_cuda is built."""
     if not os.path.exists(os.path.join(REPO_ROOT, scene)):
         pytest.skip(scene + " not generated")
     job, ours = _run_job(tmp_path / "ours", scene=scene, integrator=integrator, width=width, height=height, spp=4, wave_spp=1)
     assert ours.returncode == 0, ours.stdout + ours.stderr
+    ctx = load_scene(scene, width, height, integrator=1 if integrator == "VolumePathTracer" else 0)
+    want = (ctx.render(0x5EED, 0, 4, 0, 10) / np.float32(4))[::-1]         # the repository's host layer + the same library
+    stored = json.load(open(REF_CUDA_GOLDEN))["%s %s %dx%d" % (scene, integrator, width, height)]
+    assert want.mean() > 0 and image_digest(want) == stored["image"], (float(want.mean()), stored["mean"])
+    for name in ("final.exr", "auto-00004spp.exr"):
+        assert image_digest(read_exr(str(tmp_path / "ours" / "out" / name))) == stored[name], name
+    if not os.path.exists(REF_CUDA):
+        return
     job["output_directory"] = str(tmp_path / "ref" / "out")
     os.makedirs(str(tmp_path / "ref"), exist_ok=True)
     path = str(tmp_path / "ref" / "job.json")
@@ -194,9 +211,7 @@ def test_reference_tree_bound_to_the_cuda_library_renders_the_same_image(tmp_pat
     r = subprocess.run([REF_CUDA, "--root", REPO_ROOT, path, "--raw", raw], capture_output=True, text=True)
     assert r.returncode == 0 and "REF_CUDA_RESULT" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
     got = np.fromfile(raw, np.float32).reshape(height, width, 3)          # Image::m_raw of the reference's Image, top scanline first
-    ctx = load_scene(scene, width, height, integrator=1 if integrator == "VolumePathTracer" else 0)
-    want = (ctx.render(0x5EED, 0, 4, 0, 10) / np.float32(4))[::-1]         # the repository's host layer + the same library
-    assert want.mean() > 0 and np.array_equal(got, want)
+    assert np.array_equal(got, want)
     for name in ("final.exr", "auto-00004spp.exr"):                         # the reference's tinyexr writer against this repository's
         a = read_exr(str(tmp_path / "ref" / "out" / name)); b = read_exr(str(tmp_path / "ours" / "out" / name))
         assert np.array_equal(a, b), name
