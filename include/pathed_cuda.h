@@ -256,6 +256,34 @@ int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t 
                                  uint32_t *ticket);
 int ptc_framebuffer_gather_end(ptc_ctx *root, uint32_t ticket, float *out_rgb_host);
 
+/* ---- adaptive sampling: each pixel stops once its estimated relative error meets a target ------------------------------ */
+/* A render is a sequence of passes into the context's framebuffer.  Pass 1 gives every pixel samples 0 .. min_spp - 1; each later
+ * pass gives every pixel still ACTIVE the next min(step_spp, max_spp - n) samples, so all active pixels share one count n.  After a
+ * pass pixel p stops when, for every channel c, var_c / n <= threshold^2 * (mean_c^2 + 1e-2), with mean_c = S_c / n, var_c =
+ * max(0, (M_c - n mean_c^2) / (n - 1)), S the framebuffer's sum and M the sum of the squared samples, evaluated in fp64: the
+ * expected per-pixel term of the relMSE metric (x - r)^2 / (r^2 + 1e-2) (SURVEY 8(d)) is at most threshold^2.  A non-finite
+ * estimate never stops a pixel (a NaN sample keeps it going to max_spp); every pixel stops at max_spp.
+ * A path's random stream is keyed by (pixel, sample index) and the resolve adds a pixel's samples in sample order, so pixel p of
+ * the adaptive framebuffer holds exactly, bit for bit, what ptc_render(seed, 0, n_p, ...) accumulates there from zero.
+ * Device memory: 24 bytes per pixel besides the framebuffer (second moments 3 x fp32, count, two pixel-list entries). */
+typedef struct ptc_adaptive_desc {
+    float threshold;   /* tau > 0: the relMSE target is tau^2 */
+    uint32_t min_spp;  /* >= 2: samples of the first pass */
+    uint32_t step_spp; /* >= 1: samples per later pass */
+    uint32_t max_spp;  /* >= min_spp */
+} ptc_adaptive_desc;
+/* clears the framebuffer, the second moments and the counts; every pixel active.  PTC_ERR_INVALID for a bad descriptor.
+ * Until the next ptc_framebuffer_clear the framebuffer belongs to the adaptive render: ptc_framebuffer_render* return
+ * PTC_ERR_STATE (ptc_render, ptc_render_device and ptc_framebuffer_gather work as usual; the gather with divisor 1 reads the sums) */
+int ptc_adaptive_begin(ptc_ctx *ctx, const ptc_adaptive_desc *desc);
+/* one pass on the context's stream, returns when the stopping test is done (one host synchronisation per pass): active_out =
+ * pixels still active (0: the render is complete and further calls are no-ops), spp_out = the samples the active pixels hold
+ * after the pass.  Either pointer may be NULL.  PTC_ERR_STATE before ptc_adaptive_begin.  ptc_stats.samples counts the samples traced. */
+int ptc_adaptive_pass(ptc_ctx *ctx, uint64_t seed, int start_bounce, int last_bounce, uint32_t *active_out, uint32_t *spp_out);
+/* spp_per_pixel (W*H) = the samples each pixel holds so far, second_moment_rgb (3*W*H) = per-channel sums of the squared samples;
+ * index row*W + col, row 0 = bottom, like the framebuffer.  Either may be NULL.  PTC_ERR_STATE before ptc_adaptive_begin. */
+int ptc_adaptive_state(ptc_ctx *ctx, uint32_t *spp_per_pixel, float *second_moment_rgb);
+
 /* ---- the random streams on their own (known-answer tests; need no scene) ---------------------- */
 /* Philox4x32-10, the generator that replaces RandomGenerator (src/random_generator.cpp:4-11) and std::rand (src/camera.cpp:51-52)
  * on the device: out[4i..4i+3] = philox(counter = counters[4i..4i+3], key = keys[2i..2i+1]) */

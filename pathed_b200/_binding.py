@@ -29,6 +29,10 @@ class MaterialDesc(ctypes.Structure):
                 ("checker_off", ctypes.c_float * 3), ("checker_resolution", ctypes.c_float * 2), ("texture", ctypes.c_uint32)]
 
 
+class AdaptiveDesc(ctypes.Structure):
+    _fields_ = [("threshold", ctypes.c_float), ("min_spp", ctypes.c_uint32), ("step_spp", ctypes.c_uint32), ("max_spp", ctypes.c_uint32)]
+
+
 class Stats(ctypes.Structure):
     _fields_ = [(n, ctypes.c_uint64) for n in ("closest_rays", "shadow_rays", "samples", "kernel_launches", "bvh_nodes",
                                                "bvh_triangles", "bvh_bytes", "extend_inner_visits", "extend_triangle_tests",
@@ -255,6 +259,24 @@ class Api:
         out = np.zeros((self.height, self.width, 3), np.float32)
         self._call("framebuffer_gather_end", ctypes.c_uint32(ticket), _ptr(out))
         return out
+
+    # ---- adaptive sampling (ptc_adaptive_*): passes into the context's framebuffer until every pixel meets the relMSE target
+    def adaptive_begin(self, threshold, min_spp, step_spp, max_spp):
+        desc = AdaptiveDesc(float(threshold), int(min_spp), int(step_spp), int(max_spp))
+        self._call("adaptive_begin", ctypes.byref(desc))
+
+    def adaptive_pass(self, seed, start_bounce, last_bounce):
+        """one pass; returns (pixels still active, samples per active pixel after the pass)"""
+        active, spp = ctypes.c_uint32(), ctypes.c_uint32()
+        self._call("adaptive_pass", ctypes.c_uint64(seed), ctypes.c_int(start_bounce), ctypes.c_int(last_bounce), ctypes.byref(active), ctypes.byref(spp))
+        return active.value, spp.value
+
+    def adaptive_state(self):
+        """(samples per pixel [h, w] uint32, per-channel sums of squared samples [h, w, 3] fp32), row 0 = bottom like the sums"""
+        counts = np.zeros((self.height, self.width), np.uint32)
+        m2 = np.zeros((self.height, self.width, 3), np.float32)
+        self._call("adaptive_state", _ptr(counts), _ptr(m2))
+        return counts, m2
 
     # ---- random streams (known-answer tests)
     def philox(self, counters, keys):

@@ -17,6 +17,7 @@
 #include "volume.cuh"
 
 #include <cuda_runtime.h>
+#include <cub/device/device_select.cuh>
 
 #include <algorithm>
 #include <cstdio>
@@ -104,6 +105,7 @@ struct WaveParams {
     uint32_t nPixels;
     int32_t startBounce, lastBounce;
     uint32_t groupShift;   // log2 of the sample group (slotToPixelSample)
+    const uint32_t *pixels; // the wave's pixel list (adaptive passes: nPixels pixels still active); null = every pixel of the image
 };
 
 // Device-side bookkeeping of one wave: queue sizes and work cursors per bounce (no host synchronisation inside a wave)
@@ -128,6 +130,15 @@ __device__ __forceinline__ uint32_t slotToPixel(uint32_t q, uint32_t width, uint
     const uint32_t tile = q >> 5, within = q & 31u, tilesX = width >> 3;
     const uint32_t col = (tile % tilesX) * 8u + (within & 7u), row = (tile / tilesX) * 4u + (within >> 3);
     return row * width + col;
+}
+// Pixel slot q of a wave -> pixel, the one mapping every stage uses: an adaptive pass lists the pixels still active (a stable
+// selection from slotToPixel's order, so a warp's camera rays stay in neighbouring tiles); a wave without a list covers the image.
+// LISTED = false: compiled for waves without a list (the material kernels, whose register budget the test of the pointer would
+// strain: +8..40 B of spills per class measured with -Xptxas -v)
+template <bool LISTED = true>
+__device__ __forceinline__ uint32_t wavePixel(uint32_t q, const WaveParams &wp, uint32_t width, uint32_t height)
+{
+    return LISTED && wp.pixels ? __ldg(wp.pixels + q) : slotToPixel(q, width, height);
 }
 
 // Origin slot p of a wave -> (pixel slot q, sample s of the wave).  G = 2^groupShift consecutive slots hold consecutive samples of
@@ -177,7 +188,7 @@ __global__ void __launch_bounds__(256) generateKernel(DScene scene, PathBuffers 
     for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < nPaths; p += gridDim.x * blockDim.x) {
         uint32_t q, s;
         slotToPixelSample(p, wp, q, s);
-        const uint32_t pixel = slotToPixel(q, (uint32_t)scene.width, (uint32_t)scene.height);
+        const uint32_t pixel = wavePixel(q, wp, (uint32_t)scene.width, (uint32_t)scene.height);
         Rng rng;
         rng.initPhilox(wp.seed, pixel, wp.firstSample + s);
         rng.beginVertex(0);
@@ -554,7 +565,8 @@ __global__ void __launch_bounds__(256, PTC_LOGIC_MIN_BLOCKS) logicKernel(DScene 
 
 // ------------------------------------------------------------------------------------------------ K4 material
 // Vertex k + 1 of every surviving path whose hit surface has material class TYPE: Intersection, BSDF sample, NEE set-up.
-template <int TYPE>
+// LISTED: the wave has a pixel list (wavePixel)
+template <int TYPE, bool LISTED>
 #ifndef PTC_MATERIAL_MIN_BLOCKS
 #define PTC_MATERIAL_MIN_BLOCKS 8
 #endif
@@ -581,7 +593,7 @@ __global__ void __launch_bounds__(128, PTC_MATERIAL_MIN_BLOCKS) materialKernel(D
             Rng rng;
             uint32_t oq, os;
             slotToPixelSample(origin, wp, oq, os);
-            rng.initPhilox(wp.seed, slotToPixel(oq, (uint32_t)scene.width, (uint32_t)scene.height), wp.firstSample + os);
+            rng.initPhilox(wp.seed, wavePixel<LISTED>(oq, wp, (uint32_t)scene.width, (uint32_t)scene.height), wp.firstSample + os);
             rng.beginVertex((uint32_t)(k + 1));
             BsdfSample bs;
             bsdfSample<TYPE>(m, bi, rng, bs);
@@ -628,21 +640,55 @@ __global__ void __launch_bounds__(128, PTC_MATERIAL_MIN_BLOCKS) materialKernel(D
 // Checkpoints that fall inside a wave (src/integrator.cpp:87-92 saves the image after 1, 2, 4, ... samples): the resolve keeps a copy
 // of the running sums after `at[i]` samples of the wave in dst[i], so a wave does not have to end at every power of two
 struct CheckpointPlan { uint32_t n; uint32_t at[PTC_MAX_CHECKPOINTS]; float *dst[PTC_MAX_CHECKPOINTS]; };
-__global__ void __launch_bounds__(256) accumulateKernel(PathBuffers pb, WaveParams wp, float *accum, uint32_t width, uint32_t height, const __grid_constant__ CheckpointPlan plan)
+// MOMENTS (adaptive passes): moments[3 * pixel + c] += x_c^2 for every sample x, in sample order like the sums
+template <bool MOMENTS>
+__global__ void __launch_bounds__(256) accumulateKernel(PathBuffers pb, WaveParams wp, float *accum, float *moments, uint32_t width, uint32_t height, const __grid_constant__ CheckpointPlan plan)
 {
     for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < wp.nPixels; q += gridDim.x * blockDim.x) {
-        const size_t pixel = slotToPixel(q, width, height);
+        const size_t pixel = wavePixel(q, wp, width, height);
         float r = accum[3 * pixel], g = accum[3 * pixel + 1], b = accum[3 * pixel + 2];
+        float mr = 0.f, mg = 0.f, mb = 0.f;
+        if (MOMENTS) { mr = moments[3 * pixel]; mg = moments[3 * pixel + 1]; mb = moments[3 * pixel + 2]; }
         uint32_t next = 0;
         for (uint32_t s = 0; s < wp.sppWave; s++) { // radianceLookup += color, one sample after the other (src/sample_integrator.cpp:61-63)
             while (next < plan.n && plan.at[next] == s) { float *d = plan.dst[next++]; d[3 * pixel] = r; d[3 * pixel + 1] = g; d[3 * pixel + 2] = b; }
             const float4 c = streamLoad(pb.out + pixelSampleToSlot(q, s, wp));
             r += c.x; g += c.y; b += c.z;
+            if (MOMENTS) { mr += c.x * c.x; mg += c.y * c.y; mb += c.z * c.z; }
         }
         while (next < plan.n) { float *d = plan.dst[next++]; d[3 * pixel] = r; d[3 * pixel + 1] = g; d[3 * pixel + 2] = b; }
         accum[3 * pixel] = r; accum[3 * pixel + 1] = g; accum[3 * pixel + 2] = b;
+        if (MOMENTS) { moments[3 * pixel] = mr; moments[3 * pixel + 1] = mg; moments[3 * pixel + 2] = mb; }
     }
 }
+
+// Adaptive sampling: the stopping test after a pass that ended at n samples per listed pixel.  Pixel p stops when for every channel
+// var_c / n <= tau^2 (mean_c^2 + 1e-2) (mean = S / n, var = max(0, (M - n mean^2) / (n - 1)), in fp64): the expected per-pixel
+// term of the relMSE metric (x - r)^2 / (r^2 + 1e-2) is below the target tau^2.  A non-finite estimate never stops a pixel, and
+// every pixel stops at n = maxSpp.  counts[pixel] = n for every listed pixel; next[q] = the pixel if it goes on, else ~0u (dropped by
+// the stable selection that follows).  --fmad=false: no contraction, the test is the plain fp64 expression.
+__global__ void __launch_bounds__(256) adaptiveTestKernel(WaveParams wp, const float *sums, const float *moments, uint32_t *counts, uint32_t *next,
+                                                          uint32_t width, uint32_t height, double tau2, uint32_t n, uint32_t maxSpp)
+{
+    for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < wp.nPixels; q += gridDim.x * blockDim.x) {
+        const uint32_t pixel = wavePixel(q, wp, width, height);
+        bool stop = n >= maxSpp;
+        if (!stop) {
+            stop = true;
+            const double dn = (double)n;
+            for (int c = 0; c < 3; c++) {
+                const double mean = (double)sums[3 * (size_t)pixel + c] / dn;
+                const double sq = mean * mean;
+                double var = ((double)moments[3 * (size_t)pixel + c] - dn * sq) / (dn - 1.0);
+                if (var < 0.0) { var = 0.0; }
+                stop = stop && isfinite(mean) && isfinite(var) && var / dn <= tau2 * (sq + 1e-2);
+            }
+        }
+        counts[pixel] = n;
+        next[q] = stop ? ~0u : pixel;
+    }
+}
+struct StillActive { __device__ __forceinline__ bool operator()(uint32_t v) const { return v != ~0u; } };
 
 // ------------------------------------------------------------------------------------------------ VolumePathTracer
 // One thread follows one path from the camera to its end (volume.cuh: volumeRadiance); warps pull 32 paths at a time from a
@@ -669,7 +715,7 @@ __global__ void __launch_bounds__(128, PTC_VOLUME_MIN_BLOCKS) volumePathKernel(c
         if (p < nPaths) {
             uint32_t q, s;
             slotToPixelSample(p, wp, q, s);
-            const uint32_t pixel = slotToPixel(q, (uint32_t)scene.width, (uint32_t)scene.height);
+            const uint32_t pixel = wavePixel(q, wp, (uint32_t)scene.width, (uint32_t)scene.height);
             Rng rng;
             rng.initPhilox(wp.seed, pixel, wp.firstSample + s);
             rng.beginVertex(0);
@@ -1114,6 +1160,18 @@ struct ptc_ctx {
     uint32_t bvhNodeCount = 0, bvhTriangleCount = 0;
     bool hostBvhFetched = true;
     void *buildWorkspace = nullptr; // the device builder's working set, released with the context (bvh.h: buildWideBVHDevice)
+    // adaptive sampling (ptc_adaptive_*): between begin and the next ptc_framebuffer_clear the framebuffer belongs to the passes.
+    // Per pixel: second moments (3 x fp32, next to the framebuffer's sums), sample count, and two list entries (active pixels,
+    // the stopping test's output) = 24 B, plus cub's selection scratch
+    struct Adaptive {
+        bool on = false;
+        ptc_adaptive_desc desc = {0.f, 0, 0, 0};
+        uint32_t n = 0, active = 0; // the samples every active pixel holds; pixels still active
+        size_t pixels = 0;          // what the buffers are sized for
+        float *moments = nullptr;
+        uint32_t *counts = nullptr, *list = nullptr, *next = nullptr, *selected = nullptr, *selectedHost = nullptr;
+        void *scratch = nullptr; size_t scratchBytes = 0;
+    } adaptive;
     uint64_t samples = 0, launches = 0;
     float lastRenderMs = 0.f;
     // stage timing: CUDA events on the launching stream around every launch, summed per kernel class
@@ -1207,7 +1265,7 @@ int ptc_create(int device, ptc_ctx **out)
     ctx->gridTraverse = ctx->numSMs * std::max(perSM, 1);
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, logicKernel, 256, 0);
     ctx->gridLogic = ctx->numSMs * std::max(perSM, 1);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, materialKernel<PTC_PLASTIC>, 128, 0);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, (materialKernel<PTC_PLASTIC, false>), 128, 0);
     ctx->gridShade = ctx->numSMs * std::max(perSM, 1);
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, volumePathKernel<false>, 128, 0);
     ctx->gridVolume = ctx->numSMs * std::max(perSM, 1);
@@ -1247,6 +1305,9 @@ void ptc_destroy(ptc_ctx *ctx)
     }
     if (ctx->laneFork) { cudaEventDestroy(ctx->laneFork); }
     cudaFree(ctx->framebuffer); cudaFree(ctx->gatherStage);
+    cudaFree(ctx->adaptive.moments); cudaFree(ctx->adaptive.counts); cudaFree(ctx->adaptive.list); cudaFree(ctx->adaptive.next);
+    cudaFree(ctx->adaptive.selected); cudaFree(ctx->adaptive.scratch);
+    if (ctx->adaptive.selectedHost) { cudaFreeHost(ctx->adaptive.selectedHost); }
     for (float *snapshot : ctx->snapshots) { cudaFree(snapshot); }
     for (auto &g : ctx->gathers) { cudaFree(g.device); if (g.pinned) { cudaFreeHost(g.pinned); } if (g.done) { cudaEventDestroy(g.done); } }
     if (ctx->gatherRead) { cudaEventDestroy(ctx->gatherRead); }
@@ -1993,7 +2054,10 @@ static int ensureVolumeBuffers(ptc_ctx *ctx, uint32_t capacity)
 }
 
 #define LAUNCH_MATERIAL(TYPE) \
-    if (ctx->classMask & (1u << TYPE)) { materialKernel<TYPE><<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc, bc + 1); ctx->launches++; }
+    if (ctx->classMask & (1u << TYPE)) { \
+        if (wp.pixels) { materialKernel<TYPE, true><<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc, bc + 1); } \
+        else { materialKernel<TYPE, false><<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc, bc + 1); } \
+        ctx->launches++; }
 #define LAUNCH_VOLUME_MATERIAL(TYPE) \
     if (ctx->classMask & (1u << TYPE)) { volumeMaterialKernel<TYPE><<<ctx->gridVolumeShade, 128, 0, stream>>>(s, pb, vb, wp, bc, bc + 1); ctx->launches++; }
 
@@ -2002,7 +2066,7 @@ static int ensureVolumeBuffers(ptc_ctx *ctx, uint32_t capacity)
 // stream per lane, so that the stages of different lanes share the SMs (ptc_ctx::lanes); nLanes = 1 is the plain sequence.
 // volume: the VolumePathTracer's stages (volume_wavefront.cuh) -- merged probe / continuation rays, two kinds of shadow rays, its own
 // logic and material kernels; bounce 0 is the PathTracer's.
-static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan *plans, int nLanes, float *accumDevice, cudaStream_t callerStream, bool volume)
+static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan *plans, int nLanes, float *accumDevice, float *moments, cudaStream_t callerStream, bool volume)
 {
     const DScene &s = ctx->scene;
     struct LaneState { PathBuffers pb; VolumeBuffers vb; BounceCounters *cnt; cudaStream_t stream, shadowStream; cudaEvent_t shadeDone, shadowDone; };
@@ -2123,7 +2187,9 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
             CUDA_TRY(ctx, cudaStreamWaitEvent(callerStream, x.done, 0));
         }
         StageTimer t(ctx, callerStream, STAGE_OTHER);
-        accumulateKernel<<<std::min<uint32_t>((wps[i].nPixels + 255) / 256, (uint32_t)ctx->gridSimple * 4), 256, 0, callerStream>>>(lanes[i].pb, wps[i], accumDevice, (uint32_t)s.width, (uint32_t)s.height, plans[i]);
+        const uint32_t grid = std::min<uint32_t>((wps[i].nPixels + 255) / 256, (uint32_t)ctx->gridSimple * 4);
+        if (moments) { accumulateKernel<true><<<grid, 256, 0, callerStream>>>(lanes[i].pb, wps[i], accumDevice, moments, (uint32_t)s.width, (uint32_t)s.height, plans[i]); }
+        else { accumulateKernel<false><<<grid, 256, 0, callerStream>>>(lanes[i].pb, wps[i], accumDevice, nullptr, (uint32_t)s.width, (uint32_t)s.height, plans[i]); }
         tallyKernel<<<1, 32, 0, callerStream>>>(lanes[i].cnt, ctx->totals);
         ctx->launches += 2;
     }
@@ -2132,12 +2198,16 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
     return PTC_OK;
 }
 
+// The pixels of an adaptive pass (ptc_adaptive_pass): `count` pixels, listed on the device (null list: the whole image in slotToPixel's
+// order), whose accumulation also adds the squared samples into `moments`.  moments = null: a plain render of every pixel.
+struct PassPixels { const uint32_t *list = nullptr; uint32_t count = 0; float *moments = nullptr; };
+
 // VolumePathTracer waves: one volumePathKernel launch over pixels x sppWave paths, then the same in-order accumulation
 static int renderVolume(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp, uint32_t sppWave, int start, int last, float *accumDevice, cudaStream_t stream,
-                        const Checkpoints &checkpoints)
+                        const Checkpoints &checkpoints, const PassPixels &pass)
 {
     const DScene &s = ctx->scene;
-    const uint32_t nPixels = (uint32_t)s.width * (uint32_t)s.height;
+    const uint32_t nPixels = pass.moments ? pass.count : (uint32_t)s.width * (uint32_t)s.height;
     if (ctx->volumeCapacity < nPixels * sppWave) {
         cudaFree(ctx->volumeOut); ctx->volumeOut = nullptr; ctx->volumeCapacity = 0;
         CUDA_TRY(ctx, cudaMalloc((void **)&ctx->volumeOut, (size_t)nPixels * sppWave * sizeof(float4)));
@@ -2149,7 +2219,7 @@ static int renderVolume(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint3
     for (uint32_t done = 0; done < nSpp; done += sppWave) {
         WaveParams wp;
         wp.seed = seed; wp.firstSample = firstSample + done; wp.sppWave = std::min(sppWave, nSpp - done); wp.nPixels = nPixels; wp.groupShift = groupShiftFor(wp.sppWave);
-        wp.startBounce = start; wp.lastBounce = last;
+        wp.startBounce = start; wp.lastBounce = last; wp.pixels = pass.list;
         CUDA_TRY(ctx, cudaMemsetAsync(ctx->volumeCursor, 0, sizeof(uint32_t), stream));
         {
             StageTimer t(ctx, stream, STAGE_SHADE);
@@ -2160,7 +2230,9 @@ static int renderVolume(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint3
         {
             StageTimer t(ctx, stream, STAGE_OTHER);
             const CheckpointPlan plan = planFor(checkpoints, wp.firstSample, wp.sppWave, done == 0, done + sppWave >= nSpp);
-            accumulateKernel<<<std::min<uint32_t>((nPixels + 255) / 256, (uint32_t)ctx->gridSimple * 4), 256, 0, stream>>>(pb, wp, accumDevice, (uint32_t)s.width, (uint32_t)s.height, plan);
+            const uint32_t grid = std::min<uint32_t>((nPixels + 255) / 256, (uint32_t)ctx->gridSimple * 4);
+            if (pass.moments) { accumulateKernel<true><<<grid, 256, 0, stream>>>(pb, wp, accumDevice, pass.moments, (uint32_t)s.width, (uint32_t)s.height, plan); }
+            else { accumulateKernel<false><<<grid, 256, 0, stream>>>(pb, wp, accumDevice, nullptr, (uint32_t)s.width, (uint32_t)s.height, plan); }
         }
         ctx->launches += 2;
         CUDA_TRY(ctx, cudaGetLastError());
@@ -2171,23 +2243,23 @@ static int renderVolume(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint3
 }
 
 static int renderInternal(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp, int start, int last, float *accumDevice, cudaStream_t stream,
-                          const Checkpoints &checkpoints = Checkpoints())
+                          const Checkpoints &checkpoints = Checkpoints(), const PassPixels &pass = PassPixels())
 {
     if (start < 0 || (last != -1 && start > last)) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bad bounce window [%d, %d]", start, last); }
     if (last == -1 || last > PTC_MAX_BOUNCES) { last = PTC_MAX_BOUNCES; }
-    const uint32_t nPixels = (uint32_t)ctx->scene.width * (uint32_t)ctx->scene.height;
+    const uint32_t nPixels = pass.moments ? pass.count : (uint32_t)ctx->scene.width * (uint32_t)ctx->scene.height;
     uint32_t sppWave = (uint32_t)std::max<int64_t>(1, ctx->pathsPerWave / (int64_t)nPixels);
     sppWave = std::min(sppWave, std::max(nSpp, 1u));
     const bool volume = ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER;
     // the one-thread-per-path kernel stays for instanced scenes (the volume traversal kernels test world-space leaves only) and as an option
-    if (volume && (ctx->volumeMegakernel || ctx->scene.bvh.placements)) { return renderVolume(ctx, seed, firstSample, nSpp, sppWave, start, last, accumDevice, stream, checkpoints); }
+    if (volume && (ctx->volumeMegakernel || ctx->scene.bvh.placements)) { return renderVolume(ctx, seed, firstSample, nSpp, sppWave, start, last, accumDevice, stream, checkpoints, pass); }
     int rc = ensurePathBuffers(ctx, nPixels * sppWave);
     if (rc) { return rc; }
     if (volume && (rc = ensureVolumeBuffers(ctx, nPixels * sppWave))) { return rc; }
     for (uint32_t done = 0; done < nSpp; done += sppWave) {
         WaveParams wp;
         wp.seed = seed; wp.firstSample = firstSample + done; wp.sppWave = std::min(sppWave, nSpp - done); wp.nPixels = nPixels; wp.groupShift = groupShiftFor(wp.sppWave);
-        wp.startBounce = start; wp.lastBounce = last;
+        wp.startBounce = start; wp.lastBounce = last; wp.pixels = pass.list;
         // lanes: consecutive blocks of the wave's samples.  Two lanes, four when the wave is small (measured on five scenes,
         // profiles/r02_sweep_lanes.txt); one while a stage or traversal counter pass describes one launch sequence at a time
         int nLanes = ctx->lanes > 0 ? ctx->lanes : ((uint64_t)nPixels * wp.sppWave <= (1u << 25) ? 4 : 2);
@@ -2201,7 +2273,7 @@ static int renderInternal(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uin
             w.firstSample = wp.firstSample + at; w.sppWave = std::min(perLane, wp.sppWave - at); w.groupShift = groupShiftFor(w.sppWave);
             plans[used] = planFor(checkpoints, w.firstSample, w.sppWave, done == 0 && at == 0, done + sppWave >= nSpp && at + perLane >= wp.sppWave);
         }
-        if ((rc = launchWave(ctx, wps, plans, used, accumDevice, stream, volume))) { return rc; }
+        if ((rc = launchWave(ctx, wps, plans, used, accumDevice, pass.moments, stream, volume))) { return rc; }
     }
     ctx->samples += (uint64_t)nPixels * nSpp;
     return PTC_OK;
@@ -2276,6 +2348,7 @@ int ptc_framebuffer_clear(ptc_ctx *ctx)
     const int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer, 0, ctx->framebufferSize * sizeof(float), ctx->stream));
+    ctx->adaptive.on = false;
     return PTC_OK;
 }
 
@@ -2289,6 +2362,7 @@ int ptc_framebuffer_render_checkpoints(ptc_ctx *ctx, uint64_t seed, uint32_t fir
     NEED_COMMIT(ctx);
     if (nCounts > PTC_MAX_CHECKPOINTS || (nCounts && !sampleCounts)) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bad checkpoint list (at most %d)", PTC_MAX_CHECKPOINTS); }
     for (uint32_t i = 1; i < nCounts; i++) { if (sampleCounts[i] <= sampleCounts[i - 1]) { CTX_FAIL(ctx, PTC_ERR_INVALID, "checkpoint sample counts must ascend"); } }
+    if (ctx->adaptive.on) { CTX_FAIL(ctx, PTC_ERR_STATE, "the framebuffer holds an adaptive render: ptc_framebuffer_clear first"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
@@ -2387,6 +2461,86 @@ int ptc_framebuffer_gather(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers
     uint32_t ticket = 0;
     const int rc = ptc_framebuffer_gather_begin(root, peers, nPeers, -1, divisor, &ticket);
     return rc ? rc : ptc_framebuffer_gather_end(root, ticket, out);
+}
+
+int ptc_adaptive_begin(ptc_ctx *ctx, const ptc_adaptive_desc *desc)
+{
+    NEED_COMMIT(ctx);
+    if (!desc || !(desc->threshold > 0.f) || desc->min_spp < 2 || desc->step_spp < 1 || desc->max_spp < desc->min_spp) {
+        CTX_FAIL(ctx, PTC_ERR_INVALID, "bad adaptive sampling descriptor (threshold > 0, min_spp >= 2, step_spp >= 1, max_spp >= min_spp)");
+    }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const int rc = ensureFramebuffer(ctx);
+    if (rc) { return rc; }
+    ptc_ctx::Adaptive &a = ctx->adaptive;
+    const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
+    if (a.pixels != pixels) {
+        cudaFree(a.moments); cudaFree(a.counts); cudaFree(a.list); cudaFree(a.next); cudaFree(a.scratch);
+        a.moments = nullptr; a.counts = a.list = a.next = nullptr; a.scratch = nullptr; a.pixels = 0;
+        CUDA_TRY(ctx, cudaMalloc((void **)&a.moments, 3 * pixels * sizeof(float)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&a.counts, pixels * sizeof(uint32_t)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&a.list, pixels * sizeof(uint32_t)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&a.next, pixels * sizeof(uint32_t)));
+        if (!a.selected) { CUDA_TRY(ctx, cudaMalloc((void **)&a.selected, sizeof(uint32_t))); }
+        if (!a.selectedHost) { CUDA_TRY(ctx, cudaMallocHost((void **)&a.selectedHost, sizeof(uint32_t))); }
+        a.scratchBytes = 0;
+        CUDA_TRY(ctx, cub::DeviceSelect::If(nullptr, a.scratchBytes, a.next, a.list, a.selected, (int)pixels, StillActive(), ctx->stream));
+        CUDA_TRY(ctx, cudaMalloc(&a.scratch, std::max<size_t>(a.scratchBytes, 1)));
+        a.pixels = pixels;
+    }
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer, 0, ctx->framebufferSize * sizeof(float), ctx->stream));
+    CUDA_TRY(ctx, cudaMemsetAsync(a.moments, 0, 3 * pixels * sizeof(float), ctx->stream));
+    CUDA_TRY(ctx, cudaMemsetAsync(a.counts, 0, pixels * sizeof(uint32_t), ctx->stream));
+    a.desc = *desc; a.n = 0; a.active = (uint32_t)pixels; a.on = true;
+    return PTC_OK;
+}
+
+// One pass: samples n .. n + k - 1 of the active pixels (k = min_spp for the first pass, then min(step_spp, max_spp - n)), in
+// one or more waves over the pixel list, then the stopping test and the stable selection of the pixels that go on.  The host
+// needs the survivor count to size the next pass: one synchronisation per pass.
+int ptc_adaptive_pass(ptc_ctx *ctx, uint64_t seed, int start, int last, uint32_t *activeOut, uint32_t *sppOut)
+{
+    NEED_COMMIT(ctx);
+    ptc_ctx::Adaptive &a = ctx->adaptive;
+    if (!a.on) { CTX_FAIL(ctx, PTC_ERR_STATE, "no adaptive render on this context: ptc_adaptive_begin first"); }
+    if (a.pixels != (size_t)ctx->scene.width * ctx->scene.height || ctx->framebufferSize != 3 * a.pixels) {
+        CTX_FAIL(ctx, PTC_ERR_STATE, "the resolution changed during the adaptive render");
+    }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    if (a.active) {
+        const uint32_t k = a.n == 0 ? a.desc.min_spp : std::min(a.desc.step_spp, a.desc.max_spp - a.n);
+        PassPixels pass; pass.list = a.n == 0 ? nullptr : a.list; pass.count = a.active; pass.moments = a.moments;
+        const int rc = renderInternal(ctx, seed, a.n, k, start, last, ctx->framebuffer, ctx->stream, Checkpoints(), pass);
+        if (rc) { return rc; }
+        const uint32_t n = a.n + k;
+        WaveParams wp; memset(&wp, 0, sizeof(wp));
+        wp.nPixels = a.active; wp.pixels = pass.list;
+        const double tau = (double)a.desc.threshold;
+        adaptiveTestKernel<<<std::min<uint32_t>((a.active + 255) / 256, (uint32_t)ctx->gridSimple * 4), 256, 0, ctx->stream>>>(
+            wp, ctx->framebuffer, a.moments, a.counts, a.next, (uint32_t)ctx->scene.width, (uint32_t)ctx->scene.height, tau * tau, n, a.desc.max_spp);
+        CUDA_TRY(ctx, cudaGetLastError());
+        size_t bytes = a.scratchBytes;
+        CUDA_TRY(ctx, cub::DeviceSelect::If(a.scratch, bytes, a.next, a.list, a.selected, (int)a.active, StillActive(), ctx->stream));
+        CUDA_TRY(ctx, cudaMemcpyAsync(a.selectedHost, a.selected, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->launches += 2;
+        a.n = n; a.active = *a.selectedHost;
+    }
+    if (activeOut) { *activeOut = a.active; }
+    if (sppOut) { *sppOut = a.n; }
+    return PTC_OK;
+}
+
+int ptc_adaptive_state(ptc_ctx *ctx, uint32_t *sppPerPixel, float *secondMoment)
+{
+    NEED_COMMIT(ctx);
+    const ptc_ctx::Adaptive &a = ctx->adaptive;
+    if (!a.on) { CTX_FAIL(ctx, PTC_ERR_STATE, "no adaptive render on this context: ptc_adaptive_begin first"); }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    if (sppPerPixel) { CUDA_TRY(ctx, cudaMemcpyAsync(sppPerPixel, a.counts, a.pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream)); }
+    if (secondMoment) { CUDA_TRY(ctx, cudaMemcpyAsync(secondMoment, a.moments, 3 * a.pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream)); }
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return PTC_OK;
 }
 
 int ptc_resolve_device(ptc_ctx *ctx, const float *accum, float *out, uint32_t spp, void *stream)

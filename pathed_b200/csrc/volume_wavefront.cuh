@@ -328,7 +328,7 @@ __global__ void __launch_bounds__(128, PTC_VOLUME_MATERIAL_MIN_BLOCKS) volumeMat
             Rng rng;
             uint32_t oq, os;
             slotToPixelSample(origin, wp, oq, os);
-            rng.initPhilox(wp.seed, slotToPixel(oq, (uint32_t)scene.width, (uint32_t)scene.height), wp.firstSample + os);
+            rng.initPhilox(wp.seed, wavePixel(oq, wp, (uint32_t)scene.width, (uint32_t)scene.height), wp.firstSample + os);
             rng.beginVertex((uint32_t)b);
             V3 modulation = mk(1.f, 1.f, 1.f);
             int32_t medium = -1;

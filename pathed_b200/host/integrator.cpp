@@ -3,6 +3,7 @@
 // here one call into the C ABI covers a whole batch of samples per pixel and the framebuffer stays in HBM between checkpoints.
 #include "pathed.hpp"
 
+#include "exr_io.hpp"
 #include "scene_parser.hpp"
 
 #include <algorithm>
@@ -227,6 +228,7 @@ void CudaPathTracer::run(Image &image, Scene &scene, std::function<void(RenderSt
     const double preBegin = now();
     preprocess(scene);
     printf("Pre-process complete (%0.1fs elapsed)\n", now() - preBegin);
+    if (g_job->adaptive()) { runAdaptive(image, scene, callback, quit); return; }
 
     const int gpus = scene.gpus();
     const int start = m_bounceController.startBounce(), last = m_bounceController.lastBounce();
@@ -295,6 +297,61 @@ void CudaPathTracer::run(Image &image, Scene &scene, std::function<void(RenderSt
         if (!more) { break; }
         current = next;
     }
+}
+
+// Adaptive sampling (ptc_adaptive_pass): every pass gives the pixels still active the same number of further samples and ends with
+// the stopping test on the device.  After each pass the host fetches the sums and the per-pixel counts and shows the per-pixel means
+// S_p / n_p (divided as the K7 resolve divides); a pass that ends at a power-of-two count is saved as that checkpoint.  At the end
+// adaptive-spp.exr holds the sample count of every pixel (one fp32 channel Y).
+void CudaPathTracer::runAdaptive(Image &image, Scene &scene, std::function<void(RenderStatus)> callback, bool *quit)
+{
+    const int width = g_job->width(), height = g_job->height(), maxSpp = g_job->spp();
+    const size_t pixels = (size_t)width * height;
+    ptc_ctx *ctx = scene.context(0);
+    check(ctx, ptc_set_integrator(ctx, m_integrator), "integrator");
+    ptc_adaptive_desc desc;
+    desc.threshold = g_job->adaptiveThreshold();
+    desc.min_spp = (uint32_t)g_job->adaptiveMinSpp(); desc.step_spp = (uint32_t)g_job->adaptiveStepSpp(); desc.max_spp = (uint32_t)maxSpp;
+    check(ctx, ptc_adaptive_begin(ctx, &desc), "adaptive begin");
+    std::vector<float> sums(3 * pixels), resolved(3 * pixels);
+    std::vector<uint32_t> counts(pixels);
+    const double loopBegin = now();
+    for (int pass = 1;; pass++) {
+        const double begin = now();
+        uint32_t active = 0, n = 0;
+        check(ctx, ptc_adaptive_pass(ctx, m_seed, m_bounceController.startBounce(), m_bounceController.lastBounce(), &active, &n), "adaptive pass");
+        check(ctx, ptc_framebuffer_gather(ctx, nullptr, 0, 1, sums.data()), "framebuffer gather");
+        check(ctx, ptc_adaptive_state(ctx, counts.data(), nullptr), "adaptive state");
+        uint64_t samples = 0;
+        for (size_t p = 0; p < pixels; p++) {
+            samples += counts[p];
+            for (int c = 0; c < 3; c++) { resolved[3 * p + c] = sums[3 * p + c] / (float)counts[p]; }
+        }
+        const double end = now();
+        m_samples = samples;
+        m_nextSample = n;
+        m_renderSeconds = end - loopBegin;
+        {
+            std::lock_guard<std::mutex> guard(image.getLock());
+            image.setSpp((int)n);
+            image.setAll(resolved.data());
+            if ((n & (n - 1)) == 0) { image.saveCheckpoint("auto"); }
+        }
+        postwave(scene, (int)n);
+        RenderStatus status;
+        status.setSample((int)n);
+        callback(status);
+        std::ostringstream line;
+        line << "adaptive pass " << pass << ": " << n << "/" << maxSpp << " spp, " << active << " pixels active" << std::fixed << std::setprecision(1)
+             << " (" << (end - begin) << "s elapsed)";
+        Logger::line(line.str());
+        if (active == 0 || *quit) { break; }
+    }
+    std::vector<float> plane(pixels); // top scanline first, like every image the job writes
+    for (int row = 0; row < height; row++) {
+        for (int col = 0; col < width; col++) { plane[(size_t)(height - 1 - row) * width + col] = (float)counts[(size_t)row * width + col]; }
+    }
+    saveEXR(g_job->outputDirectory() + "adaptive-spp.exr", width, height, {"Y"}, {plane.data()}, false);
 }
 
 } // namespace pathed

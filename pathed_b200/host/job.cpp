@@ -6,6 +6,7 @@
 
 #include <algorithm>
 #include <cerrno>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <fstream>
@@ -51,7 +52,19 @@ static Json parseJobFile(std::istream &jobFile)
 Job::Job(std::istream &jobFile)
     : m_json(new Json(parseJobFile(jobFile))),
       m_bounceController((*m_json)["startBounce"].asInt(), (*m_json)["lastBounce"].asInt())
-{}
+{
+    if (!adaptive()) { return; }
+    const double threshold = (*m_json)["adaptive_threshold"].asNumber();
+    if (!(threshold > 0.0) || !std::isfinite(threshold)) { throw std::runtime_error("adaptive_threshold must be a number > 0"); }
+    for (const char *key : {"adaptive_min_spp", "adaptive_step_spp"}) {
+        const Json &value = (*m_json)[key];
+        if (!value.isNull() && (!value.isNumber() || value.asNumber() != std::floor(value.asNumber()))) { throw std::runtime_error(std::string(key) + " must be an integer"); }
+    }
+    if (adaptiveMinSpp() < 2) { throw std::runtime_error("adaptive_min_spp must be >= 2"); }
+    if (adaptiveStepSpp() < 1) { throw std::runtime_error("adaptive_step_spp must be >= 1"); }
+    if (spp() < adaptiveMinSpp()) { throw std::runtime_error("spp (the most samples a pixel gets) must be >= adaptive_min_spp"); }
+    if (gpus() != 1) { throw std::runtime_error("adaptive sampling runs on one GPU: set \"gpus\": 1 or drop adaptive_threshold"); }
+}
 
 Job::~Job() {}
 
@@ -73,6 +86,10 @@ std::string Job::scene() const { return (*m_json)["scene"].asString(); }
 int Job::gpus() const { return (*m_json)["gpus"].isNumber() ? std::max(1, (*m_json)["gpus"].asInt()) : 1; }
 uint64_t Job::seed() const { return (*m_json)["seed"].isNumber() ? (uint64_t)(*m_json)["seed"].asNumber() : 0x5EEDull; }
 int Job::waveSpp() const { return (*m_json)["wave_spp"].isNumber() ? std::max(1, (*m_json)["wave_spp"].asInt()) : 64; }
+bool Job::adaptive() const { return !(*m_json)["adaptive_threshold"].isNull(); }
+float Job::adaptiveThreshold() const { return adaptive() ? (float)(*m_json)["adaptive_threshold"].asNumber() : 0.f; }
+int Job::adaptiveMinSpp() const { return (*m_json)["adaptive_min_spp"].isNumber() ? (*m_json)["adaptive_min_spp"].asInt() : 16; }
+int Job::adaptiveStepSpp() const { return (*m_json)["adaptive_step_spp"].isNumber() ? (*m_json)["adaptive_step_spp"].asInt() : 16; }
 
 void Job::init()
 {

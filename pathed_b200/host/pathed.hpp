@@ -70,6 +70,13 @@ public:
     int gpus() const;          // "gpus": number of devices the spp are split over (default 1)
     uint64_t seed() const;     // "seed": Philox key (default 0x5EED; the reference seeds from random_device)
     int waveSpp() const;       // "wave_spp": max samples per pixel per device call between callbacks (default 64)
+    // adaptive sampling (ptc_adaptive_*): present "adaptive_threshold" (tau > 0) makes the job adaptive, "spp" is then the most
+    // samples a pixel gets; "adaptive_min_spp" (>= 2, <= spp, default 16) samples every pixel gets, "adaptive_step_spp" (>= 1,
+    // default 16) samples per later pass.  Checked by the constructor, like "gpus" == 1 (adaptive sampling runs on one GPU)
+    bool adaptive() const;
+    float adaptiveThreshold() const;
+    int adaptiveMinSpp() const;
+    int adaptiveStepSpp() const;
 
     // string -> integrator (src/job.cpp:65-97); anything but "PathTracer" throws const char* "Unimplemented"
     std::shared_ptr<Integrator> integrator() const;
@@ -195,6 +202,8 @@ private:
     uint32_t m_nextSample = 0;
     double m_renderSeconds = 0.0;
     uint64_t m_samples = 0;
+    // the job's adaptive render: passes on device 0 until every pixel has stopped
+    void runAdaptive(Image &image, Scene &scene, std::function<void(RenderStatus)> callback, bool *quit);
 };
 
 // "VolumePathTracer" (src/volume_path_tracer.cpp): the same device-resident loop with the participating-media L()
