@@ -284,6 +284,48 @@ int ptc_adaptive_pass(ptc_ctx *ctx, uint64_t seed, int start_bounce, int last_bo
  * index row*W + col, row 0 = bottom, like the framebuffer.  Either may be NULL.  PTC_ERR_STATE before ptc_adaptive_begin. */
 int ptc_adaptive_state(ptc_ctx *ctx, uint32_t *spp_per_pixel, float *second_moment_rgb);
 
+/* ---- denoising: first-hit guide buffers and a variance-guided a-trous filter (DESIGN §10) ------------------------------ */
+/* snapshot argument of ptc_framebuffer_gather_begin: sum the second-moment buffers of root + peers instead of the framebuffers
+ * (a context's adaptive render's moments, else its option "framebuffer_moments" buffer; use divisor 1).  PTC_ERR_STATE for a
+ * context whose moments do not cover every sample of its framebuffer: the option must be on at ptc_framebuffer_clear and at every
+ * framebuffer render since (a context that rendered no samples has zero moments). */
+#define PTC_GATHER_MOMENTS (-2)
+/* Adds into the host buffers (index row*W + col, row 0 = bottom, `+=` like ptc_render), for every pixel and every sample s in
+ * first_sample .. first_sample + n_spp - 1, in sample order and in fp32, what the first hit of the path tracer's camera ray for
+ * (seed, pixel, s) sees -- the same two Philox draws of vertex 0 jitter cameraRay(row + jy, col + jx), the closest hit is
+ * Scene::testIntersect's (ptc_intersect_full):
+ *   albedo_rgb (3*W*H): Lambertian / OrenNayar / Plastic: the diffuse colour, checkerboard or texture the BSDF uses; Mirror,
+ *                       Glass, Microfacet, Passthrough: (1, 1, 1); a miss: 0
+ *   normal_xyz (3*W*H): the shading normal, unflipped (in an instance's local space for instanced geometry); a miss: 0
+ *   depth      (W*H):   the hit distance t; a miss: 0
+ *   hits       (W*H):   +1 per sample that hits.
+ * The same for both integrators; draws no random numbers of the paths and leaves the framebuffer alone. */
+int ptc_render_aovs(ptc_ctx *ctx, uint64_t seed, uint32_t first_sample, uint32_t n_spp, float *albedo_rgb, float *normal_xyz,
+                    float *depth, uint32_t *hits);
+/* the spatial filter of SVGF (Schied et al., HPG 2017) with an albedo edge-stopping term; the formula is in DESIGN §10 */
+typedef struct ptc_denoise_desc {
+    uint32_t iterations; /* a-trous levels, steps 1, 2, 4, ...: 0 .. 10 (0 returns S / n) */
+    float sigma_l;       /* > 0: luminance, in units of the blurred standard deviation of the mean */
+    float sigma_n;       /* >= 0: exponent of the normal term */
+    float sigma_z;       /* > 0: relative depth difference per unit of the step */
+    float sigma_a;       /* > 0: L1 albedo difference */
+    float eps;           /* > 0 */
+} ptc_denoise_desc;
+#define PTC_DENOISE_DEFAULTS {5u, 4.f, 128.f, 1.f, 0.1f, 1e-6f}
+typedef struct ptc_denoise_input {
+    const float *sums;       /* 3*W*H: sums of the samples (the framebuffer) */
+    const float *moments;    /* 3*W*H: sums of the squared samples */
+    const uint32_t *counts;  /* W*H samples per pixel (adaptive renders), or NULL: every pixel has `spp` */
+    uint32_t spp;
+    const float *albedo_rgb, *normal_xyz, *depth; /* ptc_render_aovs over aov_spp samples */
+    const uint32_t *hits;
+    uint32_t aov_spp;
+} ptc_denoise_input;
+/* out_rgb (3*W*H) = the denoised mean colour; W, H from the context's camera; all pointers are host pointers.  Runs on the
+ * context's device and returns when the output is on the host.  Deterministic: two calls give the same bytes.  PTC_ERR_INVALID
+ * for a bad descriptor, a missing input, a pixel with fewer than 2 samples or aov_spp == 0. */
+int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_input *in, float *out_rgb);
+
 /* ---- the random streams on their own (known-answer tests; need no scene) ---------------------- */
 /* Philox4x32-10, the generator that replaces RandomGenerator (src/random_generator.cpp:4-11) and std::rand (src/camera.cpp:51-52)
  * on the device: out[4i..4i+3] = philox(counter = counters[4i..4i+3], key = keys[2i..2i+1]) */
@@ -344,7 +386,11 @@ int ptc_set_option(ptc_ctx *ctx, const char *name, int64_t value); /* "stage_tim
                                                                       0 host), "volume_megakernel" (1: VolumePathTracer as one
                                                                       thread per path instead of wavefront stages), "lanes" (a
                                                                       wave traced as n part-waves side by side on n streams; 0,
-                                                                      the default: chosen per wave; the image does not depend on n) */
+                                                                      the default: chosen per wave; the image does not depend on n),
+                                                                      "framebuffer_moments" (1: ptc_framebuffer_render* also add the
+                                                                      squared samples into a context buffer that ptc_framebuffer_clear
+                                                                      zeroes, read with PTC_GATHER_MOMENTS; set it before the clear;
+                                                                      the sums do not change) */
 /* scalar reference traversal of the device BVH on the host side of the library: counts inner-node
  * visits and triangle tests per ray (SURVEY.md §8(d): algorithmic bytes per ray) */
 int ptc_count_traversal(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, uint64_t *inner_visits, uint64_t *triangle_tests);

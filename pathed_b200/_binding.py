@@ -20,6 +20,7 @@ PATH_TRACER, VOLUME_PATH_TRACER = 0, 1
 NO_MEDIUM = 0xFFFFFFFF
 MAX_EVENTS = 8
 BECKMANN, GGX = 0, 1
+GATHER_MOMENTS = -2  # snapshot of framebuffer_gather_begin: the sums of the squared samples
 
 
 class MaterialDesc(ctypes.Structure):
@@ -31,6 +32,20 @@ class MaterialDesc(ctypes.Structure):
 
 class AdaptiveDesc(ctypes.Structure):
     _fields_ = [("threshold", ctypes.c_float), ("min_spp", ctypes.c_uint32), ("step_spp", ctypes.c_uint32), ("max_spp", ctypes.c_uint32)]
+
+
+class DenoiseDesc(ctypes.Structure):
+    _fields_ = [("iterations", ctypes.c_uint32), ("sigma_l", ctypes.c_float), ("sigma_n", ctypes.c_float), ("sigma_z", ctypes.c_float),
+                ("sigma_a", ctypes.c_float), ("eps", ctypes.c_float)]
+
+
+DENOISE_DEFAULTS = {"iterations": 5, "sigma_l": 4.0, "sigma_n": 128.0, "sigma_z": 1.0, "sigma_a": 0.1, "eps": 1e-6}  # PTC_DENOISE_DEFAULTS
+
+
+class DenoiseInput(ctypes.Structure):
+    _fields_ = [("sums", ctypes.c_void_p), ("moments", ctypes.c_void_p), ("counts", ctypes.c_void_p), ("spp", ctypes.c_uint32),
+                ("albedo_rgb", ctypes.c_void_p), ("normal_xyz", ctypes.c_void_p), ("depth", ctypes.c_void_p), ("hits", ctypes.c_void_p),
+                ("aov_spp", ctypes.c_uint32)]
 
 
 class Stats(ctypes.Structure):
@@ -238,7 +253,10 @@ class Api:
         self._call("framebuffer_render", ctypes.c_uint64(seed), ctypes.c_uint32(first_sample), ctypes.c_uint32(n_spp),
                    ctypes.c_int(start_bounce), ctypes.c_int(last_bounce))
 
-    def framebuffer_gather(self, peers=(), divisor=1):
+    def framebuffer_gather(self, peers=(), divisor=1, snapshot=-1):
+        """snapshot -1: the framebuffers; GATHER_MOMENTS (-2): the second moments (use divisor 1); i >= 0: checkpoint snapshot i"""
+        if snapshot != -1:
+            return self.framebuffer_gather_end(self.framebuffer_gather_begin(peers, snapshot, divisor))
         out = np.zeros((self.height, self.width, 3), np.float32)
         arr = (ctypes.c_void_p * max(len(peers), 1))(*[p.ctx.value for p in peers])
         self._call("framebuffer_gather", arr, ctypes.c_uint32(len(peers)), ctypes.c_uint32(divisor), _ptr(out))
@@ -277,6 +295,47 @@ class Api:
         m2 = np.zeros((self.height, self.width, 3), np.float32)
         self._call("adaptive_state", _ptr(counts), _ptr(m2))
         return counts, m2
+
+    # ---- denoising (ptc_render_aovs, ptc_denoise; DESIGN §10)
+    def render_aovs(self, seed, first_sample, n_spp, aovs=None):
+        """first-hit guide buffers of samples first_sample .. first_sample + n_spp - 1, added into `aovs` (a dict like the one returned;
+        None: zeros): albedo [h, w, 3], normal [h, w, 3], depth [h, w] fp32 sums and hits [h, w] uint32, row 0 = bottom"""
+        h, w = self.height, self.width
+        if aovs is None:
+            aovs = {"albedo": np.zeros((h, w, 3), np.float32), "normal": np.zeros((h, w, 3), np.float32),
+                    "depth": np.zeros((h, w), np.float32), "hits": np.zeros((h, w), np.uint32)}
+        for name, dtype, size in (("albedo", np.float32, 3 * h * w), ("normal", np.float32, 3 * h * w), ("depth", np.float32, h * w),
+                                  ("hits", np.uint32, h * w)):
+            a = aovs[name]
+            assert a.dtype == dtype and a.flags.c_contiguous and a.size == size, name
+        self._call("render_aovs", ctypes.c_uint64(seed), ctypes.c_uint32(first_sample), ctypes.c_uint32(n_spp), _ptr(aovs["albedo"]),
+                   _ptr(aovs["normal"]), _ptr(aovs["depth"]), _ptr(aovs["hits"]))
+        return aovs
+
+    def denoise(self, sums, moments, counts_or_spp, aovs, aov_spp, **params):
+        """ptc_denoise: the denoised mean colour [h, w, 3].  counts_or_spp: per-pixel sample counts [h, w] or one spp for every pixel;
+        params: iterations, sigma_l, sigma_n, sigma_z, sigma_a, eps (DENOISE_DEFAULTS for the ones not given)"""
+        unknown = set(params) - set(DENOISE_DEFAULTS)
+        if unknown:
+            raise TypeError("unknown denoise parameters %s" % sorted(unknown))
+        p = dict(DENOISE_DEFAULTS, **params)
+        desc = DenoiseDesc(int(p["iterations"]), *[float(p[k]) for k in ("sigma_l", "sigma_n", "sigma_z", "sigma_a", "eps")])
+        n = 3 * self.width * self.height
+        f32 = lambda a, size: np.ascontiguousarray(a, np.float32).reshape(size)
+        keep = {"sums": f32(sums, n), "moments": f32(moments, n), "albedo": f32(aovs["albedo"], n), "normal": f32(aovs["normal"], n),
+                "depth": f32(aovs["depth"], n // 3), "hits": np.ascontiguousarray(aovs["hits"], np.uint32).reshape(n // 3)}
+        inp = DenoiseInput()
+        inp.sums, inp.moments = keep["sums"].ctypes.data, keep["moments"].ctypes.data
+        if np.ndim(counts_or_spp) == 0:
+            inp.counts, inp.spp = None, int(counts_or_spp)
+        else:
+            keep["counts"] = np.ascontiguousarray(counts_or_spp, np.uint32).reshape(n // 3)
+            inp.counts, inp.spp = keep["counts"].ctypes.data, 0
+        inp.albedo_rgb, inp.normal_xyz = keep["albedo"].ctypes.data, keep["normal"].ctypes.data
+        inp.depth, inp.hits, inp.aov_spp = keep["depth"].ctypes.data, keep["hits"].ctypes.data, int(aov_spp)
+        out = np.zeros((self.height, self.width, 3), np.float32)
+        self._call("denoise", ctypes.byref(desc), ctypes.byref(inp), _ptr(out))
+        return out
 
     # ---- random streams (known-answer tests)
     def philox(self, counters, keys):

@@ -739,6 +739,7 @@ __global__ void __launch_bounds__(128, PTC_VOLUME_MIN_BLOCKS) volumePathKernel(c
 }
 
 #include "volume_wavefront.cuh"
+#include "denoise.cuh"
 
 __global__ void resolveKernel(const float *accum, float *out, uint32_t n, uint32_t spp) // src/integrator.cpp:74-85
 {
@@ -1172,6 +1173,14 @@ struct ptc_ctx {
         uint32_t *counts = nullptr, *list = nullptr, *next = nullptr, *selected = nullptr, *selectedHost = nullptr;
         void *scratch = nullptr; size_t scratchBytes = 0;
     } adaptive;
+    // option "framebuffer_moments": the framebuffer renders also add the squared samples into `moments` (3 x fp32 per pixel, zeroed
+    // by ptc_framebuffer_clear), the input of ptc_denoise that PTC_GATHER_MOMENTS gathers.  complete: the moments cover every sample
+    // the framebuffer holds (the option was on at the last clear and at every render since); the gather refuses them otherwise
+    struct FramebufferMoments { bool on = false, complete = false; float *moments = nullptr; size_t size = 0; } fbMoments;
+    // ptc_denoise's device buffers: the staged inputs (15 x 4 B per pixel), guide records (32 B), two colour records (16 B each)
+    struct Denoise { size_t pixels = 0; float *inputs = nullptr; float4 *guide = nullptr, *colour[2] = {nullptr, nullptr}; } denoise;
+    // ptc_render_aovs's device copy of the guide buffers (8 x 4 B per pixel)
+    struct Aovs { size_t pixels = 0; float *buffer = nullptr; } aovs;
     uint64_t samples = 0, launches = 0;
     float lastRenderMs = 0.f;
     // stage timing: CUDA events on the launching stream around every launch, summed per kernel class
@@ -1308,6 +1317,8 @@ void ptc_destroy(ptc_ctx *ctx)
     cudaFree(ctx->adaptive.moments); cudaFree(ctx->adaptive.counts); cudaFree(ctx->adaptive.list); cudaFree(ctx->adaptive.next);
     cudaFree(ctx->adaptive.selected); cudaFree(ctx->adaptive.scratch);
     if (ctx->adaptive.selectedHost) { cudaFreeHost(ctx->adaptive.selectedHost); }
+    cudaFree(ctx->fbMoments.moments); cudaFree(ctx->aovs.buffer);
+    cudaFree(ctx->denoise.inputs); cudaFree(ctx->denoise.guide); cudaFree(ctx->denoise.colour[0]); cudaFree(ctx->denoise.colour[1]);
     for (float *snapshot : ctx->snapshots) { cudaFree(snapshot); }
     for (auto &g : ctx->gathers) { cudaFree(g.device); if (g.pinned) { cudaFreeHost(g.pinned); } if (g.done) { cudaEventDestroy(g.done); } }
     if (ctx->gatherRead) { cudaEventDestroy(ctx->gatherRead); }
@@ -2341,6 +2352,18 @@ static int ensureFramebuffer(ptc_ctx *ctx)
     return PTC_OK;
 }
 
+// the buffer of option "framebuffer_moments", sized like the framebuffer; a new one starts at zero (like a new framebuffer)
+static int ensureFramebufferMoments(ptc_ctx *ctx)
+{
+    ptc_ctx::FramebufferMoments &m = ctx->fbMoments;
+    if (m.size == ctx->framebufferSize) { return PTC_OK; }
+    cudaFree(m.moments); m.moments = nullptr; m.size = 0;
+    CUDA_TRY(ctx, cudaMalloc((void **)&m.moments, ctx->framebufferSize * sizeof(float)));
+    CUDA_TRY(ctx, cudaMemsetAsync(m.moments, 0, ctx->framebufferSize * sizeof(float), ctx->stream));
+    m.size = ctx->framebufferSize;
+    return PTC_OK;
+}
+
 int ptc_framebuffer_clear(ptc_ctx *ctx)
 {
     NEED_COMMIT(ctx);
@@ -2348,6 +2371,13 @@ int ptc_framebuffer_clear(ptc_ctx *ctx)
     const int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer, 0, ctx->framebufferSize * sizeof(float), ctx->stream));
+    // with the option on the moments exist from here, so that a context that gets no samples still has (zero) moments to gather
+    if (ctx->fbMoments.on) {
+        const int mrc = ensureFramebufferMoments(ctx);
+        if (mrc) { return mrc; }
+        CUDA_TRY(ctx, cudaMemsetAsync(ctx->fbMoments.moments, 0, ctx->fbMoments.size * sizeof(float), ctx->stream));
+    }
+    ctx->fbMoments.complete = ctx->fbMoments.on;
     ctx->adaptive.on = false;
     return PTC_OK;
 }
@@ -2371,12 +2401,18 @@ int ptc_framebuffer_render_checkpoints(ptc_ctx *ctx, uint64_t seed, uint32_t fir
         CUDA_TRY(ctx, cudaMalloc((void **)&buffer, ctx->framebufferSize * sizeof(float)));
         ctx->snapshots.push_back(buffer);
     }
+    if (!ctx->fbMoments.on) { ctx->fbMoments.complete = false; }
+    else if ((rc = ensureFramebufferMoments(ctx))) { return rc; }
     if (nSpp == 0) { // no samples for this context in the wave: every snapshot is the framebuffer as it stands
         for (uint32_t i = 0; i < nCounts; i++) { CUDA_TRY(ctx, cudaMemcpyAsync(ctx->snapshots[i], ctx->framebuffer, ctx->framebufferSize * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream)); }
         return PTC_OK;
     }
     Checkpoints cp; cp.counts = sampleCounts; cp.n = nCounts; cp.dst = ctx->snapshots.data();
-    return renderInternal(ctx, seed, firstSample, nSpp, start, last, ctx->framebuffer, ctx->stream, cp);
+    PassPixels pass; // every pixel, no list; with the moments option the accumulation also adds the squared samples (the sums are the same)
+    if (ctx->fbMoments.on) {
+        pass.count = (uint32_t)(ctx->framebufferSize / 3); pass.moments = ctx->fbMoments.moments;
+    }
+    return renderInternal(ctx, seed, firstSample, nSpp, start, last, ctx->framebuffer, ctx->stream, cp, pass);
 }
 
 int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, int snapshot, uint32_t divisor, uint32_t *ticketOut)
@@ -2387,8 +2423,21 @@ int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t 
     int rc = ensureFramebuffer(root);
     if (rc) { return rc; }
     const size_t n = root->framebufferSize;
-    auto source = [&](ptc_ctx *c) -> const float * { return snapshot < 0 ? c->framebuffer : (size_t)snapshot < c->snapshots.size() ? c->snapshots[snapshot] : nullptr; };
-    if (!source(root)) { CTX_FAIL(root, PTC_ERR_STATE, "no snapshot %d was rendered", snapshot); }
+    // PTC_GATHER_MOMENTS: the second moments of an adaptive render, else those of the framebuffer renders
+    auto moments = [&](ptc_ctx *c) -> const float * {
+        if (c->adaptive.on) { return c->adaptive.moments; }
+        return c->fbMoments.complete && c->fbMoments.size == n ? c->fbMoments.moments : nullptr;
+    };
+    auto source = [&](ptc_ctx *c) -> const float * {
+        if (snapshot == PTC_GATHER_MOMENTS) { return moments(c); }
+        return snapshot < 0 ? c->framebuffer : (size_t)snapshot < c->snapshots.size() ? c->snapshots[snapshot] : nullptr;
+    };
+    if (!source(root)) {
+        if (snapshot == PTC_GATHER_MOMENTS) {
+            CTX_FAIL(root, PTC_ERR_STATE, "no second moments of every sample on this context (option framebuffer_moments on since the last clear, or an adaptive render)");
+        }
+        CTX_FAIL(root, PTC_ERR_STATE, "no snapshot %d was rendered", snapshot);
+    }
     FramebufferSet set;
     set.fb[0] = source(root); set.count = 1;
     size_t staged = 0;
@@ -2492,6 +2541,7 @@ int ptc_adaptive_begin(ptc_ctx *ctx, const ptc_adaptive_desc *desc)
     CUDA_TRY(ctx, cudaMemsetAsync(a.moments, 0, 3 * pixels * sizeof(float), ctx->stream));
     CUDA_TRY(ctx, cudaMemsetAsync(a.counts, 0, pixels * sizeof(uint32_t), ctx->stream));
     a.desc = *desc; a.n = 0; a.active = (uint32_t)pixels; a.on = true;
+    ctx->fbMoments.complete = false; // the framebuffer now holds what the adaptive moments cover
     return PTC_OK;
 }
 
@@ -2676,6 +2726,99 @@ int ptc_camera_rays(ptc_ctx *ctx, const float *rowCol, uint32_t n, ptc_ray *rays
     NEED_COMMIT(ctx);
     return roundTrip(ctx, rowCol, (size_t)2 * n, rays, n, [&](float *d, ptc_ray *o) { cameraRaysKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o); });
 }
+// Guide buffers (denoise.cuh: aovKernel): the caller's sums go up, the kernel adds to them, they come back
+int ptc_render_aovs(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp, float *albedo, float *normal, float *depth, uint32_t *hits)
+{
+    NEED_COMMIT(ctx);
+    if (!albedo || !normal || !depth || !hits) { CTX_FAIL(ctx, PTC_ERR_INVALID, "null guide buffer"); }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
+    ptc_ctx::Aovs &a = ctx->aovs;
+    if (a.pixels != pixels) {
+        cudaFree(a.buffer); a.buffer = nullptr; a.pixels = 0;
+        CUDA_TRY(ctx, cudaMalloc((void **)&a.buffer, 8 * pixels * sizeof(float)));
+        a.pixels = pixels;
+    }
+    float *d = a.buffer;
+    float *dAlbedo = d, *dNormal = d + 3 * pixels, *dDepth = d + 6 * pixels;
+    uint32_t *dHits = (uint32_t *)(d + 7 * pixels);
+    cudaError_t e = cudaSuccess;
+    auto step = [&](cudaError_t r) { if (e == cudaSuccess) { e = r; } };
+    step(cudaMemcpyAsync(dAlbedo, albedo, 3 * pixels * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    step(cudaMemcpyAsync(dNormal, normal, 3 * pixels * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    step(cudaMemcpyAsync(dDepth, depth, pixels * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+    step(cudaMemcpyAsync(dHits, hits, pixels * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    if (e == cudaSuccess && nSpp) {
+        aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene, seed, firstSample, nSpp, dAlbedo, dNormal, dDepth, dHits);
+        ctx->launches++;
+        step(cudaGetLastError());
+    }
+    step(cudaMemcpyAsync(albedo, dAlbedo, 3 * pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    step(cudaMemcpyAsync(normal, dNormal, 3 * pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    step(cudaMemcpyAsync(depth, dDepth, pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    step(cudaMemcpyAsync(hits, dHits, pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    step(cudaStreamSynchronize(ctx->stream));
+    if (e != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "guide buffers failed: %s", cudaGetErrorString(e)); }
+    return PTC_OK;
+}
+
+// The filter (denoise.cuh): inputs staged in one device buffer, one kernel that builds the colour and guide records, one a-trous
+// launch per iteration between the two colour buffers, the last one's colours copied back
+int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_input *in, float *out)
+{
+    NEED_COMMIT(ctx);
+    auto positive = [](float v) { return v > 0.f && std::isfinite(v); };
+    if (!desc || desc->iterations > 10 || !positive(desc->sigma_l) || !(desc->sigma_n >= 0.f && std::isfinite(desc->sigma_n)) ||
+        !positive(desc->sigma_z) || !positive(desc->sigma_a) || !positive(desc->eps)) {
+        CTX_FAIL(ctx, PTC_ERR_INVALID, "bad denoise descriptor (iterations <= 10, sigma_l, sigma_z, sigma_a, eps > 0, sigma_n >= 0)");
+    }
+    if (!in || !out || !in->sums || !in->moments || !in->albedo_rgb || !in->normal_xyz || !in->depth || !in->hits) {
+        CTX_FAIL(ctx, PTC_ERR_INVALID, "missing denoise input");
+    }
+    if (!in->aov_spp) { CTX_FAIL(ctx, PTC_ERR_INVALID, "aov_spp must be > 0"); }
+    const int width = ctx->scene.width, height = ctx->scene.height;
+    const size_t pixels = (size_t)width * height;
+    if (in->counts) {
+        for (size_t p = 0; p < pixels; p++) { if (in->counts[p] < 2) { CTX_FAIL(ctx, PTC_ERR_INVALID, "pixel %zu has %u samples: the variance needs 2", p, in->counts[p]); } }
+    } else if (in->spp < 2) { CTX_FAIL(ctx, PTC_ERR_INVALID, "spp must be >= 2: the variance needs 2 samples"); }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    ptc_ctx::Denoise &d = ctx->denoise;
+    if (d.pixels != pixels) {
+        cudaFree(d.inputs); cudaFree(d.guide); cudaFree(d.colour[0]); cudaFree(d.colour[1]);
+        d = ptc_ctx::Denoise();
+        CUDA_TRY(ctx, cudaMalloc((void **)&d.inputs, 15 * pixels * sizeof(float)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&d.guide, 2 * pixels * sizeof(float4)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[0], pixels * sizeof(float4)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[1], pixels * sizeof(float4)));
+        d.pixels = pixels;
+    }
+    DenoiseInputs di;
+    float *f = d.inputs;
+    di.sums = f; di.moments = f + 3 * pixels; di.albedo = f + 6 * pixels; di.normal = f + 9 * pixels; di.depth = f + 12 * pixels;
+    di.hits = (const uint32_t *)(f + 13 * pixels); di.counts = in->counts ? (const uint32_t *)(f + 14 * pixels) : nullptr;
+    di.spp = in->spp; di.aovSpp = in->aov_spp; di.nPixels = (uint32_t)pixels;
+    const struct { void *dst; const void *src; size_t bytes; } uploads[] = {
+        {f, in->sums, 3 * pixels * 4}, {f + 3 * pixels, in->moments, 3 * pixels * 4}, {f + 6 * pixels, in->albedo_rgb, 3 * pixels * 4},
+        {f + 9 * pixels, in->normal_xyz, 3 * pixels * 4}, {f + 12 * pixels, in->depth, pixels * 4}, {f + 13 * pixels, in->hits, pixels * 4},
+        {f + 14 * pixels, in->counts, in->counts ? pixels * 4 : 0}};
+    for (const auto &u : uploads) { if (u.bytes) { CUDA_TRY(ctx, cudaMemcpyAsync(u.dst, u.src, u.bytes, cudaMemcpyHostToDevice, ctx->stream)); } }
+    denoisePrepareKernel<<<std::min<uint32_t>((uint32_t)((pixels + 255) / 256), (uint32_t)ctx->gridSimple * 4), 256, 0, ctx->stream>>>(di, d.colour[0], d.guide);
+    ctx->launches++;
+    CUDA_TRY(ctx, cudaGetLastError());
+    DenoiseParams dp;
+    dp.sigmaL = desc->sigma_l; dp.sigmaN = desc->sigma_n; dp.sigmaZ = desc->sigma_z; dp.sigmaA = desc->sigma_a; dp.eps = desc->eps;
+    const dim3 block(32, 8), grid((unsigned)(width + 31) / 32, (unsigned)(height + 7) / 8);
+    for (uint32_t i = 0; i < desc->iterations; i++) {
+        denoiseAtrousKernel<<<grid, block, 0, ctx->stream>>>(d.colour[i & 1], d.colour[(i + 1) & 1], d.guide, width, height, 1 << i, dp);
+        ctx->launches++;
+        CUDA_TRY(ctx, cudaGetLastError());
+    }
+    std::vector<float4> result(pixels);
+    CUDA_TRY(ctx, cudaMemcpyAsync(result.data(), d.colour[desc->iterations & 1], pixels * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    for (size_t p = 0; p < pixels; p++) { out[3 * p] = result[p].x; out[3 * p + 1] = result[p].y; out[3 * p + 2] = result[p].z; }
+    return PTC_OK;
+}
 int ptc_philox4x32_10(ptc_ctx *ctx, const uint32_t *counters, const uint32_t *keys, uint32_t n, uint32_t *out)
 {
     if (!ctx || (n && (!counters || !keys || !out))) { return PTC_ERR_INVALID; }
@@ -2820,6 +2963,11 @@ int ptc_set_option(ptc_ctx *ctx, const char *name, int64_t value)
     }
     if (!strcmp(name, "count_traversal")) { ctx->countTraversal = value != 0; return PTC_OK; }
     if (!strcmp(name, "volume_megakernel")) { ctx->volumeMegakernel = value != 0; return PTC_OK; }
+    if (!strcmp(name, "framebuffer_moments")) { // takes effect for the moments at the next ptc_framebuffer_clear
+        ctx->fbMoments.on = value != 0;
+        if (!ctx->fbMoments.on) { ctx->fbMoments.complete = false; }
+        return PTC_OK;
+    }
     if (!strcmp(name, "bvh_builder")) { // before ptc_commit; 1 = device (default), 0 = host binned SAH
         if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "bvh_builder must be set before ptc_commit"); }
         if (value != 0 && value != 1) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bvh_builder must be 0 (host) or 1 (device)"); }

@@ -114,6 +114,7 @@ int pth_job_describe(const char *jobPath, char *out, int outLen, char *err, int 
           << ", \"gpus\": " << job.gpus() << ", \"seed\": " << job.seed() << ", \"wave_spp\": " << job.waveSpp()
           << ", \"adaptive\": " << (job.adaptive() ? "true" : "false") << ", \"adaptive_threshold\": " << job.adaptiveThreshold()
           << ", \"adaptive_min_spp\": " << job.adaptiveMinSpp() << ", \"adaptive_step_spp\": " << job.adaptiveStepSpp()
+          << ", \"denoise\": " << (job.denoise() ? "true" : "false")
           << ", \"scene\": \"" << job.scene() << "\", \"output_directory\": \"" << job.outputDirectory()
           << "\", \"output_name\": \"" << job.outputName() << "\", \"integrator_status\": \"" << status << "\"}";
         snprintf(out, (size_t)outLen, "%s", o.str().c_str());

@@ -234,6 +234,7 @@ void CudaPathTracer::run(Image &image, Scene &scene, std::function<void(RenderSt
     const int start = m_bounceController.startBounce(), last = m_bounceController.lastBounce();
     for (int g = 0; g < gpus; g++) {
         check(scene.context(g), ptc_set_integrator(scene.context(g), m_integrator), "integrator");
+        if (g_job->denoise()) { check(scene.context(g), ptc_set_option(scene.context(g), "framebuffer_moments", 1), "framebuffer moments"); }
         check(scene.context(g), ptc_framebuffer_clear(scene.context(g)), "framebuffer clear");
     }
     std::vector<ptc_ctx *> peers;
@@ -352,6 +353,63 @@ void CudaPathTracer::runAdaptive(Image &image, Scene &scene, std::function<void(
         for (int col = 0; col < width; col++) { plane[(size_t)(height - 1 - row) * width + col] = (float)counts[(size_t)row * width + col]; }
     }
     saveEXR(g_job->outputDirectory() + "adaptive-spp.exr", width, height, {"Y"}, {plane.data()}, false);
+}
+
+// The guide buffers need far fewer samples than the colour (a pixel's first hits differ only across its footprint): at most this many
+static const uint32_t kGuideSpp = 16;
+
+// "denoise": true -- after run(), from what the contexts still hold: the sums and second moments gathered over every GPU (an
+// adaptive job: the sums, per-pixel counts and moments of its adaptive render on device 0), the guide buffers of the first
+// min(spp, kGuideSpp) samples on device 0, and ptc_denoise with the default parameters.  denoised.exr is written like final.exr
+// (Image: HALF, B,G,R, top scanline first); albedo.exr and normal.exr hold the guide buffers' means in fp32, what an external
+// denoiser takes besides the colour.
+void CudaPathTracer::writeDenoised(Scene &scene)
+{
+    const int width = g_job->width(), height = g_job->height();
+    const size_t pixels = (size_t)width * height;
+    ptc_ctx *ctx = scene.context(0);
+    std::vector<ptc_ctx *> peers;
+    for (int g = 1; g < scene.gpus(); g++) { peers.push_back(scene.context(g)); }
+    std::vector<float> sums(3 * pixels), moments(3 * pixels);
+    std::vector<uint32_t> counts;
+    check(ctx, ptc_framebuffer_gather(ctx, peers.data(), (uint32_t)peers.size(), 1, sums.data()), "framebuffer gather");
+    if (g_job->adaptive()) {
+        counts.resize(pixels);
+        check(ctx, ptc_adaptive_state(ctx, counts.data(), moments.data()), "adaptive state");
+    } else {
+        uint32_t ticket = 0;
+        check(ctx, ptc_framebuffer_gather_begin(ctx, peers.data(), (uint32_t)peers.size(), PTC_GATHER_MOMENTS, 1, &ticket), "moments gather");
+        check(ctx, ptc_framebuffer_gather_end(ctx, ticket, moments.data()), "moments gather");
+    }
+    const uint32_t *countsOrNull = counts.empty() ? nullptr : counts.data();
+    const uint32_t spp = m_nextSample; // uniform jobs: the samples every pixel holds
+    const uint32_t aovSpp = std::min<uint32_t>((uint32_t)g_job->spp(), kGuideSpp);
+    std::vector<float> albedo(3 * pixels, 0.f), normal(3 * pixels, 0.f), depth(pixels, 0.f), out(3 * pixels);
+    std::vector<uint32_t> hits(pixels, 0);
+    check(ctx, ptc_render_aovs(ctx, m_seed, 0, aovSpp, albedo.data(), normal.data(), depth.data(), hits.data()), "guide buffers");
+    const ptc_denoise_desc desc = PTC_DENOISE_DEFAULTS;
+    ptc_denoise_input in;
+    in.sums = sums.data(); in.moments = moments.data(); in.counts = countsOrNull; in.spp = spp;
+    in.albedo_rgb = albedo.data(); in.normal_xyz = normal.data(); in.depth = depth.data(); in.hits = hits.data(); in.aov_spp = aovSpp;
+    check(ctx, ptc_denoise(ctx, &desc, &in, out.data()), "denoise");
+    {
+        Image denoised(width, height);
+        denoised.setAll(out.data());
+        denoised.save("denoised"); // the destructor waits for the file
+    }
+    for (const char *name : {"albedo", "normal"}) {
+        const std::vector<float> &sum = name[0] == 'a' ? albedo : normal;
+        std::vector<float> planes[3];
+        for (int c = 0; c < 3; c++) { planes[c].resize(pixels); }
+        for (int row = 0; row < height; row++) {
+            for (int col = 0; col < width; col++) {
+                const size_t from = (size_t)row * width + col, to = (size_t)(height - 1 - row) * width + col;
+                for (int c = 0; c < 3; c++) { planes[c][to] = sum[3 * from + c] / (float)aovSpp; }
+            }
+        }
+        saveEXR(g_job->outputDirectory() + name + ".exr", width, height, {"B", "G", "R"}, {planes[2].data(), planes[1].data(), planes[0].data()}, false);
+        printf("Saved exr file. [ %s%s.exr ] \n", g_job->outputDirectory().c_str(), name);
+    }
 }
 
 } // namespace pathed

@@ -53,6 +53,9 @@ Job::Job(std::istream &jobFile)
     : m_json(new Json(parseJobFile(jobFile))),
       m_bounceController((*m_json)["startBounce"].asInt(), (*m_json)["lastBounce"].asInt())
 {
+    const Json &denoiseKey = (*m_json)["denoise"];
+    if (!denoiseKey.isNull() && !denoiseKey.isBool()) { throw std::runtime_error("denoise must be true or false"); }
+    if (denoise() && spp() < 2) { throw std::runtime_error("denoise needs spp >= 2: the filter estimates each pixel's variance"); }
     if (!adaptive()) { return; }
     const double threshold = (*m_json)["adaptive_threshold"].asNumber();
     if (!(threshold > 0.0) || !std::isfinite(threshold)) { throw std::runtime_error("adaptive_threshold must be a number > 0"); }
@@ -86,6 +89,7 @@ std::string Job::scene() const { return (*m_json)["scene"].asString(); }
 int Job::gpus() const { return (*m_json)["gpus"].isNumber() ? std::max(1, (*m_json)["gpus"].asInt()) : 1; }
 uint64_t Job::seed() const { return (*m_json)["seed"].isNumber() ? (uint64_t)(*m_json)["seed"].asNumber() : 0x5EEDull; }
 int Job::waveSpp() const { return (*m_json)["wave_spp"].isNumber() ? std::max(1, (*m_json)["wave_spp"].asInt()) : 64; }
+bool Job::denoise() const { return (*m_json)["denoise"].isBool() && (*m_json)["denoise"].asBool(); }
 bool Job::adaptive() const { return !(*m_json)["adaptive_threshold"].isNull(); }
 float Job::adaptiveThreshold() const { return adaptive() ? (float)(*m_json)["adaptive_threshold"].asNumber() : 0.f; }
 int Job::adaptiveMinSpp() const { return (*m_json)["adaptive_min_spp"].isNumber() ? (*m_json)["adaptive_min_spp"].asInt() : 16; }

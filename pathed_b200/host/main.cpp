@@ -44,6 +44,7 @@ int main(int argc, char *argv[])
             printf("PATHED_RESULT {\"samples\": %llu, \"render_wall_s\": %.6f, \"msamples_per_s\": %.3f, \"gpus\": %d}\n",
                    (unsigned long long)tracer->samplesRendered(), tracer->renderSeconds(),
                    tracer->samplesRendered() / std::max(tracer->renderSeconds(), 1e-9) * 1e-6, scene->gpus());
+            if (job.denoise()) { tracer->writeDenoised(*scene); } // after final.exr was handed to the writer
         }
     } catch (const std::exception &e) {
         std::cout << "error: " << e.what() << std::endl;

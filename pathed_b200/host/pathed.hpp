@@ -77,6 +77,10 @@ public:
     float adaptiveThreshold() const;
     int adaptiveMinSpp() const;
     int adaptiveStepSpp() const;
+    // "denoise": true (default false) also writes denoised.exr (ptc_denoise of the final sums), albedo.exr and normal.exr (the
+    // guide buffers it used); any value but a bool is refused by the constructor, and so is true with spp < 2 (the filter needs
+    // each pixel's variance)
+    bool denoise() const;
 
     // string -> integrator (src/job.cpp:65-97); anything but "PathTracer" throws const char* "Unimplemented"
     std::shared_ptr<Integrator> integrator() const;
@@ -193,6 +197,9 @@ public:
 
     double renderSeconds() const { return m_renderSeconds; } // wall time inside run() spent rendering + reducing
     uint64_t samplesRendered() const { return m_samples; }
+    // job.json "denoise": denoised.exr, albedo.exr and normal.exr from the render run() left on the devices.  Called after the job's
+    // image is saved, so that a failure here cannot cost the job final.exr
+    void writeDenoised(Scene &scene);
 
 private:
     BounceController m_bounceController;
