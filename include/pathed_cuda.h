@@ -325,6 +325,24 @@ typedef struct ptc_denoise_input {
  * context's device and returns when the output is on the host.  Deterministic: two calls give the same bytes.  PTC_ERR_INVALID
  * for a bad descriptor, a missing input, a pixel with fewer than 2 samples or aov_spp == 0. */
 int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_input *in, float *out_rgb);
+/* Device-resident denoising of the contexts' own images.  With option "framebuffer_moments" on, ptc_framebuffer_render_checkpoints
+ * also keeps the second moments of every snapshot (12 B per pixel per snapshot, next to the snapshot's sums); a snapshot's moments
+ * count as complete under the rule of PTC_GATHER_MOMENTS at the time it was written.
+ * ptc_framebuffer_guides: ptc_render_aovs into context-owned device buffers, from zero (replaces the previous call's guides); the
+ * guide records for ptc_framebuffer_denoise_begin are built here.  Any host pointer may be NULL; non-NULL ones receive the sums
+ * (like ptc_render_aovs from zeroed buffers).  Asynchronous on the context's stream unless a host pointer is given.
+ * PTC_ERR_INVALID for n_spp == 0. */
+int ptc_framebuffer_guides(ptc_ctx *ctx, uint64_t seed, uint32_t first_sample, uint32_t n_spp, float *albedo_rgb, float *normal_xyz,
+                           float *depth, uint32_t *hits);
+/* ptc_denoise of snapshot `snapshot` (< 0: the framebuffers) of root + peers, summed as ptc_framebuffer_gather_begin sums them, with
+ * their second moments summed the same way and the root's device guides (aov_spp = the n_spp of ptc_framebuffer_guides); spp =
+ * samples per pixel of that image (ignored on a root that holds an adaptive render: its per-pixel counts are used).  Enqueues only;
+ * the image (3*W*H) is fetched with ptc_framebuffer_gather_end(root, ticket, out).  Same bytes as ptc_denoise on the gathered inputs.
+ * PTC_ERR_INVALID: a bad descriptor or arguments, spp < 2 on a uniform image.  PTC_ERR_STATE: no guides on the root or guides of
+ * another resolution, a snapshot that was not rendered (or any snapshot of an adaptive root), moments that do not cover every sample
+ * of a context, an adaptive root before its first pass. */
+int ptc_framebuffer_denoise_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t n_peers, int snapshot, uint32_t spp,
+                                  const ptc_denoise_desc *desc, uint32_t *ticket);
 
 /* ---- the random streams on their own (known-answer tests; need no scene) ---------------------- */
 /* Philox4x32-10, the generator that replaces RandomGenerator (src/random_generator.cpp:4-11) and std::rand (src/camera.cpp:51-52)

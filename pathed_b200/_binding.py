@@ -42,6 +42,14 @@ class DenoiseDesc(ctypes.Structure):
 DENOISE_DEFAULTS = {"iterations": 5, "sigma_l": 4.0, "sigma_n": 128.0, "sigma_z": 1.0, "sigma_a": 0.1, "eps": 1e-6}  # PTC_DENOISE_DEFAULTS
 
 
+def _denoise_desc(params):
+    unknown = set(params) - set(DENOISE_DEFAULTS)
+    if unknown:
+        raise TypeError("unknown denoise parameters %s" % sorted(unknown))
+    p = dict(DENOISE_DEFAULTS, **params)
+    return DenoiseDesc(int(p["iterations"]), *[float(p[k]) for k in ("sigma_l", "sigma_n", "sigma_z", "sigma_a", "eps")])
+
+
 class DenoiseInput(ctypes.Structure):
     _fields_ = [("sums", ctypes.c_void_p), ("moments", ctypes.c_void_p), ("counts", ctypes.c_void_p), ("spp", ctypes.c_uint32),
                 ("albedo_rgb", ctypes.c_void_p), ("normal_xyz", ctypes.c_void_p), ("depth", ctypes.c_void_p), ("hits", ctypes.c_void_p),
@@ -296,7 +304,7 @@ class Api:
         self._call("adaptive_state", _ptr(counts), _ptr(m2))
         return counts, m2
 
-    # ---- denoising (ptc_render_aovs, ptc_denoise; DESIGN §10)
+    # ---- denoising (ptc_render_aovs, ptc_denoise, ptc_framebuffer_guides, ptc_framebuffer_denoise_begin; DESIGN §10)
     def render_aovs(self, seed, first_sample, n_spp, aovs=None):
         """first-hit guide buffers of samples first_sample .. first_sample + n_spp - 1, added into `aovs` (a dict like the one returned;
         None: zeros): albedo [h, w, 3], normal [h, w, 3], depth [h, w] fp32 sums and hits [h, w] uint32, row 0 = bottom"""
@@ -315,11 +323,7 @@ class Api:
     def denoise(self, sums, moments, counts_or_spp, aovs, aov_spp, **params):
         """ptc_denoise: the denoised mean colour [h, w, 3].  counts_or_spp: per-pixel sample counts [h, w] or one spp for every pixel;
         params: iterations, sigma_l, sigma_n, sigma_z, sigma_a, eps (DENOISE_DEFAULTS for the ones not given)"""
-        unknown = set(params) - set(DENOISE_DEFAULTS)
-        if unknown:
-            raise TypeError("unknown denoise parameters %s" % sorted(unknown))
-        p = dict(DENOISE_DEFAULTS, **params)
-        desc = DenoiseDesc(int(p["iterations"]), *[float(p[k]) for k in ("sigma_l", "sigma_n", "sigma_z", "sigma_a", "eps")])
+        desc = _denoise_desc(params)
         n = 3 * self.width * self.height
         f32 = lambda a, size: np.ascontiguousarray(a, np.float32).reshape(size)
         keep = {"sums": f32(sums, n), "moments": f32(moments, n), "albedo": f32(aovs["albedo"], n), "normal": f32(aovs["normal"], n),
@@ -336,6 +340,34 @@ class Api:
         out = np.zeros((self.height, self.width, 3), np.float32)
         self._call("denoise", ctypes.byref(desc), ctypes.byref(inp), _ptr(out))
         return out
+
+    def framebuffer_guides(self, seed, first_sample, n_spp, fetch=False):
+        """ptc_framebuffer_guides: the guides of samples first_sample .. first_sample + n_spp - 1, from zero, kept on the device for
+        framebuffer_denoise_begin; fetch=True also returns their sums (a dict like render_aovs's), else None"""
+        if not fetch:
+            self._call("framebuffer_guides", ctypes.c_uint64(seed), ctypes.c_uint32(first_sample), ctypes.c_uint32(n_spp), None, None, None, None)
+            return None
+        h, w = self.height, self.width
+        aovs = {"albedo": np.zeros((h, w, 3), np.float32), "normal": np.zeros((h, w, 3), np.float32),
+                "depth": np.zeros((h, w), np.float32), "hits": np.zeros((h, w), np.uint32)}
+        self._call("framebuffer_guides", ctypes.c_uint64(seed), ctypes.c_uint32(first_sample), ctypes.c_uint32(n_spp), _ptr(aovs["albedo"]),
+                   _ptr(aovs["normal"]), _ptr(aovs["depth"]), _ptr(aovs["hits"]))
+        return aovs
+
+    def framebuffer_denoise_begin(self, peers=(), snapshot=-1, spp=0, **params):
+        """ptc_framebuffer_denoise_begin: enqueues the denoise of snapshot `snapshot` (-1: the framebuffers) of this context + peers
+        with the guides of framebuffer_guides; spp = the image's samples per pixel (ignored on an adaptive render).  Returns the
+        ticket for framebuffer_gather_end.  params as for denoise"""
+        desc = _denoise_desc(params)
+        arr = (ctypes.c_void_p * max(len(peers), 1))(*[p.ctx.value for p in peers])
+        ticket = ctypes.c_uint32(0)
+        self._call("framebuffer_denoise_begin", arr, ctypes.c_uint32(len(peers)), ctypes.c_int(snapshot), ctypes.c_uint32(spp),
+                   ctypes.byref(desc), ctypes.byref(ticket))
+        return ticket.value
+
+    def framebuffer_denoise(self, peers=(), snapshot=-1, spp=0, **params):
+        """framebuffer_denoise_begin, then framebuffer_gather_end: the denoised mean colour [h, w, 3]"""
+        return self.framebuffer_gather_end(self.framebuffer_denoise_begin(peers, snapshot, spp, **params))
 
     # ---- random streams (known-answer tests)
     def philox(self, counters, keys):

@@ -1,5 +1,7 @@
-// Denoising (ptc_render_aovs, ptc_denoise; DESIGN §10).  Included by pathed_cuda.cu after the probe kernels: it traces with the
-// same camera, traversal and Intersection code as the path tracer and ptc_intersect_full.
+// Denoising (ptc_render_aovs, ptc_denoise, ptc_framebuffer_guides, ptc_framebuffer_denoise_begin; DESIGN §10).  Included by
+// pathed_cuda.cu after the probe kernels: it traces with the same camera, traversal and Intersection code as the path tracer and
+// ptc_intersect_full.  The host-input filter (ptc_denoise) and the device-resident one build their records with the same functions
+// (colourRecord, writeGuideRecord), so the two give the same bytes for the same sums.
 //
 // Guide buffers.  aovKernel re-traces the first hit of the camera ray the path tracer traces for (seed, pixel, sample): draws 0 and
 // 1 of vertex 0 jitter the ray exactly as generateKernel / volumePathKernel do, and the closest hit is intersectFullKernel's.  One
@@ -68,24 +70,68 @@ struct DenoiseInputs {
     uint32_t spp, aovSpp, nPixels;
 };
 
+// The colour record of one pixel from its sums S, second moments M and sample count n
+__device__ __forceinline__ float4 colourRecord(const float S[3], const float M[3], float n)
+{
+    float c[3], var[3];
+    for (int k = 0; k < 3; k++) {
+        c[k] = S[k] / n;
+        var[k] = (M[k] - n * (c[k] * c[k])) / (n - 1.f);
+        if (var[k] < 0.f) { var[k] = 0.f; } // keeps a NaN
+    }
+    return make_float4(c[0], c[1], c[2], ((var[0] + var[1]) + var[2]) / (3.f * n));
+}
+
+// The guide record of pixel p from the guide sums over aovSpp samples
+__device__ __forceinline__ void writeGuideRecord(const float *albedo, const float *normal, const float *depth, const uint32_t *hits, uint32_t aovSppCount,
+                                                 uint32_t p, float4 *guide)
+{
+    const float aovSpp = (float)aovSppCount;
+    const float nx = normal[3 * (size_t)p], ny = normal[3 * (size_t)p + 1], nz = normal[3 * (size_t)p + 2];
+    const float len2 = (nx * nx + ny * ny) + nz * nz;
+    const float len = len2 > 0.f ? sqrtf(len2) : 0.f;
+    guide[2 * (size_t)p] = make_float4(albedo[3 * (size_t)p] / aovSpp, albedo[3 * (size_t)p + 1] / aovSpp, albedo[3 * (size_t)p + 2] / aovSpp,
+                                       depth[p] / (float)max(hits[p], 1u));
+    guide[2 * (size_t)p + 1] = len > 0.f ? make_float4(nx / len, ny / len, nz / len, 0.f) : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
 __global__ void __launch_bounds__(256) denoisePrepareKernel(DenoiseInputs in, float4 *colour, float4 *guide)
 {
     for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < in.nPixels; p += gridDim.x * blockDim.x) {
-        const float n = (float)(in.counts ? in.counts[p] : in.spp);
-        float c[3], var[3];
+        colour[p] = colourRecord(in.sums + 3 * (size_t)p, in.moments + 3 * (size_t)p, (float)(in.counts ? in.counts[p] : in.spp));
+        writeGuideRecord(in.albedo, in.normal, in.depth, in.hits, in.aovSpp, p, guide);
+    }
+}
+
+// ptc_framebuffer_guides: the guide records from the device guide sums of aovKernel
+__global__ void __launch_bounds__(256) denoiseGuideKernel(const float *albedo, const float *normal, const float *depth, const uint32_t *hits, uint32_t aovSpp,
+                                                          uint32_t nPixels, float4 *guide)
+{
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < nPixels; p += gridDim.x * blockDim.x) { writeGuideRecord(albedo, normal, depth, hits, aovSpp, p, guide); }
+}
+
+// ptc_framebuffer_denoise_begin: the colour records of the sums and second moments of root + peers, each summed in
+// gatherResolveKernel's order (set.fb[0] first, then the peers in turn); n = counts[p] (an adaptive root) or spp
+__global__ void __launch_bounds__(256) denoiseGatherKernel(FramebufferSet sums, FramebufferSet moments, const uint32_t *counts, uint32_t spp, uint32_t nPixels,
+                                                           float4 *colour)
+{
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < nPixels; p += gridDim.x * blockDim.x) {
+        float S[3], M[3];
         for (int k = 0; k < 3; k++) {
-            c[k] = in.sums[3 * (size_t)p + k] / n;
-            var[k] = (in.moments[3 * (size_t)p + k] - n * (c[k] * c[k])) / (n - 1.f);
-            if (var[k] < 0.f) { var[k] = 0.f; } // keeps a NaN
+            const size_t i = 3 * (size_t)p + k;
+            S[k] = sums.fb[0][i]; M[k] = moments.fb[0][i];
+            for (int g = 1; g < sums.count; g++) { S[k] += sums.fb[g][i]; M[k] += moments.fb[g][i]; }
         }
-        colour[p] = make_float4(c[0], c[1], c[2], ((var[0] + var[1]) + var[2]) / (3.f * n));
-        const float aovSpp = (float)in.aovSpp;
-        const float nx = in.normal[3 * (size_t)p], ny = in.normal[3 * (size_t)p + 1], nz = in.normal[3 * (size_t)p + 2];
-        const float len2 = (nx * nx + ny * ny) + nz * nz;
-        const float len = len2 > 0.f ? sqrtf(len2) : 0.f;
-        guide[2 * (size_t)p] = make_float4(in.albedo[3 * (size_t)p] / aovSpp, in.albedo[3 * (size_t)p + 1] / aovSpp, in.albedo[3 * (size_t)p + 2] / aovSpp,
-                                           in.depth[p] / (float)max(in.hits[p], 1u));
-        guide[2 * (size_t)p + 1] = len > 0.f ? make_float4(nx / len, ny / len, nz / len, 0.f) : make_float4(0.f, 0.f, 0.f, 0.f);
+        colour[p] = colourRecord(S, M, (float)(counts ? counts[p] : spp));
+    }
+}
+
+// rgb of the last a-trous output, as ptc_denoise hands it out
+__global__ void __launch_bounds__(256) denoisePackKernel(const float4 *colour, float *out, uint32_t nPixels)
+{
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < nPixels; p += gridDim.x * blockDim.x) {
+        const float4 c = colour[p];
+        out[3 * (size_t)p] = c.x; out[3 * (size_t)p + 1] = c.y; out[3 * (size_t)p + 2] = c.z;
     }
 }
 

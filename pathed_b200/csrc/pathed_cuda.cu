@@ -640,10 +640,13 @@ __global__ void __launch_bounds__(128, PTC_MATERIAL_MIN_BLOCKS) materialKernel(D
 // Checkpoints that fall inside a wave (src/integrator.cpp:87-92 saves the image after 1, 2, 4, ... samples): the resolve keeps a copy
 // of the running sums after `at[i]` samples of the wave in dst[i], so a wave does not have to end at every power of two
 struct CheckpointPlan { uint32_t n; uint32_t at[PTC_MAX_CHECKPOINTS]; float *dst[PTC_MAX_CHECKPOINTS]; };
-// MOMENTS (adaptive passes): moments[3 * pixel + c] += x_c^2 for every sample x, in sample order like the sums
+// MOMENTS (adaptive passes, option framebuffer_moments): moments[3 * pixel + c] += x_c^2 for every sample x, in sample order like the
+// sums.  A checkpoint copy then holds both: dst[i] is a buffer of 6 x W x H floats, the sums followed by the second moments (the
+// moments' destination is not a field of the plan, so the plain instance keeps its parameters and code)
 template <bool MOMENTS>
 __global__ void __launch_bounds__(256) accumulateKernel(PathBuffers pb, WaveParams wp, float *accum, float *moments, uint32_t width, uint32_t height, const __grid_constant__ CheckpointPlan plan)
 {
+    const size_t momentsAt = 3 * (size_t)width * height; // MOMENTS: offset of a checkpoint's moments in its buffer
     for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < wp.nPixels; q += gridDim.x * blockDim.x) {
         const size_t pixel = wavePixel(q, wp, width, height);
         float r = accum[3 * pixel], g = accum[3 * pixel + 1], b = accum[3 * pixel + 2];
@@ -651,12 +654,18 @@ __global__ void __launch_bounds__(256) accumulateKernel(PathBuffers pb, WavePara
         if (MOMENTS) { mr = moments[3 * pixel]; mg = moments[3 * pixel + 1]; mb = moments[3 * pixel + 2]; }
         uint32_t next = 0;
         for (uint32_t s = 0; s < wp.sppWave; s++) { // radianceLookup += color, one sample after the other (src/sample_integrator.cpp:61-63)
-            while (next < plan.n && plan.at[next] == s) { float *d = plan.dst[next++]; d[3 * pixel] = r; d[3 * pixel + 1] = g; d[3 * pixel + 2] = b; }
+            while (next < plan.n && plan.at[next] == s) {
+                float *d = plan.dst[next++]; d[3 * pixel] = r; d[3 * pixel + 1] = g; d[3 * pixel + 2] = b;
+                if (MOMENTS) { d += momentsAt; d[3 * pixel] = mr; d[3 * pixel + 1] = mg; d[3 * pixel + 2] = mb; }
+            }
             const float4 c = streamLoad(pb.out + pixelSampleToSlot(q, s, wp));
             r += c.x; g += c.y; b += c.z;
             if (MOMENTS) { mr += c.x * c.x; mg += c.y * c.y; mb += c.z * c.z; }
         }
-        while (next < plan.n) { float *d = plan.dst[next++]; d[3 * pixel] = r; d[3 * pixel + 1] = g; d[3 * pixel + 2] = b; }
+        while (next < plan.n) {
+            float *d = plan.dst[next++]; d[3 * pixel] = r; d[3 * pixel + 1] = g; d[3 * pixel + 2] = b;
+            if (MOMENTS) { d += momentsAt; d[3 * pixel] = mr; d[3 * pixel + 1] = mg; d[3 * pixel + 2] = mb; }
+        }
         accum[3 * pixel] = r; accum[3 * pixel + 1] = g; accum[3 * pixel + 2] = b;
         if (MOMENTS) { moments[3 * pixel] = mr; moments[3 * pixel + 1] = mg; moments[3 * pixel + 2] = mb; }
     }
@@ -739,6 +748,9 @@ __global__ void __launch_bounds__(128, PTC_VOLUME_MIN_BLOCKS) volumePathKernel(c
 }
 
 #include "volume_wavefront.cuh"
+// K7 resolve fused with the spp-split reduce (gatherResolveKernel) and the device-resident denoise read these: every framebuffer but the
+// first lives on another GPU and is read through its NVLink peer mapping (or a staged local copy when peer access is unavailable)
+struct FramebufferSet { const float *fb[PTC_MAX_PEERS + 1]; int count; };
 #include "denoise.cuh"
 
 __global__ void resolveKernel(const float *accum, float *out, uint32_t n, uint32_t spp) // src/integrator.cpp:74-85
@@ -746,9 +758,7 @@ __global__ void resolveKernel(const float *accum, float *out, uint32_t n, uint32
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) { out[i] = accum[i] / (int)spp; }
 }
 
-// K7 resolve fused with the spp-split reduce: every framebuffer but the first lives on another GPU and is read through
-// its NVLink peer mapping (or a staged local copy when peer access is unavailable); summed in a fixed order
-struct FramebufferSet { const float *fb[PTC_MAX_PEERS + 1]; int count; };
+// K7 resolve fused with the spp-split reduce, summed in a fixed order
 __global__ void __launch_bounds__(256) gatherResolveKernel(FramebufferSet set, float *out, uint32_t n, uint32_t divisor)
 {
     const uint32_t n4 = n >> 2;
@@ -1124,7 +1134,12 @@ struct ptc_ctx {
     float *framebuffer = nullptr, *gatherStage = nullptr; size_t framebufferSize = 0, gatherStageSize = 0;
     cudaEvent_t framebufferReady = nullptr;
     std::vector<float *> snapshots;                      // checkpoint copies of the framebuffer (ptc_framebuffer_render_checkpoints)
-    struct Gather { float *device = nullptr, *pinned = nullptr; cudaEvent_t done = nullptr; bool busy = false; };
+    // snapshots allocated with option framebuffer_moments on hold the sums and then the second moments (accumulateKernel<true>); a
+    // snapshot's moments are complete when they cover every sample its sums hold (fbMoments.complete when it was written)
+    bool snapshotsHoldMoments = false;
+    size_t snapshotSize = 0; // floats of sums per snapshot: the framebuffer size they were allocated for
+    std::vector<bool> snapshotMomentsComplete;
+    struct Gather { float *device = nullptr, *pinned = nullptr; size_t size = 0; cudaEvent_t done = nullptr; bool busy = false; };
     std::vector<Gather> gathers;                         // results of ptc_framebuffer_gather_begin in flight
     cudaEvent_t gatherRead = nullptr;                    // the last gather kernel of this (root) context finished reading the framebuffers
     float *pinned = nullptr; size_t pinnedSize = 0;
@@ -1177,10 +1192,13 @@ struct ptc_ctx {
     // by ptc_framebuffer_clear), the input of ptc_denoise that PTC_GATHER_MOMENTS gathers.  complete: the moments cover every sample
     // the framebuffer holds (the option was on at the last clear and at every render since); the gather refuses them otherwise
     struct FramebufferMoments { bool on = false, complete = false; float *moments = nullptr; size_t size = 0; } fbMoments;
-    // ptc_denoise's device buffers: the staged inputs (15 x 4 B per pixel), guide records (32 B), two colour records (16 B each)
-    struct Denoise { size_t pixels = 0; float *inputs = nullptr; float4 *guide = nullptr, *colour[2] = {nullptr, nullptr}; } denoise;
-    // ptc_render_aovs's device copy of the guide buffers (8 x 4 B per pixel)
+    // ptc_denoise's device buffers: the staged inputs (15 x 4 B per pixel) and guide records (32 B), sized for `pixels`; two colour
+    // records (16 B each, sized for colourPixels), which ptc_framebuffer_denoise_begin uses as well
+    struct Denoise { size_t pixels = 0, colourPixels = 0; float *inputs = nullptr; float4 *guide = nullptr, *colour[2] = {nullptr, nullptr}; } denoise;
+    // the device guide sums of ptc_render_aovs and ptc_framebuffer_guides (8 x 4 B per pixel)
     struct Aovs { size_t pixels = 0; float *buffer = nullptr; } aovs;
+    // ptc_framebuffer_guides: the guide records (32 B per pixel) ptc_framebuffer_denoise_begin filters with; aovSpp = 0: none
+    struct Guides { size_t pixels = 0; int width = 0, height = 0; float4 *records = nullptr; uint32_t aovSpp = 0; } guides;
     uint64_t samples = 0, launches = 0;
     float lastRenderMs = 0.f;
     // stage timing: CUDA events on the launching stream around every launch, summed per kernel class
@@ -1319,6 +1337,7 @@ void ptc_destroy(ptc_ctx *ctx)
     if (ctx->adaptive.selectedHost) { cudaFreeHost(ctx->adaptive.selectedHost); }
     cudaFree(ctx->fbMoments.moments); cudaFree(ctx->aovs.buffer);
     cudaFree(ctx->denoise.inputs); cudaFree(ctx->denoise.guide); cudaFree(ctx->denoise.colour[0]); cudaFree(ctx->denoise.colour[1]);
+    cudaFree(ctx->guides.records);
     for (float *snapshot : ctx->snapshots) { cudaFree(snapshot); }
     for (auto &g : ctx->gathers) { cudaFree(g.device); if (g.pinned) { cudaFreeHost(g.pinned); } if (g.done) { cudaEventDestroy(g.done); } }
     if (ctx->gatherRead) { cudaEventDestroy(ctx->gatherRead); }
@@ -2396,15 +2415,27 @@ int ptc_framebuffer_render_checkpoints(ptc_ctx *ctx, uint64_t seed, uint32_t fir
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
+    const size_t n = ctx->framebufferSize;
+    // the moments need room behind the sums, and a new resolution new buffers
+    if (nCounts && ((ctx->fbMoments.on && !ctx->snapshotsHoldMoments) || ctx->snapshotSize != n)) {
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); // gathers that read the old snapshots are ordered before this stream's work
+        for (float *snapshot : ctx->snapshots) { cudaFree(snapshot); }
+        ctx->snapshots.clear(); ctx->snapshotsHoldMoments = ctx->fbMoments.on; ctx->snapshotSize = n;
+    }
     while (ctx->snapshots.size() < nCounts) {
         float *buffer = nullptr;
-        CUDA_TRY(ctx, cudaMalloc((void **)&buffer, ctx->framebufferSize * sizeof(float)));
+        CUDA_TRY(ctx, cudaMalloc((void **)&buffer, (ctx->snapshotsHoldMoments ? 2 : 1) * n * sizeof(float)));
         ctx->snapshots.push_back(buffer);
     }
     if (!ctx->fbMoments.on) { ctx->fbMoments.complete = false; }
     else if ((rc = ensureFramebufferMoments(ctx))) { return rc; }
-    if (nSpp == 0) { // no samples for this context in the wave: every snapshot is the framebuffer as it stands
-        for (uint32_t i = 0; i < nCounts; i++) { CUDA_TRY(ctx, cudaMemcpyAsync(ctx->snapshots[i], ctx->framebuffer, ctx->framebufferSize * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream)); }
+    ctx->snapshotMomentsComplete.assign(ctx->snapshots.size(), false);
+    for (uint32_t i = 0; i < nCounts; i++) { ctx->snapshotMomentsComplete[i] = ctx->fbMoments.on && ctx->fbMoments.complete; }
+    if (nSpp == 0) { // no samples for this context in the wave: every snapshot is the framebuffer (and its moments) as it stands
+        for (uint32_t i = 0; i < nCounts; i++) {
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->snapshots[i], ctx->framebuffer, n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+            if (ctx->fbMoments.on) { CUDA_TRY(ctx, cudaMemcpyAsync(ctx->snapshots[i] + n, ctx->fbMoments.moments, n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream)); }
+        }
         return PTC_OK;
     }
     Checkpoints cp; cp.counts = sampleCounts; cp.n = nCounts; cp.dst = ctx->snapshots.data();
@@ -2415,6 +2446,98 @@ int ptc_framebuffer_render_checkpoints(ptc_ctx *ctx, uint64_t seed, uint32_t fir
     return renderInternal(ctx, seed, firstSample, nSpp, start, last, ctx->framebuffer, ctx->stream, cp, pass);
 }
 
+} // extern "C"
+
+// The second moments that cover every sample a context's framebuffer holds: its adaptive render's, else those of option
+// framebuffer_moments when complete; null when there are none
+static const float *framebufferMoments(const ptc_ctx *c, size_t n)
+{
+    if (c->adaptive.on) { return c->adaptive.moments; }
+    return c->fbMoments.complete && c->fbMoments.size == n ? c->fbMoments.moments : nullptr;
+}
+
+// The buffers a gather over root + peers reads: set k = sources[k](root), then sources[k] of every peer as root's device reads it --
+// the peer's own pointer on the same device or through an NVLink peer mapping, else a copy staged into root->gatherStage.  Root's
+// stream is first ordered behind each peer's pending work.  PTC_ERR_STATE for a peer without a buffer or of another size.
+typedef std::function<const float *(ptc_ctx *)> GatherSource;
+static int gatherSets(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, const GatherSource *sources, int nSets, FramebufferSet *sets)
+{
+    const size_t n = root->framebufferSize;
+    for (int k = 0; k < nSets; k++) { sets[k].fb[0] = sources[k](root); sets[k].count = 1; }
+    size_t staged = 0;
+    for (uint32_t g = 0; g < nPeers; g++) {
+        ptc_ctx *peer = peers[g];
+        bool present = peer && peer->committed && peer->framebufferSize == n;
+        for (int k = 0; present && k < nSets; k++) { present = sources[k](peer) != nullptr; }
+        if (!present) { CTX_FAIL(root, PTC_ERR_STATE, "peer %u has no framebuffer (or snapshot, or moments) of the same size", g); }
+        // order the gather after the peer's pending renders
+        CUDA_TRY(root, cudaSetDevice(peer->device));
+        CUDA_TRY(root, cudaEventRecord(peer->framebufferReady, peer->stream));
+        CUDA_TRY(root, cudaSetDevice(root->device));
+        CUDA_TRY(root, cudaStreamWaitEvent(root->stream, peer->framebufferReady, 0));
+        bool direct = peer->device == root->device;
+        int canAccess = 0;
+        if (!direct) { cudaDeviceCanAccessPeer(&canAccess, root->device, peer->device); }
+        if (canAccess) {
+            const cudaError_t e = cudaDeviceEnablePeerAccess(peer->device, 0);
+            direct = e == cudaSuccess || e == cudaErrorPeerAccessAlreadyEnabled;
+            cudaGetLastError();
+        }
+        for (int k = 0; k < nSets; k++) {
+            if (direct) { sets[k].fb[sets[k].count++] = sources[k](peer); continue; }
+            // no peer mapping: stage the peer's buffer into local memory first
+            if (root->gatherStageSize < (size_t)nSets * nPeers * n) {
+                CUDA_TRY(root, cudaStreamSynchronize(root->stream));
+                cudaFree(root->gatherStage); root->gatherStage = nullptr; root->gatherStageSize = 0;
+                CUDA_TRY(root, cudaMalloc((void **)&root->gatherStage, (size_t)nSets * nPeers * n * sizeof(float)));
+                root->gatherStageSize = (size_t)nSets * nPeers * n;
+            }
+            float *slot = root->gatherStage + staged * n; staged++;
+            CUDA_TRY(root, cudaMemcpyPeerAsync(slot, root->device, sources[k](peer), peer->device, n * sizeof(float), root->stream));
+            sets[k].fb[sets[k].count++] = slot;
+        }
+    }
+    return PTC_OK;
+}
+
+// A free result slot of root (device buffer + pinned host buffer + event), allocated on first use
+static int takeGatherSlot(ptc_ctx *root, uint32_t *ticketOut)
+{
+    uint32_t ticket = 0;
+    while (ticket < root->gathers.size() && root->gathers[ticket].busy) { ticket++; }
+    if (ticket == root->gathers.size()) { root->gathers.push_back(ptc_ctx::Gather()); }
+    ptc_ctx::Gather &slot = root->gathers[ticket];
+    if (slot.size != root->framebufferSize) { // first use, or the camera's resolution changed
+        cudaFree(slot.device); slot.device = nullptr;
+        if (slot.pinned) { cudaFreeHost(slot.pinned); slot.pinned = nullptr; }
+        slot.size = 0;
+        CUDA_TRY(root, cudaMalloc((void **)&slot.device, root->framebufferSize * sizeof(float)));
+        CUDA_TRY(root, cudaMallocHost((void **)&slot.pinned, root->framebufferSize * sizeof(float)));
+        slot.size = root->framebufferSize;
+    }
+    if (!slot.done) { CUDA_TRY(root, cudaEventCreateWithFlags(&slot.done, cudaEventDisableTiming)); }
+    *ticketOut = ticket;
+    return PTC_OK;
+}
+
+// After the kernels that read the contexts' buffers and wrote slot `ticket`'s device buffer: later work on the peers waits for those
+// reads, the result goes to the slot's pinned buffer, and ptc_framebuffer_gather_end hands it out
+static int finishGather(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, uint32_t ticket)
+{
+    CUDA_TRY(root, cudaGetLastError());
+    // renders that follow on any of the contexts must not overwrite what the kernels read
+    if (!root->gatherRead) { CUDA_TRY(root, cudaEventCreateWithFlags(&root->gatherRead, cudaEventDisableTiming)); }
+    CUDA_TRY(root, cudaEventRecord(root->gatherRead, root->stream));
+    for (uint32_t g = 0; g < nPeers; g++) { CUDA_TRY(root, cudaStreamWaitEvent(peers[g]->stream, root->gatherRead, 0)); }
+    ptc_ctx::Gather &slot = root->gathers[ticket];
+    CUDA_TRY(root, cudaMemcpyAsync(slot.pinned, slot.device, root->framebufferSize * sizeof(float), cudaMemcpyDeviceToHost, root->stream));
+    CUDA_TRY(root, cudaEventRecord(slot.done, root->stream));
+    slot.busy = true;
+    return PTC_OK;
+}
+
+extern "C" {
+
 int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, int snapshot, uint32_t divisor, uint32_t *ticketOut)
 {
     NEED_COMMIT(root);
@@ -2424,13 +2547,9 @@ int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t 
     if (rc) { return rc; }
     const size_t n = root->framebufferSize;
     // PTC_GATHER_MOMENTS: the second moments of an adaptive render, else those of the framebuffer renders
-    auto moments = [&](ptc_ctx *c) -> const float * {
-        if (c->adaptive.on) { return c->adaptive.moments; }
-        return c->fbMoments.complete && c->fbMoments.size == n ? c->fbMoments.moments : nullptr;
-    };
-    auto source = [&](ptc_ctx *c) -> const float * {
-        if (snapshot == PTC_GATHER_MOMENTS) { return moments(c); }
-        return snapshot < 0 ? c->framebuffer : (size_t)snapshot < c->snapshots.size() ? c->snapshots[snapshot] : nullptr;
+    const GatherSource source = [&](ptc_ctx *c) -> const float * {
+        if (snapshot == PTC_GATHER_MOMENTS) { return framebufferMoments(c, n); }
+        return snapshot < 0 ? c->framebuffer : (size_t)snapshot < c->snapshots.size() && c->snapshotSize == n ? c->snapshots[snapshot] : nullptr;
     };
     if (!source(root)) {
         if (snapshot == PTC_GATHER_MOMENTS) {
@@ -2439,55 +2558,12 @@ int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t 
         CTX_FAIL(root, PTC_ERR_STATE, "no snapshot %d was rendered", snapshot);
     }
     FramebufferSet set;
-    set.fb[0] = source(root); set.count = 1;
-    size_t staged = 0;
-    for (uint32_t g = 0; g < nPeers; g++) {
-        ptc_ctx *peer = peers[g];
-        if (!peer || !peer->committed || peer->framebufferSize != n || !source(peer)) { CTX_FAIL(root, PTC_ERR_STATE, "peer %u has no framebuffer (or snapshot) of the same size", g); }
-        // order the gather after the peer's pending renders
-        CUDA_TRY(root, cudaSetDevice(peer->device));
-        CUDA_TRY(root, cudaEventRecord(peer->framebufferReady, peer->stream));
-        CUDA_TRY(root, cudaSetDevice(root->device));
-        CUDA_TRY(root, cudaStreamWaitEvent(root->stream, peer->framebufferReady, 0));
-        int canAccess = 0;
-        if (peer->device != root->device) { cudaDeviceCanAccessPeer(&canAccess, root->device, peer->device); }
-        if (peer->device == root->device) { set.fb[set.count++] = source(peer); continue; }
-        if (canAccess) {
-            const cudaError_t e = cudaDeviceEnablePeerAccess(peer->device, 0);
-            if (e == cudaSuccess || e == cudaErrorPeerAccessAlreadyEnabled) { cudaGetLastError(); set.fb[set.count++] = source(peer); continue; }
-            cudaGetLastError();
-        }
-        // no peer mapping: stage the peer's framebuffer into local memory first
-        if (root->gatherStageSize < (size_t)nPeers * n) {
-            CUDA_TRY(root, cudaStreamSynchronize(root->stream));
-            cudaFree(root->gatherStage); root->gatherStage = nullptr; root->gatherStageSize = 0;
-            CUDA_TRY(root, cudaMalloc((void **)&root->gatherStage, (size_t)nPeers * n * sizeof(float)));
-            root->gatherStageSize = (size_t)nPeers * n;
-        }
-        float *slot = root->gatherStage + staged * n; staged++;
-        CUDA_TRY(root, cudaMemcpyPeerAsync(slot, root->device, source(peer), peer->device, n * sizeof(float), root->stream));
-        set.fb[set.count++] = slot;
-    }
-    // a free result slot (device buffer + pinned host buffer + event)
+    if ((rc = gatherSets(root, peers, nPeers, &source, 1, &set))) { return rc; }
     uint32_t ticket = 0;
-    while (ticket < root->gathers.size() && root->gathers[ticket].busy) { ticket++; }
-    if (ticket == root->gathers.size()) { root->gathers.push_back(ptc_ctx::Gather()); }
-    ptc_ctx::Gather &slot = root->gathers[ticket];
-    if (!slot.device) {
-        CUDA_TRY(root, cudaMalloc((void **)&slot.device, n * sizeof(float)));
-        CUDA_TRY(root, cudaMallocHost((void **)&slot.pinned, n * sizeof(float)));
-        CUDA_TRY(root, cudaEventCreateWithFlags(&slot.done, cudaEventDisableTiming));
-    }
-    gatherResolveKernel<<<std::min<uint32_t>((uint32_t)((n / 4 + 255) / 256) + 1, (uint32_t)root->gridSimple * 4), 256, 0, root->stream>>>(set, slot.device, (uint32_t)n, divisor);
+    if ((rc = takeGatherSlot(root, &ticket))) { return rc; }
+    gatherResolveKernel<<<std::min<uint32_t>((uint32_t)((n / 4 + 255) / 256) + 1, (uint32_t)root->gridSimple * 4), 256, 0, root->stream>>>(set, root->gathers[ticket].device, (uint32_t)n, divisor);
     root->launches++;
-    CUDA_TRY(root, cudaGetLastError());
-    // renders that follow on any of the contexts must not overwrite what this kernel reads
-    if (!root->gatherRead) { CUDA_TRY(root, cudaEventCreateWithFlags(&root->gatherRead, cudaEventDisableTiming)); }
-    CUDA_TRY(root, cudaEventRecord(root->gatherRead, root->stream));
-    for (uint32_t g = 0; g < nPeers; g++) { CUDA_TRY(root, cudaStreamWaitEvent(peers[g]->stream, root->gatherRead, 0)); }
-    CUDA_TRY(root, cudaMemcpyAsync(slot.pinned, slot.device, n * sizeof(float), cudaMemcpyDeviceToHost, root->stream));
-    CUDA_TRY(root, cudaEventRecord(slot.done, root->stream));
-    slot.busy = true;
+    if ((rc = finishGather(root, peers, nPeers, ticket))) { return rc; }
     *ticketOut = ticket;
     return PTC_OK;
 }
@@ -2626,6 +2702,56 @@ static int roundTrip(ptc_ctx *ctx, const In *in, size_t nIn, Out *out, size_t nO
 }
 static inline uint32_t gridFor(ptc_ctx *ctx, uint32_t n) { return std::max(1u, std::min<uint32_t>((n + 127) / 128, (uint32_t)ctx->gridSimple * 4)); }
 
+// ------------------------------------------------------------------------------------------------ denoising (denoise.cuh)
+// the device guide sums (albedo 3, normal 3, depth 1, hits 1 x 4 B per pixel) of ptc_render_aovs and ptc_framebuffer_guides
+static int ensureAovs(ptc_ctx *ctx, size_t pixels)
+{
+    ptc_ctx::Aovs &a = ctx->aovs;
+    if (a.pixels == pixels) { return PTC_OK; }
+    cudaFree(a.buffer); a.buffer = nullptr; a.pixels = 0;
+    CUDA_TRY(ctx, cudaMalloc((void **)&a.buffer, 8 * pixels * sizeof(float)));
+    a.pixels = pixels;
+    return PTC_OK;
+}
+
+static int checkDenoiseDesc(ptc_ctx *ctx, const ptc_denoise_desc *desc)
+{
+    auto positive = [](float v) { return v > 0.f && std::isfinite(v); };
+    if (!desc || desc->iterations > 10 || !positive(desc->sigma_l) || !(desc->sigma_n >= 0.f && std::isfinite(desc->sigma_n)) ||
+        !positive(desc->sigma_z) || !positive(desc->sigma_a) || !positive(desc->eps)) {
+        CTX_FAIL(ctx, PTC_ERR_INVALID, "bad denoise descriptor (iterations <= 10, sigma_l, sigma_z, sigma_a, eps > 0, sigma_n >= 0)");
+    }
+    return PTC_OK;
+}
+
+// The a-trous levels over ctx->denoise.colour[0] (the prepared colour records) on the context's stream; the result is in
+// colour[desc->iterations & 1]
+static int denoiseAtrous(ptc_ctx *ctx, const ptc_denoise_desc *desc, const float4 *guide)
+{
+    ptc_ctx::Denoise &d = ctx->denoise;
+    const int width = ctx->scene.width, height = ctx->scene.height;
+    DenoiseParams dp;
+    dp.sigmaL = desc->sigma_l; dp.sigmaN = desc->sigma_n; dp.sigmaZ = desc->sigma_z; dp.sigmaA = desc->sigma_a; dp.eps = desc->eps;
+    const dim3 block(32, 8), grid((unsigned)(width + 31) / 32, (unsigned)(height + 7) / 8);
+    for (uint32_t i = 0; i < desc->iterations; i++) {
+        denoiseAtrousKernel<<<grid, block, 0, ctx->stream>>>(d.colour[i & 1], d.colour[(i + 1) & 1], guide, width, height, 1 << i, dp);
+        ctx->launches++;
+        CUDA_TRY(ctx, cudaGetLastError());
+    }
+    return PTC_OK;
+}
+
+static int ensureDenoiseColour(ptc_ctx *ctx, size_t pixels)
+{
+    ptc_ctx::Denoise &d = ctx->denoise;
+    if (d.colourPixels == pixels) { return PTC_OK; }
+    cudaFree(d.colour[0]); cudaFree(d.colour[1]); d.colour[0] = d.colour[1] = nullptr; d.colourPixels = 0;
+    CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[0], pixels * sizeof(float4)));
+    CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[1], pixels * sizeof(float4)));
+    d.colourPixels = pixels;
+    return PTC_OK;
+}
+
 extern "C" {
 
 int ptc_intersect(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit *hits)
@@ -2733,13 +2859,9 @@ int ptc_render_aovs(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t 
     if (!albedo || !normal || !depth || !hits) { CTX_FAIL(ctx, PTC_ERR_INVALID, "null guide buffer"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
-    ptc_ctx::Aovs &a = ctx->aovs;
-    if (a.pixels != pixels) {
-        cudaFree(a.buffer); a.buffer = nullptr; a.pixels = 0;
-        CUDA_TRY(ctx, cudaMalloc((void **)&a.buffer, 8 * pixels * sizeof(float)));
-        a.pixels = pixels;
-    }
-    float *d = a.buffer;
+    const int rc = ensureAovs(ctx, pixels);
+    if (rc) { return rc; }
+    float *d = ctx->aovs.buffer;
     float *dAlbedo = d, *dNormal = d + 3 * pixels, *dDepth = d + 6 * pixels;
     uint32_t *dHits = (uint32_t *)(d + 7 * pixels);
     cudaError_t e = cudaSuccess;
@@ -2762,16 +2884,49 @@ int ptc_render_aovs(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t 
     return PTC_OK;
 }
 
+// The same guide sums from zero into the context's device buffers, then the guide records of ptc_denoise's prepare step
+int ptc_framebuffer_guides(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp, float *albedo, float *normal, float *depth, uint32_t *hits)
+{
+    NEED_COMMIT(ctx);
+    if (!nSpp) { CTX_FAIL(ctx, PTC_ERR_INVALID, "n_spp must be > 0: the guide records are means over the samples"); }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
+    int rc = ensureAovs(ctx, pixels);
+    if (rc) { return rc; }
+    ptc_ctx::Guides &g = ctx->guides;
+    g.aovSpp = 0; // no guides until this call has enqueued them
+    if (g.pixels != pixels) {
+        cudaFree(g.records); g.records = nullptr; g.pixels = 0;
+        CUDA_TRY(ctx, cudaMalloc((void **)&g.records, 2 * pixels * sizeof(float4)));
+        g.pixels = pixels;
+    }
+    float *d = ctx->aovs.buffer;
+    float *dAlbedo = d, *dNormal = d + 3 * pixels, *dDepth = d + 6 * pixels;
+    uint32_t *dHits = (uint32_t *)(d + 7 * pixels);
+    CUDA_TRY(ctx, cudaMemsetAsync(d, 0, 8 * pixels * sizeof(float), ctx->stream));
+    aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene, seed, firstSample, nSpp, dAlbedo, dNormal, dDepth, dHits);
+    denoiseGuideKernel<<<std::min<uint32_t>((uint32_t)((pixels + 255) / 256), (uint32_t)ctx->gridSimple * 4), 256, 0, ctx->stream>>>(
+        dAlbedo, dNormal, dDepth, dHits, nSpp, (uint32_t)pixels, g.records);
+    ctx->launches += 2;
+    CUDA_TRY(ctx, cudaGetLastError());
+    const struct { void *dst; const void *src; size_t bytes; } fetches[] = {
+        {albedo, dAlbedo, 3 * pixels * 4}, {normal, dNormal, 3 * pixels * 4}, {depth, dDepth, pixels * 4}, {hits, dHits, pixels * 4}};
+    bool fetched = false;
+    for (const auto &f : fetches) {
+        if (f.dst) { CUDA_TRY(ctx, cudaMemcpyAsync(f.dst, f.src, f.bytes, cudaMemcpyDeviceToHost, ctx->stream)); fetched = true; }
+    }
+    if (fetched) { CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); }
+    g.aovSpp = nSpp; g.width = ctx->scene.width; g.height = ctx->scene.height;
+    return PTC_OK;
+}
+
 // The filter (denoise.cuh): inputs staged in one device buffer, one kernel that builds the colour and guide records, one a-trous
 // launch per iteration between the two colour buffers, the last one's colours copied back
 int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_input *in, float *out)
 {
     NEED_COMMIT(ctx);
-    auto positive = [](float v) { return v > 0.f && std::isfinite(v); };
-    if (!desc || desc->iterations > 10 || !positive(desc->sigma_l) || !(desc->sigma_n >= 0.f && std::isfinite(desc->sigma_n)) ||
-        !positive(desc->sigma_z) || !positive(desc->sigma_a) || !positive(desc->eps)) {
-        CTX_FAIL(ctx, PTC_ERR_INVALID, "bad denoise descriptor (iterations <= 10, sigma_l, sigma_z, sigma_a, eps > 0, sigma_n >= 0)");
-    }
+    int rc = checkDenoiseDesc(ctx, desc);
+    if (rc) { return rc; }
     if (!in || !out || !in->sums || !in->moments || !in->albedo_rgb || !in->normal_xyz || !in->depth || !in->hits) {
         CTX_FAIL(ctx, PTC_ERR_INVALID, "missing denoise input");
     }
@@ -2784,14 +2939,12 @@ int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_in
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     ptc_ctx::Denoise &d = ctx->denoise;
     if (d.pixels != pixels) {
-        cudaFree(d.inputs); cudaFree(d.guide); cudaFree(d.colour[0]); cudaFree(d.colour[1]);
-        d = ptc_ctx::Denoise();
+        cudaFree(d.inputs); cudaFree(d.guide); d.inputs = nullptr; d.guide = nullptr; d.pixels = 0;
         CUDA_TRY(ctx, cudaMalloc((void **)&d.inputs, 15 * pixels * sizeof(float)));
         CUDA_TRY(ctx, cudaMalloc((void **)&d.guide, 2 * pixels * sizeof(float4)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[0], pixels * sizeof(float4)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[1], pixels * sizeof(float4)));
         d.pixels = pixels;
     }
+    if ((rc = ensureDenoiseColour(ctx, pixels))) { return rc; }
     DenoiseInputs di;
     float *f = d.inputs;
     di.sums = f; di.moments = f + 3 * pixels; di.albedo = f + 6 * pixels; di.normal = f + 9 * pixels; di.depth = f + 12 * pixels;
@@ -2805,20 +2958,62 @@ int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_in
     denoisePrepareKernel<<<std::min<uint32_t>((uint32_t)((pixels + 255) / 256), (uint32_t)ctx->gridSimple * 4), 256, 0, ctx->stream>>>(di, d.colour[0], d.guide);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
-    DenoiseParams dp;
-    dp.sigmaL = desc->sigma_l; dp.sigmaN = desc->sigma_n; dp.sigmaZ = desc->sigma_z; dp.sigmaA = desc->sigma_a; dp.eps = desc->eps;
-    const dim3 block(32, 8), grid((unsigned)(width + 31) / 32, (unsigned)(height + 7) / 8);
-    for (uint32_t i = 0; i < desc->iterations; i++) {
-        denoiseAtrousKernel<<<grid, block, 0, ctx->stream>>>(d.colour[i & 1], d.colour[(i + 1) & 1], d.guide, width, height, 1 << i, dp);
-        ctx->launches++;
-        CUDA_TRY(ctx, cudaGetLastError());
-    }
+    if ((rc = denoiseAtrous(ctx, desc, d.guide))) { return rc; }
     std::vector<float4> result(pixels);
     CUDA_TRY(ctx, cudaMemcpyAsync(result.data(), d.colour[desc->iterations & 1], pixels * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     for (size_t p = 0; p < pixels; p++) { out[3 * p] = result[p].x; out[3 * p + 1] = result[p].y; out[3 * p + 2] = result[p].z; }
     return PTC_OK;
 }
+
+// ptc_denoise on what the contexts hold: the colour records straight from the (peer-read) sums and moments, the guide records of
+// ptc_framebuffer_guides, the same a-trous levels, and the image out through a gather slot
+int ptc_framebuffer_denoise_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, int snapshot, uint32_t spp, const ptc_denoise_desc *desc,
+                                  uint32_t *ticketOut)
+{
+    NEED_COMMIT(root);
+    int rc = checkDenoiseDesc(root, desc);
+    if (rc) { return rc; }
+    if (!ticketOut || (nPeers && !peers) || nPeers > PTC_MAX_PEERS) { CTX_FAIL(root, PTC_ERR_INVALID, "bad denoise arguments"); }
+    const ptc_ctx::Adaptive &a = root->adaptive;
+    if (!a.on && spp < 2) { CTX_FAIL(root, PTC_ERR_INVALID, "spp must be >= 2: the variance needs 2 samples"); }
+    CUDA_TRY(root, cudaSetDevice(root->device));
+    if ((rc = ensureFramebuffer(root))) { return rc; }
+    const size_t n = root->framebufferSize, pixels = n / 3;
+    if (!root->guides.aovSpp || root->guides.width != root->scene.width || root->guides.height != root->scene.height || pixels != root->guides.pixels) { CTX_FAIL(root, PTC_ERR_STATE, "no guides of this resolution: ptc_framebuffer_guides first"); }
+    if (a.on && a.n == 0) { CTX_FAIL(root, PTC_ERR_STATE, "the adaptive render has no pass yet"); }
+    if (a.on && snapshot >= 0) { CTX_FAIL(root, PTC_ERR_STATE, "an adaptive render keeps no checkpoint snapshots"); }
+    const GatherSource sources[2] = {
+        [&](ptc_ctx *c) -> const float * {
+            return snapshot < 0 ? c->framebuffer : (size_t)snapshot < c->snapshots.size() && c->snapshotSize == n ? c->snapshots[snapshot] : nullptr;
+        },
+        [&](ptc_ctx *c) -> const float * {
+            if (snapshot < 0) { return framebufferMoments(c, n); }
+            const bool held = c->snapshotsHoldMoments && c->snapshotSize == n && (size_t)snapshot < c->snapshots.size() && c->snapshotMomentsComplete[snapshot];
+            return held ? c->snapshots[snapshot] + n : nullptr;
+        }};
+    if (!sources[0](root)) { CTX_FAIL(root, PTC_ERR_STATE, "no snapshot %d was rendered", snapshot); }
+    if (!sources[1](root)) {
+        CTX_FAIL(root, PTC_ERR_STATE, "no second moments of every sample of this image (option framebuffer_moments on since the last clear, or an adaptive render)");
+    }
+    FramebufferSet sets[2];
+    if ((rc = gatherSets(root, peers, nPeers, sources, 2, sets))) { return rc; }
+    if ((rc = ensureDenoiseColour(root, pixels))) { return rc; }
+    uint32_t ticket = 0;
+    if ((rc = takeGatherSlot(root, &ticket))) { return rc; }
+    const uint32_t grid = std::min<uint32_t>((uint32_t)((pixels + 255) / 256), (uint32_t)root->gridSimple * 4);
+    ptc_ctx::Denoise &d = root->denoise;
+    denoiseGatherKernel<<<grid, 256, 0, root->stream>>>(sets[0], sets[1], a.on ? a.counts : nullptr, spp, (uint32_t)pixels, d.colour[0]);
+    root->launches++;
+    CUDA_TRY(root, cudaGetLastError());
+    if ((rc = denoiseAtrous(root, desc, root->guides.records))) { return rc; }
+    denoisePackKernel<<<grid, 256, 0, root->stream>>>(d.colour[desc->iterations & 1], root->gathers[ticket].device, (uint32_t)pixels);
+    root->launches++;
+    if ((rc = finishGather(root, peers, nPeers, ticket))) { return rc; }
+    *ticketOut = ticket;
+    return PTC_OK;
+}
+
 int ptc_philox4x32_10(ptc_ctx *ctx, const uint32_t *counters, const uint32_t *keys, uint32_t n, uint32_t *out)
 {
     if (!ctx || (n && (!counters || !keys || !out))) { return PTC_ERR_INVALID; }

@@ -115,6 +115,7 @@ int pth_job_describe(const char *jobPath, char *out, int outLen, char *err, int 
           << ", \"adaptive\": " << (job.adaptive() ? "true" : "false") << ", \"adaptive_threshold\": " << job.adaptiveThreshold()
           << ", \"adaptive_min_spp\": " << job.adaptiveMinSpp() << ", \"adaptive_step_spp\": " << job.adaptiveStepSpp()
           << ", \"denoise\": " << (job.denoise() ? "true" : "false")
+          << ", \"denoise_checkpoints\": " << (job.denoiseCheckpoints() ? "true" : "false")
           << ", \"scene\": \"" << job.scene() << "\", \"output_directory\": \"" << job.outputDirectory()
           << "\", \"output_name\": \"" << job.outputName() << "\", \"integrator_status\": \"" << status << "\"}";
         snprintf(out, (size_t)outLen, "%s", o.str().c_str());

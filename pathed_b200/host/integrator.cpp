@@ -53,6 +53,16 @@ double now()
     return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
+// The guide buffers need far fewer samples than the colour (a pixel's first hits differ only across its footprint): at most this many
+const uint32_t kGuideSpp = 16;
+uint32_t guideSpp() { return std::min<uint32_t>((uint32_t)g_job->spp(), kGuideSpp); }
+
+// The guides of the first guideSpp() samples on device 0 for ptc_framebuffer_denoise_begin, enqueued without waiting for them
+void enqueueGuides(ptc_ctx *ctx, uint64_t seed)
+{
+    check(ctx, ptc_framebuffer_guides(ctx, seed, 0, guideSpp(), nullptr, nullptr, nullptr, nullptr), "guide buffers");
+}
+
 } // namespace
 
 // ------------------------------------------------------------------------------------------------ Scene
@@ -219,7 +229,9 @@ void CudaPathTracer::sampleImage(std::vector<float> &radianceLookup, Scene &scen
 // src/integrator.cpp:87-92) that fall inside a wave are snapshots the resolve kernel keeps on the way (ptc_framebuffer_render_
 // checkpoints): waves do not end there.  After a wave ONE kernel on GPU 0 per image sums the framebuffers (or snapshots) through peer
 // (NVLink) loads and divides by the sample count (K7 resolve); the copies to the host are asynchronous, and the next wave is
-// enqueued before the host converts, reports and saves this one -- GPU and host work overlap.
+// enqueued before the host converts, reports and saves this one -- GPU and host work overlap.  With "denoise_checkpoints" every
+// checkpoint of at least 2 samples is also denoised on GPU 0 from the same snapshots (ptc_framebuffer_denoise_begin), its image
+// fetched through the same ticket queue, and saved as denoised-auto; the guides are rendered once, after the first wave's renders.
 void CudaPathTracer::run(Image &image, Scene &scene, std::function<void(RenderStatus)> callback, bool *quit)
 {
     const int width = g_job->width(), height = g_job->height(), primarySamples = g_job->spp();
@@ -241,8 +253,11 @@ void CudaPathTracer::run(Image &image, Scene &scene, std::function<void(RenderSt
     for (int g = 1; g < gpus; g++) { peers.push_back(scene.context(g)); }
     ptc_ctx *root = scene.context(0);
     std::vector<float> resolved((size_t)3 * width * height);
+    const bool denoiseCheckpoints = g_job->denoiseCheckpoints();
+    const ptc_denoise_desc desc = PTC_DENOISE_DEFAULTS;
+    std::unique_ptr<Image> denoised(denoiseCheckpoints ? new Image(width, height) : nullptr); // the destructor waits for its files
 
-    struct Pending { int spp; uint32_t ticket; bool checkpoint; };
+    struct Pending { int spp; uint32_t ticket; bool checkpoint; bool denoised = false; };
     struct Wave { int first = 0, end = 0; std::vector<Pending> images; double enqueued = 0.0; };
     // enqueue the wave that starts at sample `first`: renders on every GPU, then one gather per image wanted from it
     auto enqueue = [&](int first) {
@@ -260,14 +275,24 @@ void CudaPathTracer::run(Image &image, Scene &scene, std::function<void(RenderSt
             check(scene.context(g), ptc_framebuffer_render_checkpoints(scene.context(g), m_seed, (uint32_t)from, (uint32_t)count, start, last,
                                                                        counts.data(), (uint32_t)counts.size()), "render");
         }
+        if (denoiseCheckpoints && first == 0) { enqueueGuides(root, m_seed); }
+        // the denoised image of snapshot `snapshot` (-1: the framebuffers), a checkpoint of `spp` samples
+        auto denoise = [&](int snapshot, int spp) {
+            if (!denoiseCheckpoints || spp < 2) { return; }
+            Pending d; d.spp = spp; d.checkpoint = true; d.denoised = true;
+            check(root, ptc_framebuffer_denoise_begin(root, peers.data(), (uint32_t)peers.size(), snapshot, (uint32_t)spp, &desc, &d.ticket), "checkpoint denoise");
+            wave.images.push_back(d);
+        };
         for (size_t i = 0; i < counts.size(); i++) {
             Pending p; p.spp = (int)counts[i]; p.checkpoint = true;
             check(root, ptc_framebuffer_gather_begin(root, peers.data(), (uint32_t)peers.size(), (int)i, counts[i], &p.ticket), "checkpoint gather");
             wave.images.push_back(p);
+            denoise((int)i, p.spp);
         }
         Pending p; p.spp = wave.end; p.checkpoint = (wave.end & (wave.end - 1)) == 0;
         check(root, ptc_framebuffer_gather_begin(root, peers.data(), (uint32_t)peers.size(), -1, (uint32_t)wave.end, &p.ticket), "framebuffer gather");
         wave.images.push_back(p);
+        if (p.checkpoint) { denoise(-1, p.spp); }
         return wave;
     };
 
@@ -279,6 +304,12 @@ void CudaPathTracer::run(Image &image, Scene &scene, std::function<void(RenderSt
         if (more) { next = enqueue(current.end); } // the GPUs go on while the host handles the images of `current`
         for (const Pending &p : current.images) {
             check(root, ptc_framebuffer_gather_end(root, p.ticket, resolved.data()), "framebuffer gather");
+            if (p.denoised) {
+                denoised->setSpp(p.spp);
+                denoised->setAll(resolved.data());
+                denoised->saveCheckpoint("denoised-auto");
+                continue;
+            }
             std::lock_guard<std::mutex> guard(image.getLock());
             image.setSpp(p.spp);
             image.setAll(resolved.data());
@@ -316,6 +347,8 @@ void CudaPathTracer::runAdaptive(Image &image, Scene &scene, std::function<void(
     check(ctx, ptc_adaptive_begin(ctx, &desc), "adaptive begin");
     std::vector<float> sums(3 * pixels), resolved(3 * pixels);
     std::vector<uint32_t> counts(pixels);
+    const ptc_denoise_desc denoiseDesc = PTC_DENOISE_DEFAULTS;
+    std::unique_ptr<Image> denoised(g_job->denoiseCheckpoints() ? new Image(width, height) : nullptr);
     const double loopBegin = now();
     for (int pass = 1;; pass++) {
         const double begin = now();
@@ -338,6 +371,17 @@ void CudaPathTracer::runAdaptive(Image &image, Scene &scene, std::function<void(
             image.setAll(resolved.data());
             if ((n & (n - 1)) == 0) { image.saveCheckpoint("auto"); }
         }
+        if (denoised) {
+            if (pass == 1) { enqueueGuides(ctx, m_seed); }
+            if ((n & (n - 1)) == 0 && n >= 2) { // n is ignored: the per-pixel counts of the adaptive render are used
+                uint32_t ticket = 0;
+                check(ctx, ptc_framebuffer_denoise_begin(ctx, nullptr, 0, -1, n, &denoiseDesc, &ticket), "checkpoint denoise");
+                check(ctx, ptc_framebuffer_gather_end(ctx, ticket, resolved.data()), "checkpoint denoise");
+                denoised->setSpp((int)n);
+                denoised->setAll(resolved.data());
+                denoised->saveCheckpoint("denoised-auto");
+            }
+        }
         postwave(scene, (int)n);
         RenderStatus status;
         status.setSample((int)n);
@@ -355,14 +399,12 @@ void CudaPathTracer::runAdaptive(Image &image, Scene &scene, std::function<void(
     saveEXR(g_job->outputDirectory() + "adaptive-spp.exr", width, height, {"Y"}, {plane.data()}, false);
 }
 
-// The guide buffers need far fewer samples than the colour (a pixel's first hits differ only across its footprint): at most this many
-static const uint32_t kGuideSpp = 16;
-
-// "denoise": true -- after run(), from what the contexts still hold: the sums and second moments gathered over every GPU (an
-// adaptive job: the sums, per-pixel counts and moments of its adaptive render on device 0), the guide buffers of the first
-// min(spp, kGuideSpp) samples on device 0, and ptc_denoise with the default parameters.  denoised.exr is written like final.exr
-// (Image: HALF, B,G,R, top scanline first); albedo.exr and normal.exr hold the guide buffers' means in fp32, what an external
-// denoiser takes besides the colour.
+// "denoise": true -- after run(), from what the contexts still hold: ptc_framebuffer_denoise_begin with the default parameters over
+// the sums and second moments of every GPU (an adaptive job: the sums, per-pixel counts and moments of its adaptive render on device
+// 0) and the guides of the first min(spp, kGuideSpp) samples on device 0, rendered here again when the checkpoints were denoised (the
+// same bytes: this call also fetches their sums, which the checkpoints' asynchronous guide pass did not wait for).
+// denoised.exr is written like final.exr (Image: HALF, B,G,R, top scanline first); albedo.exr and normal.exr hold the guide
+// buffers' means in fp32, what an external denoiser takes besides the colour.
 void CudaPathTracer::writeDenoised(Scene &scene)
 {
     const int width = g_job->width(), height = g_job->height();
@@ -370,28 +412,15 @@ void CudaPathTracer::writeDenoised(Scene &scene)
     ptc_ctx *ctx = scene.context(0);
     std::vector<ptc_ctx *> peers;
     for (int g = 1; g < scene.gpus(); g++) { peers.push_back(scene.context(g)); }
-    std::vector<float> sums(3 * pixels), moments(3 * pixels);
-    std::vector<uint32_t> counts;
-    check(ctx, ptc_framebuffer_gather(ctx, peers.data(), (uint32_t)peers.size(), 1, sums.data()), "framebuffer gather");
-    if (g_job->adaptive()) {
-        counts.resize(pixels);
-        check(ctx, ptc_adaptive_state(ctx, counts.data(), moments.data()), "adaptive state");
-    } else {
-        uint32_t ticket = 0;
-        check(ctx, ptc_framebuffer_gather_begin(ctx, peers.data(), (uint32_t)peers.size(), PTC_GATHER_MOMENTS, 1, &ticket), "moments gather");
-        check(ctx, ptc_framebuffer_gather_end(ctx, ticket, moments.data()), "moments gather");
-    }
-    const uint32_t *countsOrNull = counts.empty() ? nullptr : counts.data();
-    const uint32_t spp = m_nextSample; // uniform jobs: the samples every pixel holds
-    const uint32_t aovSpp = std::min<uint32_t>((uint32_t)g_job->spp(), kGuideSpp);
-    std::vector<float> albedo(3 * pixels, 0.f), normal(3 * pixels, 0.f), depth(pixels, 0.f), out(3 * pixels);
-    std::vector<uint32_t> hits(pixels, 0);
-    check(ctx, ptc_render_aovs(ctx, m_seed, 0, aovSpp, albedo.data(), normal.data(), depth.data(), hits.data()), "guide buffers");
+    const uint32_t aovSpp = guideSpp();
+    std::vector<float> albedo(3 * pixels, 0.f), normal(3 * pixels, 0.f);
+    check(ctx, ptc_framebuffer_guides(ctx, m_seed, 0, aovSpp, albedo.data(), normal.data(), nullptr, nullptr), "guide buffers");
     const ptc_denoise_desc desc = PTC_DENOISE_DEFAULTS;
-    ptc_denoise_input in;
-    in.sums = sums.data(); in.moments = moments.data(); in.counts = countsOrNull; in.spp = spp;
-    in.albedo_rgb = albedo.data(); in.normal_xyz = normal.data(); in.depth = depth.data(); in.hits = hits.data(); in.aov_spp = aovSpp;
-    check(ctx, ptc_denoise(ctx, &desc, &in, out.data()), "denoise");
+    std::vector<float> out(3 * pixels);
+    uint32_t ticket = 0;
+    // uniform jobs: m_nextSample = the samples every pixel holds
+    check(ctx, ptc_framebuffer_denoise_begin(ctx, peers.data(), (uint32_t)peers.size(), -1, m_nextSample, &desc, &ticket), "denoise");
+    check(ctx, ptc_framebuffer_gather_end(ctx, ticket, out.data()), "denoise");
     {
         Image denoised(width, height);
         denoised.setAll(out.data());

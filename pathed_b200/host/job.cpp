@@ -56,6 +56,9 @@ Job::Job(std::istream &jobFile)
     const Json &denoiseKey = (*m_json)["denoise"];
     if (!denoiseKey.isNull() && !denoiseKey.isBool()) { throw std::runtime_error("denoise must be true or false"); }
     if (denoise() && spp() < 2) { throw std::runtime_error("denoise needs spp >= 2: the filter estimates each pixel's variance"); }
+    const Json &checkpointsKey = (*m_json)["denoise_checkpoints"];
+    if (!checkpointsKey.isNull() && !checkpointsKey.isBool()) { throw std::runtime_error("denoise_checkpoints must be true or false"); }
+    if (denoiseCheckpoints() && !denoise()) { throw std::runtime_error("denoise_checkpoints needs \"denoise\": true"); }
     if (!adaptive()) { return; }
     const double threshold = (*m_json)["adaptive_threshold"].asNumber();
     if (!(threshold > 0.0) || !std::isfinite(threshold)) { throw std::runtime_error("adaptive_threshold must be a number > 0"); }
@@ -90,6 +93,7 @@ int Job::gpus() const { return (*m_json)["gpus"].isNumber() ? std::max(1, (*m_js
 uint64_t Job::seed() const { return (*m_json)["seed"].isNumber() ? (uint64_t)(*m_json)["seed"].asNumber() : 0x5EEDull; }
 int Job::waveSpp() const { return (*m_json)["wave_spp"].isNumber() ? std::max(1, (*m_json)["wave_spp"].asInt()) : 64; }
 bool Job::denoise() const { return (*m_json)["denoise"].isBool() && (*m_json)["denoise"].asBool(); }
+bool Job::denoiseCheckpoints() const { return (*m_json)["denoise_checkpoints"].isBool() && (*m_json)["denoise_checkpoints"].asBool(); }
 bool Job::adaptive() const { return !(*m_json)["adaptive_threshold"].isNull(); }
 float Job::adaptiveThreshold() const { return adaptive() ? (float)(*m_json)["adaptive_threshold"].asNumber() : 0.f; }
 int Job::adaptiveMinSpp() const { return (*m_json)["adaptive_min_spp"].isNumber() ? (*m_json)["adaptive_min_spp"].asInt() : 16; }

@@ -81,6 +81,9 @@ public:
     // guide buffers it used); any value but a bool is refused by the constructor, and so is true with spp < 2 (the filter needs
     // each pixel's variance)
     bool denoise() const;
+    // "denoise_checkpoints": true (default false; needs "denoise": true, any value but a bool is refused) also denoises every
+    // checkpoint of at least 2 samples on the devices: denoised-auto.exr and denoised-auto-%05dspp.exr, like auto-*.exr
+    bool denoiseCheckpoints() const;
 
     // string -> integrator (src/job.cpp:65-97); anything but "PathTracer" throws const char* "Unimplemented"
     std::shared_ptr<Integrator> integrator() const;
