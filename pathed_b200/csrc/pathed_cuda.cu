@@ -1093,6 +1093,57 @@ struct HostGeometry {
 };
 struct HostScene { uint32_t nGeoms = 0; std::vector<uint32_t> members; }; // members: indices into ptc_ctx::geometries, attach order
 
+// Owners of the CUDA resources a context (or a query's scope) holds: each is released with its owner, so no release is listed anywhere.
+// Buffer: `size()` elements of device memory, or of page-locked host memory when PINNED.  resize(n) reallocates when n differs from
+// the size, reserve(n) only when n is larger; the contents after a reallocation are undefined.
+template <typename T, bool PINNED = false>
+class Buffer {
+public:
+    Buffer() = default;
+    Buffer(T *p, size_t n) : p_(p), n_(n) {} // takes ownership of an allocation made elsewhere
+    Buffer(Buffer &&o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr; o.n_ = 0; }
+    Buffer &operator=(Buffer &&o) noexcept { std::swap(p_, o.p_); std::swap(n_, o.n_); return *this; }
+    ~Buffer() { release(); }
+    cudaError_t resize(size_t n)
+    {
+        if (n == n_) { return cudaSuccess; }
+        release();
+        const cudaError_t e = PINNED ? cudaMallocHost((void **)&p_, n * sizeof(T)) : cudaMalloc((void **)&p_, n * sizeof(T));
+        if (e == cudaSuccess) { n_ = n; } else { p_ = nullptr; }
+        return e;
+    }
+    cudaError_t reserve(size_t n) { return n > n_ ? resize(n) : cudaSuccess; }
+    T *get() const { return p_; }
+    size_t size() const { return n_; }
+private:
+    void release() { if (p_) { if (PINNED) { cudaFreeHost(p_); } else { cudaFree(p_); } } p_ = nullptr; n_ = 0; }
+    T *p_ = nullptr; size_t n_ = 0;
+};
+template <typename T> using PinnedBuffer = Buffer<T, true>;
+// A non-blocking stream and an event; create() makes the handle on its first call (events without timing unless asked)
+class Stream {
+public:
+    Stream() = default;
+    Stream(Stream &&o) noexcept : s_(o.s_) { o.s_ = nullptr; }
+    Stream &operator=(Stream &&o) noexcept { std::swap(s_, o.s_); return *this; }
+    ~Stream() { if (s_) { cudaStreamDestroy(s_); } }
+    cudaError_t create() { return s_ ? cudaSuccess : cudaStreamCreateWithFlags(&s_, cudaStreamNonBlocking); }
+    operator cudaStream_t() const { return s_; }
+private:
+    cudaStream_t s_ = nullptr;
+};
+class Event {
+public:
+    Event() = default;
+    Event(Event &&o) noexcept : e_(o.e_) { o.e_ = nullptr; }
+    Event &operator=(Event &&o) noexcept { std::swap(e_, o.e_); return *this; }
+    ~Event() { if (e_) { cudaEventDestroy(e_); } }
+    cudaError_t create(unsigned flags = cudaEventDisableTiming) { return e_ ? cudaSuccess : cudaEventCreateWithFlags(&e_, flags); }
+    operator cudaEvent_t() const { return e_; }
+private:
+    cudaEvent_t e_ = nullptr;
+};
+
 struct ptc_ctx {
     int device = 0;
     std::string error;
@@ -1110,11 +1161,11 @@ struct ptc_ctx {
     struct HostMedium { float sigmaT[3], sigmaS[3]; };
     std::vector<HostMedium> media;
     int integrator = PTC_INTEGRATOR_PATH_TRACER;
-    float4 *volumeOut = nullptr; uint32_t volumeCapacity = 0; uint32_t *volumeCursor = nullptr;
+    Buffer<float4> volumeOut; Buffer<uint32_t> volumeCursor;
     int gridVolume = 0;
     // VolumePathTracer as wavefront stages (volume_wavefront.cuh); volumeMegakernel = 1 keeps the one-thread-per-path kernel
     bool volumeMegakernel = false;
-    VolumeBuffers volumeBuffers = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}; uint32_t volumeBufferCapacity = 0; std::vector<void *> volumeAllocations;
+    VolumeBuffers volumeBuffers = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}; Buffer<uint8_t> volumeArrays[6];
     int gridVolumeTraverse = 0, gridVolumeLogic = 0, gridVolumeShade = 0;
     bool hasEnv = false, hasCamera = false;
     std::vector<float> envRgba; int envW = 0, envH = 0; float envScale = 1.f; float envM2W[16], envW2M[16];
@@ -1122,33 +1173,33 @@ struct ptc_ctx {
     WideBVH bvh;
     uint32_t nLights = 0;
     // device
-    std::vector<void *> allocations; std::vector<size_t> allocationBytes; // scene data on the device (what ptc_replicate copies)
-    std::vector<DMaterial> deviceMaterials;                              // the device material table as uploaded (holds texel pointers)
+    std::vector<Buffer<uint8_t>> allocations;  // scene data on the device (what ptc_replicate copies)
+    std::vector<DMaterial> deviceMaterials;    // the device material table as uploaded (holds texel pointers)
     DScene scene;
-    PathBuffers paths; uint32_t pathCapacity = 0; std::vector<void *> pathAllocations;
-    uint32_t classQueueCapacity = 0, classQueueMask = 0; std::vector<void *> classQueueAllocations;
-    BounceCounters *counters = nullptr;
+    PathBuffers paths; uint32_t pathCapacity = 0; Buffer<uint8_t> pathSlab;
+    Buffer<uint32_t> classQueues[PTC_MATERIAL_CLASSES];
+    Buffer<BounceCounters> counters;
     uint32_t classMask = 0; // material classes present in the scene
-    unsigned long long *totals = nullptr;
-    float *accumScratch = nullptr; size_t accumScratchSize = 0;
-    float *framebuffer = nullptr, *gatherStage = nullptr; size_t framebufferSize = 0, gatherStageSize = 0;
-    cudaEvent_t framebufferReady = nullptr;
-    std::vector<float *> snapshots;                      // checkpoint copies of the framebuffer (ptc_framebuffer_render_checkpoints)
+    Buffer<unsigned long long> totals;
+    Buffer<float> accumScratch;
+    Buffer<float> framebuffer, gatherStage;
+    Event framebufferReady;
+    std::vector<Buffer<float>> snapshots;                // checkpoint copies of the framebuffer (ptc_framebuffer_render_checkpoints)
     // snapshots allocated with option framebuffer_moments on hold the sums and then the second moments (accumulateKernel<true>); a
-    // snapshot's moments are complete when they cover every sample its sums hold (fbMoments.complete when it was written)
+    // snapshot's moments are complete when they cover every sample its sums hold (momentsComplete when it was written)
     bool snapshotsHoldMoments = false;
     size_t snapshotSize = 0; // floats of sums per snapshot: the framebuffer size they were allocated for
     std::vector<bool> snapshotMomentsComplete;
-    struct Gather { float *device = nullptr, *pinned = nullptr; size_t size = 0; cudaEvent_t done = nullptr; bool busy = false; };
+    struct Gather { Buffer<float> device; PinnedBuffer<float> pinned; Event done; bool busy = false; };
     std::vector<Gather> gathers;                         // results of ptc_framebuffer_gather_begin in flight
-    cudaEvent_t gatherRead = nullptr;                    // the last gather kernel of this (root) context finished reading the framebuffers
-    float *pinned = nullptr; size_t pinnedSize = 0;
+    Event gatherRead;                                    // the last gather kernel of this (root) context finished reading the framebuffers
+    PinnedBuffer<float> pinned;
     // ptc_render: the caller's radianceLookup is uploaded on its own stream while the wave's kernels run; only the first
     // accumulation waits for it (beforeAccumulate is called once, after the wave's other launches have been issued)
-    cudaStream_t copyStream = nullptr; cudaEvent_t uploadDone = nullptr;
+    Stream copyStream; Event uploadDone;
     std::function<int()> beforeAccumulate;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t evStart = nullptr, evStop = nullptr;
+    Stream stream;
+    Event evStart, evStop;
     int numSMs = 148;
     int gridTraverse = 0, gridShade = 0, gridLogic = 0, gridSimple = 0;
     int gridTraverseShared = 0, gridVolumeTraverseShared = 0; // traversal grids of a wave traced as several lanes: two CTAs per SM fewer
@@ -1160,100 +1211,104 @@ struct ptc_ctx {
     // the shadow rays of a bounce are traced on a second stream, concurrently with the bounce's extend rays: both grids fill the GPU, so
     // the shadow CTAs become resident as the extend kernel drains -- the tail of one launch is filled with the head of the other
     bool overlapShadow = true;
-    cudaStream_t shadowStream = nullptr; cudaEvent_t shadeDone = nullptr, shadowDone = nullptr;
+    Stream shadowStream; Event shadeDone, shadowDone;
     // A wave is traced as `lanes` interleaved part-waves (consecutive blocks of the wave's samples, each with its own share of the path
     // state, its own counters and streams): while one lane's paths are in a shading stage (waiting on dependent loads, half of the issue
     // slots idle) another lane's rays are in a traversal stage (issue-bound, hardly any DRAM traffic), and the SMs hold CTAs of both.
     // Lane 0 runs on the caller's stream; the samples are still added to the image in sample order (launchWave), so the result does
     // not depend on the number of lanes.
     int lanes = 0; // 0 = chosen per wave (renderInternal)
-    struct Lane { cudaStream_t stream = nullptr, shadowStream = nullptr; cudaEvent_t shadeDone = nullptr, shadowDone = nullptr, done = nullptr; BounceCounters *counters = nullptr; };
+    struct Lane { Stream stream, shadowStream; Event shadeDone, shadowDone, done; Buffer<BounceCounters> counters; };
     std::vector<Lane> extraLanes; // lanes 1 ..
-    cudaEvent_t laneFork = nullptr;
+    Event laneFork;
     int bvhBuilder = 1; // 1: device builder (bvh_build_gpu.cu), 0: host binned-SAH builder (bvh_build.cu)
     float bvhBuildMs = 0.f; uint32_t bvhPlocIterations = 0;
     // the device builder leaves nodes and leaf triangles in HBM; the host copy (only ptc_count_traversal walks it) is fetched on demand
     uint32_t bvhNodeCount = 0, bvhTriangleCount = 0;
     bool hostBvhFetched = true;
-    void *buildWorkspace = nullptr; // the device builder's working set, released with the context (bvh.h: buildWideBVHDevice)
+    Buffer<uint8_t> buildWorkspace; // the device builder's working set, released with the context (bvh.h: buildWideBVHDevice)
     // adaptive sampling (ptc_adaptive_*): between begin and the next ptc_framebuffer_clear the framebuffer belongs to the passes.
-    // Per pixel: second moments (3 x fp32, next to the framebuffer's sums), sample count, and two list entries (active pixels,
-    // the stopping test's output) = 24 B, plus cub's selection scratch
+    // Per pixel: second moments (`moments` below), sample count, and two list entries (active pixels, the stopping test's output)
+    // = 24 B, plus cub's selection scratch
     struct Adaptive {
         bool on = false;
         ptc_adaptive_desc desc = {0.f, 0, 0, 0};
         uint32_t n = 0, active = 0; // the samples every active pixel holds; pixels still active
         size_t pixels = 0;          // what the buffers are sized for
-        float *moments = nullptr;
-        uint32_t *counts = nullptr, *list = nullptr, *next = nullptr, *selected = nullptr, *selectedHost = nullptr;
-        void *scratch = nullptr; size_t scratchBytes = 0;
+        Buffer<uint32_t> counts, list, next, selected;
+        PinnedBuffer<uint32_t> selectedHost;
+        Buffer<uint8_t> scratch;
     } adaptive;
-    // option "framebuffer_moments": the framebuffer renders also add the squared samples into `moments` (3 x fp32 per pixel, zeroed
-    // by ptc_framebuffer_clear), the input of ptc_denoise that PTC_GATHER_MOMENTS gathers.  complete: the moments cover every sample
-    // the framebuffer holds (the option was on at the last clear and at every render since); the gather refuses them otherwise
-    struct FramebufferMoments { bool on = false, complete = false; float *moments = nullptr; size_t size = 0; } fbMoments;
-    // ptc_denoise's device buffers: the staged inputs (15 x 4 B per pixel) and guide records (32 B), sized for `pixels`; two colour
-    // records (16 B each, sized for colourPixels), which ptc_framebuffer_denoise_begin uses as well
-    struct Denoise { size_t pixels = 0, colourPixels = 0; float *inputs = nullptr; float4 *guide = nullptr, *colour[2] = {nullptr, nullptr}; } denoise;
+    // The second moments (3 x fp32 per pixel, next to the framebuffer's sums): the squared samples that the adaptive passes add, and,
+    // with option "framebuffer_moments" (momentsOption), the framebuffer renders; zeroed by ptc_adaptive_begin and, with the option
+    // on, by ptc_framebuffer_clear.  The input of ptc_denoise that PTC_GATHER_MOMENTS gathers.  momentsComplete: they cover every
+    // sample the framebuffer holds (an adaptive render, or the option on at the last clear and at every render since); the gather
+    // refuses them otherwise
+    bool momentsOption = false, momentsComplete = false;
+    Buffer<float> moments;
+    // ptc_denoise's device buffers: the staged inputs (15 x 4 B per pixel) and guide records (32 B); two colour records (16 B each),
+    // which ptc_framebuffer_denoise_begin uses as well
+    struct Denoise { Buffer<float> inputs; Buffer<float4> guide, colour[2]; } denoise;
     // the device guide sums of ptc_render_aovs and ptc_framebuffer_guides (8 x 4 B per pixel)
-    struct Aovs { size_t pixels = 0; float *buffer = nullptr; } aovs;
+    Buffer<float> aovs;
     // ptc_framebuffer_guides: the guide records (32 B per pixel) ptc_framebuffer_denoise_begin filters with; aovSpp = 0: none
-    struct Guides { size_t pixels = 0; int width = 0, height = 0; float4 *records = nullptr; uint32_t aovSpp = 0; } guides;
+    struct Guides { int width = 0, height = 0; Buffer<float4> records; uint32_t aovSpp = 0; } guides;
     uint64_t samples = 0, launches = 0;
     float lastRenderMs = 0.f;
     // stage timing: CUDA events on the launching stream around every launch, summed per kernel class
-    struct Timed { cudaEvent_t a, b; int kind; };
+    struct Timed { Event a, b; int kind; };
     std::vector<Timed> pending;
-    std::vector<cudaEvent_t> eventPool;
+    std::vector<Event> eventPool;
     double stageMs[4] = {0, 0, 0, 0};
     uint64_t stageLaunches[4] = {0, 0, 0, 0};
 };
 
 enum { STAGE_EXTEND = 0, STAGE_SHADOW = 1, STAGE_SHADE = 2, STAGE_OTHER = 3 };
 
-static cudaEvent_t takeEvent(ptc_ctx *ctx)
+static Event takeEvent(ptc_ctx *ctx)
 {
-    if (!ctx->eventPool.empty()) { cudaEvent_t e = ctx->eventPool.back(); ctx->eventPool.pop_back(); return e; }
-    cudaEvent_t e = nullptr;
-    cudaEventCreate(&e);
+    Event e;
+    if (!ctx->eventPool.empty()) { e = std::move(ctx->eventPool.back()); ctx->eventPool.pop_back(); }
+    else { e.create(cudaEventDefault); }
     return e;
 }
 static void collectTimings(ptc_ctx *ctx)
 {
-    for (const ptc_ctx::Timed &t : ctx->pending) {
+    for (ptc_ctx::Timed &t : ctx->pending) {
         float ms = 0.f;
         cudaEventSynchronize(t.b);
         cudaEventElapsedTime(&ms, t.a, t.b);
         ctx->stageMs[t.kind] += ms; ctx->stageLaunches[t.kind]++;
-        ctx->eventPool.push_back(t.a); ctx->eventPool.push_back(t.b);
+        ctx->eventPool.push_back(std::move(t.a)); ctx->eventPool.push_back(std::move(t.b));
     }
     ctx->pending.clear();
 }
 struct StageTimer { // brackets one launch when stage timing is on
-    ptc_ctx *ctx; cudaStream_t stream; cudaEvent_t a = nullptr; int kind;
+    ptc_ctx *ctx; cudaStream_t stream; Event a; int kind;
     StageTimer(ptc_ctx *c, cudaStream_t s, int k) : ctx(c), stream(s), kind(k)
     {
         if (ctx->stageTiming) { a = takeEvent(ctx); cudaEventRecord(a, stream); }
     }
     ~StageTimer()
     {
-        if (a) { cudaEvent_t b = takeEvent(ctx); cudaEventRecord(b, stream); ctx->pending.push_back({a, b, kind}); }
+        if (a) { Event b = takeEvent(ctx); cudaEventRecord(b, stream); ctx->pending.push_back({std::move(a), std::move(b), kind}); }
     }
 };
 
 #define CTX_FAIL(ctx, code, ...) do { char _b[512]; snprintf(_b, sizeof(_b), __VA_ARGS__); (ctx)->error = _b; return (code); } while (0)
 #define CUDA_TRY(ctx, call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(_e)); } } while (0)
 
+// grid of a grid-stride launch over n >= 1 items
+static inline uint32_t gridFor(ptc_ctx *ctx, uint32_t n, uint32_t block = 128) { return std::max(1u, std::min<uint32_t>((n + block - 1) / block, (uint32_t)ctx->gridSimple * 4)); }
+
 template <typename T>
-static int upload(ptc_ctx *ctx, const T *src, size_t count, const T **dst, std::vector<void *> &track)
+static int upload(ptc_ctx *ctx, const T *src, size_t count, const T **dst)
 {
-    void *p = nullptr;
-    const size_t bytes = std::max<size_t>(count, 1) * sizeof(T);
-    CUDA_TRY(ctx, cudaMalloc(&p, bytes));
-    track.push_back(p);
-    if (&track == &ctx->allocations) { ctx->allocationBytes.push_back(bytes); }
-    if (count) { CUDA_TRY(ctx, cudaMemcpy(p, src, count * sizeof(T), cudaMemcpyHostToDevice)); }
-    *dst = (const T *)p;
+    Buffer<uint8_t> b;
+    CUDA_TRY(ctx, b.resize(std::max<size_t>(count, 1) * sizeof(T)));
+    *dst = (const T *)b.get();
+    ctx->allocations.push_back(std::move(b));
+    if (count) { CUDA_TRY(ctx, cudaMemcpy((void *)*dst, src, count * sizeof(T), cudaMemcpyHostToDevice)); }
     return PTC_OK;
 }
 
@@ -1276,17 +1331,14 @@ int ptc_create(int device, ptc_ctx **out)
     memset(&ctx->paths, 0, sizeof(ctx->paths));
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) { ctx->numSMs = prop.multiProcessorCount; }
-    if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaStreamCreateWithFlags(&ctx->shadowStream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaStreamCreateWithFlags(&ctx->copyStream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&ctx->uploadDone, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&ctx->shadeDone, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&ctx->shadowDone, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreate(&ctx->evStart) != cudaSuccess || cudaEventCreate(&ctx->evStop) != cudaSuccess ||
-        cudaMalloc((void **)&ctx->counters, CNT_STRIDE * sizeof(BounceCounters)) != cudaSuccess ||
-        cudaMalloc((void **)&ctx->totals, 6 * sizeof(unsigned long long)) != cudaSuccess) {
+    if (ctx->stream.create() != cudaSuccess || ctx->shadowStream.create() != cudaSuccess || ctx->copyStream.create() != cudaSuccess ||
+        ctx->uploadDone.create() != cudaSuccess || ctx->shadeDone.create() != cudaSuccess || ctx->shadowDone.create() != cudaSuccess ||
+        ctx->evStart.create(cudaEventDefault) != cudaSuccess || ctx->evStop.create(cudaEventDefault) != cudaSuccess ||
+        ctx->counters.resize(CNT_STRIDE) != cudaSuccess || ctx->totals.resize(6) != cudaSuccess) {
         delete ctx;
         return PTC_ERR_CUDA;
     }
-    cudaMemset(ctx->totals, 0, 6 * sizeof(unsigned long long));
+    cudaMemset(ctx->totals.get(), 0, 6 * sizeof(unsigned long long));
     int perSM = 0;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, (traverseKernel<false, false>), 128, 0);
     ctx->gridTraverse = ctx->numSMs * std::max(perSM, 1);
@@ -1320,43 +1372,8 @@ void ptc_destroy(ptc_ctx *ctx)
     if (!ctx) { return; }
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
-    for (void *p : ctx->allocations) { cudaFree(p); }
-    ctx->allocations.clear(); ctx->allocationBytes.clear();
-    for (void *p : ctx->pathAllocations) { cudaFree(p); }
-    for (void *p : ctx->classQueueAllocations) { cudaFree(p); }
-    cudaFree(ctx->counters); cudaFree(ctx->totals); cudaFree(ctx->accumScratch);
-    for (ptc_ctx::Lane &lane : ctx->extraLanes) {
-        if (lane.stream) { cudaStreamDestroy(lane.stream); } if (lane.shadowStream) { cudaStreamDestroy(lane.shadowStream); }
-        for (cudaEvent_t e : {lane.shadeDone, lane.shadowDone, lane.done}) { if (e) { cudaEventDestroy(e); } }
-        cudaFree(lane.counters);
-    }
-    if (ctx->laneFork) { cudaEventDestroy(ctx->laneFork); }
-    cudaFree(ctx->framebuffer); cudaFree(ctx->gatherStage);
-    cudaFree(ctx->adaptive.moments); cudaFree(ctx->adaptive.counts); cudaFree(ctx->adaptive.list); cudaFree(ctx->adaptive.next);
-    cudaFree(ctx->adaptive.selected); cudaFree(ctx->adaptive.scratch);
-    if (ctx->adaptive.selectedHost) { cudaFreeHost(ctx->adaptive.selectedHost); }
-    cudaFree(ctx->fbMoments.moments); cudaFree(ctx->aovs.buffer);
-    cudaFree(ctx->denoise.inputs); cudaFree(ctx->denoise.guide); cudaFree(ctx->denoise.colour[0]); cudaFree(ctx->denoise.colour[1]);
-    cudaFree(ctx->guides.records);
-    for (float *snapshot : ctx->snapshots) { cudaFree(snapshot); }
-    for (auto &g : ctx->gathers) { cudaFree(g.device); if (g.pinned) { cudaFreeHost(g.pinned); } if (g.done) { cudaEventDestroy(g.done); } }
-    if (ctx->gatherRead) { cudaEventDestroy(ctx->gatherRead); }
-    cudaFree(ctx->volumeOut); cudaFree(ctx->volumeCursor);
-    for (void *p : ctx->volumeAllocations) { cudaFree(p); }
-    cudaFree(ctx->buildWorkspace);
-    if (ctx->framebufferReady) { cudaEventDestroy(ctx->framebufferReady); }
-    if (ctx->pinned) { cudaFreeHost(ctx->pinned); }
-    if (ctx->stream) { cudaStreamDestroy(ctx->stream); }
-    if (ctx->shadowStream) { cudaStreamDestroy(ctx->shadowStream); }
-    if (ctx->copyStream) { cudaStreamDestroy(ctx->copyStream); }
-    if (ctx->uploadDone) { cudaEventDestroy(ctx->uploadDone); }
-    if (ctx->shadeDone) { cudaEventDestroy(ctx->shadeDone); }
-    if (ctx->shadowDone) { cudaEventDestroy(ctx->shadowDone); }
-    if (ctx->evStart) { cudaEventDestroy(ctx->evStart); }
-    if (ctx->evStop) { cudaEventDestroy(ctx->evStop); }
     collectTimings(ctx);
-    for (cudaEvent_t e : ctx->eventPool) { cudaEventDestroy(e); }
-    delete ctx;
+    delete ctx; // the members release the context's buffers, streams and events
 }
 
 const char *ptc_last_error(ptc_ctx *ctx) { return ctx ? ctx->error.c_str() : "null context"; }
@@ -1675,27 +1692,28 @@ int ptc_commit(ptc_ctx *ctx)
     // rtcCommitScene: BVH over all triangle geometries; spheres are kept in a flat list.  The geometry goes to the device first:
     // the default builder runs there (option "bvh_builder" = 0 selects the host binned-SAH builder instead).
     int rc;
-    auto &A = ctx->allocations;
-    if ((rc = upload(ctx, (const float4 *)ctx->positions4.data(), ctx->positions4.size() / 4, &s.positions, A))) { return rc; }
-    if ((rc = upload(ctx, (const uint4 *)prims4.data(), prims4.size() / 4, &s.prims, A))) { return rc; }
+    if ((rc = upload(ctx, (const float4 *)ctx->positions4.data(), ctx->positions4.size() / 4, &s.positions))) { return rc; }
+    if ((rc = upload(ctx, (const uint4 *)prims4.data(), prims4.size() / 4, &s.prims))) { return rc; }
     const float4 *buildPositions = s.positions; const uint4 *buildPrims = s.prims; // what the BVH is built over: world-space triangles
     const std::vector<float> &hostBuildPositions = instanced ? worldPos4 : ctx->positions4;
     const std::vector<uint32_t> &hostBuildPrims = instanced ? worldPrims4 : ctx->prims4;
     if (instanced) {
-        if ((rc = upload(ctx, (const float4 *)worldPos4.data(), worldPos4.size() / 4, &buildPositions, A))) { return rc; }
-        if ((rc = upload(ctx, (const uint4 *)worldPrims4.data(), worldPrims4.size() / 4, &buildPrims, A))) { return rc; }
+        if ((rc = upload(ctx, (const float4 *)worldPos4.data(), worldPos4.size() / 4, &buildPositions))) { return rc; }
+        if ((rc = upload(ctx, (const uint4 *)worldPrims4.data(), worldPrims4.size() / 4, &buildPrims))) { return rc; }
         s.instIds = nullptr;
-        if ((rc = upload(ctx, (const uint2 *)flatInst2.data(), flatInst2.size() / 2, &s.instIds, A))) { return rc; }
+        if ((rc = upload(ctx, (const uint2 *)flatInst2.data(), flatInst2.size() / 2, &s.instIds))) { return rc; }
     } else { s.instIds = nullptr; }
     {
         const auto buildStart = std::chrono::steady_clock::now();
         try {
             if (ctx->bvhBuilder == 1) {
                 DeviceWideBVH built;
-                if (ctx->buildWorkspace) { cudaFree(ctx->buildWorkspace); ctx->buildWorkspace = nullptr; }
-                buildWideBVHDevice(buildPositions, buildPrims, nPrims, ctx->stream, built, &ctx->buildWorkspace);
-                if (built.nodes) { A.push_back(built.nodes); ctx->allocationBytes.push_back((size_t)built.nNodes * sizeof(WideNode)); }
-                if (built.triangles) { A.push_back(built.triangles); ctx->allocationBytes.push_back((size_t)built.nTriangles * sizeof(LeafTriangle)); }
+                void *workspace = nullptr;
+                ctx->buildWorkspace = Buffer<uint8_t>(); // an earlier build's working set goes before this build allocates its own
+                buildWideBVHDevice(buildPositions, buildPrims, nPrims, ctx->stream, built, &workspace);
+                ctx->buildWorkspace = Buffer<uint8_t>((uint8_t *)workspace, 0); // the builder does not report its size
+                if (built.nodes) { ctx->allocations.emplace_back((uint8_t *)built.nodes, (size_t)built.nNodes * sizeof(WideNode)); }
+                if (built.triangles) { ctx->allocations.emplace_back((uint8_t *)built.triangles, (size_t)built.nTriangles * sizeof(LeafTriangle)); }
                 s.bvh.nodes = built.nodes; s.bvh.triangles = built.triangles; s.bvh.nNodes = built.nNodes;
                 ctx->bvhPlocIterations = built.plocIterations;
                 // no host copy here (49 MB through pageable memory cost more than the build): fetchHostBvh brings it when
@@ -1704,8 +1722,8 @@ int ptc_commit(ptc_ctx *ctx)
                 ctx->bvhNodeCount = built.nNodes; ctx->bvhTriangleCount = built.nTriangles; ctx->hostBvhFetched = false;
             } else {
                 buildWideBVH(hostBuildPositions.data(), hostBuildPrims.data(), nPrims, ctx->bvh);
-                if ((rc = upload(ctx, (const float4 *)ctx->bvh.nodes.data(), ctx->bvh.nodes.size() * 5, &s.bvh.nodes, A))) { return rc; }
-                if ((rc = upload(ctx, (const float4 *)ctx->bvh.triangles.data(), ctx->bvh.triangles.size() * 3, &s.bvh.triangles, A))) { return rc; }
+                if ((rc = upload(ctx, (const float4 *)ctx->bvh.nodes.data(), ctx->bvh.nodes.size() * 5, &s.bvh.nodes))) { return rc; }
+                if ((rc = upload(ctx, (const float4 *)ctx->bvh.triangles.data(), ctx->bvh.triangles.size() * 3, &s.bvh.triangles))) { return rc; }
                 s.bvh.nNodes = (uint32_t)ctx->bvh.nodes.size();
                 ctx->bvhNodeCount = (uint32_t)ctx->bvh.nodes.size(); ctx->bvhTriangleCount = (uint32_t)ctx->bvh.triangles.size(); ctx->hostBvhFetched = true;
             }
@@ -1714,8 +1732,8 @@ int ptc_commit(ptc_ctx *ctx)
         ctx->bvh.placements = placements;
         if (!placements.empty() && ctx->bvhTriangleCount) {
             const uint32_t *tags = nullptr;
-            if ((rc = upload(ctx, flatTag.data(), flatTag.size(), &tags, A))) { return rc; }
-            if ((rc = upload(ctx, (const float4 *)placements.data(), placements.size() / 4, &s.bvh.placements, A))) { return rc; }
+            if ((rc = upload(ctx, flatTag.data(), flatTag.size(), &tags))) { return rc; }
+            if ((rc = upload(ctx, (const float4 *)placements.data(), placements.size() / 4, &s.bvh.placements))) { return rc; }
             const uint32_t nTriangles = ctx->bvhTriangleCount;
             LeafTriangle *leaves = (LeafTriangle *)s.bvh.triangles;
             localizeLeavesKernel<<<(nTriangles + 255) / 256, 256, 0, ctx->stream>>>(leaves, nTriangles, s.positions, s.prims, tags);
@@ -1728,7 +1746,7 @@ int ptc_commit(ptc_ctx *ctx)
     // textures: packed texels per image, one gamma table for all (Texture::lookup's powf(c / 255.f, 2.2f), src/texture.cpp:44-48)
     std::vector<const uint32_t *> deviceTexels(ctx->textures.size(), nullptr);
     for (size_t t = 0; t < ctx->textures.size(); t++) {
-        const int rcTex = upload(ctx, ctx->textures[t].texels.data(), ctx->textures[t].texels.size(), &deviceTexels[t], ctx->allocations);
+        const int rcTex = upload(ctx, ctx->textures[t].texels.data(), ctx->textures[t].texels.size(), &deviceTexels[t]);
         if (rcTex) { return rcTex; }
     }
     {
@@ -1787,10 +1805,10 @@ int ptc_commit(ptc_ctx *ctx)
     if (ctx->hasEnv) { DLight l; memset(&l, 0, sizeof(l)); l.kind = 2; lights.push_back(l); }
     ctx->nLights = (uint32_t)lights.size();
 
-    if ((rc = upload(ctx, (const float4 *)spheres4.data(), spheres4.size() / 4, &s.bvh.spheres, A))) { return rc; }
+    if ((rc = upload(ctx, (const float4 *)spheres4.data(), spheres4.size() / 4, &s.bvh.spheres))) { return rc; }
     s.bvh.nSpheres = (uint32_t)(spheres4.size() / 4);
-    if ((rc = upload(ctx, (const float4 *)ctx->normals4.data(), ctx->normals4.size() / 4, &s.normals, A))) { return rc; }
-    if ((rc = upload(ctx, (const float2 *)ctx->uvs2.data(), ctx->uvs2.size() / 2, &s.uvs, A))) { return rc; }
+    if ((rc = upload(ctx, (const float4 *)ctx->normals4.data(), ctx->normals4.size() / 4, &s.normals))) { return rc; }
+    if ((rc = upload(ctx, (const float2 *)ctx->uvs2.data(), ctx->uvs2.size() / 2, &s.uvs))) { return rc; }
     { // per-triangle shading records (shading.cuh: DScene::triShade); Ng = e2 x e1 with the fused multiply-subtracts of triangleNg
         std::vector<float> rec((size_t)nPrims * 20, 0.f);
         for (uint32_t p = 0; p < nPrims; p++) {
@@ -1808,20 +1826,20 @@ int ptc_commit(ptc_ctx *ctx)
                 r[13 + 2 * k] = t[0]; r[14 + 2 * k] = t[1];
             }
         }
-        if ((rc = upload(ctx, (const float4 *)rec.data(), rec.size() / 4, &s.triShade, A))) { return rc; }
+        if ((rc = upload(ctx, (const float4 *)rec.data(), rec.size() / 4, &s.triShade))) { return rc; }
     }
-    if ((rc = upload(ctx, (const uint2 *)primIds2.data(), primIds2.size() / 2, &s.primIds, A))) { return rc; }
-    if ((rc = upload(ctx, (const uint2 *)sphereIds2.data(), sphereIds2.size() / 2, &s.sphereIds, A))) { return rc; }
-    if ((rc = upload(ctx, dm.data(), dm.size(), &s.materials, A))) { return rc; }
+    if ((rc = upload(ctx, (const uint2 *)primIds2.data(), primIds2.size() / 2, &s.primIds))) { return rc; }
+    if ((rc = upload(ctx, (const uint2 *)sphereIds2.data(), sphereIds2.size() / 2, &s.sphereIds))) { return rc; }
+    if ((rc = upload(ctx, dm.data(), dm.size(), &s.materials))) { return rc; }
     ctx->deviceMaterials = dm;
     { // one byte per primitive / sphere for the logic stage: material type | emitter << 3
         std::vector<uint8_t> primClass(nPrims), sphereClass(sphereIds2.size() / 2);
         for (uint32_t p = 0; p < nPrims; p++) { const DMaterial &m = dm[prims4[4 * (size_t)p + 3]]; primClass[p] = (uint8_t)(m.type | (m.emitter ? 8 : 0)); }
         for (size_t i = 0; i < sphereClass.size(); i++) { const DMaterial &m = dm[sphereIds2[2 * i + 1]]; sphereClass[i] = (uint8_t)(m.type | (m.emitter ? 8 : 0)); }
-        if ((rc = upload(ctx, primClass.data(), primClass.size(), &s.primClass, A))) { return rc; }
-        if ((rc = upload(ctx, sphereClass.data(), sphereClass.size(), &s.sphereClass, A))) { return rc; }
+        if ((rc = upload(ctx, primClass.data(), primClass.size(), &s.primClass))) { return rc; }
+        if ((rc = upload(ctx, sphereClass.data(), sphereClass.size(), &s.sphereClass))) { return rc; }
     }
-    if ((rc = upload(ctx, lights.data(), lights.size(), &s.lights, A))) { return rc; }
+    if ((rc = upload(ctx, lights.data(), lights.size(), &s.lights))) { return rc; }
     s.nLights = ctx->nLights;
 
     // participating media: sigma_t / sigma_s, the internal medium of every geometry, and the occlusion filter's table (a
@@ -1846,10 +1864,10 @@ int ptc_commit(ptc_ctx *ctx)
                 if (dm[ctx->prims4[4 * (size_t)p + 3]].type == PTC_PASSTHROUGH) { primEvent[p] = ge.medium; s.hasFilter = 1; }
             }
         }
-        if ((rc = upload(ctx, (const float4 *)media4.data(), media4.size() / 4, &s.media, A))) { return rc; }
-        if ((rc = upload(ctx, geomMedium.data(), geomMedium.size(), &s.geomMedium, A))) { return rc; }
-        if ((rc = upload(ctx, primEvent.data(), primEvent.size(), &s.bvh.primEvent, A))) { return rc; }
-        if ((rc = upload(ctx, sphereEvent.data(), sphereEvent.size(), &s.bvh.sphereEvent, A))) { return rc; }
+        if ((rc = upload(ctx, (const float4 *)media4.data(), media4.size() / 4, &s.media))) { return rc; }
+        if ((rc = upload(ctx, geomMedium.data(), geomMedium.size(), &s.geomMedium))) { return rc; }
+        if ((rc = upload(ctx, primEvent.data(), primEvent.size(), &s.bvh.primEvent))) { return rc; }
+        if ((rc = upload(ctx, sphereEvent.data(), sphereEvent.size(), &s.bvh.sphereEvent))) { return rc; }
     }
 
     s.hasEnv = ctx->hasEnv ? 1 : 0;
@@ -1874,12 +1892,12 @@ int ptc_commit(ptc_ctx *ctx)
         std::vector<uint16_t> thetaGuide((size_t)s.envThetaG + 1), phiGuide((size_t)h * (s.envPhiG + 1));
         buildGuide(thetaCdf.data(), h, s.envThetaG, thetaGuide.data());
         for (int t = 0; t < h; t++) { buildGuide(&phiCdf[(size_t)t * w], w, s.envPhiG, &phiGuide[(size_t)t * (s.envPhiG + 1)]); }
-        if ((rc = upload(ctx, thetaGuide.data(), thetaGuide.size(), &s.envThetaGuide, A))) { return rc; }
-        if ((rc = upload(ctx, phiGuide.data(), phiGuide.size(), &s.envPhiGuide, A))) { return rc; }
-        if ((rc = upload(ctx, (const float4 *)ctx->envRgba.data(), (size_t)w * h, &s.envRgba, A))) { return rc; }
-        if ((rc = upload(ctx, thetaCdf.data(), thetaCdf.size(), &s.envThetaCdf, A))) { return rc; }
-        if ((rc = upload(ctx, phiCdf.data(), phiCdf.size(), &s.envPhiCdf, A))) { return rc; }
-        if ((rc = upload(ctx, phiEmpty.data(), phiEmpty.size(), &s.envPhiEmpty, A))) { return rc; }
+        if ((rc = upload(ctx, thetaGuide.data(), thetaGuide.size(), &s.envThetaGuide))) { return rc; }
+        if ((rc = upload(ctx, phiGuide.data(), phiGuide.size(), &s.envPhiGuide))) { return rc; }
+        if ((rc = upload(ctx, (const float4 *)ctx->envRgba.data(), (size_t)w * h, &s.envRgba))) { return rc; }
+        if ((rc = upload(ctx, thetaCdf.data(), thetaCdf.size(), &s.envThetaCdf))) { return rc; }
+        if ((rc = upload(ctx, phiCdf.data(), phiCdf.size(), &s.envPhiCdf))) { return rc; }
+        if ((rc = upload(ctx, phiEmpty.data(), phiEmpty.size(), &s.envPhiEmpty))) { return rc; }
         s.envW = w; s.envH = h; s.envScale = ctx->envScale;
         for (int r = 0; r < 3; r++) { for (int c = 0; c < 4; c++) { s.envM2W[4 * r + c] = ctx->envM2W[4 * r + c]; s.envW2M[4 * r + c] = ctx->envW2M[4 * r + c]; } }
     }
@@ -1930,16 +1948,16 @@ int ptc_replicate(ptc_ctx *src, int device, ptc_ctx **out)
     dst->scene = src->scene;
     auto fail = [&](const char *what) { src->error = std::string("ptc_replicate: ") + what + ": " + cudaGetErrorString(cudaGetLastError()); ptc_destroy(dst); return PTC_ERR_CUDA; };
     if (cudaSetDevice(device) != cudaSuccess) { return fail("cudaSetDevice"); }
-    for (size_t i = 0; i < src->allocations.size(); i++) {
-        void *copy = nullptr;
-        if (cudaMalloc(&copy, src->allocationBytes[i]) != cudaSuccess) { return fail("cudaMalloc"); }
-        dst->allocations.push_back(copy); dst->allocationBytes.push_back(src->allocationBytes[i]);
-        if (cudaMemcpyPeerAsync(copy, device, src->allocations[i], src->device, src->allocationBytes[i], dst->stream) != cudaSuccess) { return fail("cudaMemcpyPeerAsync"); }
+    for (const Buffer<uint8_t> &a : src->allocations) {
+        Buffer<uint8_t> copy;
+        if (copy.resize(a.size()) != cudaSuccess) { return fail("cudaMalloc"); }
+        dst->allocations.push_back(std::move(copy));
+        if (cudaMemcpyPeerAsync(dst->allocations.back().get(), device, a.get(), src->device, a.size(), dst->stream) != cudaSuccess) { return fail("cudaMemcpyPeerAsync"); }
     }
     bool rebased = true;
     auto rebase = [&](const void **field) {
         if (!*field) { return; }
-        for (size_t i = 0; i < src->allocations.size(); i++) { if (src->allocations[i] == *field) { *field = dst->allocations[i]; return; } }
+        for (size_t i = 0; i < src->allocations.size(); i++) { if (src->allocations[i].get() == *field) { *field = dst->allocations[i].get(); return; } }
         rebased = false;
     };
     forEachScenePointer(dst->scene, rebase);
@@ -1967,8 +1985,7 @@ static int ensurePathBuffers(ptc_ctx *ctx, uint32_t capacity, bool withClassQueu
 {
     PathBuffers &pb = ctx->paths;
     if (capacity > ctx->pathCapacity) {
-        for (void *p : ctx->pathAllocations) { cudaFree(p); }
-        ctx->pathAllocations.clear(); ctx->pathCapacity = 0;
+        ctx->pathCapacity = 0;
         struct { void **slot; size_t bytesPerPath; } arrays[] = {
             {(void **)&pb.out, 16}, {(void **)&pb.ray, 32}, {(void **)&pb.nRay, 32}, {(void **)&pb.modThr, 32}, {(void **)&pb.nModThr, 32}, {(void **)&pb.nee, 32},
             {(void **)&pb.hit, 16}, {(void **)&pb.result, 16}, {(void **)&pb.nResult, 16}, {(void **)&pb.occluded, 1}, {(void **)&pb.shadowQueue, 4}};
@@ -1977,23 +1994,17 @@ static int ensurePathBuffers(ptc_ctx *ctx, uint32_t capacity, bool withClassQueu
         // allocations change the throughput (profiles/r02_path_state_layout.txt).
         size_t total = 0;
         for (auto &a : arrays) { total += ((size_t)capacity * a.bytesPerPath + 255u) & ~(size_t)255u; }
-        char *base = nullptr;
-        CUDA_TRY(ctx, cudaMalloc((void **)&base, total));
-        ctx->pathAllocations.push_back(base);
+        CUDA_TRY(ctx, ctx->pathSlab.reserve(total));
         size_t offset = 0;
-        for (auto &a : arrays) { *a.slot = base + offset; offset += ((size_t)capacity * a.bytesPerPath + 255u) & ~(size_t)255u; }
+        for (auto &a : arrays) { *a.slot = ctx->pathSlab.get() + offset; offset += ((size_t)capacity * a.bytesPerPath + 255u) & ~(size_t)255u; }
         ctx->pathCapacity = capacity;
     }
-    if (withClassQueues && (ctx->pathCapacity > ctx->classQueueCapacity || ctx->classQueueMask != ctx->classMask)) {
-        for (void *p : ctx->classQueueAllocations) { cudaFree(p); }
-        ctx->classQueueAllocations.clear(); ctx->classQueueCapacity = 0;
-        for (int t = 0; t < PTC_MATERIAL_CLASSES; t++) {
-            pb.classQueue[t] = nullptr;
-            if (!(ctx->classMask & (1u << t))) { continue; }
-            CUDA_TRY(ctx, cudaMalloc((void **)&pb.classQueue[t], (size_t)ctx->pathCapacity * sizeof(uint32_t)));
-            ctx->classQueueAllocations.push_back(pb.classQueue[t]);
-        }
-        ctx->classQueueCapacity = ctx->pathCapacity; ctx->classQueueMask = ctx->classMask;
+    if (!withClassQueues) { return PTC_OK; }
+    for (int t = 0; t < PTC_MATERIAL_CLASSES; t++) {
+        pb.classQueue[t] = nullptr;
+        if (!(ctx->classMask & (1u << t))) { continue; }
+        CUDA_TRY(ctx, ctx->classQueues[t].reserve(ctx->pathCapacity));
+        pb.classQueue[t] = ctx->classQueues[t].get();
     }
     return PTC_OK;
 }
@@ -2045,16 +2056,16 @@ static PathBuffers laneBuffers(const PathBuffers &all, size_t offset)
 
 static int ensureLanes(ptc_ctx *ctx, int lanes)
 {
-    if (!ctx->laneFork) { CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->laneFork, cudaEventDisableTiming)); }
+    CUDA_TRY(ctx, ctx->laneFork.create());
     while ((int)ctx->extraLanes.size() < lanes - 1) {
         ptc_ctx::Lane lane;
-        CUDA_TRY(ctx, cudaStreamCreateWithFlags(&lane.stream, cudaStreamNonBlocking));
-        CUDA_TRY(ctx, cudaStreamCreateWithFlags(&lane.shadowStream, cudaStreamNonBlocking));
-        CUDA_TRY(ctx, cudaEventCreateWithFlags(&lane.shadeDone, cudaEventDisableTiming));
-        CUDA_TRY(ctx, cudaEventCreateWithFlags(&lane.shadowDone, cudaEventDisableTiming));
-        CUDA_TRY(ctx, cudaEventCreateWithFlags(&lane.done, cudaEventDisableTiming));
-        CUDA_TRY(ctx, cudaMalloc((void **)&lane.counters, CNT_STRIDE * sizeof(BounceCounters)));
-        ctx->extraLanes.push_back(lane);
+        CUDA_TRY(ctx, lane.stream.create());
+        CUDA_TRY(ctx, lane.shadowStream.create());
+        CUDA_TRY(ctx, lane.shadeDone.create());
+        CUDA_TRY(ctx, lane.shadowDone.create());
+        CUDA_TRY(ctx, lane.done.create());
+        CUDA_TRY(ctx, lane.counters.resize(CNT_STRIDE));
+        ctx->extraLanes.push_back(std::move(lane));
     }
     return PTC_OK;
 }
@@ -2069,17 +2080,13 @@ static VolumeBuffers laneVolumeBuffers(const VolumeBuffers &all, size_t offset)
 // VolumePathTracer, wavefront form (volume_wavefront.cuh)
 static int ensureVolumeBuffers(ptc_ctx *ctx, uint32_t capacity)
 {
-    if (capacity <= ctx->volumeBufferCapacity) { return PTC_OK; }
-    for (void *p : ctx->volumeAllocations) { cudaFree(p); }
-    ctx->volumeAllocations.clear(); ctx->volumeBufferCapacity = 0;
     VolumeBuffers &vb = ctx->volumeBuffers;
     struct { void **slot; size_t bytesPerPath; } arrays[] = {
         {(void **)&vb.probeHit, 16}, {(void **)&vb.shadowTr, 16}, {(void **)&vb.scatter, 48}, {(void **)&vb.scatterTr, 16}, {(void **)&vb.extendQueue, 4}, {(void **)&vb.scatterQueue, 4}};
-    for (auto &a : arrays) {
-        CUDA_TRY(ctx, cudaMalloc(a.slot, (size_t)capacity * a.bytesPerPath));
-        ctx->volumeAllocations.push_back(*a.slot);
+    for (int i = 0; i < 6; i++) {
+        CUDA_TRY(ctx, ctx->volumeArrays[i].reserve((size_t)capacity * arrays[i].bytesPerPath));
+        *arrays[i].slot = ctx->volumeArrays[i].get();
     }
-    ctx->volumeBufferCapacity = capacity;
     return PTC_OK;
 }
 
@@ -2115,21 +2122,21 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
         l.pb = laneBuffers(ctx->paths, offset); // by value: the current / next buffers swap after every bounce
         l.vb = laneVolumeBuffers(ctx->volumeBuffers, offset);
         offset += (size_t)wps[i].nPixels * wps[i].sppWave;
-        if (i == 0) { l.cnt = ctx->counters; l.stream = callerStream; l.shadowStream = ctx->shadowStream; l.shadeDone = ctx->shadeDone; l.shadowDone = ctx->shadowDone; }
+        if (i == 0) { l.cnt = ctx->counters.get(); l.stream = callerStream; l.shadowStream = ctx->shadowStream; l.shadeDone = ctx->shadeDone; l.shadowDone = ctx->shadowDone; }
         else {
             const ptc_ctx::Lane &x = ctx->extraLanes[(size_t)i - 1];
-            l.cnt = x.counters; l.stream = x.stream; l.shadowStream = x.shadowStream; l.shadeDone = x.shadeDone; l.shadowDone = x.shadowDone;
+            l.cnt = x.counters.get(); l.stream = x.stream; l.shadowStream = x.shadowStream; l.shadeDone = x.shadeDone; l.shadowDone = x.shadowDone;
             CUDA_TRY(ctx, cudaStreamWaitEvent(l.stream, ctx->laneFork, 0));
         }
         CUDA_TRY(ctx, cudaMemsetAsync(l.cnt, 0, CNT_STRIDE * sizeof(BounceCounters), l.stream));
         const uint32_t nPaths = wps[i].nPixels * wps[i].sppWave;
         {
             StageTimer t(ctx, l.stream, STAGE_OTHER);
-            generateKernel<<<std::min<uint32_t>((nPaths + 255) / 256, (uint32_t)ctx->gridSimple * 4), 256, 0, l.stream>>>(s, l.pb, wps[i], l.cnt);
+            generateKernel<<<gridFor(ctx, nPaths, 256), 256, 0, l.stream>>>(s, l.pb, wps[i], l.cnt);
         }
         ctx->launches++;
     }
-    unsigned long long *work = ctx->totals + 2;
+    unsigned long long *work = ctx->totals.get() + 2;
     const bool count = ctx->countTraversal;
     const int lastBounce = wps[0].lastBounce;
     // ray k leaves vertex k (k = 0: camera ray).  Ray k feeds direct() of vertex k and creates vertex k + 1, so rays
@@ -2217,10 +2224,10 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
             CUDA_TRY(ctx, cudaStreamWaitEvent(callerStream, x.done, 0));
         }
         StageTimer t(ctx, callerStream, STAGE_OTHER);
-        const uint32_t grid = std::min<uint32_t>((wps[i].nPixels + 255) / 256, (uint32_t)ctx->gridSimple * 4);
+        const uint32_t grid = gridFor(ctx, wps[i].nPixels, 256);
         if (moments) { accumulateKernel<true><<<grid, 256, 0, callerStream>>>(lanes[i].pb, wps[i], accumDevice, moments, (uint32_t)s.width, (uint32_t)s.height, plans[i]); }
         else { accumulateKernel<false><<<grid, 256, 0, callerStream>>>(lanes[i].pb, wps[i], accumDevice, nullptr, (uint32_t)s.width, (uint32_t)s.height, plans[i]); }
-        tallyKernel<<<1, 32, 0, callerStream>>>(lanes[i].cnt, ctx->totals);
+        tallyKernel<<<1, 32, 0, callerStream>>>(lanes[i].cnt, ctx->totals.get());
         ctx->launches += 2;
     }
     if (ctx->pending.size() > 4096) { collectTimings(ctx); }
@@ -2238,29 +2245,27 @@ static int renderVolume(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint3
 {
     const DScene &s = ctx->scene;
     const uint32_t nPixels = pass.moments ? pass.count : (uint32_t)s.width * (uint32_t)s.height;
-    if (ctx->volumeCapacity < nPixels * sppWave) {
-        cudaFree(ctx->volumeOut); ctx->volumeOut = nullptr; ctx->volumeCapacity = 0;
-        CUDA_TRY(ctx, cudaMalloc((void **)&ctx->volumeOut, (size_t)nPixels * sppWave * sizeof(float4)));
-        ctx->volumeCapacity = nPixels * sppWave;
-    }
-    if (!ctx->volumeCursor) { CUDA_TRY(ctx, cudaMalloc((void **)&ctx->volumeCursor, sizeof(uint32_t))); }
+    CUDA_TRY(ctx, ctx->volumeOut.reserve((size_t)nPixels * sppWave));
+    CUDA_TRY(ctx, ctx->volumeCursor.resize(1));
+    float4 *out = ctx->volumeOut.get();
+    uint32_t *cursor = ctx->volumeCursor.get();
     PathBuffers pb = ctx->paths;
-    pb.out = ctx->volumeOut;
+    pb.out = out;
     for (uint32_t done = 0; done < nSpp; done += sppWave) {
         WaveParams wp;
         wp.seed = seed; wp.firstSample = firstSample + done; wp.sppWave = std::min(sppWave, nSpp - done); wp.nPixels = nPixels; wp.groupShift = groupShiftFor(wp.sppWave);
         wp.startBounce = start; wp.lastBounce = last; wp.pixels = pass.list;
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->volumeCursor, 0, sizeof(uint32_t), stream));
+        CUDA_TRY(ctx, cudaMemsetAsync(cursor, 0, sizeof(uint32_t), stream));
         {
             StageTimer t(ctx, stream, STAGE_SHADE);
-            if (ctx->countTraversal) { volumePathKernel<true><<<ctx->gridVolume, 128, 0, stream>>>(s, ctx->volumeOut, wp, ctx->volumeCursor, ctx->totals); }
-            else { volumePathKernel<false><<<ctx->gridVolume, 128, 0, stream>>>(s, ctx->volumeOut, wp, ctx->volumeCursor, ctx->totals); }
+            if (ctx->countTraversal) { volumePathKernel<true><<<ctx->gridVolume, 128, 0, stream>>>(s, out, wp, cursor, ctx->totals.get()); }
+            else { volumePathKernel<false><<<ctx->gridVolume, 128, 0, stream>>>(s, out, wp, cursor, ctx->totals.get()); }
         }
         { const int rcUpload = runBeforeAccumulate(ctx); if (rcUpload) { return rcUpload; } }
         {
             StageTimer t(ctx, stream, STAGE_OTHER);
             const CheckpointPlan plan = planFor(checkpoints, wp.firstSample, wp.sppWave, done == 0, done + sppWave >= nSpp);
-            const uint32_t grid = std::min<uint32_t>((nPixels + 255) / 256, (uint32_t)ctx->gridSimple * 4);
+            const uint32_t grid = gridFor(ctx, nPixels, 256);
             if (pass.moments) { accumulateKernel<true><<<grid, 256, 0, stream>>>(pb, wp, accumDevice, pass.moments, (uint32_t)s.width, (uint32_t)s.height, plan); }
             else { accumulateKernel<false><<<grid, 256, 0, stream>>>(pb, wp, accumDevice, nullptr, (uint32_t)s.width, (uint32_t)s.height, plan); }
         }
@@ -2323,35 +2328,31 @@ int ptc_render(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp,
     if (!accum) { CTX_FAIL(ctx, PTC_ERR_INVALID, "null accumulation buffer"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)3 * ctx->scene.width * ctx->scene.height;
-    if (ctx->accumScratchSize < n) {
-        cudaFree(ctx->accumScratch); ctx->accumScratch = nullptr;
-        if (ctx->pinned) { cudaFreeHost(ctx->pinned); ctx->pinned = nullptr; }
-        CUDA_TRY(ctx, cudaMalloc((void **)&ctx->accumScratch, n * sizeof(float)));
-        CUDA_TRY(ctx, cudaMallocHost((void **)&ctx->pinned, n * sizeof(float)));
-        ctx->accumScratchSize = ctx->pinnedSize = n;
-    }
+    CUDA_TRY(ctx, ctx->accumScratch.reserve(n));
+    CUDA_TRY(ctx, ctx->pinned.reserve(n));
+    float *accumDevice = ctx->accumScratch.get();
     // A radianceLookup in page-locked memory (cudaHostAlloc / cudaHostRegister by the caller) is copied from and to directly; a pageable
     // one goes through the context's pinned staging buffer (two host copies of the framebuffer more per call).
     cudaPointerAttributes attr;
     const bool callerPinned = cudaPointerGetAttributes(&attr, accum) == cudaSuccess && attr.type == cudaMemoryTypeHost;
     cudaGetLastError(); // older drivers report unregistered host memory as an error
-    float *hostSide = callerPinned ? accum : ctx->pinned;
+    float *hostSide = callerPinned ? accum : ctx->pinned.get();
     // radianceLookup is accumulated, not overwritten (src/sample_integrator.cpp:61-63): upload, add, download.  The sums are first
     // needed by the accumulation at the end of the first wave, so the host copy into pinned memory and the upload are issued on a second
     // stream AFTER the wave's other launches (they are asynchronous) and run while the GPU traces the wave.
     CUDA_TRY(ctx, cudaEventRecord(ctx->evStart, ctx->stream));
-    ctx->beforeAccumulate = [ctx, accum, hostSide, n]() -> int {
+    ctx->beforeAccumulate = [ctx, accum, accumDevice, hostSide, n]() -> int {
         if (hostSide != accum) { memcpy(hostSide, accum, n * sizeof(float)); }
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->accumScratch, hostSide, n * sizeof(float), cudaMemcpyHostToDevice, ctx->copyStream));
+        CUDA_TRY(ctx, cudaMemcpyAsync(accumDevice, hostSide, n * sizeof(float), cudaMemcpyHostToDevice, ctx->copyStream));
         CUDA_TRY(ctx, cudaEventRecord(ctx->uploadDone, ctx->copyStream));
         CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->uploadDone, 0));
         return PTC_OK;
     };
-    int rc = renderInternal(ctx, seed, firstSample, nSpp, start, last, ctx->accumScratch, ctx->stream);
+    int rc = renderInternal(ctx, seed, firstSample, nSpp, start, last, accumDevice, ctx->stream);
     if (!rc) { rc = runBeforeAccumulate(ctx); } // no wave at all (zero samples): the sums pass through
     ctx->beforeAccumulate = nullptr;
     if (rc) { return rc; }
-    CUDA_TRY(ctx, cudaMemcpyAsync(hostSide, ctx->accumScratch, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(hostSide, accumDevice, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaEventRecord(ctx->evStop, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     cudaEventElapsedTime(&ctx->lastRenderMs, ctx->evStart, ctx->evStop);
@@ -2359,27 +2360,14 @@ int ptc_render(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp,
     return PTC_OK;
 }
 
+// The framebuffer at the camera's resolution; a new one starts at zero
 static int ensureFramebuffer(ptc_ctx *ctx)
 {
     const size_t n = (size_t)3 * ctx->scene.width * ctx->scene.height;
-    if (ctx->framebufferSize == n) { return PTC_OK; }
-    cudaFree(ctx->framebuffer); ctx->framebuffer = nullptr; ctx->framebufferSize = 0;
-    CUDA_TRY(ctx, cudaMalloc((void **)&ctx->framebuffer, n * sizeof(float)));
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer, 0, n * sizeof(float), ctx->stream));
-    if (!ctx->framebufferReady) { CUDA_TRY(ctx, cudaEventCreateWithFlags(&ctx->framebufferReady, cudaEventDisableTiming)); }
-    ctx->framebufferSize = n;
-    return PTC_OK;
-}
-
-// the buffer of option "framebuffer_moments", sized like the framebuffer; a new one starts at zero (like a new framebuffer)
-static int ensureFramebufferMoments(ptc_ctx *ctx)
-{
-    ptc_ctx::FramebufferMoments &m = ctx->fbMoments;
-    if (m.size == ctx->framebufferSize) { return PTC_OK; }
-    cudaFree(m.moments); m.moments = nullptr; m.size = 0;
-    CUDA_TRY(ctx, cudaMalloc((void **)&m.moments, ctx->framebufferSize * sizeof(float)));
-    CUDA_TRY(ctx, cudaMemsetAsync(m.moments, 0, ctx->framebufferSize * sizeof(float), ctx->stream));
-    m.size = ctx->framebufferSize;
+    if (ctx->framebuffer.size() == n) { return PTC_OK; }
+    CUDA_TRY(ctx, ctx->framebuffer.resize(n));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer.get(), 0, n * sizeof(float), ctx->stream));
+    CUDA_TRY(ctx, ctx->framebufferReady.create());
     return PTC_OK;
 }
 
@@ -2389,14 +2377,14 @@ int ptc_framebuffer_clear(ptc_ctx *ctx)
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer, 0, ctx->framebufferSize * sizeof(float), ctx->stream));
+    const size_t n = ctx->framebuffer.size();
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer.get(), 0, n * sizeof(float), ctx->stream));
     // with the option on the moments exist from here, so that a context that gets no samples still has (zero) moments to gather
-    if (ctx->fbMoments.on) {
-        const int mrc = ensureFramebufferMoments(ctx);
-        if (mrc) { return mrc; }
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->fbMoments.moments, 0, ctx->fbMoments.size * sizeof(float), ctx->stream));
+    if (ctx->momentsOption) {
+        CUDA_TRY(ctx, ctx->moments.resize(n));
+        CUDA_TRY(ctx, cudaMemsetAsync(ctx->moments.get(), 0, n * sizeof(float), ctx->stream));
     }
-    ctx->fbMoments.complete = ctx->fbMoments.on;
+    ctx->momentsComplete = ctx->momentsOption;
     ctx->adaptive.on = false;
     return PTC_OK;
 }
@@ -2415,45 +2403,50 @@ int ptc_framebuffer_render_checkpoints(ptc_ctx *ctx, uint64_t seed, uint32_t fir
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
-    const size_t n = ctx->framebufferSize;
+    const size_t n = ctx->framebuffer.size();
+    const bool withMoments = ctx->momentsOption;
     // the moments need room behind the sums, and a new resolution new buffers
-    if (nCounts && ((ctx->fbMoments.on && !ctx->snapshotsHoldMoments) || ctx->snapshotSize != n)) {
+    if (nCounts && ((withMoments && !ctx->snapshotsHoldMoments) || ctx->snapshotSize != n)) {
         CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); // gathers that read the old snapshots are ordered before this stream's work
-        for (float *snapshot : ctx->snapshots) { cudaFree(snapshot); }
-        ctx->snapshots.clear(); ctx->snapshotsHoldMoments = ctx->fbMoments.on; ctx->snapshotSize = n;
+        ctx->snapshots.clear(); ctx->snapshotsHoldMoments = withMoments; ctx->snapshotSize = n;
     }
     while (ctx->snapshots.size() < nCounts) {
-        float *buffer = nullptr;
-        CUDA_TRY(ctx, cudaMalloc((void **)&buffer, (ctx->snapshotsHoldMoments ? 2 : 1) * n * sizeof(float)));
-        ctx->snapshots.push_back(buffer);
+        Buffer<float> buffer;
+        CUDA_TRY(ctx, buffer.resize((ctx->snapshotsHoldMoments ? 2 : 1) * n));
+        ctx->snapshots.push_back(std::move(buffer));
     }
-    if (!ctx->fbMoments.on) { ctx->fbMoments.complete = false; }
-    else if ((rc = ensureFramebufferMoments(ctx))) { return rc; }
+    if (!withMoments) { ctx->momentsComplete = false; }
+    else if (ctx->moments.size() != n) { // a new buffer starts at zero, like a new framebuffer
+        CUDA_TRY(ctx, ctx->moments.resize(n));
+        CUDA_TRY(ctx, cudaMemsetAsync(ctx->moments.get(), 0, n * sizeof(float), ctx->stream));
+    }
     ctx->snapshotMomentsComplete.assign(ctx->snapshots.size(), false);
-    for (uint32_t i = 0; i < nCounts; i++) { ctx->snapshotMomentsComplete[i] = ctx->fbMoments.on && ctx->fbMoments.complete; }
+    float *dst[PTC_MAX_CHECKPOINTS];
+    for (uint32_t i = 0; i < nCounts; i++) { ctx->snapshotMomentsComplete[i] = withMoments && ctx->momentsComplete; dst[i] = ctx->snapshots[i].get(); }
     if (nSpp == 0) { // no samples for this context in the wave: every snapshot is the framebuffer (and its moments) as it stands
         for (uint32_t i = 0; i < nCounts; i++) {
-            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->snapshots[i], ctx->framebuffer, n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
-            if (ctx->fbMoments.on) { CUDA_TRY(ctx, cudaMemcpyAsync(ctx->snapshots[i] + n, ctx->fbMoments.moments, n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream)); }
+            CUDA_TRY(ctx, cudaMemcpyAsync(dst[i], ctx->framebuffer.get(), n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+            if (withMoments) { CUDA_TRY(ctx, cudaMemcpyAsync(dst[i] + n, ctx->moments.get(), n * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream)); }
         }
         return PTC_OK;
     }
-    Checkpoints cp; cp.counts = sampleCounts; cp.n = nCounts; cp.dst = ctx->snapshots.data();
+    Checkpoints cp; cp.counts = sampleCounts; cp.n = nCounts; cp.dst = dst;
     PassPixels pass; // every pixel, no list; with the moments option the accumulation also adds the squared samples (the sums are the same)
-    if (ctx->fbMoments.on) {
-        pass.count = (uint32_t)(ctx->framebufferSize / 3); pass.moments = ctx->fbMoments.moments;
-    }
-    return renderInternal(ctx, seed, firstSample, nSpp, start, last, ctx->framebuffer, ctx->stream, cp, pass);
+    if (withMoments) { pass.count = (uint32_t)(n / 3); pass.moments = ctx->moments.get(); }
+    return renderInternal(ctx, seed, firstSample, nSpp, start, last, ctx->framebuffer.get(), ctx->stream, cp, pass);
 }
 
 } // extern "C"
 
-// The second moments that cover every sample a context's framebuffer holds: its adaptive render's, else those of option
-// framebuffer_moments when complete; null when there are none
-static const float *framebufferMoments(const ptc_ctx *c, size_t n)
+// What a gather reads on context c for a framebuffer of n floats: the sums of checkpoint snapshot i, or of the framebuffer when i < 0,
+// or with `moments` the second moments that cover every sample those sums hold; null when there are none
+static const float *gatherInput(const ptc_ctx *c, int i, size_t n, bool moments)
 {
-    if (c->adaptive.on) { return c->adaptive.moments; }
-    return c->fbMoments.complete && c->fbMoments.size == n ? c->fbMoments.moments : nullptr;
+    if (i < 0 && !moments) { return c->framebuffer.get(); }
+    if (i < 0) { return c->momentsComplete && c->moments.size() == n ? c->moments.get() : nullptr; }
+    if ((size_t)i >= c->snapshots.size() || c->snapshotSize != n) { return nullptr; }
+    if (!moments) { return c->snapshots[i].get(); }
+    return c->snapshotsHoldMoments && c->snapshotMomentsComplete[i] ? c->snapshots[i].get() + n : nullptr;
 }
 
 // The buffers a gather over root + peers reads: set k = sources[k](root), then sources[k] of every peer as root's device reads it --
@@ -2462,12 +2455,12 @@ static const float *framebufferMoments(const ptc_ctx *c, size_t n)
 typedef std::function<const float *(ptc_ctx *)> GatherSource;
 static int gatherSets(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, const GatherSource *sources, int nSets, FramebufferSet *sets)
 {
-    const size_t n = root->framebufferSize;
+    const size_t n = root->framebuffer.size();
     for (int k = 0; k < nSets; k++) { sets[k].fb[0] = sources[k](root); sets[k].count = 1; }
     size_t staged = 0;
     for (uint32_t g = 0; g < nPeers; g++) {
         ptc_ctx *peer = peers[g];
-        bool present = peer && peer->committed && peer->framebufferSize == n;
+        bool present = peer && peer->committed && peer->framebuffer.size() == n;
         for (int k = 0; present && k < nSets; k++) { present = sources[k](peer) != nullptr; }
         if (!present) { CTX_FAIL(root, PTC_ERR_STATE, "peer %u has no framebuffer (or snapshot, or moments) of the same size", g); }
         // order the gather after the peer's pending renders
@@ -2486,13 +2479,11 @@ static int gatherSets(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, con
         for (int k = 0; k < nSets; k++) {
             if (direct) { sets[k].fb[sets[k].count++] = sources[k](peer); continue; }
             // no peer mapping: stage the peer's buffer into local memory first
-            if (root->gatherStageSize < (size_t)nSets * nPeers * n) {
-                CUDA_TRY(root, cudaStreamSynchronize(root->stream));
-                cudaFree(root->gatherStage); root->gatherStage = nullptr; root->gatherStageSize = 0;
-                CUDA_TRY(root, cudaMalloc((void **)&root->gatherStage, (size_t)nSets * nPeers * n * sizeof(float)));
-                root->gatherStageSize = (size_t)nSets * nPeers * n;
+            if (root->gatherStage.size() < (size_t)nSets * nPeers * n) {
+                CUDA_TRY(root, cudaStreamSynchronize(root->stream)); // earlier gathers may still read the old buffer
+                CUDA_TRY(root, root->gatherStage.reserve((size_t)nSets * nPeers * n));
             }
-            float *slot = root->gatherStage + staged * n; staged++;
+            float *slot = root->gatherStage.get() + staged * n; staged++;
             CUDA_TRY(root, cudaMemcpyPeerAsync(slot, root->device, sources[k](peer), peer->device, n * sizeof(float), root->stream));
             sets[k].fb[sets[k].count++] = slot;
         }
@@ -2505,17 +2496,12 @@ static int takeGatherSlot(ptc_ctx *root, uint32_t *ticketOut)
 {
     uint32_t ticket = 0;
     while (ticket < root->gathers.size() && root->gathers[ticket].busy) { ticket++; }
-    if (ticket == root->gathers.size()) { root->gathers.push_back(ptc_ctx::Gather()); }
+    if (ticket == root->gathers.size()) { root->gathers.emplace_back(); }
     ptc_ctx::Gather &slot = root->gathers[ticket];
-    if (slot.size != root->framebufferSize) { // first use, or the camera's resolution changed
-        cudaFree(slot.device); slot.device = nullptr;
-        if (slot.pinned) { cudaFreeHost(slot.pinned); slot.pinned = nullptr; }
-        slot.size = 0;
-        CUDA_TRY(root, cudaMalloc((void **)&slot.device, root->framebufferSize * sizeof(float)));
-        CUDA_TRY(root, cudaMallocHost((void **)&slot.pinned, root->framebufferSize * sizeof(float)));
-        slot.size = root->framebufferSize;
-    }
-    if (!slot.done) { CUDA_TRY(root, cudaEventCreateWithFlags(&slot.done, cudaEventDisableTiming)); }
+    // sized on first use, and again when the camera's resolution changed
+    CUDA_TRY(root, slot.device.resize(root->framebuffer.size()));
+    CUDA_TRY(root, slot.pinned.resize(root->framebuffer.size()));
+    CUDA_TRY(root, slot.done.create());
     *ticketOut = ticket;
     return PTC_OK;
 }
@@ -2526,11 +2512,11 @@ static int finishGather(ptc_ctx *root, ptc_ctx *const *peers, uint32_t nPeers, u
 {
     CUDA_TRY(root, cudaGetLastError());
     // renders that follow on any of the contexts must not overwrite what the kernels read
-    if (!root->gatherRead) { CUDA_TRY(root, cudaEventCreateWithFlags(&root->gatherRead, cudaEventDisableTiming)); }
+    CUDA_TRY(root, root->gatherRead.create());
     CUDA_TRY(root, cudaEventRecord(root->gatherRead, root->stream));
     for (uint32_t g = 0; g < nPeers; g++) { CUDA_TRY(root, cudaStreamWaitEvent(peers[g]->stream, root->gatherRead, 0)); }
     ptc_ctx::Gather &slot = root->gathers[ticket];
-    CUDA_TRY(root, cudaMemcpyAsync(slot.pinned, slot.device, root->framebufferSize * sizeof(float), cudaMemcpyDeviceToHost, root->stream));
+    CUDA_TRY(root, cudaMemcpyAsync(slot.pinned.get(), slot.device.get(), slot.device.size() * sizeof(float), cudaMemcpyDeviceToHost, root->stream));
     CUDA_TRY(root, cudaEventRecord(slot.done, root->stream));
     slot.busy = true;
     return PTC_OK;
@@ -2545,14 +2531,12 @@ int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t 
     CUDA_TRY(root, cudaSetDevice(root->device));
     int rc = ensureFramebuffer(root);
     if (rc) { return rc; }
-    const size_t n = root->framebufferSize;
-    // PTC_GATHER_MOMENTS: the second moments of an adaptive render, else those of the framebuffer renders
-    const GatherSource source = [&](ptc_ctx *c) -> const float * {
-        if (snapshot == PTC_GATHER_MOMENTS) { return framebufferMoments(c, n); }
-        return snapshot < 0 ? c->framebuffer : (size_t)snapshot < c->snapshots.size() && c->snapshotSize == n ? c->snapshots[snapshot] : nullptr;
-    };
+    const size_t n = root->framebuffer.size();
+    // PTC_GATHER_MOMENTS: the second moments of an adaptive render or of the framebuffer renders
+    const bool moments = snapshot == PTC_GATHER_MOMENTS;
+    const GatherSource source = [&](ptc_ctx *c) { return gatherInput(c, snapshot, n, moments); };
     if (!source(root)) {
-        if (snapshot == PTC_GATHER_MOMENTS) {
+        if (moments) {
             CTX_FAIL(root, PTC_ERR_STATE, "no second moments of every sample on this context (option framebuffer_moments on since the last clear, or an adaptive render)");
         }
         CTX_FAIL(root, PTC_ERR_STATE, "no snapshot %d was rendered", snapshot);
@@ -2561,7 +2545,7 @@ int ptc_framebuffer_gather_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t 
     if ((rc = gatherSets(root, peers, nPeers, &source, 1, &set))) { return rc; }
     uint32_t ticket = 0;
     if ((rc = takeGatherSlot(root, &ticket))) { return rc; }
-    gatherResolveKernel<<<std::min<uint32_t>((uint32_t)((n / 4 + 255) / 256) + 1, (uint32_t)root->gridSimple * 4), 256, 0, root->stream>>>(set, root->gathers[ticket].device, (uint32_t)n, divisor);
+    gatherResolveKernel<<<std::min<uint32_t>((uint32_t)((n / 4 + 255) / 256) + 1, (uint32_t)root->gridSimple * 4), 256, 0, root->stream>>>(set, root->gathers[ticket].device.get(), (uint32_t)n, divisor);
     root->launches++;
     if ((rc = finishGather(root, peers, nPeers, ticket))) { return rc; }
     *ticketOut = ticket;
@@ -2575,7 +2559,7 @@ int ptc_framebuffer_gather_end(ptc_ctx *root, uint32_t ticket, float *out)
     CUDA_TRY(root, cudaSetDevice(root->device));
     ptc_ctx::Gather &slot = root->gathers[ticket];
     CUDA_TRY(root, cudaEventSynchronize(slot.done));
-    memcpy(out, slot.pinned, root->framebufferSize * sizeof(float));
+    memcpy(out, slot.pinned.get(), root->framebuffer.size() * sizeof(float));
     slot.busy = false;
     return PTC_OK;
 }
@@ -2599,25 +2583,22 @@ int ptc_adaptive_begin(ptc_ctx *ctx, const ptc_adaptive_desc *desc)
     if (rc) { return rc; }
     ptc_ctx::Adaptive &a = ctx->adaptive;
     const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
-    if (a.pixels != pixels) {
-        cudaFree(a.moments); cudaFree(a.counts); cudaFree(a.list); cudaFree(a.next); cudaFree(a.scratch);
-        a.moments = nullptr; a.counts = a.list = a.next = nullptr; a.scratch = nullptr; a.pixels = 0;
-        CUDA_TRY(ctx, cudaMalloc((void **)&a.moments, 3 * pixels * sizeof(float)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&a.counts, pixels * sizeof(uint32_t)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&a.list, pixels * sizeof(uint32_t)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&a.next, pixels * sizeof(uint32_t)));
-        if (!a.selected) { CUDA_TRY(ctx, cudaMalloc((void **)&a.selected, sizeof(uint32_t))); }
-        if (!a.selectedHost) { CUDA_TRY(ctx, cudaMallocHost((void **)&a.selectedHost, sizeof(uint32_t))); }
-        a.scratchBytes = 0;
-        CUDA_TRY(ctx, cub::DeviceSelect::If(nullptr, a.scratchBytes, a.next, a.list, a.selected, (int)pixels, StillActive(), ctx->stream));
-        CUDA_TRY(ctx, cudaMalloc(&a.scratch, std::max<size_t>(a.scratchBytes, 1)));
-        a.pixels = pixels;
-    }
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer, 0, ctx->framebufferSize * sizeof(float), ctx->stream));
-    CUDA_TRY(ctx, cudaMemsetAsync(a.moments, 0, 3 * pixels * sizeof(float), ctx->stream));
-    CUDA_TRY(ctx, cudaMemsetAsync(a.counts, 0, pixels * sizeof(uint32_t), ctx->stream));
+    a.pixels = 0; // until every buffer is sized for `pixels`
+    CUDA_TRY(ctx, ctx->moments.resize(3 * pixels));
+    CUDA_TRY(ctx, a.counts.resize(pixels));
+    CUDA_TRY(ctx, a.list.resize(pixels));
+    CUDA_TRY(ctx, a.next.resize(pixels));
+    CUDA_TRY(ctx, a.selected.resize(1));
+    CUDA_TRY(ctx, a.selectedHost.resize(1));
+    size_t scratchBytes = 0;
+    CUDA_TRY(ctx, cub::DeviceSelect::If(nullptr, scratchBytes, a.next.get(), a.list.get(), a.selected.get(), (int)pixels, StillActive(), ctx->stream));
+    CUDA_TRY(ctx, a.scratch.resize(std::max<size_t>(scratchBytes, 1)));
+    a.pixels = pixels;
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer.get(), 0, ctx->framebuffer.size() * sizeof(float), ctx->stream));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->moments.get(), 0, 3 * pixels * sizeof(float), ctx->stream));
+    CUDA_TRY(ctx, cudaMemsetAsync(a.counts.get(), 0, pixels * sizeof(uint32_t), ctx->stream));
     a.desc = *desc; a.n = 0; a.active = (uint32_t)pixels; a.on = true;
-    ctx->fbMoments.complete = false; // the framebuffer now holds what the adaptive moments cover
+    ctx->momentsComplete = true; // the passes add the squares of every sample they add to the framebuffer
     return PTC_OK;
 }
 
@@ -2629,28 +2610,28 @@ int ptc_adaptive_pass(ptc_ctx *ctx, uint64_t seed, int start, int last, uint32_t
     NEED_COMMIT(ctx);
     ptc_ctx::Adaptive &a = ctx->adaptive;
     if (!a.on) { CTX_FAIL(ctx, PTC_ERR_STATE, "no adaptive render on this context: ptc_adaptive_begin first"); }
-    if (a.pixels != (size_t)ctx->scene.width * ctx->scene.height || ctx->framebufferSize != 3 * a.pixels) {
+    if (a.pixels != (size_t)ctx->scene.width * ctx->scene.height || ctx->framebuffer.size() != 3 * a.pixels) {
         CTX_FAIL(ctx, PTC_ERR_STATE, "the resolution changed during the adaptive render");
     }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     if (a.active) {
         const uint32_t k = a.n == 0 ? a.desc.min_spp : std::min(a.desc.step_spp, a.desc.max_spp - a.n);
-        PassPixels pass; pass.list = a.n == 0 ? nullptr : a.list; pass.count = a.active; pass.moments = a.moments;
-        const int rc = renderInternal(ctx, seed, a.n, k, start, last, ctx->framebuffer, ctx->stream, Checkpoints(), pass);
+        PassPixels pass; pass.list = a.n == 0 ? nullptr : a.list.get(); pass.count = a.active; pass.moments = ctx->moments.get();
+        const int rc = renderInternal(ctx, seed, a.n, k, start, last, ctx->framebuffer.get(), ctx->stream, Checkpoints(), pass);
         if (rc) { return rc; }
         const uint32_t n = a.n + k;
         WaveParams wp; memset(&wp, 0, sizeof(wp));
         wp.nPixels = a.active; wp.pixels = pass.list;
         const double tau = (double)a.desc.threshold;
-        adaptiveTestKernel<<<std::min<uint32_t>((a.active + 255) / 256, (uint32_t)ctx->gridSimple * 4), 256, 0, ctx->stream>>>(
-            wp, ctx->framebuffer, a.moments, a.counts, a.next, (uint32_t)ctx->scene.width, (uint32_t)ctx->scene.height, tau * tau, n, a.desc.max_spp);
+        adaptiveTestKernel<<<gridFor(ctx, a.active, 256), 256, 0, ctx->stream>>>(
+            wp, ctx->framebuffer.get(), ctx->moments.get(), a.counts.get(), a.next.get(), (uint32_t)ctx->scene.width, (uint32_t)ctx->scene.height, tau * tau, n, a.desc.max_spp);
         CUDA_TRY(ctx, cudaGetLastError());
-        size_t bytes = a.scratchBytes;
-        CUDA_TRY(ctx, cub::DeviceSelect::If(a.scratch, bytes, a.next, a.list, a.selected, (int)a.active, StillActive(), ctx->stream));
-        CUDA_TRY(ctx, cudaMemcpyAsync(a.selectedHost, a.selected, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        size_t bytes = a.scratch.size();
+        CUDA_TRY(ctx, cub::DeviceSelect::If(a.scratch.get(), bytes, a.next.get(), a.list.get(), a.selected.get(), (int)a.active, StillActive(), ctx->stream));
+        CUDA_TRY(ctx, cudaMemcpyAsync(a.selectedHost.get(), a.selected.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
         CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
         ctx->launches += 2;
-        a.n = n; a.active = *a.selectedHost;
+        a.n = n; a.active = *a.selectedHost.get();
     }
     if (activeOut) { *activeOut = a.active; }
     if (sppOut) { *sppOut = a.n; }
@@ -2663,8 +2644,8 @@ int ptc_adaptive_state(ptc_ctx *ctx, uint32_t *sppPerPixel, float *secondMoment)
     const ptc_ctx::Adaptive &a = ctx->adaptive;
     if (!a.on) { CTX_FAIL(ctx, PTC_ERR_STATE, "no adaptive render on this context: ptc_adaptive_begin first"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    if (sppPerPixel) { CUDA_TRY(ctx, cudaMemcpyAsync(sppPerPixel, a.counts, a.pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream)); }
-    if (secondMoment) { CUDA_TRY(ctx, cudaMemcpyAsync(secondMoment, a.moments, 3 * a.pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream)); }
+    if (sppPerPixel) { CUDA_TRY(ctx, cudaMemcpyAsync(sppPerPixel, a.counts.get(), a.pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream)); }
+    if (secondMoment) { CUDA_TRY(ctx, cudaMemcpyAsync(secondMoment, ctx->moments.get(), 3 * a.pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream)); }
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return PTC_OK;
 }
@@ -2674,7 +2655,7 @@ int ptc_resolve_device(ptc_ctx *ctx, const float *accum, float *out, uint32_t sp
     NEED_COMMIT(ctx);
     if (!accum || !out || !spp) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bad resolve arguments"); }
     const uint32_t n = 3u * (uint32_t)ctx->scene.width * (uint32_t)ctx->scene.height;
-    resolveKernel<<<std::min<uint32_t>((n + 255) / 256, (uint32_t)ctx->gridSimple * 4), 256, 0, (cudaStream_t)stream>>>(accum, out, n, spp);
+    resolveKernel<<<gridFor(ctx, n, 256), 256, 0, (cudaStream_t)stream>>>(accum, out, n, spp);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
     return PTC_OK;
@@ -2686,34 +2667,21 @@ int ptc_resolve_device(ptc_ctx *ctx, const float *accum, float *out, uint32_t sp
 template <typename In, typename Out, typename Launch>
 static int roundTrip(ptc_ctx *ctx, const In *in, size_t nIn, Out *out, size_t nOut, Launch launch)
 {
-    In *dIn = nullptr; Out *dOut = nullptr;
+    Buffer<In> dIn; Buffer<Out> dOut;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, cudaMalloc((void **)&dIn, std::max<size_t>(nIn, 1) * sizeof(In)));
-    if (cudaMalloc((void **)&dOut, std::max<size_t>(nOut, 1) * sizeof(Out)) != cudaSuccess) { cudaFree(dIn); CTX_FAIL(ctx, PTC_ERR_NOMEM, "cudaMalloc failed"); }
-    cudaMemcpyAsync(dIn, in, nIn * sizeof(In), cudaMemcpyHostToDevice, ctx->stream);
-    launch(dIn, dOut);
+    CUDA_TRY(ctx, dIn.resize(std::max<size_t>(nIn, 1)));
+    if (dOut.resize(std::max<size_t>(nOut, 1)) != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_NOMEM, "cudaMalloc failed"); }
+    cudaMemcpyAsync(dIn.get(), in, nIn * sizeof(In), cudaMemcpyHostToDevice, ctx->stream);
+    launch(dIn.get(), dOut.get());
     ctx->launches++;
-    cudaMemcpyAsync(out, dOut, nOut * sizeof(Out), cudaMemcpyDeviceToHost, ctx->stream);
+    cudaMemcpyAsync(out, dOut.get(), nOut * sizeof(Out), cudaMemcpyDeviceToHost, ctx->stream);
     const cudaError_t e = cudaStreamSynchronize(ctx->stream);
     const cudaError_t e2 = cudaGetLastError();
-    cudaFree(dIn); cudaFree(dOut);
     if (e != cudaSuccess || e2 != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "kernel failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2)); }
     return PTC_OK;
 }
-static inline uint32_t gridFor(ptc_ctx *ctx, uint32_t n) { return std::max(1u, std::min<uint32_t>((n + 127) / 128, (uint32_t)ctx->gridSimple * 4)); }
 
 // ------------------------------------------------------------------------------------------------ denoising (denoise.cuh)
-// the device guide sums (albedo 3, normal 3, depth 1, hits 1 x 4 B per pixel) of ptc_render_aovs and ptc_framebuffer_guides
-static int ensureAovs(ptc_ctx *ctx, size_t pixels)
-{
-    ptc_ctx::Aovs &a = ctx->aovs;
-    if (a.pixels == pixels) { return PTC_OK; }
-    cudaFree(a.buffer); a.buffer = nullptr; a.pixels = 0;
-    CUDA_TRY(ctx, cudaMalloc((void **)&a.buffer, 8 * pixels * sizeof(float)));
-    a.pixels = pixels;
-    return PTC_OK;
-}
-
 static int checkDenoiseDesc(ptc_ctx *ctx, const ptc_denoise_desc *desc)
 {
     auto positive = [](float v) { return v > 0.f && std::isfinite(v); };
@@ -2734,21 +2702,10 @@ static int denoiseAtrous(ptc_ctx *ctx, const ptc_denoise_desc *desc, const float
     dp.sigmaL = desc->sigma_l; dp.sigmaN = desc->sigma_n; dp.sigmaZ = desc->sigma_z; dp.sigmaA = desc->sigma_a; dp.eps = desc->eps;
     const dim3 block(32, 8), grid((unsigned)(width + 31) / 32, (unsigned)(height + 7) / 8);
     for (uint32_t i = 0; i < desc->iterations; i++) {
-        denoiseAtrousKernel<<<grid, block, 0, ctx->stream>>>(d.colour[i & 1], d.colour[(i + 1) & 1], guide, width, height, 1 << i, dp);
+        denoiseAtrousKernel<<<grid, block, 0, ctx->stream>>>(d.colour[i & 1].get(), d.colour[(i + 1) & 1].get(), guide, width, height, 1 << i, dp);
         ctx->launches++;
         CUDA_TRY(ctx, cudaGetLastError());
     }
-    return PTC_OK;
-}
-
-static int ensureDenoiseColour(ptc_ctx *ctx, size_t pixels)
-{
-    ptc_ctx::Denoise &d = ctx->denoise;
-    if (d.colourPixels == pixels) { return PTC_OK; }
-    cudaFree(d.colour[0]); cudaFree(d.colour[1]); d.colour[0] = d.colour[1] = nullptr; d.colourPixels = 0;
-    CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[0], pixels * sizeof(float4)));
-    CUDA_TRY(ctx, cudaMalloc((void **)&d.colour[1], pixels * sizeof(float4)));
-    d.colourPixels = pixels;
     return PTC_OK;
 }
 
@@ -2764,12 +2721,11 @@ int ptc_intersect_instanced(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_h
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !hits || !instIds)) { return PTC_ERR_INVALID; }
-    uint2 *dInst = nullptr;
+    Buffer<uint2> dInst;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, cudaMalloc((void **)&dInst, std::max<size_t>(n, 1) * sizeof(uint2)));
-    const int rc = roundTrip(ctx, rays, n, hits, n, [&](ptc_ray *d, ptc_hit *o) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o, dInst); });
-    if (!rc) { cudaMemcpy(instIds, dInst, (size_t)n * sizeof(uint2), cudaMemcpyDeviceToHost); }
-    cudaFree(dInst);
+    CUDA_TRY(ctx, dInst.resize(std::max<size_t>(n, 1)));
+    const int rc = roundTrip(ctx, rays, n, hits, n, [&](ptc_ray *d, ptc_hit *o) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o, dInst.get()); });
+    if (!rc) { cudaMemcpy(instIds, dInst.get(), (size_t)n * sizeof(uint2), cudaMemcpyDeviceToHost); }
     return rc;
 }
 int ptc_intersect_full(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_isect *out)
@@ -2782,42 +2738,37 @@ int ptc_occluded(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t 
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !maxT || !occluded)) { return PTC_ERR_INVALID; }
-    float *dT = nullptr;
-    CUDA_TRY(ctx, cudaMalloc((void **)&dT, std::max<size_t>(n, 1) * sizeof(float)));
-    cudaMemcpyAsync(dT, maxT, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, rays, n, occluded, n, [&](ptc_ray *d, uint8_t *o) { occludedKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dT, n, o); });
-    cudaFree(dT);
-    return rc;
+    Buffer<float> dT;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    CUDA_TRY(ctx, dT.resize(std::max<size_t>(n, 1)));
+    cudaMemcpyAsync(dT.get(), maxT, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    return roundTrip(ctx, rays, n, occluded, n, [&](ptc_ray *d, uint8_t *o) { occludedKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dT.get(), n, o); });
 }
 // volumetric queries: the per-ray event lists come back through device scratch buffers
 static int volumetricQuery(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t n, uint8_t *occluded, ptc_isect *isects, uint32_t *nEvents,
                            float *eventT, uint32_t *eventMedium)
 {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    ptc_ray *dRays = nullptr; float *dMaxT = nullptr, *dT = nullptr; uint8_t *dOcc = nullptr; ptc_isect *dIs = nullptr; uint32_t *dN = nullptr, *dM = nullptr;
+    Buffer<ptc_ray> dRays; Buffer<float> dMaxT, dT; Buffer<uint8_t> dOcc; Buffer<ptc_isect> dIs; Buffer<uint32_t> dN, dM;
     const size_t m = std::max<size_t>(n, 1);
-    int rc = PTC_OK;
-    if (cudaMalloc((void **)&dRays, m * sizeof(ptc_ray)) != cudaSuccess || cudaMalloc((void **)&dMaxT, m * sizeof(float)) != cudaSuccess ||
-        cudaMalloc((void **)&dOcc, m) != cudaSuccess || cudaMalloc((void **)&dIs, m * sizeof(ptc_isect)) != cudaSuccess ||
-        cudaMalloc((void **)&dN, m * sizeof(uint32_t)) != cudaSuccess || cudaMalloc((void **)&dT, m * PTC_MAX_EVENTS * sizeof(float)) != cudaSuccess ||
-        cudaMalloc((void **)&dM, m * PTC_MAX_EVENTS * sizeof(uint32_t)) != cudaSuccess) { rc = PTC_ERR_NOMEM; ctx->error = "cudaMalloc failed"; }
-    if (!rc) {
-        cudaMemcpyAsync(dRays, rays, n * sizeof(ptc_ray), cudaMemcpyHostToDevice, ctx->stream);
-        if (maxT) { cudaMemcpyAsync(dMaxT, maxT, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream); }
-        if (occluded) { occludedVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, dRays, dMaxT, n, dOcc, dN, dT, dM); }
-        else { intersectVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, dRays, n, dIs, dN, dT, dM); }
-        ctx->launches++;
-        if (occluded) { cudaMemcpyAsync(occluded, dOcc, n, cudaMemcpyDeviceToHost, ctx->stream); }
-        if (isects) { cudaMemcpyAsync(isects, dIs, n * sizeof(ptc_isect), cudaMemcpyDeviceToHost, ctx->stream); }
-        if (nEvents) { cudaMemcpyAsync(nEvents, dN, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream); }
-        if (eventT) { cudaMemcpyAsync(eventT, dT, (size_t)n * PTC_MAX_EVENTS * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream); }
-        if (eventMedium) { cudaMemcpyAsync(eventMedium, dM, (size_t)n * PTC_MAX_EVENTS * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream); }
-        const cudaError_t e = cudaStreamSynchronize(ctx->stream);
-        const cudaError_t e2 = cudaGetLastError();
-        if (e != cudaSuccess || e2 != cudaSuccess) { rc = PTC_ERR_CUDA; ctx->error = std::string("kernel failed: ") + cudaGetErrorString(e != cudaSuccess ? e : e2); }
+    if (dRays.resize(m) != cudaSuccess || dMaxT.resize(m) != cudaSuccess || dOcc.resize(m) != cudaSuccess || dIs.resize(m) != cudaSuccess ||
+        dN.resize(m) != cudaSuccess || dT.resize(m * PTC_MAX_EVENTS) != cudaSuccess || dM.resize(m * PTC_MAX_EVENTS) != cudaSuccess) {
+        CTX_FAIL(ctx, PTC_ERR_NOMEM, "cudaMalloc failed");
     }
-    cudaFree(dRays); cudaFree(dMaxT); cudaFree(dT); cudaFree(dOcc); cudaFree(dIs); cudaFree(dN); cudaFree(dM);
-    return rc;
+    cudaMemcpyAsync(dRays.get(), rays, n * sizeof(ptc_ray), cudaMemcpyHostToDevice, ctx->stream);
+    if (maxT) { cudaMemcpyAsync(dMaxT.get(), maxT, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream); }
+    if (occluded) { occludedVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, dRays.get(), dMaxT.get(), n, dOcc.get(), dN.get(), dT.get(), dM.get()); }
+    else { intersectVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, dRays.get(), n, dIs.get(), dN.get(), dT.get(), dM.get()); }
+    ctx->launches++;
+    if (occluded) { cudaMemcpyAsync(occluded, dOcc.get(), n, cudaMemcpyDeviceToHost, ctx->stream); }
+    if (isects) { cudaMemcpyAsync(isects, dIs.get(), n * sizeof(ptc_isect), cudaMemcpyDeviceToHost, ctx->stream); }
+    if (nEvents) { cudaMemcpyAsync(nEvents, dN.get(), n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream); }
+    if (eventT) { cudaMemcpyAsync(eventT, dT.get(), (size_t)n * PTC_MAX_EVENTS * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream); }
+    if (eventMedium) { cudaMemcpyAsync(eventMedium, dM.get(), (size_t)n * PTC_MAX_EVENTS * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream); }
+    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+    const cudaError_t e2 = cudaGetLastError();
+    if (e != cudaSuccess || e2 != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "kernel failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2)); }
+    return PTC_OK;
 }
 int ptc_occluded_volumetric(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t n, uint8_t *occluded, uint32_t *nEvents, float *eventT, uint32_t *eventMedium)
 {
@@ -2859,9 +2810,8 @@ int ptc_render_aovs(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t 
     if (!albedo || !normal || !depth || !hits) { CTX_FAIL(ctx, PTC_ERR_INVALID, "null guide buffer"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
-    const int rc = ensureAovs(ctx, pixels);
-    if (rc) { return rc; }
-    float *d = ctx->aovs.buffer;
+    CUDA_TRY(ctx, ctx->aovs.resize(8 * pixels));
+    float *d = ctx->aovs.get();
     float *dAlbedo = d, *dNormal = d + 3 * pixels, *dDepth = d + 6 * pixels;
     uint32_t *dHits = (uint32_t *)(d + 7 * pixels);
     cudaError_t e = cudaSuccess;
@@ -2891,22 +2841,16 @@ int ptc_framebuffer_guides(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, ui
     if (!nSpp) { CTX_FAIL(ctx, PTC_ERR_INVALID, "n_spp must be > 0: the guide records are means over the samples"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
-    int rc = ensureAovs(ctx, pixels);
-    if (rc) { return rc; }
+    CUDA_TRY(ctx, ctx->aovs.resize(8 * pixels));
     ptc_ctx::Guides &g = ctx->guides;
     g.aovSpp = 0; // no guides until this call has enqueued them
-    if (g.pixels != pixels) {
-        cudaFree(g.records); g.records = nullptr; g.pixels = 0;
-        CUDA_TRY(ctx, cudaMalloc((void **)&g.records, 2 * pixels * sizeof(float4)));
-        g.pixels = pixels;
-    }
-    float *d = ctx->aovs.buffer;
+    CUDA_TRY(ctx, g.records.resize(2 * pixels));
+    float *d = ctx->aovs.get();
     float *dAlbedo = d, *dNormal = d + 3 * pixels, *dDepth = d + 6 * pixels;
     uint32_t *dHits = (uint32_t *)(d + 7 * pixels);
     CUDA_TRY(ctx, cudaMemsetAsync(d, 0, 8 * pixels * sizeof(float), ctx->stream));
     aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene, seed, firstSample, nSpp, dAlbedo, dNormal, dDepth, dHits);
-    denoiseGuideKernel<<<std::min<uint32_t>((uint32_t)((pixels + 255) / 256), (uint32_t)ctx->gridSimple * 4), 256, 0, ctx->stream>>>(
-        dAlbedo, dNormal, dDepth, dHits, nSpp, (uint32_t)pixels, g.records);
+    denoiseGuideKernel<<<gridFor(ctx, (uint32_t)pixels, 256), 256, 0, ctx->stream>>>(dAlbedo, dNormal, dDepth, dHits, nSpp, (uint32_t)pixels, g.records.get());
     ctx->launches += 2;
     CUDA_TRY(ctx, cudaGetLastError());
     const struct { void *dst; const void *src; size_t bytes; } fetches[] = {
@@ -2938,15 +2882,12 @@ int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_in
     } else if (in->spp < 2) { CTX_FAIL(ctx, PTC_ERR_INVALID, "spp must be >= 2: the variance needs 2 samples"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     ptc_ctx::Denoise &d = ctx->denoise;
-    if (d.pixels != pixels) {
-        cudaFree(d.inputs); cudaFree(d.guide); d.inputs = nullptr; d.guide = nullptr; d.pixels = 0;
-        CUDA_TRY(ctx, cudaMalloc((void **)&d.inputs, 15 * pixels * sizeof(float)));
-        CUDA_TRY(ctx, cudaMalloc((void **)&d.guide, 2 * pixels * sizeof(float4)));
-        d.pixels = pixels;
-    }
-    if ((rc = ensureDenoiseColour(ctx, pixels))) { return rc; }
+    CUDA_TRY(ctx, d.inputs.resize(15 * pixels));
+    CUDA_TRY(ctx, d.guide.resize(2 * pixels));
+    CUDA_TRY(ctx, d.colour[0].resize(pixels));
+    CUDA_TRY(ctx, d.colour[1].resize(pixels));
     DenoiseInputs di;
-    float *f = d.inputs;
+    float *f = d.inputs.get();
     di.sums = f; di.moments = f + 3 * pixels; di.albedo = f + 6 * pixels; di.normal = f + 9 * pixels; di.depth = f + 12 * pixels;
     di.hits = (const uint32_t *)(f + 13 * pixels); di.counts = in->counts ? (const uint32_t *)(f + 14 * pixels) : nullptr;
     di.spp = in->spp; di.aovSpp = in->aov_spp; di.nPixels = (uint32_t)pixels;
@@ -2955,12 +2896,12 @@ int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_in
         {f + 9 * pixels, in->normal_xyz, 3 * pixels * 4}, {f + 12 * pixels, in->depth, pixels * 4}, {f + 13 * pixels, in->hits, pixels * 4},
         {f + 14 * pixels, in->counts, in->counts ? pixels * 4 : 0}};
     for (const auto &u : uploads) { if (u.bytes) { CUDA_TRY(ctx, cudaMemcpyAsync(u.dst, u.src, u.bytes, cudaMemcpyHostToDevice, ctx->stream)); } }
-    denoisePrepareKernel<<<std::min<uint32_t>((uint32_t)((pixels + 255) / 256), (uint32_t)ctx->gridSimple * 4), 256, 0, ctx->stream>>>(di, d.colour[0], d.guide);
+    denoisePrepareKernel<<<gridFor(ctx, (uint32_t)pixels, 256), 256, 0, ctx->stream>>>(di, d.colour[0].get(), d.guide.get());
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
-    if ((rc = denoiseAtrous(ctx, desc, d.guide))) { return rc; }
+    if ((rc = denoiseAtrous(ctx, desc, d.guide.get()))) { return rc; }
     std::vector<float4> result(pixels);
-    CUDA_TRY(ctx, cudaMemcpyAsync(result.data(), d.colour[desc->iterations & 1], pixels * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(result.data(), d.colour[desc->iterations & 1].get(), pixels * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     for (size_t p = 0; p < pixels; p++) { out[3 * p] = result[p].x; out[3 * p + 1] = result[p].y; out[3 * p + 2] = result[p].z; }
     return PTC_OK;
@@ -2979,35 +2920,28 @@ int ptc_framebuffer_denoise_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t
     if (!a.on && spp < 2) { CTX_FAIL(root, PTC_ERR_INVALID, "spp must be >= 2: the variance needs 2 samples"); }
     CUDA_TRY(root, cudaSetDevice(root->device));
     if ((rc = ensureFramebuffer(root))) { return rc; }
-    const size_t n = root->framebufferSize, pixels = n / 3;
-    if (!root->guides.aovSpp || root->guides.width != root->scene.width || root->guides.height != root->scene.height || pixels != root->guides.pixels) { CTX_FAIL(root, PTC_ERR_STATE, "no guides of this resolution: ptc_framebuffer_guides first"); }
+    const size_t n = root->framebuffer.size(), pixels = n / 3;
+    if (!root->guides.aovSpp || root->guides.width != root->scene.width || root->guides.height != root->scene.height || 2 * pixels != root->guides.records.size()) { CTX_FAIL(root, PTC_ERR_STATE, "no guides of this resolution: ptc_framebuffer_guides first"); }
     if (a.on && a.n == 0) { CTX_FAIL(root, PTC_ERR_STATE, "the adaptive render has no pass yet"); }
     if (a.on && snapshot >= 0) { CTX_FAIL(root, PTC_ERR_STATE, "an adaptive render keeps no checkpoint snapshots"); }
-    const GatherSource sources[2] = {
-        [&](ptc_ctx *c) -> const float * {
-            return snapshot < 0 ? c->framebuffer : (size_t)snapshot < c->snapshots.size() && c->snapshotSize == n ? c->snapshots[snapshot] : nullptr;
-        },
-        [&](ptc_ctx *c) -> const float * {
-            if (snapshot < 0) { return framebufferMoments(c, n); }
-            const bool held = c->snapshotsHoldMoments && c->snapshotSize == n && (size_t)snapshot < c->snapshots.size() && c->snapshotMomentsComplete[snapshot];
-            return held ? c->snapshots[snapshot] + n : nullptr;
-        }};
+    const GatherSource sources[2] = {[&](ptc_ctx *c) { return gatherInput(c, snapshot, n, false); }, [&](ptc_ctx *c) { return gatherInput(c, snapshot, n, true); }};
     if (!sources[0](root)) { CTX_FAIL(root, PTC_ERR_STATE, "no snapshot %d was rendered", snapshot); }
     if (!sources[1](root)) {
         CTX_FAIL(root, PTC_ERR_STATE, "no second moments of every sample of this image (option framebuffer_moments on since the last clear, or an adaptive render)");
     }
     FramebufferSet sets[2];
     if ((rc = gatherSets(root, peers, nPeers, sources, 2, sets))) { return rc; }
-    if ((rc = ensureDenoiseColour(root, pixels))) { return rc; }
+    ptc_ctx::Denoise &d = root->denoise;
+    CUDA_TRY(root, d.colour[0].resize(pixels));
+    CUDA_TRY(root, d.colour[1].resize(pixels));
     uint32_t ticket = 0;
     if ((rc = takeGatherSlot(root, &ticket))) { return rc; }
-    const uint32_t grid = std::min<uint32_t>((uint32_t)((pixels + 255) / 256), (uint32_t)root->gridSimple * 4);
-    ptc_ctx::Denoise &d = root->denoise;
-    denoiseGatherKernel<<<grid, 256, 0, root->stream>>>(sets[0], sets[1], a.on ? a.counts : nullptr, spp, (uint32_t)pixels, d.colour[0]);
+    const uint32_t grid = gridFor(root, (uint32_t)pixels, 256);
+    denoiseGatherKernel<<<grid, 256, 0, root->stream>>>(sets[0], sets[1], a.on ? a.counts.get() : nullptr, spp, (uint32_t)pixels, d.colour[0].get());
     root->launches++;
     CUDA_TRY(root, cudaGetLastError());
-    if ((rc = denoiseAtrous(root, desc, root->guides.records))) { return rc; }
-    denoisePackKernel<<<grid, 256, 0, root->stream>>>(d.colour[desc->iterations & 1], root->gathers[ticket].device, (uint32_t)pixels);
+    if ((rc = denoiseAtrous(root, desc, root->guides.records.get()))) { return rc; }
+    denoisePackKernel<<<grid, 256, 0, root->stream>>>(d.colour[desc->iterations & 1].get(), root->gathers[ticket].device.get(), (uint32_t)pixels);
     root->launches++;
     if ((rc = finishGather(root, peers, nPeers, ticket))) { return rc; }
     *ticketOut = ticket;
@@ -3017,13 +2951,11 @@ int ptc_framebuffer_denoise_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t
 int ptc_philox4x32_10(ptc_ctx *ctx, const uint32_t *counters, const uint32_t *keys, uint32_t n, uint32_t *out)
 {
     if (!ctx || (n && (!counters || !keys || !out))) { return PTC_ERR_INVALID; }
-    uint32_t *dKeys = nullptr;
+    Buffer<uint32_t> dKeys;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, cudaMalloc((void **)&dKeys, std::max<size_t>(n, 1) * 2 * sizeof(uint32_t)));
-    cudaMemcpyAsync(dKeys, keys, (size_t)n * 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, counters, (size_t)4 * n, out, (size_t)4 * n, [&](uint32_t *d, uint32_t *o) { philoxKernel<<<std::max(1u, (n + 127) / 128), 128, 0, ctx->stream>>>(d, dKeys, n, o); });
-    cudaFree(dKeys);
-    return rc;
+    CUDA_TRY(ctx, dKeys.resize(std::max<size_t>(n, 1) * 2));
+    cudaMemcpyAsync(dKeys.get(), keys, (size_t)n * 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
+    return roundTrip(ctx, counters, (size_t)4 * n, out, (size_t)4 * n, [&](uint32_t *d, uint32_t *o) { philoxKernel<<<std::max(1u, (n + 127) / 128), 128, 0, ctx->stream>>>(d, dKeys.get(), n, o); });
 }
 int ptc_uniforms(ptc_ctx *ctx, uint64_t seed, const uint32_t *streams, uint32_t nStreams, uint32_t draws, float *out)
 {
@@ -3035,39 +2967,39 @@ int ptc_bsdf_eval(ptc_ctx *ctx, uint32_t material, const ptc_isect *isects, cons
 {
     NEED_COMMIT(ctx);
     if (material >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
-    float *dWi = nullptr, *dPdf = nullptr;
-    CUDA_TRY(ctx, cudaMalloc((void **)&dWi, std::max<size_t>(n, 1) * 3 * sizeof(float)));
-    CUDA_TRY(ctx, cudaMalloc((void **)&dPdf, std::max<size_t>(n, 1) * sizeof(float)));
-    cudaMemcpyAsync(dWi, wi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, isects, n, f, (size_t)3 * n, [&](ptc_isect *d, float *o) { bsdfEvalKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, d, dWi, n, o, dPdf); });
-    if (!rc) { cudaMemcpy(pdf, dPdf, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost); }
-    cudaFree(dWi); cudaFree(dPdf);
+    Buffer<float> dWi, dPdf;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    CUDA_TRY(ctx, dWi.resize(std::max<size_t>(n, 1) * 3));
+    CUDA_TRY(ctx, dPdf.resize(std::max<size_t>(n, 1)));
+    cudaMemcpyAsync(dWi.get(), wi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    const int rc = roundTrip(ctx, isects, n, f, (size_t)3 * n, [&](ptc_isect *d, float *o) { bsdfEvalKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, d, dWi.get(), n, o, dPdf.get()); });
+    if (!rc) { cudaMemcpy(pdf, dPdf.get(), (size_t)n * sizeof(float), cudaMemcpyDeviceToHost); }
     return rc;
 }
 int ptc_bsdf_sample(ptc_ctx *ctx, uint32_t material, const ptc_isect *isects, const float *xi, uint32_t n, float *wi, float *pdf, float *thr)
 {
     NEED_COMMIT(ctx);
     if (material >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
-    float *dXi = nullptr, *dPdf = nullptr, *dThr = nullptr;
-    CUDA_TRY(ctx, cudaMalloc((void **)&dXi, std::max<size_t>(n, 1) * 3 * sizeof(float)));
-    CUDA_TRY(ctx, cudaMalloc((void **)&dPdf, std::max<size_t>(n, 1) * sizeof(float)));
-    CUDA_TRY(ctx, cudaMalloc((void **)&dThr, std::max<size_t>(n, 1) * 3 * sizeof(float)));
-    cudaMemcpyAsync(dXi, xi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, isects, n, wi, (size_t)3 * n, [&](ptc_isect *d, float *o) { bsdfSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, d, dXi, n, o, dPdf, dThr); });
-    if (!rc) { cudaMemcpy(pdf, dPdf, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost); cudaMemcpy(thr, dThr, (size_t)n * 3 * sizeof(float), cudaMemcpyDeviceToHost); }
-    cudaFree(dXi); cudaFree(dPdf); cudaFree(dThr);
+    Buffer<float> dXi, dPdf, dThr;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    CUDA_TRY(ctx, dXi.resize(std::max<size_t>(n, 1) * 3));
+    CUDA_TRY(ctx, dPdf.resize(std::max<size_t>(n, 1)));
+    CUDA_TRY(ctx, dThr.resize(std::max<size_t>(n, 1) * 3));
+    cudaMemcpyAsync(dXi.get(), xi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    const int rc = roundTrip(ctx, isects, n, wi, (size_t)3 * n,
+                             [&](ptc_isect *d, float *o) { bsdfSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, d, dXi.get(), n, o, dPdf.get(), dThr.get()); });
+    if (!rc) { cudaMemcpy(pdf, dPdf.get(), (size_t)n * sizeof(float), cudaMemcpyDeviceToHost); cudaMemcpy(thr, dThr.get(), (size_t)n * 3 * sizeof(float), cudaMemcpyDeviceToHost); }
     return rc;
 }
 int ptc_light_sample(ptc_ctx *ctx, const float *ref, const float *xi, uint32_t n, ptc_light_sample_t *out)
 {
     NEED_COMMIT(ctx);
     if (!ctx->nLights) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene has no lights"); }
-    float *dXi = nullptr;
-    CUDA_TRY(ctx, cudaMalloc((void **)&dXi, std::max<size_t>(n, 1) * 3 * sizeof(float)));
-    cudaMemcpyAsync(dXi, xi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, ref, (size_t)3 * n, out, n, [&](float *d, ptc_light_sample_t *o) { lightSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi, n, o); });
-    cudaFree(dXi);
-    return rc;
+    Buffer<float> dXi;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    CUDA_TRY(ctx, dXi.resize(std::max<size_t>(n, 1) * 3));
+    cudaMemcpyAsync(dXi.get(), xi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    return roundTrip(ctx, ref, (size_t)3 * n, out, n, [&](float *d, ptc_light_sample_t *o) { lightSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi.get(), n, o); });
 }
 int ptc_light_pdf(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, float *pdf)
 {
@@ -3083,15 +3015,14 @@ int ptc_radiance_replay(ptc_ctx *ctx, const ptc_ray *rays, const float *xi, uint
 {
     NEED_COMMIT(ctx);
     if (last == -1 || last > PTC_MAX_BOUNCES) { last = PTC_MAX_BOUNCES; }
-    float *dXi = nullptr;
-    CUDA_TRY(ctx, cudaMalloc((void **)&dXi, std::max<size_t>((size_t)n * stride, 1) * sizeof(float)));
-    cudaMemcpyAsync(dXi, xi, (size_t)n * stride * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, rays, n, rgb, (size_t)3 * n, [&](ptc_ray *d, float *o) {
-        if (ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER) { volumeReplayKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi, stride, n, start, last, o); }
-        else { radianceReplayKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi, stride, n, start, last, o); }
+    Buffer<float> dXi;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    CUDA_TRY(ctx, dXi.resize(std::max<size_t>((size_t)n * stride, 1)));
+    cudaMemcpyAsync(dXi.get(), xi, (size_t)n * stride * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
+    return roundTrip(ctx, rays, n, rgb, (size_t)3 * n, [&](ptc_ray *d, float *o) {
+        if (ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER) { volumeReplayKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi.get(), stride, n, start, last, o); }
+        else { radianceReplayKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi.get(), stride, n, start, last, o); }
     });
-    cudaFree(dXi);
-    return rc;
 }
 
 int ptc_num_lights(ptc_ctx *ctx, uint32_t *out) { NEED_COMMIT(ctx); *out = ctx->nLights; return PTC_OK; }
@@ -3104,7 +3035,7 @@ int ptc_get_stats(ptc_ctx *ctx, ptc_stats *out)
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     collectTimings(ctx);
-    cudaMemcpy(totals, ctx->totals, sizeof(totals), cudaMemcpyDeviceToHost);
+    cudaMemcpy(totals, ctx->totals.get(), sizeof(totals), cudaMemcpyDeviceToHost);
     out->closest_rays = totals[0]; out->shadow_rays = totals[1]; out->samples = ctx->samples; out->kernel_launches = ctx->launches;
     out->extend_inner_visits = totals[2]; out->extend_triangle_tests = totals[3];
     out->shadow_inner_visits = totals[4]; out->shadow_triangle_tests = totals[5];
@@ -3126,7 +3057,7 @@ int ptc_get_wave_counts(ptc_ctx *ctx, uint32_t *extend, uint32_t *shadow, uint32
     std::vector<BounceCounters> host(CNT_STRIDE);
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
-    if (cudaMemcpy(host.data(), ctx->counters, CNT_STRIDE * sizeof(BounceCounters), cudaMemcpyDeviceToHost) != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "cudaMemcpy failed"); }
+    if (cudaMemcpy(host.data(), ctx->counters.get(), CNT_STRIDE * sizeof(BounceCounters), cudaMemcpyDeviceToHost) != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "cudaMemcpy failed"); }
     for (uint32_t k = 0; k < capacity && k < CNT_STRIDE; k++) { extend[k] = host[k].extendCount; shadow[k] = host[k].shadowCount + host[k].scatterCount; }
     return PTC_OK;
 }
@@ -3137,7 +3068,7 @@ int ptc_reset_stats(ptc_ctx *ctx)
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     collectTimings(ctx);
-    cudaMemset(ctx->totals, 0, 6 * sizeof(unsigned long long));
+    cudaMemset(ctx->totals.get(), 0, 6 * sizeof(unsigned long long));
     ctx->samples = 0; ctx->launches = 0;
     for (int i = 0; i < 4; i++) { ctx->stageMs[i] = 0; ctx->stageLaunches[i] = 0; }
     return PTC_OK;
@@ -3159,8 +3090,8 @@ int ptc_set_option(ptc_ctx *ctx, const char *name, int64_t value)
     if (!strcmp(name, "count_traversal")) { ctx->countTraversal = value != 0; return PTC_OK; }
     if (!strcmp(name, "volume_megakernel")) { ctx->volumeMegakernel = value != 0; return PTC_OK; }
     if (!strcmp(name, "framebuffer_moments")) { // takes effect for the moments at the next ptc_framebuffer_clear
-        ctx->fbMoments.on = value != 0;
-        if (!ctx->fbMoments.on) { ctx->fbMoments.complete = false; }
+        ctx->momentsOption = value != 0;
+        if (!ctx->momentsOption && !ctx->adaptive.on) { ctx->momentsComplete = false; } // an adaptive render's moments stay complete
         return PTC_OK;
     }
     if (!strcmp(name, "bvh_builder")) { // before ptc_commit; 1 = device (default), 0 = host binned SAH
