@@ -1194,10 +1194,8 @@ struct ptc_ctx {
     std::vector<Gather> gathers;                         // results of ptc_framebuffer_gather_begin in flight
     Event gatherRead;                                    // the last gather kernel of this (root) context finished reading the framebuffers
     PinnedBuffer<float> pinned;
-    // ptc_render: the caller's radianceLookup is uploaded on its own stream while the wave's kernels run; only the first
-    // accumulation waits for it (beforeAccumulate is called once, after the wave's other launches have been issued)
+    // ptc_render: the caller's radianceLookup is uploaded on its own stream while the first wave's kernels run (uploadSums)
     Stream copyStream; Event uploadDone;
-    std::function<int()> beforeAccumulate;
     Stream stream;
     Event evStart, evStop;
     int numSMs = 148;
@@ -1249,7 +1247,7 @@ struct ptc_ctx {
     // ptc_denoise's device buffers: the staged inputs (15 x 4 B per pixel) and guide records (32 B); two colour records (16 B each),
     // which ptc_framebuffer_denoise_begin uses as well
     struct Denoise { Buffer<float> inputs; Buffer<float4> guide, colour[2]; } denoise;
-    // the device guide sums of ptc_render_aovs and ptc_framebuffer_guides (8 x 4 B per pixel)
+    // the device guide sums of ptc_framebuffer_guides (8 x 4 B per pixel)
     Buffer<float> aovs;
     // ptc_framebuffer_guides: the guide records (32 B per pixel) ptc_framebuffer_denoise_begin filters with; aovSpp = 0: none
     struct Guides { int width = 0, height = 0; Buffer<float4> records; uint32_t aovSpp = 0; } guides;
@@ -2035,13 +2033,17 @@ static CheckpointPlan planFor(const Checkpoints &cp, uint32_t F, uint32_t S, boo
     return plan;
 }
 
-// ptc_render: the upload of the caller's sums, issued behind the launches of the first wave (ptc_ctx::beforeAccumulate)
-static int runBeforeAccumulate(ptc_ctx *ctx)
+// ptc_render's upload of the caller's sums (through `staging`, page-locked, when that is another buffer) into `device`.  The first
+// wave issues it on copyStream behind its other launches, so that it runs while the GPU traces the wave; only the wave's first
+// accumulation waits for it.
+struct SumsUpload { const float *caller; float *staging, *device; size_t n; };
+static int uploadSums(ptc_ctx *ctx, const SumsUpload &u)
 {
-    if (!ctx->beforeAccumulate) { return PTC_OK; }
-    const std::function<int()> f = ctx->beforeAccumulate;
-    ctx->beforeAccumulate = nullptr;
-    return f();
+    if (u.staging != u.caller) { memcpy(u.staging, u.caller, u.n * sizeof(float)); }
+    CUDA_TRY(ctx, cudaMemcpyAsync(u.device, u.staging, u.n * sizeof(float), cudaMemcpyHostToDevice, ctx->copyStream));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->uploadDone, ctx->copyStream));
+    CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->uploadDone, 0));
+    return PTC_OK;
 }
 
 // The arrays of lane `lane`: every array of the wave's path state starts `offset` paths further on
@@ -2090,20 +2092,75 @@ static int ensureVolumeBuffers(ptc_ctx *ctx, uint32_t capacity)
     return PTC_OK;
 }
 
-#define LAUNCH_MATERIAL(TYPE) \
-    if (ctx->classMask & (1u << TYPE)) { \
-        if (wp.pixels) { materialKernel<TYPE, true><<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc, bc + 1); } \
-        else { materialKernel<TYPE, false><<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc, bc + 1); } \
-        ctx->launches++; }
-#define LAUNCH_VOLUME_MATERIAL(TYPE) \
-    if (ctx->classMask & (1u << TYPE)) { volumeMaterialKernel<TYPE><<<ctx->gridVolumeShade, 128, 0, stream>>>(s, pb, vb, wp, bc, bc + 1); ctx->launches++; }
+// A traversal stage of a wave: a traverseKernel, or a volumeTraverseKernel (it also reads the VolumePathTracer's buffers), and its grid
+typedef void (*TraverseFn)(DScene, PathBuffers, const uint32_t *, const uint32_t *, uint32_t *, unsigned long long *);
+typedef void (*VolumeTraverseFn)(DScene, PathBuffers, VolumeBuffers, const uint32_t *, const uint32_t *, uint32_t *, unsigned long long *);
+struct Traversal {
+    TraverseFn plain = nullptr; VolumeTraverseFn volume = nullptr; int grid = 0;
+    void launch(cudaStream_t stream, const DScene &s, const PathBuffers &pb, const VolumeBuffers &vb, const uint32_t *queue, const uint32_t *count,
+                uint32_t *cursor, unsigned long long *work) const
+    {
+        if (volume) { volume<<<grid, 128, 0, stream>>>(s, pb, vb, queue, count, cursor, work); }
+        else { plain<<<grid, 128, 0, stream>>>(s, pb, queue, count, cursor, work); }
+    }
+};
+// extend0: the camera rays; extend: the rays of bounces >= 1; shadow and, in participating media, scatter: the shadow rays of bounces >= 1
+struct WaveTraversals { Traversal extend0, extend, shadow, scatter; };
+// sharedSMs: the wave is traced as several lanes, whose persistent traversal grids leave room for the CTAs of another lane's stage
+// (profiles/r02_sweep_lanes.txt)
+static WaveTraversals pickTraversals(const ptc_ctx *ctx, bool volume, bool sharedSMs)
+{
+    const DScene &s = ctx->scene;
+    const bool count = ctx->countTraversal;
+    const int grid = sharedSMs ? ctx->gridTraverseShared : ctx->gridTraverse;
+    const int volumeGrid = sharedSMs ? ctx->gridVolumeTraverseShared : ctx->gridVolumeTraverse;
+    WaveTraversals t;
+    const TraverseFn closest = count ? traverseKernel<false, true> : traverseKernel<false, false>;
+    t.extend0 = {s.bvh.placements ? traverseKernel<false, false, false, true> : closest, nullptr, grid}; // instanced: never counted
+    if (!volume) {
+        t.extend = t.extend0;
+        const TraverseFn shadow = s.bvh.placements ? traverseKernel<true, false, false, true> : s.hasFilter ? traverseKernel<true, false, true>
+                                  : count ? traverseKernel<true, true> : traverseKernel<true, false>;
+        t.shadow = {shadow, nullptr, grid};
+        return t;
+    }
+    // the VolumePathTracer's bounces: probe + continuation ray in one traversal (no container surface: the two rules coincide), both
+    // kinds of shadow rays next to them
+    if (s.hasFilter) { t.extend = {nullptr, count ? volumeTraverseKernel<VOL_EXTEND, true> : volumeTraverseKernel<VOL_EXTEND, false>, volumeGrid}; }
+    else { t.extend = {closest, nullptr, grid}; }
+    t.shadow = {nullptr, count ? volumeTraverseKernel<VOL_SHADOW, true> : volumeTraverseKernel<VOL_SHADOW, false>, volumeGrid};
+    if (s.nMedia) { t.scatter = {nullptr, count ? volumeTraverseKernel<VOL_SCATTER, true> : volumeTraverseKernel<VOL_SCATTER, false>, volumeGrid}; }
+    return t;
+}
+
+// The material stage's kernels by class; [LISTED]: the wave's pixels are listed (WaveParams::pixels)
+typedef void (*MaterialFn)(DScene, PathBuffers, WaveParams, BounceCounters *, BounceCounters *);
+static const MaterialFn materialKernels[2][PTC_MATERIAL_CLASSES] = {
+    {materialKernel<PTC_LAMBERTIAN, false>, materialKernel<PTC_OREN_NAYAR, false>, materialKernel<PTC_MIRROR, false>, materialKernel<PTC_GLASS, false>,
+     materialKernel<PTC_MICROFACET, false>, materialKernel<PTC_PLASTIC, false>, materialKernel<PTC_PASSTHROUGH, false>},
+    {materialKernel<PTC_LAMBERTIAN, true>, materialKernel<PTC_OREN_NAYAR, true>, materialKernel<PTC_MIRROR, true>, materialKernel<PTC_GLASS, true>,
+     materialKernel<PTC_MICROFACET, true>, materialKernel<PTC_PLASTIC, true>, materialKernel<PTC_PASSTHROUGH, true>}};
+typedef void (*VolumeMaterialFn)(DScene, PathBuffers, VolumeBuffers, WaveParams, BounceCounters *, BounceCounters *);
+static const VolumeMaterialFn volumeMaterialKernels[PTC_MATERIAL_CLASSES] = {
+    volumeMaterialKernel<PTC_LAMBERTIAN>, volumeMaterialKernel<PTC_OREN_NAYAR>, volumeMaterialKernel<PTC_MIRROR>, volumeMaterialKernel<PTC_GLASS>,
+    volumeMaterialKernel<PTC_MICROFACET>, volumeMaterialKernel<PTC_PLASTIC>, volumeMaterialKernel<PTC_PASSTHROUGH>};
+
+// radianceLookup += the samples of one (part-)wave, in sample order; with `moments` also their squares
+static void launchAccumulate(ptc_ctx *ctx, cudaStream_t stream, const PathBuffers &pb, const WaveParams &wp, float *accumDevice, float *moments,
+                             const CheckpointPlan &plan)
+{
+    const auto kernel = moments ? accumulateKernel<true> : accumulateKernel<false>;
+    kernel<<<gridFor(ctx, wp.nPixels, 256), 256, 0, stream>>>(pb, wp, accumDevice, moments, (uint32_t)ctx->scene.width, (uint32_t)ctx->scene.height, plan);
+    ctx->launches++;
+}
 
 // One wave = fixed launch sequence; all queue sizes stay on the device.  The wave's samples are traced as nLanes part-waves (wps[i]:
 // consecutive sample blocks, plans[i]: the checkpoints that fall into them) whose launch sequences are issued bounce by bounce on one
 // stream per lane, so that the stages of different lanes share the SMs (ptc_ctx::lanes); nLanes = 1 is the plain sequence.
 // volume: the VolumePathTracer's stages (volume_wavefront.cuh) -- merged probe / continuation rays, two kinds of shadow rays, its own
-// logic and material kernels; bounce 0 is the PathTracer's.
-static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan *plans, int nLanes, float *accumDevice, float *moments, cudaStream_t callerStream, bool volume)
+// logic and material kernels; bounce 0 is the PathTracer's.  upload: issued behind the wave's other launches (uploadSums).
+static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan *plans, int nLanes, float *accumDevice, float *moments, cudaStream_t callerStream,
+                      bool volume, const SumsUpload *upload)
 {
     const DScene &s = ctx->scene;
     struct LaneState { PathBuffers pb; VolumeBuffers vb; BounceCounters *cnt; cudaStream_t stream, shadowStream; cudaEvent_t shadeDone, shadowDone; };
@@ -2113,9 +2170,7 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
         if (rc) { return rc; }
         CUDA_TRY(ctx, cudaEventRecord(ctx->laneFork, callerStream)); // the other lanes start behind whatever the caller's stream holds so far
     }
-    // lanes share the SMs: the persistent traversal grids leave room for the CTAs of another lane's stage (profiles/r02_sweep_lanes.txt)
-    const int gridTraverse = nLanes > 1 ? ctx->gridTraverseShared : ctx->gridTraverse;
-    const int gridVolumeTraverse = nLanes > 1 ? ctx->gridVolumeTraverseShared : ctx->gridVolumeTraverse;
+    const WaveTraversals traversals = pickTraversals(ctx, volume, nLanes > 1);
     size_t offset = 0;
     for (int i = 0; i < nLanes; i++) {
         LaneState &l = lanes[i];
@@ -2137,7 +2192,6 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
         ctx->launches++;
     }
     unsigned long long *work = ctx->totals.get() + 2;
-    const bool count = ctx->countTraversal;
     const int lastBounce = wps[0].lastBounce;
     // ray k leaves vertex k (k = 0: camera ray).  Ray k feeds direct() of vertex k and creates vertex k + 1, so rays
     // 0 .. lastBounce are traced; shadow rays cast at vertex k are traced alongside ray k.
@@ -2157,39 +2211,20 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
                 CUDA_TRY(ctx, cudaStreamWaitEvent(l.shadowStream, l.shadeDone, 0));
             }
             {
+                // the rays of bounce k are the current buffers' slots 0 .. extendCount - 1: no queue (camera rays of either integrator:
+                // Scene::testIntersect), except the VolumePathTracer's bounces
                 StageTimer t(ctx, stream, STAGE_EXTEND);
-                if (volume && k > 0) {
-                    if (s.hasFilter) { // probe + continuation ray in one traversal
-                        if (count) { volumeTraverseKernel<VOL_EXTEND, true><<<gridVolumeTraverse, 128, 0, stream>>>(s, pb, vb, vb.extendQueue, &bc->extendCount, &bc->extendCursor, work); }
-                        else { volumeTraverseKernel<VOL_EXTEND, false><<<gridVolumeTraverse, 128, 0, stream>>>(s, pb, vb, vb.extendQueue, &bc->extendCount, &bc->extendCursor, work); }
-                    } else {           // no container surface: the two rules coincide
-                        if (count) { traverseKernel<false, true><<<gridTraverse, 128, 0, stream>>>(s, pb, vb.extendQueue, &bc->extendCount, &bc->extendCursor, work); }
-                        else { traverseKernel<false, false><<<gridTraverse, 128, 0, stream>>>(s, pb, vb.extendQueue, &bc->extendCount, &bc->extendCursor, work); }
-                    }
-                }
-                // the rays of bounce k are the current buffers' slots 0 .. extendCount - 1: no queue (camera rays of either integrator: Scene::testIntersect)
-                else if (s.bvh.placements) { traverseKernel<false, false, false, true><<<gridTraverse, 128, 0, stream>>>(s, pb, nullptr, &bc->extendCount, &bc->extendCursor, work); }
-                else if (count) { traverseKernel<false, true><<<gridTraverse, 128, 0, stream>>>(s, pb, nullptr, &bc->extendCount, &bc->extendCursor, work); }
-                else { traverseKernel<false, false><<<gridTraverse, 128, 0, stream>>>(s, pb, nullptr, &bc->extendCount, &bc->extendCursor, work); }
+                (k > 0 ? traversals.extend : traversals.extend0).launch(stream, s, pb, vb, volume && k > 0 ? vb.extendQueue : nullptr, &bc->extendCount, &bc->extendCursor, work);
             }
             ctx->launches++;
-            if (k > 0 && volume) { // both kinds of shadow rays of bounce k, next to the bounce's merged rays
+            if (k > 0) {
                 StageTimer t(ctx, shadowOn, STAGE_SHADOW);
-                if (count) {
-                    volumeTraverseKernel<VOL_SHADOW, true><<<gridVolumeTraverse, 128, 0, shadowOn>>>(s, pb, vb, pb.shadowQueue, &bc->shadowCount, &bc->shadowCursor, work + 2);
-                    if (s.nMedia) { volumeTraverseKernel<VOL_SCATTER, true><<<gridVolumeTraverse, 128, 0, shadowOn>>>(s, pb, vb, vb.scatterQueue, &bc->scatterCount, &bc->scatterCursor, work + 2); }
-                } else {
-                    volumeTraverseKernel<VOL_SHADOW, false><<<gridVolumeTraverse, 128, 0, shadowOn>>>(s, pb, vb, pb.shadowQueue, &bc->shadowCount, &bc->shadowCursor, work + 2);
-                    if (s.nMedia) { volumeTraverseKernel<VOL_SCATTER, false><<<gridVolumeTraverse, 128, 0, shadowOn>>>(s, pb, vb, vb.scatterQueue, &bc->scatterCount, &bc->scatterCursor, work + 2); }
-                }
-                ctx->launches += s.nMedia ? 2 : 1;
-            } else if (k > 0) {
-                StageTimer t(ctx, shadowOn, STAGE_SHADOW);
-                if (s.bvh.placements) { traverseKernel<true, false, false, true><<<gridTraverse, 128, 0, shadowOn>>>(s, pb, pb.shadowQueue, &bc->shadowCount, &bc->shadowCursor, work + 2); }
-                else if (s.hasFilter) { traverseKernel<true, false, true><<<gridTraverse, 128, 0, shadowOn>>>(s, pb, pb.shadowQueue, &bc->shadowCount, &bc->shadowCursor, work + 2); }
-                else if (count) { traverseKernel<true, true><<<gridTraverse, 128, 0, shadowOn>>>(s, pb, pb.shadowQueue, &bc->shadowCount, &bc->shadowCursor, work + 2); }
-                else { traverseKernel<true, false><<<gridTraverse, 128, 0, shadowOn>>>(s, pb, pb.shadowQueue, &bc->shadowCount, &bc->shadowCursor, work + 2); }
+                traversals.shadow.launch(shadowOn, s, pb, vb, pb.shadowQueue, &bc->shadowCount, &bc->shadowCursor, work + 2);
                 ctx->launches++;
+                if (traversals.scatter.volume) {
+                    traversals.scatter.launch(shadowOn, s, pb, vb, vb.scatterQueue, &bc->scatterCount, &bc->scatterCursor, work + 2);
+                    ctx->launches++;
+                }
             }
             if (overlap) { // the logic stage reads the occlusion bytes / shadow outcomes
                 CUDA_TRY(ctx, cudaEventRecord(l.shadowDone, l.shadowStream));
@@ -2203,19 +2238,18 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
                     if (k == 0 && s.hasFilter) { containerKernel<<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc); ctx->launches++; }
                 }
                 ctx->launches++;
-                if (volume) {
-                    LAUNCH_VOLUME_MATERIAL(PTC_LAMBERTIAN) LAUNCH_VOLUME_MATERIAL(PTC_OREN_NAYAR) LAUNCH_VOLUME_MATERIAL(PTC_MIRROR) LAUNCH_VOLUME_MATERIAL(PTC_GLASS)
-                    LAUNCH_VOLUME_MATERIAL(PTC_MICROFACET) LAUNCH_VOLUME_MATERIAL(PTC_PLASTIC) LAUNCH_VOLUME_MATERIAL(PTC_PASSTHROUGH)
-                } else {
-                    LAUNCH_MATERIAL(PTC_LAMBERTIAN) LAUNCH_MATERIAL(PTC_OREN_NAYAR) LAUNCH_MATERIAL(PTC_MIRROR) LAUNCH_MATERIAL(PTC_GLASS)
-                    LAUNCH_MATERIAL(PTC_MICROFACET) LAUNCH_MATERIAL(PTC_PLASTIC) LAUNCH_MATERIAL(PTC_PASSTHROUGH)
+                for (int c = 0; c < PTC_MATERIAL_CLASSES; c++) {
+                    if (!(ctx->classMask & (1u << c))) { continue; }
+                    if (volume) { volumeMaterialKernels[c]<<<ctx->gridVolumeShade, 128, 0, stream>>>(s, pb, vb, wp, bc, bc + 1); }
+                    else { materialKernels[wp.pixels != nullptr][c]<<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc, bc + 1); }
+                    ctx->launches++;
                 }
             }
             // the material stage moved every surviving path to its slot of bounce k + 1 in the `next` buffers
             std::swap(pb.ray, pb.nRay); std::swap(pb.modThr, pb.nModThr); std::swap(pb.result, pb.nResult);
         }
     }
-    { const int rcUpload = runBeforeAccumulate(ctx); if (rcUpload) { return rcUpload; } }
+    if (upload) { const int rc = uploadSums(ctx, *upload); if (rc) { return rc; } }
     // radianceLookup += in sample order: the lanes' samples are added one lane after the other on the caller's stream
     for (int i = 0; i < nLanes; i++) {
         if (i > 0) {
@@ -2224,11 +2258,9 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
             CUDA_TRY(ctx, cudaStreamWaitEvent(callerStream, x.done, 0));
         }
         StageTimer t(ctx, callerStream, STAGE_OTHER);
-        const uint32_t grid = gridFor(ctx, wps[i].nPixels, 256);
-        if (moments) { accumulateKernel<true><<<grid, 256, 0, callerStream>>>(lanes[i].pb, wps[i], accumDevice, moments, (uint32_t)s.width, (uint32_t)s.height, plans[i]); }
-        else { accumulateKernel<false><<<grid, 256, 0, callerStream>>>(lanes[i].pb, wps[i], accumDevice, nullptr, (uint32_t)s.width, (uint32_t)s.height, plans[i]); }
+        launchAccumulate(ctx, callerStream, lanes[i].pb, wps[i], accumDevice, moments, plans[i]);
         tallyKernel<<<1, 32, 0, callerStream>>>(lanes[i].cnt, ctx->totals.get());
-        ctx->launches += 2;
+        ctx->launches++;
     }
     if (ctx->pending.size() > 4096) { collectTimings(ctx); }
     CUDA_TRY(ctx, cudaGetLastError());
@@ -2239,46 +2271,31 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
 // order), whose accumulation also adds the squared samples into `moments`.  moments = null: a plain render of every pixel.
 struct PassPixels { const uint32_t *list = nullptr; uint32_t count = 0; float *moments = nullptr; };
 
-// VolumePathTracer waves: one volumePathKernel launch over pixels x sppWave paths, then the same in-order accumulation
-static int renderVolume(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp, uint32_t sppWave, int start, int last, float *accumDevice, cudaStream_t stream,
-                        const Checkpoints &checkpoints, const PassPixels &pass)
+// One wave of the VolumePathTracer as one thread per path: a volumePathKernel launch over pixels x sppWave paths, then the same
+// in-order accumulation
+static int volumeWave(ptc_ctx *ctx, const WaveParams &wp, const CheckpointPlan &plan, float *accumDevice, float *moments, cudaStream_t stream, const SumsUpload *upload)
 {
-    const DScene &s = ctx->scene;
-    const uint32_t nPixels = pass.moments ? pass.count : (uint32_t)s.width * (uint32_t)s.height;
-    CUDA_TRY(ctx, ctx->volumeOut.reserve((size_t)nPixels * sppWave));
-    CUDA_TRY(ctx, ctx->volumeCursor.resize(1));
-    float4 *out = ctx->volumeOut.get();
-    uint32_t *cursor = ctx->volumeCursor.get();
     PathBuffers pb = ctx->paths;
-    pb.out = out;
-    for (uint32_t done = 0; done < nSpp; done += sppWave) {
-        WaveParams wp;
-        wp.seed = seed; wp.firstSample = firstSample + done; wp.sppWave = std::min(sppWave, nSpp - done); wp.nPixels = nPixels; wp.groupShift = groupShiftFor(wp.sppWave);
-        wp.startBounce = start; wp.lastBounce = last; wp.pixels = pass.list;
-        CUDA_TRY(ctx, cudaMemsetAsync(cursor, 0, sizeof(uint32_t), stream));
-        {
-            StageTimer t(ctx, stream, STAGE_SHADE);
-            if (ctx->countTraversal) { volumePathKernel<true><<<ctx->gridVolume, 128, 0, stream>>>(s, out, wp, cursor, ctx->totals.get()); }
-            else { volumePathKernel<false><<<ctx->gridVolume, 128, 0, stream>>>(s, out, wp, cursor, ctx->totals.get()); }
-        }
-        { const int rcUpload = runBeforeAccumulate(ctx); if (rcUpload) { return rcUpload; } }
-        {
-            StageTimer t(ctx, stream, STAGE_OTHER);
-            const CheckpointPlan plan = planFor(checkpoints, wp.firstSample, wp.sppWave, done == 0, done + sppWave >= nSpp);
-            const uint32_t grid = gridFor(ctx, nPixels, 256);
-            if (pass.moments) { accumulateKernel<true><<<grid, 256, 0, stream>>>(pb, wp, accumDevice, pass.moments, (uint32_t)s.width, (uint32_t)s.height, plan); }
-            else { accumulateKernel<false><<<grid, 256, 0, stream>>>(pb, wp, accumDevice, nullptr, (uint32_t)s.width, (uint32_t)s.height, plan); }
-        }
-        ctx->launches += 2;
-        CUDA_TRY(ctx, cudaGetLastError());
+    pb.out = ctx->volumeOut.get();
+    uint32_t *cursor = ctx->volumeCursor.get();
+    CUDA_TRY(ctx, cudaMemsetAsync(cursor, 0, sizeof(uint32_t), stream));
+    {
+        StageTimer t(ctx, stream, STAGE_SHADE);
+        const auto kernel = ctx->countTraversal ? volumePathKernel<true> : volumePathKernel<false>;
+        kernel<<<ctx->gridVolume, 128, 0, stream>>>(ctx->scene, pb.out, wp, cursor, ctx->totals.get());
+        ctx->launches++;
     }
-    if (ctx->pending.size() > 4096) { collectTimings(ctx); }
-    ctx->samples += (uint64_t)nPixels * nSpp;
+    if (upload) { const int rc = uploadSums(ctx, *upload); if (rc) { return rc; } }
+    {
+        StageTimer t(ctx, stream, STAGE_OTHER);
+        launchAccumulate(ctx, stream, pb, wp, accumDevice, moments, plan);
+    }
+    CUDA_TRY(ctx, cudaGetLastError());
     return PTC_OK;
 }
 
 static int renderInternal(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp, int start, int last, float *accumDevice, cudaStream_t stream,
-                          const Checkpoints &checkpoints = Checkpoints(), const PassPixels &pass = PassPixels())
+                          const Checkpoints &checkpoints = Checkpoints(), const PassPixels &pass = PassPixels(), const SumsUpload *upload = nullptr)
 {
     if (start < 0 || (last != -1 && start > last)) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bad bounce window [%d, %d]", start, last); }
     if (last == -1 || last > PTC_MAX_BOUNCES) { last = PTC_MAX_BOUNCES; }
@@ -2287,18 +2304,24 @@ static int renderInternal(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uin
     sppWave = std::min(sppWave, std::max(nSpp, 1u));
     const bool volume = ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER;
     // the one-thread-per-path kernel stays for instanced scenes (the volume traversal kernels test world-space leaves only) and as an option
-    if (volume && (ctx->volumeMegakernel || ctx->scene.bvh.placements)) { return renderVolume(ctx, seed, firstSample, nSpp, sppWave, start, last, accumDevice, stream, checkpoints, pass); }
-    int rc = ensurePathBuffers(ctx, nPixels * sppWave);
-    if (rc) { return rc; }
-    if (volume && (rc = ensureVolumeBuffers(ctx, nPixels * sppWave))) { return rc; }
+    const bool megakernel = volume && (ctx->volumeMegakernel || ctx->scene.bvh.placements);
+    if (megakernel) {
+        CUDA_TRY(ctx, ctx->volumeOut.reserve((size_t)nPixels * sppWave));
+        CUDA_TRY(ctx, ctx->volumeCursor.resize(1));
+    } else {
+        int rc = ensurePathBuffers(ctx, nPixels * sppWave);
+        if (rc) { return rc; }
+        if (volume && (rc = ensureVolumeBuffers(ctx, nPixels * sppWave))) { return rc; }
+    }
     for (uint32_t done = 0; done < nSpp; done += sppWave) {
         WaveParams wp;
         wp.seed = seed; wp.firstSample = firstSample + done; wp.sppWave = std::min(sppWave, nSpp - done); wp.nPixels = nPixels; wp.groupShift = groupShiftFor(wp.sppWave);
         wp.startBounce = start; wp.lastBounce = last; wp.pixels = pass.list;
         // lanes: consecutive blocks of the wave's samples.  Two lanes, four when the wave is small (measured on five scenes,
-        // profiles/r02_sweep_lanes.txt); one while a stage or traversal counter pass describes one launch sequence at a time
+        // profiles/r02_sweep_lanes.txt); one for the megakernel, and while a stage or traversal counter pass describes one launch
+        // sequence at a time
         int nLanes = ctx->lanes > 0 ? ctx->lanes : ((uint64_t)nPixels * wp.sppWave <= (1u << 25) ? 4 : 2);
-        if (ctx->stageTiming || ctx->countTraversal) { nLanes = 1; }
+        if (megakernel || ctx->stageTiming || ctx->countTraversal) { nLanes = 1; }
         nLanes = (int)std::min<uint32_t>((uint32_t)nLanes, wp.sppWave);
         WaveParams wps[PTC_MAX_LANES]; CheckpointPlan plans[PTC_MAX_LANES];
         const uint32_t perLane = (wp.sppWave + (uint32_t)nLanes - 1) / (uint32_t)nLanes;
@@ -2308,8 +2331,12 @@ static int renderInternal(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uin
             w.firstSample = wp.firstSample + at; w.sppWave = std::min(perLane, wp.sppWave - at); w.groupShift = groupShiftFor(w.sppWave);
             plans[used] = planFor(checkpoints, w.firstSample, w.sppWave, done == 0 && at == 0, done + sppWave >= nSpp && at + perLane >= wp.sppWave);
         }
-        if ((rc = launchWave(ctx, wps, plans, used, accumDevice, pass.moments, stream, volume))) { return rc; }
+        const SumsUpload *waveUpload = done == 0 ? upload : nullptr;
+        const int rc = megakernel ? volumeWave(ctx, wps[0], plans[0], accumDevice, pass.moments, stream, waveUpload)
+                                  : launchWave(ctx, wps, plans, used, accumDevice, pass.moments, stream, volume, waveUpload);
+        if (rc) { return rc; }
     }
+    if (ctx->pending.size() > 4096) { collectTimings(ctx); } // launchWave also collects after every wave
     ctx->samples += (uint64_t)nPixels * nSpp;
     return PTC_OK;
 }
@@ -2341,16 +2368,9 @@ int ptc_render(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp,
     // needed by the accumulation at the end of the first wave, so the host copy into pinned memory and the upload are issued on a second
     // stream AFTER the wave's other launches (they are asynchronous) and run while the GPU traces the wave.
     CUDA_TRY(ctx, cudaEventRecord(ctx->evStart, ctx->stream));
-    ctx->beforeAccumulate = [ctx, accum, accumDevice, hostSide, n]() -> int {
-        if (hostSide != accum) { memcpy(hostSide, accum, n * sizeof(float)); }
-        CUDA_TRY(ctx, cudaMemcpyAsync(accumDevice, hostSide, n * sizeof(float), cudaMemcpyHostToDevice, ctx->copyStream));
-        CUDA_TRY(ctx, cudaEventRecord(ctx->uploadDone, ctx->copyStream));
-        CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, ctx->uploadDone, 0));
-        return PTC_OK;
-    };
-    int rc = renderInternal(ctx, seed, firstSample, nSpp, start, last, accumDevice, ctx->stream);
-    if (!rc) { rc = runBeforeAccumulate(ctx); } // no wave at all (zero samples): the sums pass through
-    ctx->beforeAccumulate = nullptr;
+    const SumsUpload upload = {accum, hostSide, accumDevice, n};
+    int rc = renderInternal(ctx, seed, firstSample, nSpp, start, last, accumDevice, ctx->stream, Checkpoints(), PassPixels(), &upload);
+    if (!rc && nSpp == 0) { rc = uploadSums(ctx, upload); } // no wave at all: the sums pass through
     if (rc) { return rc; }
     CUDA_TRY(ctx, cudaMemcpyAsync(hostSide, accumDevice, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaEventRecord(ctx->evStop, ctx->stream));
@@ -2664,20 +2684,35 @@ int ptc_resolve_device(ptc_ctx *ctx, const float *accum, float *out, uint32_t sp
 } // extern "C"
 
 // ------------------------------------------------------------------------------------------------ queries (host buffers)
-template <typename In, typename Out, typename Launch>
-static int roundTrip(ptc_ctx *ctx, const In *in, size_t nIn, Out *out, size_t nOut, Launch launch)
+// A host array of a query, `n` elements, and its device scratch.  An input is uploaded before the launch, an output downloaded after
+// it; an optional output with a null pointer is not downloaded (the kernel still writes its scratch).
+template <typename T> struct HostArray { T *host; size_t n; bool up, down; Buffer<T> device; };
+namespace host {
+template <typename T> static HostArray<T> in(const T *p, size_t n) { return {const_cast<T *>(p), n, true, false}; } // never written
+template <typename T> static HostArray<T> out(T *p, size_t n) { return {p, n, false, true}; }
+template <typename T> static HostArray<T> inout(T *p, size_t n) { return {p, n, true, true}; }
+template <typename T> static HostArray<T> optionalOut(T *p, size_t n) { return {p, n, false, p != nullptr}; }
+}
+
+// One query on host arrays, on the context's device and stream: scratch of at least one element per array (n = 0 works), the inputs
+// uploaded, launch(the arrays' device pointers, in order) -- one kernel --, every output downloaded, one synchronisation.
+// PTC_ERR_NOMEM when the scratch cannot be allocated, PTC_ERR_CUDA for any other failure.
+template <typename Launch, typename... T>
+static int query(ptc_ctx *ctx, Launch launch, HostArray<T>... a)
 {
-    Buffer<In> dIn; Buffer<Out> dOut;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dIn.resize(std::max<size_t>(nIn, 1)));
-    if (dOut.resize(std::max<size_t>(nOut, 1)) != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_NOMEM, "cudaMalloc failed"); }
-    cudaMemcpyAsync(dIn.get(), in, nIn * sizeof(In), cudaMemcpyHostToDevice, ctx->stream);
-    launch(dIn.get(), dOut.get());
+    cudaError_t e = cudaSuccess;
+    if (!(((e = a.device.resize(std::max<size_t>(a.n, 1))) == cudaSuccess) && ...)) { CTX_FAIL(ctx, PTC_ERR_NOMEM, "query scratch: %s", cudaGetErrorString(e)); }
+    if (!((!a.up || !a.n || (e = cudaMemcpyAsync(a.device.get(), a.host, a.n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream)) == cudaSuccess) && ...)) {
+        CTX_FAIL(ctx, PTC_ERR_CUDA, "query upload: %s", cudaGetErrorString(e));
+    }
+    launch(a.device.get()...);
     ctx->launches++;
-    cudaMemcpyAsync(out, dOut.get(), nOut * sizeof(Out), cudaMemcpyDeviceToHost, ctx->stream);
-    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    const cudaError_t e2 = cudaGetLastError();
-    if (e != cudaSuccess || e2 != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "kernel failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2)); }
+    CUDA_TRY(ctx, cudaGetLastError());
+    if (!((!a.down || !a.n || (e = cudaMemcpyAsync(a.host, a.device.get(), a.n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream)) == cudaSuccess) && ...)) {
+        CTX_FAIL(ctx, PTC_ERR_CUDA, "query download: %s", cudaGetErrorString(e));
+    }
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return PTC_OK;
 }
 
@@ -2715,72 +2750,52 @@ int ptc_intersect(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit *hits)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !hits)) { return PTC_ERR_INVALID; }
-    return roundTrip(ctx, rays, n, hits, n, [&](ptc_ray *d, ptc_hit *o) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o, nullptr); });
+    return query(ctx, [&](const ptc_ray *r, ptc_hit *h) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, h, nullptr); },
+                 host::in(rays, n), host::out(hits, n));
 }
 int ptc_intersect_instanced(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit *hits, uint32_t *instIds)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !hits || !instIds)) { return PTC_ERR_INVALID; }
-    Buffer<uint2> dInst;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dInst.resize(std::max<size_t>(n, 1)));
-    const int rc = roundTrip(ctx, rays, n, hits, n, [&](ptc_ray *d, ptc_hit *o) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o, dInst.get()); });
-    if (!rc) { cudaMemcpy(instIds, dInst.get(), (size_t)n * sizeof(uint2), cudaMemcpyDeviceToHost); }
-    return rc;
+    return query(ctx, [&](const ptc_ray *r, ptc_hit *h, uint32_t *inst) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, h, (uint2 *)inst); },
+                 host::in(rays, n), host::out(hits, n), host::out(instIds, (size_t)2 * n));
 }
 int ptc_intersect_full(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_isect *out)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !out)) { return PTC_ERR_INVALID; }
-    return roundTrip(ctx, rays, n, out, n, [&](ptc_ray *d, ptc_isect *o) { intersectFullKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o); });
+    return query(ctx, [&](const ptc_ray *r, ptc_isect *o) { intersectFullKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, o); },
+                 host::in(rays, n), host::out(out, n));
 }
 int ptc_occluded(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t n, uint8_t *occluded)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !maxT || !occluded)) { return PTC_ERR_INVALID; }
-    Buffer<float> dT;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dT.resize(std::max<size_t>(n, 1)));
-    cudaMemcpyAsync(dT.get(), maxT, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    return roundTrip(ctx, rays, n, occluded, n, [&](ptc_ray *d, uint8_t *o) { occludedKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dT.get(), n, o); });
+    return query(ctx, [&](const ptc_ray *r, const float *t, uint8_t *o) { occludedKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, t, n, o); },
+                 host::in(rays, n), host::in(maxT, n), host::out(occluded, n));
 }
-// volumetric queries: the per-ray event lists come back through device scratch buffers
-static int volumetricQuery(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t n, uint8_t *occluded, ptc_isect *isects, uint32_t *nEvents,
-                           float *eventT, uint32_t *eventMedium)
-{
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    Buffer<ptc_ray> dRays; Buffer<float> dMaxT, dT; Buffer<uint8_t> dOcc; Buffer<ptc_isect> dIs; Buffer<uint32_t> dN, dM;
-    const size_t m = std::max<size_t>(n, 1);
-    if (dRays.resize(m) != cudaSuccess || dMaxT.resize(m) != cudaSuccess || dOcc.resize(m) != cudaSuccess || dIs.resize(m) != cudaSuccess ||
-        dN.resize(m) != cudaSuccess || dT.resize(m * PTC_MAX_EVENTS) != cudaSuccess || dM.resize(m * PTC_MAX_EVENTS) != cudaSuccess) {
-        CTX_FAIL(ctx, PTC_ERR_NOMEM, "cudaMalloc failed");
-    }
-    cudaMemcpyAsync(dRays.get(), rays, n * sizeof(ptc_ray), cudaMemcpyHostToDevice, ctx->stream);
-    if (maxT) { cudaMemcpyAsync(dMaxT.get(), maxT, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream); }
-    if (occluded) { occludedVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, dRays.get(), dMaxT.get(), n, dOcc.get(), dN.get(), dT.get(), dM.get()); }
-    else { intersectVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, dRays.get(), n, dIs.get(), dN.get(), dT.get(), dM.get()); }
-    ctx->launches++;
-    if (occluded) { cudaMemcpyAsync(occluded, dOcc.get(), n, cudaMemcpyDeviceToHost, ctx->stream); }
-    if (isects) { cudaMemcpyAsync(isects, dIs.get(), n * sizeof(ptc_isect), cudaMemcpyDeviceToHost, ctx->stream); }
-    if (nEvents) { cudaMemcpyAsync(nEvents, dN.get(), n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream); }
-    if (eventT) { cudaMemcpyAsync(eventT, dT.get(), (size_t)n * PTC_MAX_EVENTS * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream); }
-    if (eventMedium) { cudaMemcpyAsync(eventMedium, dM.get(), (size_t)n * PTC_MAX_EVENTS * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream); }
-    const cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    const cudaError_t e2 = cudaGetLastError();
-    if (e != cudaSuccess || e2 != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "kernel failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2)); }
-    return PTC_OK;
-}
+// the volumetric queries' per-ray event lists are optional outputs
 int ptc_occluded_volumetric(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t n, uint8_t *occluded, uint32_t *nEvents, float *eventT, uint32_t *eventMedium)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !maxT || !occluded)) { return PTC_ERR_INVALID; }
-    return volumetricQuery(ctx, rays, maxT, n, occluded, nullptr, nEvents, eventT, eventMedium);
+    return query(ctx,
+                 [&](const ptc_ray *r, const float *t, uint8_t *o, uint32_t *en, float *et, uint32_t *em) {
+                     occludedVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, t, n, o, en, et, em);
+                 },
+                 host::in(rays, n), host::in(maxT, n), host::out(occluded, n), host::optionalOut(nEvents, n),
+                 host::optionalOut(eventT, (size_t)n * PTC_MAX_EVENTS), host::optionalOut(eventMedium, (size_t)n * PTC_MAX_EVENTS));
 }
 int ptc_intersect_volumetric(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_isect *out, uint32_t *nEvents, float *eventT, uint32_t *eventMedium)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !out)) { return PTC_ERR_INVALID; }
-    return volumetricQuery(ctx, rays, nullptr, n, nullptr, out, nEvents, eventT, eventMedium);
+    return query(ctx,
+                 [&](const ptc_ray *r, ptc_isect *o, uint32_t *en, float *et, uint32_t *em) {
+                     intersectVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, o, en, et, em);
+                 },
+                 host::in(rays, n), host::out(out, n), host::optionalOut(nEvents, n), host::optionalOut(eventT, (size_t)n * PTC_MAX_EVENTS),
+                 host::optionalOut(eventMedium, (size_t)n * PTC_MAX_EVENTS));
 }
 int ptc_intersect_device(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit *hits, void *stream)
 {
@@ -2801,37 +2816,21 @@ int ptc_occluded_device(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, ui
 int ptc_camera_rays(ptc_ctx *ctx, const float *rowCol, uint32_t n, ptc_ray *rays)
 {
     NEED_COMMIT(ctx);
-    return roundTrip(ctx, rowCol, (size_t)2 * n, rays, n, [&](float *d, ptc_ray *o) { cameraRaysKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o); });
+    return query(ctx, [&](const float *rc, ptc_ray *r) { cameraRaysKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, rc, n, r); },
+                 host::in(rowCol, (size_t)2 * n), host::out(rays, n));
 }
 // Guide buffers (denoise.cuh: aovKernel): the caller's sums go up, the kernel adds to them, they come back
 int ptc_render_aovs(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp, float *albedo, float *normal, float *depth, uint32_t *hits)
 {
     NEED_COMMIT(ctx);
     if (!albedo || !normal || !depth || !hits) { CTX_FAIL(ctx, PTC_ERR_INVALID, "null guide buffer"); }
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    if (!nSpp) { return PTC_OK; } // no samples: the sums stay as they are
     const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
-    CUDA_TRY(ctx, ctx->aovs.resize(8 * pixels));
-    float *d = ctx->aovs.get();
-    float *dAlbedo = d, *dNormal = d + 3 * pixels, *dDepth = d + 6 * pixels;
-    uint32_t *dHits = (uint32_t *)(d + 7 * pixels);
-    cudaError_t e = cudaSuccess;
-    auto step = [&](cudaError_t r) { if (e == cudaSuccess) { e = r; } };
-    step(cudaMemcpyAsync(dAlbedo, albedo, 3 * pixels * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    step(cudaMemcpyAsync(dNormal, normal, 3 * pixels * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    step(cudaMemcpyAsync(dDepth, depth, pixels * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    step(cudaMemcpyAsync(dHits, hits, pixels * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    if (e == cudaSuccess && nSpp) {
-        aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene, seed, firstSample, nSpp, dAlbedo, dNormal, dDepth, dHits);
-        ctx->launches++;
-        step(cudaGetLastError());
-    }
-    step(cudaMemcpyAsync(albedo, dAlbedo, 3 * pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    step(cudaMemcpyAsync(normal, dNormal, 3 * pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    step(cudaMemcpyAsync(depth, dDepth, pixels * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    step(cudaMemcpyAsync(hits, dHits, pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    step(cudaStreamSynchronize(ctx->stream));
-    if (e != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "guide buffers failed: %s", cudaGetErrorString(e)); }
-    return PTC_OK;
+    return query(ctx,
+                 [&](float *a, float *nrm, float *z, uint32_t *h) {
+                     aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene, seed, firstSample, nSpp, a, nrm, z, h);
+                 },
+                 host::inout(albedo, 3 * pixels), host::inout(normal, 3 * pixels), host::inout(depth, pixels), host::inout(hits, pixels));
 }
 
 // The same guide sums from zero into the context's device buffers, then the guide records of ptc_denoise's prepare step
@@ -2951,78 +2950,61 @@ int ptc_framebuffer_denoise_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t
 int ptc_philox4x32_10(ptc_ctx *ctx, const uint32_t *counters, const uint32_t *keys, uint32_t n, uint32_t *out)
 {
     if (!ctx || (n && (!counters || !keys || !out))) { return PTC_ERR_INVALID; }
-    Buffer<uint32_t> dKeys;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dKeys.resize(std::max<size_t>(n, 1) * 2));
-    cudaMemcpyAsync(dKeys.get(), keys, (size_t)n * 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream);
-    return roundTrip(ctx, counters, (size_t)4 * n, out, (size_t)4 * n, [&](uint32_t *d, uint32_t *o) { philoxKernel<<<std::max(1u, (n + 127) / 128), 128, 0, ctx->stream>>>(d, dKeys.get(), n, o); });
+    return query(ctx, [&](const uint32_t *c, const uint32_t *k, uint32_t *o) { philoxKernel<<<std::max(1u, (n + 127) / 128), 128, 0, ctx->stream>>>(c, k, n, o); },
+                 host::in(counters, (size_t)4 * n), host::in(keys, (size_t)2 * n), host::out(out, (size_t)4 * n));
 }
 int ptc_uniforms(ptc_ctx *ctx, uint64_t seed, const uint32_t *streams, uint32_t nStreams, uint32_t draws, float *out)
 {
     if (!ctx || (nStreams && draws && (!streams || !out))) { return PTC_ERR_INVALID; }
-    return roundTrip(ctx, streams, (size_t)3 * nStreams, out, (size_t)nStreams * draws,
-                     [&](uint32_t *d, float *o) { uniformsKernel<<<std::max(1u, (nStreams + 127) / 128), 128, 0, ctx->stream>>>(seed, d, nStreams, draws, o); });
+    return query(ctx, [&](const uint32_t *s, float *o) { uniformsKernel<<<std::max(1u, (nStreams + 127) / 128), 128, 0, ctx->stream>>>(seed, s, nStreams, draws, o); },
+                 host::in(streams, (size_t)3 * nStreams), host::out(out, (size_t)nStreams * draws));
 }
 int ptc_bsdf_eval(ptc_ctx *ctx, uint32_t material, const ptc_isect *isects, const float *wi, uint32_t n, float *f, float *pdf)
 {
     NEED_COMMIT(ctx);
     if (material >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
-    Buffer<float> dWi, dPdf;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dWi.resize(std::max<size_t>(n, 1) * 3));
-    CUDA_TRY(ctx, dPdf.resize(std::max<size_t>(n, 1)));
-    cudaMemcpyAsync(dWi.get(), wi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, isects, n, f, (size_t)3 * n, [&](ptc_isect *d, float *o) { bsdfEvalKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, d, dWi.get(), n, o, dPdf.get()); });
-    if (!rc) { cudaMemcpy(pdf, dPdf.get(), (size_t)n * sizeof(float), cudaMemcpyDeviceToHost); }
-    return rc;
+    return query(ctx,
+                 [&](const ptc_isect *is, const float *w, float *fo, float *p) {
+                     bsdfEvalKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, is, w, n, fo, p);
+                 },
+                 host::in(isects, n), host::in(wi, (size_t)3 * n), host::out(f, (size_t)3 * n), host::out(pdf, n));
 }
 int ptc_bsdf_sample(ptc_ctx *ctx, uint32_t material, const ptc_isect *isects, const float *xi, uint32_t n, float *wi, float *pdf, float *thr)
 {
     NEED_COMMIT(ctx);
     if (material >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
-    Buffer<float> dXi, dPdf, dThr;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dXi.resize(std::max<size_t>(n, 1) * 3));
-    CUDA_TRY(ctx, dPdf.resize(std::max<size_t>(n, 1)));
-    CUDA_TRY(ctx, dThr.resize(std::max<size_t>(n, 1) * 3));
-    cudaMemcpyAsync(dXi.get(), xi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    const int rc = roundTrip(ctx, isects, n, wi, (size_t)3 * n,
-                             [&](ptc_isect *d, float *o) { bsdfSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, d, dXi.get(), n, o, dPdf.get(), dThr.get()); });
-    if (!rc) { cudaMemcpy(pdf, dPdf.get(), (size_t)n * sizeof(float), cudaMemcpyDeviceToHost); cudaMemcpy(thr, dThr.get(), (size_t)n * 3 * sizeof(float), cudaMemcpyDeviceToHost); }
-    return rc;
+    return query(ctx,
+                 [&](const ptc_isect *is, const float *x, float *w, float *p, float *t) {
+                     bsdfSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, is, x, n, w, p, t);
+                 },
+                 host::in(isects, n), host::in(xi, (size_t)3 * n), host::out(wi, (size_t)3 * n), host::out(pdf, n), host::out(thr, (size_t)3 * n));
 }
 int ptc_light_sample(ptc_ctx *ctx, const float *ref, const float *xi, uint32_t n, ptc_light_sample_t *out)
 {
     NEED_COMMIT(ctx);
     if (!ctx->nLights) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene has no lights"); }
-    Buffer<float> dXi;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dXi.resize(std::max<size_t>(n, 1) * 3));
-    cudaMemcpyAsync(dXi.get(), xi, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    return roundTrip(ctx, ref, (size_t)3 * n, out, n, [&](float *d, ptc_light_sample_t *o) { lightSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi.get(), n, o); });
+    return query(ctx, [&](const float *r, const float *x, ptc_light_sample_t *o) { lightSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, x, n, o); },
+                 host::in(ref, (size_t)3 * n), host::in(xi, (size_t)3 * n), host::out(out, n));
 }
 int ptc_light_pdf(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, float *pdf)
 {
     NEED_COMMIT(ctx);
-    return roundTrip(ctx, rays, n, pdf, n, [&](ptc_ray *d, float *o) { lightPdfKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o); });
+    return query(ctx, [&](const ptc_ray *r, float *p) { lightPdfKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, p); },
+                 host::in(rays, n), host::out(pdf, n));
 }
 int ptc_environment_radiance(ptc_ctx *ctx, const float *dirs, uint32_t n, float *rgb)
 {
     NEED_COMMIT(ctx);
-    return roundTrip(ctx, dirs, (size_t)3 * n, rgb, (size_t)3 * n, [&](float *d, float *o) { envRadianceKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o); });
+    return query(ctx, [&](const float *d, float *o) { envRadianceKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o); },
+                 host::in(dirs, (size_t)3 * n), host::out(rgb, (size_t)3 * n));
 }
 int ptc_radiance_replay(ptc_ctx *ctx, const ptc_ray *rays, const float *xi, uint32_t stride, uint32_t n, int start, int last, float *rgb)
 {
     NEED_COMMIT(ctx);
     if (last == -1 || last > PTC_MAX_BOUNCES) { last = PTC_MAX_BOUNCES; }
-    Buffer<float> dXi;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    CUDA_TRY(ctx, dXi.resize(std::max<size_t>((size_t)n * stride, 1)));
-    cudaMemcpyAsync(dXi.get(), xi, (size_t)n * stride * sizeof(float), cudaMemcpyHostToDevice, ctx->stream);
-    return roundTrip(ctx, rays, n, rgb, (size_t)3 * n, [&](ptc_ray *d, float *o) {
-        if (ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER) { volumeReplayKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi.get(), stride, n, start, last, o); }
-        else { radianceReplayKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, dXi.get(), stride, n, start, last, o); }
-    });
+    const auto kernel = ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER ? volumeReplayKernel : radianceReplayKernel;
+    return query(ctx, [&](const ptc_ray *r, const float *x, float *o) { kernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, x, stride, n, start, last, o); },
+                 host::in(rays, n), host::in(xi, (size_t)n * stride), host::out(rgb, (size_t)3 * n));
 }
 
 int ptc_num_lights(ptc_ctx *ctx, uint32_t *out) { NEED_COMMIT(ctx); *out = ctx->nLights; return PTC_OK; }
