@@ -41,7 +41,6 @@ struct WideBVH {
     std::vector<WideNode> nodes;         // nodes[0] is the root
     std::vector<LeafTriangle> triangles; // in leaf order
     std::vector<float> placements;       // instanced scenes: 24 floats per flattened placement (traverse.cuh: BvhView::placements)
-    float sceneLo[3], sceneHi[3];
     uint32_t maxDepth = 0;
 };
 

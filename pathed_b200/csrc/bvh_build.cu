@@ -139,7 +139,6 @@ uint8_t exponentFor(float extent)
 void buildWideBVH(const float *positions4, const uint32_t *indices4, uint32_t nPrims, WideBVH &out)
 {
     out.nodes.clear(); out.triangles.clear(); out.maxDepth = 0;
-    for (int a = 0; a < 3; a++) { out.sceneLo[a] = 0.f; out.sceneHi[a] = 0.f; }
     if (nPrims == 0) { return; }
 
     const auto t0 = std::chrono::steady_clock::now();
@@ -157,7 +156,6 @@ void buildWideBVH(const float *positions4, const uint32_t *indices4, uint32_t nP
     b.maxThreads = (int)std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
     const uint32_t root = b.alloc();
     b.build(root, 0, nPrims, 0);
-    for (int a = 0; a < 3; a++) { out.sceneLo[a] = b.nodes[root].box.lo[a]; out.sceneHi[a] = b.nodes[root].box.hi[a]; }
 
     const auto t1 = std::chrono::steady_clock::now();
     // ---- SAH-optimal collapse to 8-wide (Ylitie, Karras, Laine 2017, section 3.1): C(n, i) = cheapest way to represent the

@@ -896,7 +896,6 @@ void buildWideBVHDevice(const float4 *dPositions, const uint4 *dPrims, uint32_t 
 void buildWideBVHEmulated(const float *positions4, const uint32_t *indices4, uint32_t nPrims, WideBVH &out)
 {
     out.nodes.clear(); out.triangles.clear(); out.maxDepth = 0;
-    for (int k = 0; k < 3; k++) { out.sceneLo[k] = 0.f; out.sceneHi[k] = 0.f; }
     if (nPrims == 0) { return; }
     HostExec exec;
     BuildArrays a;

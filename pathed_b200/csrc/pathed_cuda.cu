@@ -23,6 +23,7 @@
 #include <cstdio>
 #include <cstring>
 #include <functional>
+#include <optional>
 #include <string>
 #include <chrono>
 #include <vector>
@@ -1144,11 +1145,8 @@ private:
     cudaEvent_t e_ = nullptr;
 };
 
-struct ptc_ctx {
-    int device = 0;
-    std::string error;
-    bool committed = false;
-    // staging (host)
+// What ptc_add_* / ptc_set_environment / ptc_begin|end_instance accumulate for ptc_commit, which releases it
+struct Staging {
     std::vector<ptc_material_desc> materials;
     struct HostTexture { std::vector<uint32_t> texels; int width, height; };
     std::vector<HostTexture> textures;
@@ -1160,26 +1158,62 @@ struct ptc_ctx {
     std::vector<uint32_t> rootGeometry;                        // root geometry id -> index into geometries
     struct HostMedium { float sigmaT[3], sigmaS[3]; };
     std::vector<HostMedium> media;
+    bool hasEnv = false; std::vector<float> envRgba; int envW = 0, envH = 0; float envScale = 1.f; float envM2W[16], envW2M[16];
+};
+
+// One device allocation of a committed scene and what points at it: the DScene field at byte offset `field` (NO_FIELD: none), and
+// for texels the material-table entries whose `texels` it holds.  ptc_replicate points them at its copy.
+static constexpr size_t NO_FIELD = ~(size_t)0; struct SceneAllocation { Buffer<uint8_t> data; size_t field; std::vector<uint32_t> materials; };
+
+// The committed scene as the renders and queries read it.  ptc_commit assembles a Committed and moves it into the context once every
+// step succeeded; ptc_replicate assigns this part to the replica.
+struct SceneState {
+    DScene view = {};                 // the kernels' parameter; before ptc_commit only its camera is set
+    std::vector<DMaterial> materials; // the material table as uploaded (texel pointers included)
+    uint32_t classMask = 0;           // material classes present in the scene
+    uint32_t bvhTriangles = 0, bvhDepth = 0, bvhPlocIterations = 0; float bvhBuildMs = 0.f; // ptc_get_stats (nodes: view.bvh.nNodes)
+    std::vector<float> placements;    // host copy of view.bvh.placements (ptc_count_traversal)
+};
+struct Committed : SceneState {
+    std::vector<SceneAllocation> allocations; // the device memory `view` and `materials` point into
+    Buffer<uint8_t> buildWorkspace;           // the device builder's working set, released with the context (bvh.h: buildWideBVHDevice)
+};
+
+// ptc_set_option's settings and the integrator: what a replica inherits
+struct Options {
     int integrator = PTC_INTEGRATOR_PATH_TRACER;
-    Buffer<float4> volumeOut; Buffer<uint32_t> volumeCursor;
-    int gridVolume = 0;
+    int64_t pathsPerWave = 1 << 27; // up to 134 M paths x 237 B = 31.8 GB of path state per wave (of 180 GB; allocated for the paths a render call needs):
+                                    // the queues of the late bounces (1 % of the paths) stay long enough to keep 148 SMs busy.  Dragon workload: 613 / 648 / 653
+                                    // Msamples/s with 2^24 / 2^26 / 2^27; teapot 1920x1080, 64-spp steps: 2306 (two waves of 32 spp at 2^26) vs 2374 (one wave)
+    bool stageTiming = false, countTraversal = false;
+    // the shadow rays of a bounce are traced on a second stream, concurrently with the bounce's extend rays: both grids fill the GPU, so
+    // the shadow CTAs become resident as the extend kernel drains -- the tail of one launch is filled with the head of the other
+    bool overlapShadow = true;
+    // A wave is traced as `lanes` interleaved part-waves (consecutive blocks of the wave's samples, each with its own share of the path
+    // state, its own counters and streams): while one lane's paths are in a shading stage (waiting on dependent loads, half of the issue
+    // slots idle) another lane's rays are in a traversal stage (issue-bound, hardly any DRAM traffic), and the SMs hold CTAs of both.
+    // Lane 0 runs on the caller's stream; the samples are still added to the image in sample order (launchWave), so the result does
+    // not depend on the number of lanes.
+    int lanes = 0; // 0 = chosen per wave (renderInternal)
     // VolumePathTracer as wavefront stages (volume_wavefront.cuh); volumeMegakernel = 1 keeps the one-thread-per-path kernel
     bool volumeMegakernel = false;
+    int bvhBuilder = 1; // 1: device builder (bvh_build_gpu.cu), 0: host binned-SAH builder (bvh_build.cu)
+    bool framebufferMoments = false; // see ptc_ctx::moments
+};
+
+struct ptc_ctx {
+    int device = 0;
+    std::string error;
+    bool committed = false, hasCamera = false;
+    Staging staged; Committed scene; Options options;
+    std::optional<WideBVH> hostBvh; // host copy of the device BVH, fetched when ptc_count_traversal first walks it
+    Buffer<float4> volumeOut; Buffer<uint32_t> volumeCursor;
+    int gridVolume = 0;
     VolumeBuffers volumeBuffers = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}; Buffer<uint8_t> volumeArrays[6];
     int gridVolumeTraverse = 0, gridVolumeLogic = 0, gridVolumeShade = 0;
-    bool hasEnv = false, hasCamera = false;
-    std::vector<float> envRgba; int envW = 0, envH = 0; float envScale = 1.f; float envM2W[16], envW2M[16];
-    float camToWorld[12]; float vfov = 0.f; int width = 0, height = 0;
-    WideBVH bvh;
-    uint32_t nLights = 0;
-    // device
-    std::vector<Buffer<uint8_t>> allocations;  // scene data on the device (what ptc_replicate copies)
-    std::vector<DMaterial> deviceMaterials;    // the device material table as uploaded (holds texel pointers)
-    DScene scene;
     PathBuffers paths; uint32_t pathCapacity = 0; Buffer<uint8_t> pathSlab;
     Buffer<uint32_t> classQueues[PTC_MATERIAL_CLASSES];
     Buffer<BounceCounters> counters;
-    uint32_t classMask = 0; // material classes present in the scene
     Buffer<unsigned long long> totals;
     Buffer<float> accumScratch;
     Buffer<float> framebuffer, gatherStage;
@@ -1201,30 +1235,10 @@ struct ptc_ctx {
     int numSMs = 148;
     int gridTraverse = 0, gridShade = 0, gridLogic = 0, gridSimple = 0;
     int gridTraverseShared = 0, gridVolumeTraverseShared = 0; // traversal grids of a wave traced as several lanes: two CTAs per SM fewer
-    // options / stats
-    int64_t pathsPerWave = 1 << 27; // up to 134 M paths x 237 B = 31.8 GB of path state per wave (of 180 GB; allocated for the paths a render call needs):
-                                    // the queues of the late bounces (1 % of the paths) stay long enough to keep 148 SMs busy.  Dragon workload: 613 / 648 / 653
-                                    // Msamples/s with 2^24 / 2^26 / 2^27; teapot 1920x1080, 64-spp steps: 2306 (two waves of 32 spp at 2^26) vs 2374 (one wave)
-    bool stageTiming = false, countTraversal = false;
-    // the shadow rays of a bounce are traced on a second stream, concurrently with the bounce's extend rays: both grids fill the GPU, so
-    // the shadow CTAs become resident as the extend kernel drains -- the tail of one launch is filled with the head of the other
-    bool overlapShadow = true;
     Stream shadowStream; Event shadeDone, shadowDone;
-    // A wave is traced as `lanes` interleaved part-waves (consecutive blocks of the wave's samples, each with its own share of the path
-    // state, its own counters and streams): while one lane's paths are in a shading stage (waiting on dependent loads, half of the issue
-    // slots idle) another lane's rays are in a traversal stage (issue-bound, hardly any DRAM traffic), and the SMs hold CTAs of both.
-    // Lane 0 runs on the caller's stream; the samples are still added to the image in sample order (launchWave), so the result does
-    // not depend on the number of lanes.
-    int lanes = 0; // 0 = chosen per wave (renderInternal)
     struct Lane { Stream stream, shadowStream; Event shadeDone, shadowDone, done; Buffer<BounceCounters> counters; };
     std::vector<Lane> extraLanes; // lanes 1 ..
     Event laneFork;
-    int bvhBuilder = 1; // 1: device builder (bvh_build_gpu.cu), 0: host binned-SAH builder (bvh_build.cu)
-    float bvhBuildMs = 0.f; uint32_t bvhPlocIterations = 0;
-    // the device builder leaves nodes and leaf triangles in HBM; the host copy (only ptc_count_traversal walks it) is fetched on demand
-    uint32_t bvhNodeCount = 0, bvhTriangleCount = 0;
-    bool hostBvhFetched = true;
-    Buffer<uint8_t> buildWorkspace; // the device builder's working set, released with the context (bvh.h: buildWideBVHDevice)
     // adaptive sampling (ptc_adaptive_*): between begin and the next ptc_framebuffer_clear the framebuffer belongs to the passes.
     // Per pixel: second moments (`moments` below), sample count, and two list entries (active pixels, the stopping test's output)
     // = 24 B, plus cub's selection scratch
@@ -1238,7 +1252,7 @@ struct ptc_ctx {
         Buffer<uint8_t> scratch;
     } adaptive;
     // The second moments (3 x fp32 per pixel, next to the framebuffer's sums): the squared samples that the adaptive passes add, and,
-    // with option "framebuffer_moments" (momentsOption), the framebuffer renders; zeroed by ptc_adaptive_begin and, with the option
+    // with option "framebuffer_moments" (options.framebufferMoments), the framebuffer renders; zeroed by ptc_adaptive_begin and, with the option
     // on, by ptc_framebuffer_clear.  The input of ptc_denoise that PTC_GATHER_MOMENTS gathers.  momentsComplete: they cover every
     // sample the framebuffer holds (an adaptive render, or the option on at the last clear and at every render since); the gather
     // refuses them otherwise
@@ -1285,7 +1299,7 @@ struct StageTimer { // brackets one launch when stage timing is on
     ptc_ctx *ctx; cudaStream_t stream; Event a; int kind;
     StageTimer(ptc_ctx *c, cudaStream_t s, int k) : ctx(c), stream(s), kind(k)
     {
-        if (ctx->stageTiming) { a = takeEvent(ctx); cudaEventRecord(a, stream); }
+        if (ctx->options.stageTiming) { a = takeEvent(ctx); cudaEventRecord(a, stream); }
     }
     ~StageTimer()
     {
@@ -1295,19 +1309,36 @@ struct StageTimer { // brackets one launch when stage timing is on
 
 #define CTX_FAIL(ctx, code, ...) do { char _b[512]; snprintf(_b, sizeof(_b), __VA_ARGS__); (ctx)->error = _b; return (code); } while (0)
 #define CUDA_TRY(ctx, call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { CTX_FAIL(ctx, PTC_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(_e)); } } while (0)
+#define TRY(call) do { const int _rc = (call); if (_rc) { return _rc; } } while (0)
 
 // grid of a grid-stride launch over n >= 1 items
 static inline uint32_t gridFor(ptc_ctx *ctx, uint32_t n, uint32_t block = 128) { return std::max(1u, std::min<uint32_t>((n + block - 1) / block, (uint32_t)ctx->gridSimple * 4)); }
 
+// byte offset of `field` inside `s` (SceneAllocation::field)
+static size_t fieldOf(const DScene &s, const void *field) { return (size_t)((const char *)field - (const char *)&s); }
+// A new device allocation holding `count` elements of `src` (at least one element is allocated), appended to `to`
 template <typename T>
-static int upload(ptc_ctx *ctx, const T *src, size_t count, const T **dst)
+static int upload(ptc_ctx *ctx, std::vector<SceneAllocation> &to, const T *src, size_t count, const T **dst, size_t field = NO_FIELD)
 {
     Buffer<uint8_t> b;
     CUDA_TRY(ctx, b.resize(std::max<size_t>(count, 1) * sizeof(T)));
     *dst = (const T *)b.get();
-    ctx->allocations.push_back(std::move(b));
+    to.push_back({std::move(b), field, {}});
     if (count) { CUDA_TRY(ctx, cudaMemcpy((void *)*dst, src, count * sizeof(T), cudaMemcpyHostToDevice)); }
     return PTC_OK;
+}
+// ... into the scene `c`, recorded as what its DScene's `field` points at
+template <typename T>
+static int upload(ptc_ctx *ctx, Committed &c, const T *src, size_t count, const T *&field)
+{
+    return upload(ctx, c.allocations, src, count, &field, fieldOf(c.view, &field));
+}
+
+// Texture::lookup's powf(c / 255.f, 2.2f) (src/texture.cpp:44-48), one table for all textures on the current device
+static cudaError_t uploadGammaTable()
+{
+    float gamma[256]; for (int c = 0; c < 256; c++) { gamma[c] = powf(c / 255.f, 2.2f); }
+    return cudaMemcpyToSymbol(c_gammaTable, gamma, sizeof(gamma));
 }
 
 extern "C" {
@@ -1325,7 +1356,6 @@ int ptc_create(int device, ptc_ctx **out)
     if (cudaSetDevice(device) != cudaSuccess) { return PTC_ERR_CUDA; }
     ptc_ctx *ctx = new ptc_ctx();
     ctx->device = device;
-    memset(&ctx->scene, 0, sizeof(ctx->scene));
     memset(&ctx->paths, 0, sizeof(ctx->paths));
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) { ctx->numSMs = prop.multiProcessorCount; }
@@ -1356,7 +1386,7 @@ int ptc_create(int device, ptc_ctx **out)
     ctx->gridTraverseShared = std::max(ctx->numSMs, ctx->gridTraverse - 2 * ctx->numSMs);
     ctx->gridVolumeTraverseShared = std::max(ctx->numSMs, ctx->gridVolumeTraverse - 2 * ctx->numSMs);
     // tuning hooks (tools/sweep_lanes.sh): number of interleaved lanes and CTAs per SM of the persistent grids
-    if (const char *e = getenv("PTC_LANES")) { ctx->lanes = std::min(PTC_MAX_LANES, std::max(0, atoi(e))); }
+    if (const char *e = getenv("PTC_LANES")) { ctx->options.lanes = std::min(PTC_MAX_LANES, std::max(0, atoi(e))); }
     if (const char *e = getenv("PTC_TRAVERSE_PER_SM")) { ctx->gridTraverse = ctx->gridTraverseShared = ctx->numSMs * std::max(1, atoi(e)); }
     if (const char *e = getenv("PTC_VOLUME_TRAVERSE_PER_SM")) { ctx->gridVolumeTraverse = ctx->gridVolumeTraverseShared = ctx->numSMs * std::max(1, atoi(e)); }
     if (const char *e = getenv("PTC_LOGIC_PER_SM")) { ctx->gridLogic = ctx->numSMs * std::max(1, atoi(e)); }
@@ -1381,12 +1411,12 @@ int ptc_add_texture(ptc_ctx *ctx, const uint8_t *rgb, int width, int height, uin
     if (!ctx || !rgb) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
     if (width <= 0 || height <= 0) { CTX_FAIL(ctx, PTC_ERR_INVALID, "Error loading texture: %d x %d", width, height); }
-    ptc_ctx::HostTexture t;
+    Staging::HostTexture t;
     t.width = width; t.height = height;
     t.texels.resize((size_t)width * height);
     for (size_t i = 0; i < t.texels.size(); i++) { t.texels[i] = (uint32_t)rgb[3 * i] | ((uint32_t)rgb[3 * i + 1] << 8) | ((uint32_t)rgb[3 * i + 2] << 16); }
-    ctx->textures.push_back(std::move(t));
-    if (id) { *id = (uint32_t)ctx->textures.size() - 1; }
+    ctx->staged.textures.push_back(std::move(t));
+    if (id) { *id = (uint32_t)ctx->staged.textures.size() - 1; }
     return PTC_OK;
 }
 
@@ -1397,15 +1427,15 @@ int ptc_add_material(ptc_ctx *ctx, const ptc_material_desc *desc, uint32_t *id)
     if (desc->type < PTC_LAMBERTIAN || desc->type > PTC_PASSTHROUGH) { CTX_FAIL(ctx, PTC_ERR_INVALID, "Unimplemented material type %d", desc->type); }
     if (desc->albedo_kind == PTC_ALBEDO_TEXTURE) {
         if (desc->type != PTC_LAMBERTIAN && desc->type != PTC_PLASTIC) { CTX_FAIL(ctx, PTC_ERR_INVALID, "only Lambertian and Plastic take a texture (src/scene_parser.cpp:625-647)"); }
-        if (desc->texture >= ctx->textures.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "texture id %u out of range", desc->texture); }
+        if (desc->texture >= ctx->staged.textures.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "texture id %u out of range", desc->texture); }
     } else if (desc->albedo_kind != PTC_ALBEDO_CONSTANT && desc->albedo_kind != PTC_ALBEDO_CHECKERBOARD) {
         CTX_FAIL(ctx, PTC_ERR_INVALID, "Unimplemented albedo kind %d", desc->albedo_kind);
     }
     if ((desc->type == PTC_MICROFACET || desc->type == PTC_PLASTIC) && desc->distribution != PTC_BECKMANN && desc->distribution != PTC_GGX) {
         CTX_FAIL(ctx, PTC_ERR_INVALID, "Unimplemented distribution %d", desc->distribution);
     }
-    ctx->materials.push_back(*desc);
-    if (id) { *id = (uint32_t)ctx->materials.size() - 1; }
+    ctx->staged.materials.push_back(*desc);
+    if (id) { *id = (uint32_t)ctx->staged.materials.size() - 1; }
     return PTC_OK;
 }
 
@@ -1413,10 +1443,10 @@ int ptc_add_medium(ptc_ctx *ctx, const float sigmaT[3], const float sigmaS[3], u
 {
     if (!ctx || !sigmaT) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    ptc_ctx::HostMedium m;
+    Staging::HostMedium m;
     for (int c = 0; c < 3; c++) { m.sigmaT[c] = sigmaT[c]; m.sigmaS[c] = sigmaS ? sigmaS[c] : 0.f; }
-    ctx->media.push_back(m);
-    if (id) { *id = (uint32_t)ctx->media.size() - 1; }
+    ctx->staged.media.push_back(m);
+    if (id) { *id = (uint32_t)ctx->staged.media.size() - 1; }
     return PTC_OK;
 }
 
@@ -1424,9 +1454,9 @@ int ptc_set_internal_medium(ptc_ctx *ctx, uint32_t geom, uint32_t medium)
 {
     if (!ctx) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    if (geom >= ctx->rootGeometry.size() || ctx->geometries[ctx->rootGeometry[geom]].isInstance) { CTX_FAIL(ctx, PTC_ERR_INVALID, "geometry id %u out of range", geom); }
-    if (medium != PTC_NO_MEDIUM && medium >= ctx->media.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "medium id %u out of range", medium); }
-    ctx->geometries[ctx->rootGeometry[geom]].medium = medium == PTC_NO_MEDIUM ? -1 : (int32_t)medium;
+    if (geom >= ctx->staged.rootGeometry.size() || ctx->staged.geometries[ctx->staged.rootGeometry[geom]].isInstance) { CTX_FAIL(ctx, PTC_ERR_INVALID, "geometry id %u out of range", geom); }
+    if (medium != PTC_NO_MEDIUM && medium >= ctx->staged.media.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "medium id %u out of range", medium); }
+    ctx->staged.geometries[ctx->staged.rootGeometry[geom]].medium = medium == PTC_NO_MEDIUM ? -1 : (int32_t)medium;
     return PTC_OK;
 }
 
@@ -1434,18 +1464,18 @@ int ptc_set_integrator(ptc_ctx *ctx, int integrator)
 {
     if (!ctx) { return PTC_ERR_INVALID; }
     if (integrator != PTC_INTEGRATOR_PATH_TRACER && integrator != PTC_INTEGRATOR_VOLUME_PATH_TRACER) { CTX_FAIL(ctx, PTC_ERR_INVALID, "Unimplemented integrator %d", integrator); }
-    ctx->integrator = integrator;
+    ctx->options.integrator = integrator;
     return PTC_OK;
 }
 
 // rtcAttachGeometry: the next geometry id of the scene being described
 static uint32_t attachGeometry(ptc_ctx *ctx, HostGeometry &g)
 {
-    g.scene = ctx->sceneStack.empty() ? 0u : ctx->sceneStack.back();
-    g.localId = ctx->scenes[g.scene].nGeoms++;
-    ctx->scenes[g.scene].members.push_back((uint32_t)ctx->geometries.size());
-    if (g.scene == 0) { ctx->rootGeometry.push_back((uint32_t)ctx->geometries.size()); }
-    ctx->geometries.push_back(g);
+    g.scene = ctx->staged.sceneStack.empty() ? 0u : ctx->staged.sceneStack.back();
+    g.localId = ctx->staged.scenes[g.scene].nGeoms++;
+    ctx->staged.scenes[g.scene].members.push_back((uint32_t)ctx->staged.geometries.size());
+    if (g.scene == 0) { ctx->staged.rootGeometry.push_back((uint32_t)ctx->staged.geometries.size()); }
+    ctx->staged.geometries.push_back(g);
     return g.localId;
 }
 
@@ -1453,10 +1483,10 @@ int ptc_begin_instance(ptc_ctx *ctx, uint32_t *sceneOut)
 {
     if (!ctx) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    if (ctx->sceneStack.size() >= 8) { CTX_FAIL(ctx, PTC_ERR_INVALID, "instance definitions nested too deeply"); }
-    ctx->scenes.push_back(HostScene());
-    ctx->sceneStack.push_back((uint32_t)ctx->scenes.size() - 1);
-    if (sceneOut) { *sceneOut = ctx->sceneStack.back(); }
+    if (ctx->staged.sceneStack.size() >= 8) { CTX_FAIL(ctx, PTC_ERR_INVALID, "instance definitions nested too deeply"); }
+    ctx->staged.scenes.push_back(HostScene());
+    ctx->staged.sceneStack.push_back((uint32_t)ctx->staged.scenes.size() - 1);
+    if (sceneOut) { *sceneOut = ctx->staged.sceneStack.back(); }
     return PTC_OK;
 }
 
@@ -1464,8 +1494,8 @@ int ptc_end_instance(ptc_ctx *ctx)
 {
     if (!ctx) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    if (ctx->sceneStack.empty()) { CTX_FAIL(ctx, PTC_ERR_STATE, "ptc_end_instance without ptc_begin_instance"); }
-    ctx->sceneStack.pop_back();
+    if (ctx->staged.sceneStack.empty()) { CTX_FAIL(ctx, PTC_ERR_STATE, "ptc_end_instance without ptc_begin_instance"); }
+    ctx->staged.sceneStack.pop_back();
     return PTC_OK;
 }
 
@@ -1495,8 +1525,8 @@ int ptc_add_instance(ptc_ctx *ctx, uint32_t scene, const float m[16], uint32_t *
 {
     if (!ctx || !m) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    if (scene == 0 || scene >= ctx->scenes.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "unknown instance scene %u", scene); }
-    for (uint32_t open : ctx->sceneStack) { if (open == scene) { CTX_FAIL(ctx, PTC_ERR_INVALID, "an instance scene cannot contain itself"); } }
+    if (scene == 0 || scene >= ctx->staged.scenes.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "unknown instance scene %u", scene); }
+    for (uint32_t open : ctx->staged.sceneStack) { if (open == scene) { CTX_FAIL(ctx, PTC_ERR_INVALID, "an instance scene cannot contain itself"); } }
     HostGeometry g;
     g.isInstance = true; g.instanceScene = scene;
     for (int row = 0; row < 3; row++) { for (int col = 0; col < 4; col++) { g.l2w[4 * row + col] = m[4 * col + row]; } } // RTC_FORMAT_FLOAT4X4_COLUMN_MAJOR
@@ -1512,25 +1542,25 @@ int ptc_add_triangle_mesh(ptc_ctx *ctx, const float *P, const float *N, const fl
     if (!ctx || (nv && !P) || (nt && (!I || !mat))) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
     for (uint32_t t = 0; t < nt; t++) {
-        if (mat[t] >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id %u out of range", mat[t]); }
+        if (mat[t] >= ctx->staged.materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id %u out of range", mat[t]); }
         for (int k = 0; k < 3; k++) { if (I[3 * (size_t)t + k] >= nv) { CTX_FAIL(ctx, PTC_ERR_INVALID, "vertex index out of range in triangle %u", t); } }
     }
     HostGeometry g;
-    g.firstVertex = (uint32_t)(ctx->positions4.size() / 4);
+    g.firstVertex = (uint32_t)(ctx->staged.positions4.size() / 4);
     g.nVertices = nv;
-    g.firstPrim = (uint32_t)(ctx->prims4.size() / 4);
+    g.firstPrim = (uint32_t)(ctx->staged.prims4.size() / 4);
     g.nPrims = nt;
-    const uint32_t geom = ctx->scenes[ctx->sceneStack.empty() ? 0u : ctx->sceneStack.back()].nGeoms; // the id attachGeometry hands out below
+    const uint32_t geom = ctx->staged.scenes[ctx->staged.sceneStack.empty() ? 0u : ctx->staged.sceneStack.back()].nGeoms; // the id attachGeometry hands out below
     for (uint32_t v = 0; v < nv; v++) {
-        ctx->positions4.insert(ctx->positions4.end(), {P[3 * (size_t)v], P[3 * (size_t)v + 1], P[3 * (size_t)v + 2], 0.f});
-        if (N) { ctx->normals4.insert(ctx->normals4.end(), {N[3 * (size_t)v], N[3 * (size_t)v + 1], N[3 * (size_t)v + 2], 0.f}); }
-        else { ctx->normals4.insert(ctx->normals4.end(), {0.f, 0.f, 0.f, 0.f}); }
-        if (UV) { ctx->uvs2.insert(ctx->uvs2.end(), {UV[2 * (size_t)v], UV[2 * (size_t)v + 1]}); }
-        else { ctx->uvs2.insert(ctx->uvs2.end(), {0.f, 0.f}); }
+        ctx->staged.positions4.insert(ctx->staged.positions4.end(), {P[3 * (size_t)v], P[3 * (size_t)v + 1], P[3 * (size_t)v + 2], 0.f});
+        if (N) { ctx->staged.normals4.insert(ctx->staged.normals4.end(), {N[3 * (size_t)v], N[3 * (size_t)v + 1], N[3 * (size_t)v + 2], 0.f}); }
+        else { ctx->staged.normals4.insert(ctx->staged.normals4.end(), {0.f, 0.f, 0.f, 0.f}); }
+        if (UV) { ctx->staged.uvs2.insert(ctx->staged.uvs2.end(), {UV[2 * (size_t)v], UV[2 * (size_t)v + 1]}); }
+        else { ctx->staged.uvs2.insert(ctx->staged.uvs2.end(), {0.f, 0.f}); }
     }
     for (uint32_t t = 0; t < nt; t++) {
-        ctx->prims4.insert(ctx->prims4.end(), {I[3 * (size_t)t] + g.firstVertex, I[3 * (size_t)t + 1] + g.firstVertex, I[3 * (size_t)t + 2] + g.firstVertex, mat[t]});
-        ctx->primIds2.insert(ctx->primIds2.end(), {geom, t});
+        ctx->staged.prims4.insert(ctx->staged.prims4.end(), {I[3 * (size_t)t] + g.firstVertex, I[3 * (size_t)t + 1] + g.firstVertex, I[3 * (size_t)t + 2] + g.firstVertex, mat[t]});
+        ctx->staged.primIds2.insert(ctx->staged.primIds2.end(), {geom, t});
     }
     attachGeometry(ctx, g);
     if (geomId) { *geomId = geom; }
@@ -1541,8 +1571,8 @@ int ptc_add_sphere(ptc_ctx *ctx, const float cr[4], uint32_t material, uint32_t 
 {
     if (!ctx || !cr) { return PTC_ERR_INVALID; }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    if (material >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id %u out of range", material); }
-    if (!ctx->sceneStack.empty()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "only triangle meshes can be instanced (src/sphere.cpp:46 attaches spheres to the global scene)"); }
+    if (material >= ctx->staged.materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id %u out of range", material); }
+    if (!ctx->staged.sceneStack.empty()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "only triangle meshes can be instanced (src/sphere.cpp:46 attaches spheres to the global scene)"); }
     HostGeometry g;
     g.isSphere = true; g.nPrims = 1; memcpy(g.centerRadius, cr, sizeof(g.centerRadius)); g.sphereMaterial = material;
     const uint32_t id = attachGeometry(ctx, g);
@@ -1555,10 +1585,10 @@ int ptc_set_environment(ptc_ctx *ctx, const float *rgba, int w, int h, float sca
     if (!ctx || !rgba || w <= 0 || h <= 0 || !m2w || !w2m) { return PTC_ERR_INVALID; }
     if (w > 65535 || h > 65535) { CTX_FAIL(ctx, PTC_ERR_INVALID, "environment map larger than 65535 texels on a side"); }
     if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    ctx->envRgba.assign(rgba, rgba + (size_t)w * h * 4);
-    ctx->envW = w; ctx->envH = h; ctx->envScale = scale;
-    memcpy(ctx->envM2W, m2w, sizeof(ctx->envM2W)); memcpy(ctx->envW2M, w2m, sizeof(ctx->envW2M));
-    ctx->hasEnv = true;
+    ctx->staged.envRgba.assign(rgba, rgba + (size_t)w * h * 4);
+    ctx->staged.envW = w; ctx->staged.envH = h; ctx->staged.envScale = scale;
+    memcpy(ctx->staged.envM2W, m2w, sizeof(ctx->staged.envM2W)); memcpy(ctx->staged.envW2M, w2m, sizeof(ctx->staged.envW2M));
+    ctx->staged.hasEnv = true;
     return PTC_OK;
 }
 
@@ -1575,12 +1605,9 @@ int ptc_set_camera(ptc_ctx *ctx, const float o[3], const float t[3], const float
     norm(up, upn); crossp(upn, dir, xr); norm(xr, xa); crossp(dir, xa, ya);
     const float sign = flip ? -1.f : 1.f;
     const float m[12] = {sign * xa[0], ya[0], dir[0], o[0], sign * xa[1], ya[1], dir[1], o[1], sign * xa[2], ya[2], dir[2], o[2]};
-    memcpy(ctx->camToWorld, m, sizeof(m));
-    ctx->vfov = vfov; ctx->width = w; ctx->height = h; ctx->hasCamera = true;
-    if (ctx->committed) { // the camera may be re-aimed after commit
-        memcpy(ctx->scene.camToWorld, m, sizeof(m));
-        ctx->scene.vfov = vfov; ctx->scene.width = w; ctx->scene.height = h;
-    }
+    DScene &s = ctx->scene.view; // the camera may be re-aimed after commit
+    memcpy(s.camToWorld, m, sizeof(m));
+    s.vfov = vfov; s.width = w; s.height = h; ctx->hasCamera = true;
     return PTC_OK;
 }
 
@@ -1613,170 +1640,148 @@ static bool buildCdf(const float *values, int n, float *cdf)
     return false;
 }
 
-int ptc_commit(ptc_ctx *ctx)
+// SURVEY 8(f) N4.  180 GB of HBM make flattening the B200-native form of Embree's two-level instancing: every placement of an
+// instance scene becomes world-space boxes of the ONE wide BVH (single-level traversal, no second stack).  The leaf triangles
+// keep the instance's LOCAL-space corners and the traversal moves the ray into the placement's space for the triangle test only
+// (traverse.cuh: rayToPlacement -- Embree's own arithmetic, so t, u, v round as they do in the reference), and everything
+// Scene::testIntersect reads after the hit -- Ng, vertex normals, uvs, the emitter triangle's corners -- stays in LOCAL space as
+// well, exactly as the reference leaves it (src/scene.cpp:122-219 never transforms back).
+// flat prim = one triangle of the BVH: (local vertex ids, material) | (geomID, primID inside its scene) | (instID[0], instID[1])
+struct Flattened {
+    std::vector<uint32_t> prims4, ids2, inst2, worldPrims4, tags;
+    std::vector<float> worldPos4, placements; // placements: per flattened placement, world-to-local rows of the outer, then of the inner level
+};
+static const float identity3x4[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
+// Adds the triangles of `scene` placed by T; returns an error message, or null
+static const char *flatten(const Staging &st, Flattened &f, uint32_t scene, const float *T, uint32_t inst0, uint32_t inst1, int level,
+                           const float *outerW2L, const float *innerW2L)
 {
-    if (!ctx) { return PTC_ERR_INVALID; }
-    if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
-    if (!ctx->hasCamera) { CTX_FAIL(ctx, PTC_ERR_STATE, "no camera set"); }
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    DScene &s = ctx->scene;
-    if (!ctx->sceneStack.empty()) { CTX_FAIL(ctx, PTC_ERR_STATE, "ptc_begin_instance without ptc_end_instance"); }
-    const bool instanced = ctx->scenes.size() > 1;
-    if (instanced && !ctx->media.empty()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "instancing together with participating media is not supported"); }
-
-    // SURVEY 8(f) N4.  180 GB of HBM make flattening the B200-native form of Embree's two-level instancing: every placement of an
-    // instance scene becomes world-space boxes of the ONE wide BVH (single-level traversal, no second stack).  The leaf triangles
-    // keep the instance's LOCAL-space corners and the traversal moves the ray into the placement's space for the triangle test only
-    // (traverse.cuh: rayToPlacement -- Embree's own arithmetic, so t, u, v round as they do in the reference), and everything
-    // Scene::testIntersect reads after the hit -- Ng, vertex normals, uvs, the emitter triangle's corners -- stays in LOCAL space as
-    // well, exactly as the reference leaves it (src/scene.cpp:122-219 never transforms back).
-    // flat prim = one triangle of the BVH: (local vertex ids, material) | (geomID, primID inside its scene) | (instID[0], instID[1])
-    std::vector<uint32_t> flatPrims4, flatIds2, flatInst2, worldPrims4, flatTag;
-    std::vector<float> worldPos4;
-    std::vector<float> placements; // per flattened placement: world-to-local rows of the outer, then of the inner level
-    if (instanced) {
-        struct Expand {
-            ptc_ctx *ctx; std::vector<uint32_t> &flatPrims4, &flatIds2, &flatInst2, &worldPrims4, &flatTag; std::vector<float> &worldPos4, &placements; std::string error;
-            void run(uint32_t scene, const float *T, uint32_t inst0, uint32_t inst1, int level, const float *outerW2L = nullptr, const float *innerW2L = nullptr)
-            {
-                uint32_t tag = 0; // what the leaf triangles of this placement carry (0: root-scene geometry, tested in world space)
-                if (level > 0) {
-                    static const float identity[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
-                    placements.insert(placements.end(), outerW2L, outerW2L + 12);
-                    placements.insert(placements.end(), innerW2L ? innerW2L : identity, (innerW2L ? innerW2L : identity) + 12);
-                    tag = (uint32_t)(placements.size() / 24) | (level == 2 ? 0x80000000u : 0u);
-                }
-                for (uint32_t index : ctx->scenes[scene].members) {
-                    const HostGeometry &g = ctx->geometries[index];
-                    if (g.isSphere) { continue; }
-                    if (g.isInstance) {
-                        if (level >= 2) { error = "more than RTC_MAX_INSTANCE_LEVEL_COUNT = 2 instance levels"; return; }
-                        float C[12]; // T o g.l2w: the inner placement is applied first
-                        for (int r = 0; r < 3; r++) {
-                            for (int c = 0; c < 4; c++) {
-                                C[4 * r + c] = T[4 * r] * g.l2w[c] + T[4 * r + 1] * g.l2w[4 + c] + T[4 * r + 2] * g.l2w[8 + c] + (c == 3 ? T[4 * r + 3] : 0.f);
-                            }
-                        }
-                        run(g.instanceScene, C, level == 0 ? g.localId : inst0, level == 0 ? PTC_INVALID_ID : g.localId, level + 1,
-                            level == 0 ? g.w2l : outerW2L, level == 0 ? nullptr : g.w2l);
-                        if (!error.empty()) { return; }
-                        continue;
-                    }
-                    const uint32_t base = (uint32_t)(worldPos4.size() / 4);
-                    for (uint32_t v = 0; v < g.nVertices; v++) {
-                        const float *q = &ctx->positions4[4 * (size_t)(g.firstVertex + v)];
-                        worldPos4.insert(worldPos4.end(), {T[0] * q[0] + T[1] * q[1] + T[2] * q[2] + T[3], T[4] * q[0] + T[5] * q[1] + T[6] * q[2] + T[7],
-                                                           T[8] * q[0] + T[9] * q[1] + T[10] * q[2] + T[11], 0.f});
-                    }
-                    for (uint32_t t = 0; t < g.nPrims; t++) {
-                        const uint32_t *ix = &ctx->prims4[4 * (size_t)(g.firstPrim + t)];
-                        flatPrims4.insert(flatPrims4.end(), ix, ix + 4);
-                        worldPrims4.insert(worldPrims4.end(), {ix[0] - g.firstVertex + base, ix[1] - g.firstVertex + base, ix[2] - g.firstVertex + base, ix[3]});
-                        flatIds2.insert(flatIds2.end(), {g.localId, t});
-                        flatInst2.insert(flatInst2.end(), {inst0, inst1});
-                        flatTag.push_back(tag);
-                    }
-                }
-            }
-        } expand{ctx, flatPrims4, flatIds2, flatInst2, worldPrims4, flatTag, worldPos4, placements, std::string()};
-        const float identity[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};
-        expand.run(0, identity, PTC_INVALID_ID, PTC_INVALID_ID, 0);
-        if (!expand.error.empty()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "%s", expand.error.c_str()); }
+    uint32_t tag = 0; // what the leaf triangles of this placement carry (0: root-scene geometry, tested in world space)
+    if (level > 0) {
+        f.placements.insert(f.placements.end(), outerW2L, outerW2L + 12);
+        f.placements.insert(f.placements.end(), innerW2L ? innerW2L : identity3x4, (innerW2L ? innerW2L : identity3x4) + 12);
+        tag = (uint32_t)(f.placements.size() / 24) | (level == 2 ? 0x80000000u : 0u);
     }
-    const std::vector<uint32_t> &prims4 = instanced ? flatPrims4 : ctx->prims4;
-    const std::vector<uint32_t> &primIds2 = instanced ? flatIds2 : ctx->primIds2;
-    const uint32_t nPrims = (uint32_t)(prims4.size() / 4);
-
-    // rtcCommitScene: BVH over all triangle geometries; spheres are kept in a flat list.  The geometry goes to the device first:
-    // the default builder runs there (option "bvh_builder" = 0 selects the host binned-SAH builder instead).
-    int rc;
-    if ((rc = upload(ctx, (const float4 *)ctx->positions4.data(), ctx->positions4.size() / 4, &s.positions))) { return rc; }
-    if ((rc = upload(ctx, (const uint4 *)prims4.data(), prims4.size() / 4, &s.prims))) { return rc; }
-    const float4 *buildPositions = s.positions; const uint4 *buildPrims = s.prims; // what the BVH is built over: world-space triangles
-    const std::vector<float> &hostBuildPositions = instanced ? worldPos4 : ctx->positions4;
-    const std::vector<uint32_t> &hostBuildPrims = instanced ? worldPrims4 : ctx->prims4;
-    if (instanced) {
-        if ((rc = upload(ctx, (const float4 *)worldPos4.data(), worldPos4.size() / 4, &buildPositions))) { return rc; }
-        if ((rc = upload(ctx, (const uint4 *)worldPrims4.data(), worldPrims4.size() / 4, &buildPrims))) { return rc; }
-        s.instIds = nullptr;
-        if ((rc = upload(ctx, (const uint2 *)flatInst2.data(), flatInst2.size() / 2, &s.instIds))) { return rc; }
-    } else { s.instIds = nullptr; }
-    {
-        const auto buildStart = std::chrono::steady_clock::now();
-        try {
-            if (ctx->bvhBuilder == 1) {
-                DeviceWideBVH built;
-                void *workspace = nullptr;
-                ctx->buildWorkspace = Buffer<uint8_t>(); // an earlier build's working set goes before this build allocates its own
-                buildWideBVHDevice(buildPositions, buildPrims, nPrims, ctx->stream, built, &workspace);
-                ctx->buildWorkspace = Buffer<uint8_t>((uint8_t *)workspace, 0); // the builder does not report its size
-                if (built.nodes) { ctx->allocations.emplace_back((uint8_t *)built.nodes, (size_t)built.nNodes * sizeof(WideNode)); }
-                if (built.triangles) { ctx->allocations.emplace_back((uint8_t *)built.triangles, (size_t)built.nTriangles * sizeof(LeafTriangle)); }
-                s.bvh.nodes = built.nodes; s.bvh.triangles = built.triangles; s.bvh.nNodes = built.nNodes;
-                ctx->bvhPlocIterations = built.plocIterations;
-                // no host copy here (49 MB through pageable memory cost more than the build): fetchHostBvh brings it when
-                // the scalar counting traversal asks for it
-                ctx->bvh.nodes.clear(); ctx->bvh.triangles.clear(); ctx->bvh.maxDepth = built.maxDepth;
-                ctx->bvhNodeCount = built.nNodes; ctx->bvhTriangleCount = built.nTriangles; ctx->hostBvhFetched = false;
-            } else {
-                buildWideBVH(hostBuildPositions.data(), hostBuildPrims.data(), nPrims, ctx->bvh);
-                if ((rc = upload(ctx, (const float4 *)ctx->bvh.nodes.data(), ctx->bvh.nodes.size() * 5, &s.bvh.nodes))) { return rc; }
-                if ((rc = upload(ctx, (const float4 *)ctx->bvh.triangles.data(), ctx->bvh.triangles.size() * 3, &s.bvh.triangles))) { return rc; }
-                s.bvh.nNodes = (uint32_t)ctx->bvh.nodes.size();
-                ctx->bvhNodeCount = (uint32_t)ctx->bvh.nodes.size(); ctx->bvhTriangleCount = (uint32_t)ctx->bvh.triangles.size(); ctx->hostBvhFetched = true;
+    for (uint32_t index : st.scenes[scene].members) {
+        const HostGeometry &g = st.geometries[index];
+        if (g.isSphere) { continue; }
+        if (g.isInstance) {
+            if (level >= 2) { return "more than RTC_MAX_INSTANCE_LEVEL_COUNT = 2 instance levels"; }
+            float C[12]; // T o g.l2w: the inner placement is applied first
+            for (int r = 0; r < 3; r++) {
+                for (int c = 0; c < 4; c++) {
+                    C[4 * r + c] = T[4 * r] * g.l2w[c] + T[4 * r + 1] * g.l2w[4 + c] + T[4 * r + 2] * g.l2w[8 + c] + (c == 3 ? T[4 * r + 3] : 0.f);
+                }
             }
-        } catch (const std::exception &e) { CTX_FAIL(ctx, PTC_ERR_INVALID, "BVH build failed: %s", e.what()); }
-        s.bvh.placements = nullptr;
-        ctx->bvh.placements = placements;
-        if (!placements.empty() && ctx->bvhTriangleCount) {
-            const uint32_t *tags = nullptr;
-            if ((rc = upload(ctx, flatTag.data(), flatTag.size(), &tags))) { return rc; }
-            if ((rc = upload(ctx, (const float4 *)placements.data(), placements.size() / 4, &s.bvh.placements))) { return rc; }
-            const uint32_t nTriangles = ctx->bvhTriangleCount;
-            LeafTriangle *leaves = (LeafTriangle *)s.bvh.triangles;
-            localizeLeavesKernel<<<(nTriangles + 255) / 256, 256, 0, ctx->stream>>>(leaves, nTriangles, s.positions, s.prims, tags);
-            CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-            ctx->bvh.nodes.clear(); ctx->bvh.triangles.clear(); ctx->hostBvhFetched = false; // the leaves changed on the device
+            const char *error = flatten(st, f, g.instanceScene, C, level == 0 ? g.localId : inst0, level == 0 ? PTC_INVALID_ID : g.localId, level + 1,
+                                        level == 0 ? g.w2l : outerW2L, level == 0 ? nullptr : g.w2l);
+            if (error) { return error; }
+            continue;
         }
-        ctx->bvhBuildMs = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - buildStart).count();
+        const uint32_t base = (uint32_t)(f.worldPos4.size() / 4);
+        for (uint32_t v = 0; v < g.nVertices; v++) {
+            const float *q = &st.positions4[4 * (size_t)(g.firstVertex + v)];
+            f.worldPos4.insert(f.worldPos4.end(), {T[0] * q[0] + T[1] * q[1] + T[2] * q[2] + T[3], T[4] * q[0] + T[5] * q[1] + T[6] * q[2] + T[7],
+                                                   T[8] * q[0] + T[9] * q[1] + T[10] * q[2] + T[11], 0.f});
+        }
+        for (uint32_t t = 0; t < g.nPrims; t++) {
+            const uint32_t *ix = &st.prims4[4 * (size_t)(g.firstPrim + t)];
+            f.prims4.insert(f.prims4.end(), ix, ix + 4);
+            f.worldPrims4.insert(f.worldPrims4.end(), {ix[0] - g.firstVertex + base, ix[1] - g.firstVertex + base, ix[2] - g.firstVertex + base, ix[3]});
+            f.ids2.insert(f.ids2.end(), {g.localId, t});
+            f.inst2.insert(f.inst2.end(), {inst0, inst1});
+            f.tags.push_back(tag);
+        }
     }
+    return nullptr;
+}
 
-    // textures: packed texels per image, one gamma table for all (Texture::lookup's powf(c / 255.f, 2.2f), src/texture.cpp:44-48)
-    std::vector<const uint32_t *> deviceTexels(ctx->textures.size(), nullptr);
-    for (size_t t = 0; t < ctx->textures.size(); t++) {
-        const int rcTex = upload(ctx, ctx->textures[t].texels.data(), ctx->textures[t].texels.size(), &deviceTexels[t]);
-        if (rcTex) { return rcTex; }
+// rtcCommitScene: BVH over all triangle geometries; spheres are kept in a flat list.  The geometry goes to the device first:
+// the default builder runs there (option "bvh_builder" = 0 selects the host binned-SAH builder instead).  An instanced scene is
+// built over world-space copies of its triangles (`buildInputs`) whose leaves are then moved back to local space.
+static int buildBvh(ptc_ctx *ctx, const Flattened *flat, const std::vector<uint32_t> &prims4, Committed &c, std::vector<SceneAllocation> &buildInputs)
+{
+    const Staging &st = ctx->staged; DScene &s = c.view;
+    const uint32_t nPrims = (uint32_t)(prims4.size() / 4);
+    TRY(upload(ctx, c, (const float4 *)st.positions4.data(), st.positions4.size() / 4, s.positions));
+    TRY(upload(ctx, c, (const uint4 *)prims4.data(), prims4.size() / 4, s.prims));
+    const float4 *buildPositions = s.positions; const uint4 *buildPrims = s.prims; // what the BVH is built over: world-space triangles
+    if (flat) {
+        TRY(upload(ctx, buildInputs, (const float4 *)flat->worldPos4.data(), flat->worldPos4.size() / 4, &buildPositions));
+        TRY(upload(ctx, buildInputs, (const uint4 *)flat->worldPrims4.data(), flat->worldPrims4.size() / 4, &buildPrims));
+        TRY(upload(ctx, c, (const uint2 *)flat->inst2.data(), flat->inst2.size() / 2, s.instIds));
     }
-    {
-        float gamma[256];
-        for (int c = 0; c < 256; c++) { gamma[c] = powf(c / 255.f, 2.2f); }
-        CUDA_TRY(ctx, cudaMemcpyToSymbol(c_gammaTable, gamma, sizeof(gamma)));
+    const auto buildStart = std::chrono::steady_clock::now();
+    try {
+        if (ctx->options.bvhBuilder == 1) {
+            DeviceWideBVH built; void *workspace = nullptr;
+            buildWideBVHDevice(buildPositions, buildPrims, nPrims, ctx->stream, built, &workspace);
+            c.buildWorkspace = Buffer<uint8_t>((uint8_t *)workspace, 0); // the builder does not report its size
+            s.bvh.nodes = built.nodes; s.bvh.triangles = built.triangles; s.bvh.nNodes = built.nNodes;
+            if (built.nodes) { c.allocations.push_back({Buffer<uint8_t>((uint8_t *)built.nodes, (size_t)built.nNodes * sizeof(WideNode)), fieldOf(s, &s.bvh.nodes), {}}); }
+            if (built.triangles) { c.allocations.push_back({Buffer<uint8_t>((uint8_t *)built.triangles, (size_t)built.nTriangles * sizeof(LeafTriangle)), fieldOf(s, &s.bvh.triangles), {}}); }
+            c.bvhTriangles = built.nTriangles; c.bvhDepth = built.maxDepth; c.bvhPlocIterations = built.plocIterations;
+        } else {
+            WideBVH bvh;
+            buildWideBVH((flat ? flat->worldPos4 : st.positions4).data(), (flat ? flat->worldPrims4 : st.prims4).data(), nPrims, bvh);
+            TRY(upload(ctx, c, (const float4 *)bvh.nodes.data(), bvh.nodes.size() * 5, s.bvh.nodes));
+            TRY(upload(ctx, c, (const float4 *)bvh.triangles.data(), bvh.triangles.size() * 3, s.bvh.triangles));
+            s.bvh.nNodes = (uint32_t)bvh.nodes.size(); c.bvhTriangles = (uint32_t)bvh.triangles.size(); c.bvhDepth = bvh.maxDepth;
+        }
+    } catch (const std::exception &e) { CTX_FAIL(ctx, PTC_ERR_INVALID, "BVH build failed: %s", e.what()); }
+    if (flat) { c.placements = flat->placements; }
+    if (!c.placements.empty() && c.bvhTriangles) {
+        const uint32_t *tags = nullptr;
+        TRY(upload(ctx, buildInputs, flat->tags.data(), flat->tags.size(), &tags));
+        TRY(upload(ctx, c, (const float4 *)c.placements.data(), c.placements.size() / 4, s.bvh.placements));
+        localizeLeavesKernel<<<(c.bvhTriangles + 255) / 256, 256, 0, ctx->stream>>>((LeafTriangle *)s.bvh.triangles, c.bvhTriangles, s.positions, s.prims, tags);
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     }
+    c.bvhBuildMs = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - buildStart).count();
+    return PTC_OK;
+}
 
-    std::vector<DMaterial> dm(ctx->materials.size());
-    ctx->classMask = 0;
-    for (size_t i = 0; i < dm.size(); i++) {
-        const ptc_material_desc &d = ctx->materials[i];
-        DMaterial &m = dm[i];
-        ctx->classMask |= 1u << d.type;
-        memset(&m, 0, sizeof(m));
+// packed texels per image, in consecutive allocations
+static int uploadTextures(ptc_ctx *ctx, Committed &c)
+{
+    const uint32_t *texels;
+    for (const Staging::HostTexture &t : ctx->staged.textures) { TRY(upload(ctx, c.allocations, t.texels.data(), t.texels.size(), &texels)); }
+    return PTC_OK;
+}
+
+// the device material table (uploaded by uploadSurfaces) and the material classes present; texture t is c.allocations[firstTexture + t]
+static void materialTable(const Staging &st, size_t firstTexture, Committed &c)
+{
+    c.materials.resize(st.materials.size());
+    for (size_t i = 0; i < c.materials.size(); i++) {
+        const ptc_material_desc &d = st.materials[i];
+        DMaterial &m = c.materials[i]; // zeroed by resize
+        c.classMask |= 1u << d.type;
         m.type = d.type; m.distribution = d.distribution; m.albedoKind = d.albedo_kind;
         m.emitter = !(d.emit[0] == 0.f && d.emit[1] == 0.f && d.emit[2] == 0.f);
-        for (int c = 0; c < 3; c++) { m.diffuse[c] = d.diffuse[c]; m.emit[c] = d.emit[c]; m.on[c] = d.checker_on[c]; m.off[c] = d.checker_off[c]; }
+        for (int k = 0; k < 3; k++) { m.diffuse[k] = d.diffuse[k]; m.emit[k] = d.emit[k]; m.on[k] = d.checker_on[k]; m.off[k] = d.checker_off[k]; }
         const float sigma2 = d.sigma * d.sigma; // OrenNayar::OrenNayar, src/oren_nayar.cpp:11-19
         m.sigmaA = 1.f - (sigma2 / (2.f * (sigma2 + 0.33f)));
         m.sigmaB = (0.45f * sigma2) / (sigma2 + 0.09f);
         m.ior = d.ior; m.alpha = d.alpha; m.resU = d.checker_resolution[0]; m.resV = d.checker_resolution[1];
         if (d.albedo_kind == PTC_ALBEDO_TEXTURE) {
-            m.texW = ctx->textures[d.texture].width; m.texH = ctx->textures[d.texture].height; m.texels = deviceTexels[d.texture];
+            SceneAllocation &texels = c.allocations[firstTexture + d.texture];
+            m.texW = st.textures[d.texture].width; m.texH = st.textures[d.texture].height; m.texels = (const uint32_t *)texels.data.get();
+            texels.materials.push_back((uint32_t)i);
         }
     }
+}
 
-    // light table: emissive surfaces in registration order, environment light last (src/scene_parser.cpp:173-190)
+// the per-surface tables: lights and spheres, vertex attributes, triangle records, ids, the material table and class bytes
+static int uploadSurfaces(ptc_ctx *ctx, const std::vector<uint32_t> &prims4, const std::vector<uint32_t> &primIds2, Committed &c)
+{
+    const Staging &st = ctx->staged; DScene &s = c.view;
+    const std::vector<DMaterial> &dm = c.materials;
+    // light table: emissive surfaces in registration order, environment light last (src/scene_parser.cpp:173-190); the sphere list
     std::vector<DLight> lights;
     std::vector<float> spheres4; std::vector<uint32_t> sphereIds2;
-    for (uint32_t member : ctx->scenes[0].members) { // only root-scene surfaces become lights (src/scene_parser.cpp:173-182)
-        const HostGeometry &ge = ctx->geometries[member];
+    for (uint32_t member : st.scenes[0].members) { // only root-scene surfaces become lights (src/scene_parser.cpp:173-182)
+        const HostGeometry &ge = st.geometries[member];
         if (ge.isInstance) { continue; }
         if (ge.isSphere) {
             spheres4.insert(spheres4.end(), ge.centerRadius, ge.centerRadius + 4);
@@ -1790,117 +1795,149 @@ int ptc_commit(ptc_ctx *ctx)
             continue;
         }
         for (uint32_t p = ge.firstPrim; p < ge.firstPrim + ge.nPrims; p++) {
-            const uint32_t *ix = &ctx->prims4[4 * (size_t)p];
+            const uint32_t *ix = &st.prims4[4 * (size_t)p];
             if (!dm[ix[3]].emitter) { continue; }
             DLight l; memset(&l, 0, sizeof(l)); l.kind = 0;
             for (int c = 0; c < 3; c++) {
-                l.p0[c] = ctx->positions4[4 * (size_t)ix[0] + c]; l.p1[c] = ctx->positions4[4 * (size_t)ix[1] + c]; l.p2[c] = ctx->positions4[4 * (size_t)ix[2] + c];
+                l.p0[c] = st.positions4[4 * (size_t)ix[0] + c]; l.p1[c] = st.positions4[4 * (size_t)ix[1] + c]; l.p2[c] = st.positions4[4 * (size_t)ix[2] + c];
                 l.emit[c] = dm[ix[3]].emit[c];
             }
             lights.push_back(l);
         }
     }
-    if (ctx->hasEnv) { DLight l; memset(&l, 0, sizeof(l)); l.kind = 2; lights.push_back(l); }
-    ctx->nLights = (uint32_t)lights.size();
-
-    if ((rc = upload(ctx, (const float4 *)spheres4.data(), spheres4.size() / 4, &s.bvh.spheres))) { return rc; }
+    if (st.hasEnv) { DLight l; memset(&l, 0, sizeof(l)); l.kind = 2; lights.push_back(l); }
+    TRY(upload(ctx, c, (const float4 *)spheres4.data(), spheres4.size() / 4, s.bvh.spheres));
     s.bvh.nSpheres = (uint32_t)(spheres4.size() / 4);
-    if ((rc = upload(ctx, (const float4 *)ctx->normals4.data(), ctx->normals4.size() / 4, &s.normals))) { return rc; }
-    if ((rc = upload(ctx, (const float2 *)ctx->uvs2.data(), ctx->uvs2.size() / 2, &s.uvs))) { return rc; }
+    TRY(upload(ctx, c, (const float4 *)st.normals4.data(), st.normals4.size() / 4, s.normals));
+    TRY(upload(ctx, c, (const float2 *)st.uvs2.data(), st.uvs2.size() / 2, s.uvs));
+    const uint32_t nPrims = (uint32_t)(prims4.size() / 4);
     { // per-triangle shading records (shading.cuh: DScene::triShade); Ng = e2 x e1 with the fused multiply-subtracts of triangleNg
         std::vector<float> rec((size_t)nPrims * 20, 0.f);
         for (uint32_t p = 0; p < nPrims; p++) {
             const uint32_t *ix = &prims4[4 * (size_t)p];
-            const float *v0 = &ctx->positions4[4 * (size_t)ix[0]], *v1 = &ctx->positions4[4 * (size_t)ix[1]], *v2 = &ctx->positions4[4 * (size_t)ix[2]];
+            const float *v0 = &st.positions4[4 * (size_t)ix[0]], *v1 = &st.positions4[4 * (size_t)ix[1]], *v2 = &st.positions4[4 * (size_t)ix[2]];
             const float e1x = v0[0] - v1[0], e1y = v0[1] - v1[1], e1z = v0[2] - v1[2];
             const float e2x = v2[0] - v0[0], e2y = v2[1] - v0[1], e2z = v2[2] - v0[2];
             float *r = &rec[(size_t)p * 20];
             r[0] = fmaf(e2y, e1z, -(e2z * e1y)); r[1] = fmaf(e2z, e1x, -(e2x * e1z)); r[2] = fmaf(e2x, e1y, -(e2y * e1x));
             memcpy(&r[3], &ix[3], sizeof(float));
             for (int k = 0; k < 3; k++) {
-                const float *n = &ctx->normals4[4 * (size_t)ix[k]];
-                const float *t = &ctx->uvs2[2 * (size_t)ix[k]];
+                const float *n = &st.normals4[4 * (size_t)ix[k]];
+                const float *t = &st.uvs2[2 * (size_t)ix[k]];
                 r[4 + 3 * k] = n[0]; r[5 + 3 * k] = n[1]; r[6 + 3 * k] = n[2];
                 r[13 + 2 * k] = t[0]; r[14 + 2 * k] = t[1];
             }
         }
-        if ((rc = upload(ctx, (const float4 *)rec.data(), rec.size() / 4, &s.triShade))) { return rc; }
+        TRY(upload(ctx, c, (const float4 *)rec.data(), rec.size() / 4, s.triShade));
     }
-    if ((rc = upload(ctx, (const uint2 *)primIds2.data(), primIds2.size() / 2, &s.primIds))) { return rc; }
-    if ((rc = upload(ctx, (const uint2 *)sphereIds2.data(), sphereIds2.size() / 2, &s.sphereIds))) { return rc; }
-    if ((rc = upload(ctx, dm.data(), dm.size(), &s.materials))) { return rc; }
-    ctx->deviceMaterials = dm;
-    { // one byte per primitive / sphere for the logic stage: material type | emitter << 3
-        std::vector<uint8_t> primClass(nPrims), sphereClass(sphereIds2.size() / 2);
-        for (uint32_t p = 0; p < nPrims; p++) { const DMaterial &m = dm[prims4[4 * (size_t)p + 3]]; primClass[p] = (uint8_t)(m.type | (m.emitter ? 8 : 0)); }
-        for (size_t i = 0; i < sphereClass.size(); i++) { const DMaterial &m = dm[sphereIds2[2 * i + 1]]; sphereClass[i] = (uint8_t)(m.type | (m.emitter ? 8 : 0)); }
-        if ((rc = upload(ctx, primClass.data(), primClass.size(), &s.primClass))) { return rc; }
-        if ((rc = upload(ctx, sphereClass.data(), sphereClass.size(), &s.sphereClass))) { return rc; }
-    }
-    if ((rc = upload(ctx, lights.data(), lights.size(), &s.lights))) { return rc; }
-    s.nLights = ctx->nLights;
+    TRY(upload(ctx, c, (const uint2 *)primIds2.data(), primIds2.size() / 2, s.primIds));
+    TRY(upload(ctx, c, (const uint2 *)sphereIds2.data(), sphereIds2.size() / 2, s.sphereIds));
+    TRY(upload(ctx, c, dm.data(), dm.size(), s.materials));
+    // one byte per primitive / sphere for the logic stage: material type | emitter << 3
+    std::vector<uint8_t> primClass(nPrims), sphereClass(sphereIds2.size() / 2);
+    for (uint32_t p = 0; p < nPrims; p++) { const DMaterial &m = dm[prims4[4 * (size_t)p + 3]]; primClass[p] = (uint8_t)(m.type | (m.emitter ? 8 : 0)); }
+    for (size_t i = 0; i < sphereClass.size(); i++) { const DMaterial &m = dm[sphereIds2[2 * i + 1]]; sphereClass[i] = (uint8_t)(m.type | (m.emitter ? 8 : 0)); }
+    TRY(upload(ctx, c, primClass.data(), primClass.size(), s.primClass));
+    TRY(upload(ctx, c, sphereClass.data(), sphereClass.size(), s.sphereClass));
+    TRY(upload(ctx, c, lights.data(), lights.size(), s.lights));
+    s.nLights = (uint32_t)lights.size();
+    return PTC_OK;
+}
 
-    // participating media: sigma_t / sigma_s, the internal medium of every geometry, and the occlusion filter's table (a
-    // Passthrough surface that encloses a medium is not a hit for testOcclusion / the volumetric queries, src/scene.cpp:42-84)
-    s.nMedia = (int32_t)ctx->media.size(); s.hasFilter = 0;
-    s.media = nullptr; s.geomMedium = nullptr; s.bvh.primEvent = nullptr; s.bvh.sphereEvent = nullptr;
-    if (s.nMedia) {
-        std::vector<float> media4;
-        for (const ptc_ctx::HostMedium &m : ctx->media) { media4.insert(media4.end(), {m.sigmaT[0], m.sigmaT[1], m.sigmaT[2], 0.f, m.sigmaS[0], m.sigmaS[1], m.sigmaS[2], 0.f}); }
-        std::vector<int32_t> geomMedium(ctx->geometries.size()), primEvent(nPrims, -1), sphereEvent;
-        for (size_t g = 0; g < ctx->geometries.size(); g++) {
-            const HostGeometry &ge = ctx->geometries[g];
-            geomMedium[g] = ge.medium;
-            if (ge.isSphere) {
-                const bool filtered = ge.medium >= 0 && dm[ge.sphereMaterial].type == PTC_PASSTHROUGH;
-                sphereEvent.push_back(filtered ? ge.medium : -1);
-                if (filtered) { s.hasFilter = 1; }
-                continue;
-            }
-            if (ge.medium < 0) { continue; }
-            for (uint32_t p = ge.firstPrim; p < ge.firstPrim + ge.nPrims; p++) {
-                if (dm[ctx->prims4[4 * (size_t)p + 3]].type == PTC_PASSTHROUGH) { primEvent[p] = ge.medium; s.hasFilter = 1; }
-            }
+// participating media: sigma_t / sigma_s, the internal medium of every geometry, and the occlusion filter's table (a
+// Passthrough surface that encloses a medium is not a hit for testOcclusion / the volumetric queries, src/scene.cpp:42-84)
+static int uploadMedia(ptc_ctx *ctx, uint32_t nPrims, Committed &c)
+{
+    const Staging &st = ctx->staged; DScene &s = c.view;
+    s.nMedia = (int32_t)st.media.size();
+    if (!s.nMedia) { return PTC_OK; }
+    std::vector<float> media4;
+    for (const Staging::HostMedium &m : st.media) { media4.insert(media4.end(), {m.sigmaT[0], m.sigmaT[1], m.sigmaT[2], 0.f, m.sigmaS[0], m.sigmaS[1], m.sigmaS[2], 0.f}); }
+    std::vector<int32_t> geomMedium(st.geometries.size()), primEvent(nPrims, -1), sphereEvent;
+    for (size_t g = 0; g < st.geometries.size(); g++) {
+        const HostGeometry &ge = st.geometries[g];
+        geomMedium[g] = ge.medium;
+        if (ge.isSphere) {
+            const bool filtered = ge.medium >= 0 && c.materials[ge.sphereMaterial].type == PTC_PASSTHROUGH;
+            sphereEvent.push_back(filtered ? ge.medium : -1);
+            if (filtered) { s.hasFilter = 1; }
+            continue;
         }
-        if ((rc = upload(ctx, (const float4 *)media4.data(), media4.size() / 4, &s.media))) { return rc; }
-        if ((rc = upload(ctx, geomMedium.data(), geomMedium.size(), &s.geomMedium))) { return rc; }
-        if ((rc = upload(ctx, primEvent.data(), primEvent.size(), &s.bvh.primEvent))) { return rc; }
-        if ((rc = upload(ctx, sphereEvent.data(), sphereEvent.size(), &s.bvh.sphereEvent))) { return rc; }
+        if (ge.medium < 0) { continue; }
+        for (uint32_t p = ge.firstPrim; p < ge.firstPrim + ge.nPrims; p++) {
+            if (c.materials[st.prims4[4 * (size_t)p + 3]].type == PTC_PASSTHROUGH) { primEvent[p] = ge.medium; s.hasFilter = 1; }
+        }
     }
+    TRY(upload(ctx, c, (const float4 *)media4.data(), media4.size() / 4, s.media));
+    TRY(upload(ctx, c, geomMedium.data(), geomMedium.size(), s.geomMedium));
+    TRY(upload(ctx, c, primEvent.data(), primEvent.size(), s.bvh.primEvent));
+    return upload(ctx, c, sphereEvent.data(), sphereEvent.size(), s.bvh.sphereEvent);
+}
 
-    s.hasEnv = ctx->hasEnv ? 1 : 0;
-    if (ctx->hasEnv) {
-        // EnvironmentLight::EnvironmentLight, src/environment_light.cpp:29-53: weight = R+G+B, no sin(theta) (Q9)
-        const int w = ctx->envW, h = ctx->envH;
-        std::vector<float> row(w), theta(h), phiCdf((size_t)w * h), thetaCdf(h);
-        std::vector<uint8_t> phiEmpty(h);
-        for (int t = 0; t < h; t++) {
-            float thetaSum = 0.f;
-            for (int p = 0; p < w; p++) {
-                const float *px = &ctx->envRgba[4 * ((size_t)t * w + p)];
-                float value = 0.f;
-                value += px[0]; value += px[1]; value += px[2];
-                thetaSum += value; row[p] = value;
-            }
-            phiEmpty[t] = buildCdf(row.data(), w, &phiCdf[(size_t)t * w]) ? 1 : 0;
-            theta[t] = thetaSum;
+// EnvironmentLight::EnvironmentLight, src/environment_light.cpp:29-53: weight = R+G+B, no sin(theta) (Q9)
+static int uploadEnvironment(ptc_ctx *ctx, Committed &c)
+{
+    const Staging &st = ctx->staged; DScene &s = c.view;
+    s.hasEnv = st.hasEnv ? 1 : 0;
+    if (!st.hasEnv) { return PTC_OK; }
+    const int w = st.envW, h = st.envH;
+    std::vector<float> row(w), theta(h), phiCdf((size_t)w * h), thetaCdf(h);
+    std::vector<uint8_t> phiEmpty(h);
+    for (int t = 0; t < h; t++) {
+        float thetaSum = 0.f;
+        for (int p = 0; p < w; p++) {
+            const float *px = &st.envRgba[4 * ((size_t)t * w + p)];
+            float value = 0.f;
+            value += px[0]; value += px[1]; value += px[2];
+            thetaSum += value; row[p] = value;
         }
-        s.envThetaEmpty = buildCdf(theta.data(), h, thetaCdf.data()) ? 1 : 0;
-        s.envThetaG = guideSize(h); s.envPhiG = guideSize(w);
-        std::vector<uint16_t> thetaGuide((size_t)s.envThetaG + 1), phiGuide((size_t)h * (s.envPhiG + 1));
-        buildGuide(thetaCdf.data(), h, s.envThetaG, thetaGuide.data());
-        for (int t = 0; t < h; t++) { buildGuide(&phiCdf[(size_t)t * w], w, s.envPhiG, &phiGuide[(size_t)t * (s.envPhiG + 1)]); }
-        if ((rc = upload(ctx, thetaGuide.data(), thetaGuide.size(), &s.envThetaGuide))) { return rc; }
-        if ((rc = upload(ctx, phiGuide.data(), phiGuide.size(), &s.envPhiGuide))) { return rc; }
-        if ((rc = upload(ctx, (const float4 *)ctx->envRgba.data(), (size_t)w * h, &s.envRgba))) { return rc; }
-        if ((rc = upload(ctx, thetaCdf.data(), thetaCdf.size(), &s.envThetaCdf))) { return rc; }
-        if ((rc = upload(ctx, phiCdf.data(), phiCdf.size(), &s.envPhiCdf))) { return rc; }
-        if ((rc = upload(ctx, phiEmpty.data(), phiEmpty.size(), &s.envPhiEmpty))) { return rc; }
-        s.envW = w; s.envH = h; s.envScale = ctx->envScale;
-        for (int r = 0; r < 3; r++) { for (int c = 0; c < 4; c++) { s.envM2W[4 * r + c] = ctx->envM2W[4 * r + c]; s.envW2M[4 * r + c] = ctx->envW2M[4 * r + c]; } }
+        phiEmpty[t] = buildCdf(row.data(), w, &phiCdf[(size_t)t * w]) ? 1 : 0;
+        theta[t] = thetaSum;
     }
-    memcpy(s.camToWorld, ctx->camToWorld, sizeof(s.camToWorld));
-    s.vfov = ctx->vfov; s.width = ctx->width; s.height = ctx->height;
+    s.envThetaEmpty = buildCdf(theta.data(), h, thetaCdf.data()) ? 1 : 0;
+    s.envThetaG = guideSize(h); s.envPhiG = guideSize(w);
+    std::vector<uint16_t> thetaGuide((size_t)s.envThetaG + 1), phiGuide((size_t)h * (s.envPhiG + 1));
+    buildGuide(thetaCdf.data(), h, s.envThetaG, thetaGuide.data());
+    for (int t = 0; t < h; t++) { buildGuide(&phiCdf[(size_t)t * w], w, s.envPhiG, &phiGuide[(size_t)t * (s.envPhiG + 1)]); }
+    TRY(upload(ctx, c, thetaGuide.data(), thetaGuide.size(), s.envThetaGuide));
+    TRY(upload(ctx, c, phiGuide.data(), phiGuide.size(), s.envPhiGuide));
+    TRY(upload(ctx, c, (const float4 *)st.envRgba.data(), (size_t)w * h, s.envRgba));
+    TRY(upload(ctx, c, thetaCdf.data(), thetaCdf.size(), s.envThetaCdf));
+    TRY(upload(ctx, c, phiCdf.data(), phiCdf.size(), s.envPhiCdf));
+    TRY(upload(ctx, c, phiEmpty.data(), phiEmpty.size(), s.envPhiEmpty));
+    s.envW = w; s.envH = h; s.envScale = st.envScale;
+    memcpy(s.envM2W, st.envM2W, sizeof(s.envM2W)); memcpy(s.envW2M, st.envW2M, sizeof(s.envW2M)); // the 3 x 4 rows
+    return PTC_OK;
+}
+
+// The staged scene becomes a Committed value step by step; the context takes it, and releases the staging, only when every step
+// succeeded, so a failed commit leaves no allocation behind
+int ptc_commit(ptc_ctx *ctx)
+{
+    if (!ctx) { return PTC_ERR_INVALID; }
+    if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene already committed"); }
+    if (!ctx->hasCamera) { CTX_FAIL(ctx, PTC_ERR_STATE, "no camera set"); }
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    const Staging &st = ctx->staged;
+    if (!st.sceneStack.empty()) { CTX_FAIL(ctx, PTC_ERR_STATE, "ptc_begin_instance without ptc_end_instance"); }
+    const bool instanced = st.scenes.size() > 1;
+    if (instanced && !st.media.empty()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "instancing together with participating media is not supported"); }
+
+    Flattened flat;
+    if (const char *error = instanced ? flatten(st, flat, 0, identity3x4, PTC_INVALID_ID, PTC_INVALID_ID, 0, nullptr, nullptr) : nullptr) { CTX_FAIL(ctx, PTC_ERR_INVALID, "%s", error); }
+    const std::vector<uint32_t> &prims4 = instanced ? flat.prims4 : st.prims4, &primIds2 = instanced ? flat.ids2 : st.primIds2;
+    Committed c; c.view = ctx->scene.view; // the camera
+    std::vector<SceneAllocation> buildInputs; // released when the commit returns
+    TRY(buildBvh(ctx, instanced ? &flat : nullptr, prims4, c, buildInputs));
+    const size_t firstTexture = c.allocations.size();
+    TRY(uploadTextures(ctx, c));
+    CUDA_TRY(ctx, uploadGammaTable());
+    materialTable(st, firstTexture, c);
+    TRY(uploadSurfaces(ctx, prims4, primIds2, c));
+    TRY(uploadMedia(ctx, (uint32_t)(prims4.size() / 4), c));
+    TRY(uploadEnvironment(ctx, c));
+    ctx->scene = std::move(c);
+    ctx->staged = Staging();
     ctx->committed = true;
     return PTC_OK;
 }
@@ -1909,19 +1946,7 @@ int ptc_commit(ptc_ctx *ctx)
 
 // SURVEY 8(e): the scene is parsed, fed and its BVH built ONCE; every further GPU of the spp split gets a copy of the finished
 // device data over NVLink (cudaMemcpyPeer) instead of a second feed + build.  Everything ptc_commit uploaded is position-independent
-// except the pointers of DScene and the texel pointers inside the material table, which are rebased here.
-static void forEachScenePointer(DScene &s, const std::function<void(const void **)> &f)
-{
-    const void **fields[] = {(const void **)&s.bvh.nodes, (const void **)&s.bvh.triangles, (const void **)&s.bvh.spheres, (const void **)&s.bvh.primEvent,
-                             (const void **)&s.bvh.sphereEvent, (const void **)&s.bvh.placements, (const void **)&s.positions, (const void **)&s.normals,
-                             (const void **)&s.uvs, (const void **)&s.prims, (const void **)&s.primIds, (const void **)&s.instIds, (const void **)&s.sphereIds,
-                             (const void **)&s.triShade, (const void **)&s.materials, (const void **)&s.lights, (const void **)&s.envRgba,
-                             (const void **)&s.envThetaCdf, (const void **)&s.envPhiCdf, (const void **)&s.envPhiEmpty, (const void **)&s.envThetaGuide,
-                             (const void **)&s.envPhiGuide, (const void **)&s.media, (const void **)&s.geomMedium, (const void **)&s.primClass,
-                             (const void **)&s.sphereClass};
-    for (const void **field : fields) { f(field); }
-}
-
+// except the pointers that lead to it, which each allocation records: they are pointed at the copies here.
 int ptc_replicate(ptc_ctx *src, int device, ptc_ctx **out)
 {
     if (!out) { return PTC_ERR_INVALID; }
@@ -1930,46 +1955,22 @@ int ptc_replicate(ptc_ctx *src, int device, ptc_ctx **out)
     ptc_ctx *dst = nullptr;
     int rc = ptc_create(device, &dst);
     if (rc) { CTX_FAIL(src, rc, "cannot create a context on device %d", device); }
-    // host-side state the calls after ptc_commit consult (the staged geometry itself is not needed any more)
-    dst->materials = src->materials; dst->media = src->media; dst->geometries = src->geometries; dst->scenes = src->scenes; dst->rootGeometry = src->rootGeometry;
-    dst->integrator = src->integrator; dst->hasEnv = src->hasEnv; dst->hasCamera = src->hasCamera;
-    dst->envW = src->envW; dst->envH = src->envH; dst->envScale = src->envScale;
-    memcpy(dst->envM2W, src->envM2W, sizeof(dst->envM2W)); memcpy(dst->envW2M, src->envW2M, sizeof(dst->envW2M));
-    memcpy(dst->camToWorld, src->camToWorld, sizeof(dst->camToWorld)); dst->vfov = src->vfov; dst->width = src->width; dst->height = src->height;
-    dst->bvh.placements = src->bvh.placements; dst->bvh.maxDepth = src->bvh.maxDepth; // nodes / triangles: fetchHostBvh, from this GPU's copy
-    memcpy(dst->bvh.sceneLo, src->bvh.sceneLo, sizeof(dst->bvh.sceneLo)); memcpy(dst->bvh.sceneHi, src->bvh.sceneHi, sizeof(dst->bvh.sceneHi));
-    dst->bvhNodeCount = src->bvhNodeCount; dst->bvhTriangleCount = src->bvhTriangleCount; dst->hostBvhFetched = false;
-    dst->nLights = src->nLights; dst->classMask = src->classMask;
-    dst->pathsPerWave = src->pathsPerWave; dst->stageTiming = src->stageTiming; dst->countTraversal = src->countTraversal; dst->volumeMegakernel = src->volumeMegakernel; dst->lanes = src->lanes;
-    dst->bvhBuilder = src->bvhBuilder; dst->bvhBuildMs = 0.f; dst->bvhPlocIterations = src->bvhPlocIterations;
-    dst->deviceMaterials = src->deviceMaterials;
-    dst->scene = src->scene;
+    static_cast<SceneState &>(dst->scene) = src->scene;
+    dst->scene.bvhBuildMs = 0.f; // nothing was built here
+    dst->options = src->options;
     auto fail = [&](const char *what) { src->error = std::string("ptc_replicate: ") + what + ": " + cudaGetErrorString(cudaGetLastError()); ptc_destroy(dst); return PTC_ERR_CUDA; };
     if (cudaSetDevice(device) != cudaSuccess) { return fail("cudaSetDevice"); }
-    for (const Buffer<uint8_t> &a : src->allocations) {
+    for (const SceneAllocation &a : src->scene.allocations) {
         Buffer<uint8_t> copy;
-        if (copy.resize(a.size()) != cudaSuccess) { return fail("cudaMalloc"); }
-        dst->allocations.push_back(std::move(copy));
-        if (cudaMemcpyPeerAsync(dst->allocations.back().get(), device, a.get(), src->device, a.size(), dst->stream) != cudaSuccess) { return fail("cudaMemcpyPeerAsync"); }
+        if (copy.resize(a.data.size()) != cudaSuccess) { return fail("cudaMalloc"); }
+        if (cudaMemcpyPeerAsync(copy.get(), device, a.data.get(), src->device, a.data.size(), dst->stream) != cudaSuccess) { return fail("cudaMemcpyPeerAsync"); }
+        if (a.field != NO_FIELD) { *(const void **)((char *)&dst->scene.view + a.field) = copy.get(); }
+        for (uint32_t m : a.materials) { dst->scene.materials[m].texels = (const uint32_t *)copy.get(); }
+        dst->scene.allocations.push_back({std::move(copy), a.field, a.materials});
     }
-    bool rebased = true;
-    auto rebase = [&](const void **field) {
-        if (!*field) { return; }
-        for (size_t i = 0; i < src->allocations.size(); i++) { if (src->allocations[i].get() == *field) { *field = dst->allocations[i].get(); return; } }
-        rebased = false;
-    };
-    forEachScenePointer(dst->scene, rebase);
-    for (DMaterial &m : dst->deviceMaterials) { rebase((const void **)&m.texels); }
-    if (!rebased) { src->error = "ptc_replicate: a scene pointer does not start one of the context's allocations"; ptc_destroy(dst); return PTC_ERR_STATE; }
-    if (!dst->deviceMaterials.empty() &&
-        cudaMemcpyAsync((void *)dst->scene.materials, dst->deviceMaterials.data(), dst->deviceMaterials.size() * sizeof(DMaterial), cudaMemcpyHostToDevice, dst->stream) != cudaSuccess) {
-        return fail("material table");
-    }
-    {
-        float gamma[256];
-        for (int c = 0; c < 256; c++) { gamma[c] = powf(c / 255.f, 2.2f); }
-        if (cudaMemcpyToSymbolAsync(c_gammaTable, gamma, sizeof(gamma), 0, cudaMemcpyHostToDevice, dst->stream) != cudaSuccess) { return fail("gamma table"); }
-    }
+    const std::vector<DMaterial> &dm = dst->scene.materials;
+    if (!dm.empty() && cudaMemcpyAsync((void *)dst->scene.view.materials, dm.data(), dm.size() * sizeof(DMaterial), cudaMemcpyHostToDevice, dst->stream) != cudaSuccess) { return fail("material table"); }
+    if (uploadGammaTable() != cudaSuccess) { return fail("gamma table"); }
     // the source's data must be complete before it is read (ptc_commit is synchronous, so it is) and the copies before `dst` is used
     if (cudaStreamSynchronize(dst->stream) != cudaSuccess) { return fail("copy"); }
     dst->committed = true;
@@ -2000,7 +2001,7 @@ static int ensurePathBuffers(ptc_ctx *ctx, uint32_t capacity, bool withClassQueu
     if (!withClassQueues) { return PTC_OK; }
     for (int t = 0; t < PTC_MATERIAL_CLASSES; t++) {
         pb.classQueue[t] = nullptr;
-        if (!(ctx->classMask & (1u << t))) { continue; }
+        if (!(ctx->scene.classMask & (1u << t))) { continue; }
         CUDA_TRY(ctx, ctx->classQueues[t].reserve(ctx->pathCapacity));
         pb.classQueue[t] = ctx->classQueues[t].get();
     }
@@ -2011,7 +2012,7 @@ int ptc_reserve_paths(ptc_ctx *ctx, uint64_t nPaths)
 {
     if (!ctx) { return PTC_ERR_INVALID; }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const uint64_t capacity = std::min<uint64_t>(std::max<uint64_t>(nPaths, 1), (uint64_t)ctx->pathsPerWave);
+    const uint64_t capacity = std::min<uint64_t>(std::max<uint64_t>(nPaths, 1), (uint64_t)ctx->options.pathsPerWave);
     return ensurePathBuffers(ctx, (uint32_t)capacity, false);
 }
 
@@ -2110,8 +2111,8 @@ struct WaveTraversals { Traversal extend0, extend, shadow, scatter; };
 // (profiles/r02_sweep_lanes.txt)
 static WaveTraversals pickTraversals(const ptc_ctx *ctx, bool volume, bool sharedSMs)
 {
-    const DScene &s = ctx->scene;
-    const bool count = ctx->countTraversal;
+    const DScene &s = ctx->scene.view;
+    const bool count = ctx->options.countTraversal;
     const int grid = sharedSMs ? ctx->gridTraverseShared : ctx->gridTraverse;
     const int volumeGrid = sharedSMs ? ctx->gridVolumeTraverseShared : ctx->gridVolumeTraverse;
     WaveTraversals t;
@@ -2150,7 +2151,7 @@ static void launchAccumulate(ptc_ctx *ctx, cudaStream_t stream, const PathBuffer
                              const CheckpointPlan &plan)
 {
     const auto kernel = moments ? accumulateKernel<true> : accumulateKernel<false>;
-    kernel<<<gridFor(ctx, wp.nPixels, 256), 256, 0, stream>>>(pb, wp, accumDevice, moments, (uint32_t)ctx->scene.width, (uint32_t)ctx->scene.height, plan);
+    kernel<<<gridFor(ctx, wp.nPixels, 256), 256, 0, stream>>>(pb, wp, accumDevice, moments, (uint32_t)ctx->scene.view.width, (uint32_t)ctx->scene.view.height, plan);
     ctx->launches++;
 }
 
@@ -2162,7 +2163,7 @@ static void launchAccumulate(ptc_ctx *ctx, cudaStream_t stream, const PathBuffer
 static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan *plans, int nLanes, float *accumDevice, float *moments, cudaStream_t callerStream,
                       bool volume, const SumsUpload *upload)
 {
-    const DScene &s = ctx->scene;
+    const DScene &s = ctx->scene.view;
     struct LaneState { PathBuffers pb; VolumeBuffers vb; BounceCounters *cnt; cudaStream_t stream, shadowStream; cudaEvent_t shadeDone, shadowDone; };
     LaneState lanes[PTC_MAX_LANES];
     if (nLanes > 1) {
@@ -2204,7 +2205,7 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
             cudaStream_t stream = l.stream;
             BounceCounters *bc = l.cnt + k;
             // shadow rays cast at vertex k (queued by material(k - 1)) go to the second stream, behind everything enqueued so far
-            const bool overlap = ctx->overlapShadow && k > 0;
+            const bool overlap = ctx->options.overlapShadow && k > 0;
             cudaStream_t shadowOn = overlap ? l.shadowStream : stream;
             if (overlap) {
                 CUDA_TRY(ctx, cudaEventRecord(l.shadeDone, stream));
@@ -2232,14 +2233,14 @@ static int launchWave(ptc_ctx *ctx, const WaveParams *wps, const CheckpointPlan 
             }
             {
                 StageTimer t(ctx, stream, STAGE_SHADE);
-                if (volume && k > 0) { volumeLogicKernel<<<ctx->gridVolumeLogic, 256, 0, stream>>>(s, pb, vb, wp, bc, ctx->classMask); }
+                if (volume && k > 0) { volumeLogicKernel<<<ctx->gridVolumeLogic, 256, 0, stream>>>(s, pb, vb, wp, bc, ctx->scene.classMask); }
                 else { // k = 0 of the VolumePathTracer: SampleIntegrator::samplePixel's own terms, as in the PathTracer wavefront
-                    logicKernel<<<ctx->gridLogic, 256, 0, stream>>>(s, pb, wp, bc, ctx->classMask, k);
+                    logicKernel<<<ctx->gridLogic, 256, 0, stream>>>(s, pb, wp, bc, ctx->scene.classMask, k);
                     if (k == 0 && s.hasFilter) { containerKernel<<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc); ctx->launches++; }
                 }
                 ctx->launches++;
                 for (int c = 0; c < PTC_MATERIAL_CLASSES; c++) {
-                    if (!(ctx->classMask & (1u << c))) { continue; }
+                    if (!(ctx->scene.classMask & (1u << c))) { continue; }
                     if (volume) { volumeMaterialKernels[c]<<<ctx->gridVolumeShade, 128, 0, stream>>>(s, pb, vb, wp, bc, bc + 1); }
                     else { materialKernels[wp.pixels != nullptr][c]<<<ctx->gridShade, 128, 0, stream>>>(s, pb, wp, bc, bc + 1); }
                     ctx->launches++;
@@ -2281,8 +2282,8 @@ static int volumeWave(ptc_ctx *ctx, const WaveParams &wp, const CheckpointPlan &
     CUDA_TRY(ctx, cudaMemsetAsync(cursor, 0, sizeof(uint32_t), stream));
     {
         StageTimer t(ctx, stream, STAGE_SHADE);
-        const auto kernel = ctx->countTraversal ? volumePathKernel<true> : volumePathKernel<false>;
-        kernel<<<ctx->gridVolume, 128, 0, stream>>>(ctx->scene, pb.out, wp, cursor, ctx->totals.get());
+        const auto kernel = ctx->options.countTraversal ? volumePathKernel<true> : volumePathKernel<false>;
+        kernel<<<ctx->gridVolume, 128, 0, stream>>>(ctx->scene.view, pb.out, wp, cursor, ctx->totals.get());
         ctx->launches++;
     }
     if (upload) { const int rc = uploadSums(ctx, *upload); if (rc) { return rc; } }
@@ -2299,12 +2300,12 @@ static int renderInternal(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uin
 {
     if (start < 0 || (last != -1 && start > last)) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bad bounce window [%d, %d]", start, last); }
     if (last == -1 || last > PTC_MAX_BOUNCES) { last = PTC_MAX_BOUNCES; }
-    const uint32_t nPixels = pass.moments ? pass.count : (uint32_t)ctx->scene.width * (uint32_t)ctx->scene.height;
-    uint32_t sppWave = (uint32_t)std::max<int64_t>(1, ctx->pathsPerWave / (int64_t)nPixels);
+    const uint32_t nPixels = pass.moments ? pass.count : (uint32_t)ctx->scene.view.width * (uint32_t)ctx->scene.view.height;
+    uint32_t sppWave = (uint32_t)std::max<int64_t>(1, ctx->options.pathsPerWave / (int64_t)nPixels);
     sppWave = std::min(sppWave, std::max(nSpp, 1u));
-    const bool volume = ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER;
+    const bool volume = ctx->options.integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER;
     // the one-thread-per-path kernel stays for instanced scenes (the volume traversal kernels test world-space leaves only) and as an option
-    const bool megakernel = volume && (ctx->volumeMegakernel || ctx->scene.bvh.placements);
+    const bool megakernel = volume && (ctx->options.volumeMegakernel || ctx->scene.view.bvh.placements);
     if (megakernel) {
         CUDA_TRY(ctx, ctx->volumeOut.reserve((size_t)nPixels * sppWave));
         CUDA_TRY(ctx, ctx->volumeCursor.resize(1));
@@ -2320,8 +2321,8 @@ static int renderInternal(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uin
         // lanes: consecutive blocks of the wave's samples.  Two lanes, four when the wave is small (measured on five scenes,
         // profiles/r02_sweep_lanes.txt); one for the megakernel, and while a stage or traversal counter pass describes one launch
         // sequence at a time
-        int nLanes = ctx->lanes > 0 ? ctx->lanes : ((uint64_t)nPixels * wp.sppWave <= (1u << 25) ? 4 : 2);
-        if (megakernel || ctx->stageTiming || ctx->countTraversal) { nLanes = 1; }
+        int nLanes = ctx->options.lanes > 0 ? ctx->options.lanes : ((uint64_t)nPixels * wp.sppWave <= (1u << 25) ? 4 : 2);
+        if (megakernel || ctx->options.stageTiming || ctx->options.countTraversal) { nLanes = 1; }
         nLanes = (int)std::min<uint32_t>((uint32_t)nLanes, wp.sppWave);
         WaveParams wps[PTC_MAX_LANES]; CheckpointPlan plans[PTC_MAX_LANES];
         const uint32_t perLane = (wp.sppWave + (uint32_t)nLanes - 1) / (uint32_t)nLanes;
@@ -2354,7 +2355,7 @@ int ptc_render(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp,
     NEED_COMMIT(ctx);
     if (!accum) { CTX_FAIL(ctx, PTC_ERR_INVALID, "null accumulation buffer"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)3 * ctx->scene.width * ctx->scene.height;
+    const size_t n = (size_t)3 * ctx->scene.view.width * ctx->scene.view.height;
     CUDA_TRY(ctx, ctx->accumScratch.reserve(n));
     CUDA_TRY(ctx, ctx->pinned.reserve(n));
     float *accumDevice = ctx->accumScratch.get();
@@ -2383,7 +2384,7 @@ int ptc_render(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t nSpp,
 // The framebuffer at the camera's resolution; a new one starts at zero
 static int ensureFramebuffer(ptc_ctx *ctx)
 {
-    const size_t n = (size_t)3 * ctx->scene.width * ctx->scene.height;
+    const size_t n = (size_t)3 * ctx->scene.view.width * ctx->scene.view.height;
     if (ctx->framebuffer.size() == n) { return PTC_OK; }
     CUDA_TRY(ctx, ctx->framebuffer.resize(n));
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer.get(), 0, n * sizeof(float), ctx->stream));
@@ -2400,11 +2401,11 @@ int ptc_framebuffer_clear(ptc_ctx *ctx)
     const size_t n = ctx->framebuffer.size();
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->framebuffer.get(), 0, n * sizeof(float), ctx->stream));
     // with the option on the moments exist from here, so that a context that gets no samples still has (zero) moments to gather
-    if (ctx->momentsOption) {
+    if (ctx->options.framebufferMoments) {
         CUDA_TRY(ctx, ctx->moments.resize(n));
         CUDA_TRY(ctx, cudaMemsetAsync(ctx->moments.get(), 0, n * sizeof(float), ctx->stream));
     }
-    ctx->momentsComplete = ctx->momentsOption;
+    ctx->momentsComplete = ctx->options.framebufferMoments;
     ctx->adaptive.on = false;
     return PTC_OK;
 }
@@ -2424,7 +2425,7 @@ int ptc_framebuffer_render_checkpoints(ptc_ctx *ctx, uint64_t seed, uint32_t fir
     int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
     const size_t n = ctx->framebuffer.size();
-    const bool withMoments = ctx->momentsOption;
+    const bool withMoments = ctx->options.framebufferMoments;
     // the moments need room behind the sums, and a new resolution new buffers
     if (nCounts && ((withMoments && !ctx->snapshotsHoldMoments) || ctx->snapshotSize != n)) {
         CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); // gathers that read the old snapshots are ordered before this stream's work
@@ -2602,7 +2603,7 @@ int ptc_adaptive_begin(ptc_ctx *ctx, const ptc_adaptive_desc *desc)
     const int rc = ensureFramebuffer(ctx);
     if (rc) { return rc; }
     ptc_ctx::Adaptive &a = ctx->adaptive;
-    const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
+    const size_t pixels = (size_t)ctx->scene.view.width * ctx->scene.view.height;
     a.pixels = 0; // until every buffer is sized for `pixels`
     CUDA_TRY(ctx, ctx->moments.resize(3 * pixels));
     CUDA_TRY(ctx, a.counts.resize(pixels));
@@ -2630,7 +2631,7 @@ int ptc_adaptive_pass(ptc_ctx *ctx, uint64_t seed, int start, int last, uint32_t
     NEED_COMMIT(ctx);
     ptc_ctx::Adaptive &a = ctx->adaptive;
     if (!a.on) { CTX_FAIL(ctx, PTC_ERR_STATE, "no adaptive render on this context: ptc_adaptive_begin first"); }
-    if (a.pixels != (size_t)ctx->scene.width * ctx->scene.height || ctx->framebuffer.size() != 3 * a.pixels) {
+    if (a.pixels != (size_t)ctx->scene.view.width * ctx->scene.view.height || ctx->framebuffer.size() != 3 * a.pixels) {
         CTX_FAIL(ctx, PTC_ERR_STATE, "the resolution changed during the adaptive render");
     }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
@@ -2644,7 +2645,7 @@ int ptc_adaptive_pass(ptc_ctx *ctx, uint64_t seed, int start, int last, uint32_t
         wp.nPixels = a.active; wp.pixels = pass.list;
         const double tau = (double)a.desc.threshold;
         adaptiveTestKernel<<<gridFor(ctx, a.active, 256), 256, 0, ctx->stream>>>(
-            wp, ctx->framebuffer.get(), ctx->moments.get(), a.counts.get(), a.next.get(), (uint32_t)ctx->scene.width, (uint32_t)ctx->scene.height, tau * tau, n, a.desc.max_spp);
+            wp, ctx->framebuffer.get(), ctx->moments.get(), a.counts.get(), a.next.get(), (uint32_t)ctx->scene.view.width, (uint32_t)ctx->scene.view.height, tau * tau, n, a.desc.max_spp);
         CUDA_TRY(ctx, cudaGetLastError());
         size_t bytes = a.scratch.size();
         CUDA_TRY(ctx, cub::DeviceSelect::If(a.scratch.get(), bytes, a.next.get(), a.list.get(), a.selected.get(), (int)a.active, StillActive(), ctx->stream));
@@ -2674,7 +2675,7 @@ int ptc_resolve_device(ptc_ctx *ctx, const float *accum, float *out, uint32_t sp
 {
     NEED_COMMIT(ctx);
     if (!accum || !out || !spp) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bad resolve arguments"); }
-    const uint32_t n = 3u * (uint32_t)ctx->scene.width * (uint32_t)ctx->scene.height;
+    const uint32_t n = 3u * (uint32_t)ctx->scene.view.width * (uint32_t)ctx->scene.view.height;
     resolveKernel<<<gridFor(ctx, n, 256), 256, 0, (cudaStream_t)stream>>>(accum, out, n, spp);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
@@ -2732,7 +2733,7 @@ static int checkDenoiseDesc(ptc_ctx *ctx, const ptc_denoise_desc *desc)
 static int denoiseAtrous(ptc_ctx *ctx, const ptc_denoise_desc *desc, const float4 *guide)
 {
     ptc_ctx::Denoise &d = ctx->denoise;
-    const int width = ctx->scene.width, height = ctx->scene.height;
+    const int width = ctx->scene.view.width, height = ctx->scene.view.height;
     DenoiseParams dp;
     dp.sigmaL = desc->sigma_l; dp.sigmaN = desc->sigma_n; dp.sigmaZ = desc->sigma_z; dp.sigmaA = desc->sigma_a; dp.eps = desc->eps;
     const dim3 block(32, 8), grid((unsigned)(width + 31) / 32, (unsigned)(height + 7) / 8);
@@ -2750,28 +2751,28 @@ int ptc_intersect(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit *hits)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !hits)) { return PTC_ERR_INVALID; }
-    return query(ctx, [&](const ptc_ray *r, ptc_hit *h) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, h, nullptr); },
+    return query(ctx, [&](const ptc_ray *r, ptc_hit *h) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, n, h, nullptr); },
                  host::in(rays, n), host::out(hits, n));
 }
 int ptc_intersect_instanced(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit *hits, uint32_t *instIds)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !hits || !instIds)) { return PTC_ERR_INVALID; }
-    return query(ctx, [&](const ptc_ray *r, ptc_hit *h, uint32_t *inst) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, h, (uint2 *)inst); },
+    return query(ctx, [&](const ptc_ray *r, ptc_hit *h, uint32_t *inst) { intersectKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, n, h, (uint2 *)inst); },
                  host::in(rays, n), host::out(hits, n), host::out(instIds, (size_t)2 * n));
 }
 int ptc_intersect_full(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_isect *out)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !out)) { return PTC_ERR_INVALID; }
-    return query(ctx, [&](const ptc_ray *r, ptc_isect *o) { intersectFullKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, o); },
+    return query(ctx, [&](const ptc_ray *r, ptc_isect *o) { intersectFullKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, n, o); },
                  host::in(rays, n), host::out(out, n));
 }
 int ptc_occluded(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t n, uint8_t *occluded)
 {
     NEED_COMMIT(ctx);
     if (n && (!rays || !maxT || !occluded)) { return PTC_ERR_INVALID; }
-    return query(ctx, [&](const ptc_ray *r, const float *t, uint8_t *o) { occludedKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, t, n, o); },
+    return query(ctx, [&](const ptc_ray *r, const float *t, uint8_t *o) { occludedKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, t, n, o); },
                  host::in(rays, n), host::in(maxT, n), host::out(occluded, n));
 }
 // the volumetric queries' per-ray event lists are optional outputs
@@ -2781,7 +2782,7 @@ int ptc_occluded_volumetric(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT
     if (n && (!rays || !maxT || !occluded)) { return PTC_ERR_INVALID; }
     return query(ctx,
                  [&](const ptc_ray *r, const float *t, uint8_t *o, uint32_t *en, float *et, uint32_t *em) {
-                     occludedVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, t, n, o, en, et, em);
+                     occludedVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, t, n, o, en, et, em);
                  },
                  host::in(rays, n), host::in(maxT, n), host::out(occluded, n), host::optionalOut(nEvents, n),
                  host::optionalOut(eventT, (size_t)n * PTC_MAX_EVENTS), host::optionalOut(eventMedium, (size_t)n * PTC_MAX_EVENTS));
@@ -2792,7 +2793,7 @@ int ptc_intersect_volumetric(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_
     if (n && (!rays || !out)) { return PTC_ERR_INVALID; }
     return query(ctx,
                  [&](const ptc_ray *r, ptc_isect *o, uint32_t *en, float *et, uint32_t *em) {
-                     intersectVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, o, en, et, em);
+                     intersectVolumetricKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, n, o, en, et, em);
                  },
                  host::in(rays, n), host::out(out, n), host::optionalOut(nEvents, n), host::optionalOut(eventT, (size_t)n * PTC_MAX_EVENTS),
                  host::optionalOut(eventMedium, (size_t)n * PTC_MAX_EVENTS));
@@ -2800,7 +2801,7 @@ int ptc_intersect_volumetric(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_
 int ptc_intersect_device(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit *hits, void *stream)
 {
     NEED_COMMIT(ctx);
-    intersectKernel<<<gridFor(ctx, n), 128, 0, (cudaStream_t)stream>>>(ctx->scene, rays, n, hits, nullptr);
+    intersectKernel<<<gridFor(ctx, n), 128, 0, (cudaStream_t)stream>>>(ctx->scene.view, rays, n, hits, nullptr);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
     return PTC_OK;
@@ -2808,7 +2809,7 @@ int ptc_intersect_device(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, ptc_hit 
 int ptc_occluded_device(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, uint32_t n, uint8_t *occluded, void *stream)
 {
     NEED_COMMIT(ctx);
-    occludedKernel<<<gridFor(ctx, n), 128, 0, (cudaStream_t)stream>>>(ctx->scene, rays, maxT, n, occluded);
+    occludedKernel<<<gridFor(ctx, n), 128, 0, (cudaStream_t)stream>>>(ctx->scene.view, rays, maxT, n, occluded);
     ctx->launches++;
     CUDA_TRY(ctx, cudaGetLastError());
     return PTC_OK;
@@ -2816,7 +2817,7 @@ int ptc_occluded_device(ptc_ctx *ctx, const ptc_ray *rays, const float *maxT, ui
 int ptc_camera_rays(ptc_ctx *ctx, const float *rowCol, uint32_t n, ptc_ray *rays)
 {
     NEED_COMMIT(ctx);
-    return query(ctx, [&](const float *rc, ptc_ray *r) { cameraRaysKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, rc, n, r); },
+    return query(ctx, [&](const float *rc, ptc_ray *r) { cameraRaysKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, rc, n, r); },
                  host::in(rowCol, (size_t)2 * n), host::out(rays, n));
 }
 // Guide buffers (denoise.cuh: aovKernel): the caller's sums go up, the kernel adds to them, they come back
@@ -2825,10 +2826,10 @@ int ptc_render_aovs(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, uint32_t 
     NEED_COMMIT(ctx);
     if (!albedo || !normal || !depth || !hits) { CTX_FAIL(ctx, PTC_ERR_INVALID, "null guide buffer"); }
     if (!nSpp) { return PTC_OK; } // no samples: the sums stay as they are
-    const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
+    const size_t pixels = (size_t)ctx->scene.view.width * ctx->scene.view.height;
     return query(ctx,
                  [&](float *a, float *nrm, float *z, uint32_t *h) {
-                     aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene, seed, firstSample, nSpp, a, nrm, z, h);
+                     aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene.view, seed, firstSample, nSpp, a, nrm, z, h);
                  },
                  host::inout(albedo, 3 * pixels), host::inout(normal, 3 * pixels), host::inout(depth, pixels), host::inout(hits, pixels));
 }
@@ -2839,7 +2840,7 @@ int ptc_framebuffer_guides(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, ui
     NEED_COMMIT(ctx);
     if (!nSpp) { CTX_FAIL(ctx, PTC_ERR_INVALID, "n_spp must be > 0: the guide records are means over the samples"); }
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    const size_t pixels = (size_t)ctx->scene.width * ctx->scene.height;
+    const size_t pixels = (size_t)ctx->scene.view.width * ctx->scene.view.height;
     CUDA_TRY(ctx, ctx->aovs.resize(8 * pixels));
     ptc_ctx::Guides &g = ctx->guides;
     g.aovSpp = 0; // no guides until this call has enqueued them
@@ -2848,7 +2849,7 @@ int ptc_framebuffer_guides(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, ui
     float *dAlbedo = d, *dNormal = d + 3 * pixels, *dDepth = d + 6 * pixels;
     uint32_t *dHits = (uint32_t *)(d + 7 * pixels);
     CUDA_TRY(ctx, cudaMemsetAsync(d, 0, 8 * pixels * sizeof(float), ctx->stream));
-    aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene, seed, firstSample, nSpp, dAlbedo, dNormal, dDepth, dHits);
+    aovKernel<<<gridFor(ctx, (uint32_t)pixels), 128, 0, ctx->stream>>>(ctx->scene.view, seed, firstSample, nSpp, dAlbedo, dNormal, dDepth, dHits);
     denoiseGuideKernel<<<gridFor(ctx, (uint32_t)pixels, 256), 256, 0, ctx->stream>>>(dAlbedo, dNormal, dDepth, dHits, nSpp, (uint32_t)pixels, g.records.get());
     ctx->launches += 2;
     CUDA_TRY(ctx, cudaGetLastError());
@@ -2859,7 +2860,7 @@ int ptc_framebuffer_guides(ptc_ctx *ctx, uint64_t seed, uint32_t firstSample, ui
         if (f.dst) { CUDA_TRY(ctx, cudaMemcpyAsync(f.dst, f.src, f.bytes, cudaMemcpyDeviceToHost, ctx->stream)); fetched = true; }
     }
     if (fetched) { CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream)); }
-    g.aovSpp = nSpp; g.width = ctx->scene.width; g.height = ctx->scene.height;
+    g.aovSpp = nSpp; g.width = ctx->scene.view.width; g.height = ctx->scene.view.height;
     return PTC_OK;
 }
 
@@ -2874,7 +2875,7 @@ int ptc_denoise(ptc_ctx *ctx, const ptc_denoise_desc *desc, const ptc_denoise_in
         CTX_FAIL(ctx, PTC_ERR_INVALID, "missing denoise input");
     }
     if (!in->aov_spp) { CTX_FAIL(ctx, PTC_ERR_INVALID, "aov_spp must be > 0"); }
-    const int width = ctx->scene.width, height = ctx->scene.height;
+    const int width = ctx->scene.view.width, height = ctx->scene.view.height;
     const size_t pixels = (size_t)width * height;
     if (in->counts) {
         for (size_t p = 0; p < pixels; p++) { if (in->counts[p] < 2) { CTX_FAIL(ctx, PTC_ERR_INVALID, "pixel %zu has %u samples: the variance needs 2", p, in->counts[p]); } }
@@ -2920,7 +2921,7 @@ int ptc_framebuffer_denoise_begin(ptc_ctx *root, ptc_ctx *const *peers, uint32_t
     CUDA_TRY(root, cudaSetDevice(root->device));
     if ((rc = ensureFramebuffer(root))) { return rc; }
     const size_t n = root->framebuffer.size(), pixels = n / 3;
-    if (!root->guides.aovSpp || root->guides.width != root->scene.width || root->guides.height != root->scene.height || 2 * pixels != root->guides.records.size()) { CTX_FAIL(root, PTC_ERR_STATE, "no guides of this resolution: ptc_framebuffer_guides first"); }
+    if (!root->guides.aovSpp || root->guides.width != root->scene.view.width || root->guides.height != root->scene.view.height || 2 * pixels != root->guides.records.size()) { CTX_FAIL(root, PTC_ERR_STATE, "no guides of this resolution: ptc_framebuffer_guides first"); }
     if (a.on && a.n == 0) { CTX_FAIL(root, PTC_ERR_STATE, "the adaptive render has no pass yet"); }
     if (a.on && snapshot >= 0) { CTX_FAIL(root, PTC_ERR_STATE, "an adaptive render keeps no checkpoint snapshots"); }
     const GatherSource sources[2] = {[&](ptc_ctx *c) { return gatherInput(c, snapshot, n, false); }, [&](ptc_ctx *c) { return gatherInput(c, snapshot, n, true); }};
@@ -2962,52 +2963,52 @@ int ptc_uniforms(ptc_ctx *ctx, uint64_t seed, const uint32_t *streams, uint32_t 
 int ptc_bsdf_eval(ptc_ctx *ctx, uint32_t material, const ptc_isect *isects, const float *wi, uint32_t n, float *f, float *pdf)
 {
     NEED_COMMIT(ctx);
-    if (material >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
+    if (material >= ctx->scene.materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
     return query(ctx,
                  [&](const ptc_isect *is, const float *w, float *fo, float *p) {
-                     bsdfEvalKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, is, w, n, fo, p);
+                     bsdfEvalKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, material, is, w, n, fo, p);
                  },
                  host::in(isects, n), host::in(wi, (size_t)3 * n), host::out(f, (size_t)3 * n), host::out(pdf, n));
 }
 int ptc_bsdf_sample(ptc_ctx *ctx, uint32_t material, const ptc_isect *isects, const float *xi, uint32_t n, float *wi, float *pdf, float *thr)
 {
     NEED_COMMIT(ctx);
-    if (material >= ctx->materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
+    if (material >= ctx->scene.materials.size()) { CTX_FAIL(ctx, PTC_ERR_INVALID, "material id out of range"); }
     return query(ctx,
                  [&](const ptc_isect *is, const float *x, float *w, float *p, float *t) {
-                     bsdfSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, material, is, x, n, w, p, t);
+                     bsdfSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, material, is, x, n, w, p, t);
                  },
                  host::in(isects, n), host::in(xi, (size_t)3 * n), host::out(wi, (size_t)3 * n), host::out(pdf, n), host::out(thr, (size_t)3 * n));
 }
 int ptc_light_sample(ptc_ctx *ctx, const float *ref, const float *xi, uint32_t n, ptc_light_sample_t *out)
 {
     NEED_COMMIT(ctx);
-    if (!ctx->nLights) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene has no lights"); }
-    return query(ctx, [&](const float *r, const float *x, ptc_light_sample_t *o) { lightSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, x, n, o); },
+    if (!ctx->scene.view.nLights) { CTX_FAIL(ctx, PTC_ERR_STATE, "scene has no lights"); }
+    return query(ctx, [&](const float *r, const float *x, ptc_light_sample_t *o) { lightSampleKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, x, n, o); },
                  host::in(ref, (size_t)3 * n), host::in(xi, (size_t)3 * n), host::out(out, n));
 }
 int ptc_light_pdf(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, float *pdf)
 {
     NEED_COMMIT(ctx);
-    return query(ctx, [&](const ptc_ray *r, float *p) { lightPdfKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, n, p); },
+    return query(ctx, [&](const ptc_ray *r, float *p) { lightPdfKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, n, p); },
                  host::in(rays, n), host::out(pdf, n));
 }
 int ptc_environment_radiance(ptc_ctx *ctx, const float *dirs, uint32_t n, float *rgb)
 {
     NEED_COMMIT(ctx);
-    return query(ctx, [&](const float *d, float *o) { envRadianceKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, d, n, o); },
+    return query(ctx, [&](const float *d, float *o) { envRadianceKernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, d, n, o); },
                  host::in(dirs, (size_t)3 * n), host::out(rgb, (size_t)3 * n));
 }
 int ptc_radiance_replay(ptc_ctx *ctx, const ptc_ray *rays, const float *xi, uint32_t stride, uint32_t n, int start, int last, float *rgb)
 {
     NEED_COMMIT(ctx);
     if (last == -1 || last > PTC_MAX_BOUNCES) { last = PTC_MAX_BOUNCES; }
-    const auto kernel = ctx->integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER ? volumeReplayKernel : radianceReplayKernel;
-    return query(ctx, [&](const ptc_ray *r, const float *x, float *o) { kernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene, r, x, stride, n, start, last, o); },
+    const auto kernel = ctx->options.integrator == PTC_INTEGRATOR_VOLUME_PATH_TRACER ? volumeReplayKernel : radianceReplayKernel;
+    return query(ctx, [&](const ptc_ray *r, const float *x, float *o) { kernel<<<gridFor(ctx, n), 128, 0, ctx->stream>>>(ctx->scene.view, r, x, stride, n, start, last, o); },
                  host::in(rays, n), host::in(xi, (size_t)n * stride), host::out(rgb, (size_t)3 * n));
 }
 
-int ptc_num_lights(ptc_ctx *ctx, uint32_t *out) { NEED_COMMIT(ctx); *out = ctx->nLights; return PTC_OK; }
+int ptc_num_lights(ptc_ctx *ctx, uint32_t *out) { NEED_COMMIT(ctx); *out = ctx->scene.view.nLights; return PTC_OK; }
 
 int ptc_get_stats(ptc_ctx *ctx, ptc_stats *out)
 {
@@ -3021,15 +3022,16 @@ int ptc_get_stats(ptc_ctx *ctx, ptc_stats *out)
     out->closest_rays = totals[0]; out->shadow_rays = totals[1]; out->samples = ctx->samples; out->kernel_launches = ctx->launches;
     out->extend_inner_visits = totals[2]; out->extend_triangle_tests = totals[3];
     out->shadow_inner_visits = totals[4]; out->shadow_triangle_tests = totals[5];
-    out->bvh_nodes = ctx->bvhNodeCount; out->bvh_triangles = ctx->bvhTriangleCount;
-    out->bvh_bytes = (size_t)ctx->bvhNodeCount * sizeof(WideNode) + (size_t)ctx->bvhTriangleCount * sizeof(LeafTriangle);
+    const Committed &sc = ctx->scene; // before ptc_commit: zeros
+    out->bvh_nodes = sc.view.bvh.nNodes; out->bvh_triangles = sc.bvhTriangles;
+    out->bvh_bytes = (size_t)sc.view.bvh.nNodes * sizeof(WideNode) + (size_t)sc.bvhTriangles * sizeof(LeafTriangle);
     out->extend_launches = ctx->stageLaunches[STAGE_EXTEND]; out->shadow_launches = ctx->stageLaunches[STAGE_SHADOW];
     out->shade_launches = ctx->stageLaunches[STAGE_SHADE];
     out->extend_ms = (float)ctx->stageMs[STAGE_EXTEND]; out->shadow_ms = (float)ctx->stageMs[STAGE_SHADOW];
     out->shade_ms = (float)ctx->stageMs[STAGE_SHADE]; out->other_ms = (float)ctx->stageMs[STAGE_OTHER];
     out->last_render_ms = ctx->lastRenderMs;
-    out->bvh_build_ms = ctx->bvhBuildMs; out->bvh_builder = (uint32_t)ctx->bvhBuilder; out->bvh_depth = ctx->bvh.maxDepth;
-    out->bvh_ploc_iterations = ctx->bvhPlocIterations;
+    out->bvh_build_ms = sc.bvhBuildMs; out->bvh_builder = (uint32_t)ctx->options.bvhBuilder; out->bvh_depth = sc.bvhDepth;
+    out->bvh_ploc_iterations = sc.bvhPlocIterations;
     return PTC_OK;
 }
 
@@ -3061,49 +3063,45 @@ int ptc_set_option(ptc_ctx *ctx, const char *name, int64_t value)
     if (!ctx || !name) { return PTC_ERR_INVALID; }
     if (!strcmp(name, "paths_per_wave")) { // path indices are 32-bit
         if (value < 1024 || value > (int64_t)1 << 30) { CTX_FAIL(ctx, PTC_ERR_INVALID, "paths_per_wave must be in [1024, 2^30]"); }
-        ctx->pathsPerWave = value; return PTC_OK;
+        ctx->options.pathsPerWave = value; return PTC_OK;
     }
-    if (!strcmp(name, "stage_timing")) { ctx->stageTiming = value != 0; return PTC_OK; }
-    if (!strcmp(name, "overlap_shadow")) { ctx->overlapShadow = value != 0; return PTC_OK; }
+    if (!strcmp(name, "stage_timing")) { ctx->options.stageTiming = value != 0; return PTC_OK; }
+    if (!strcmp(name, "overlap_shadow")) { ctx->options.overlapShadow = value != 0; return PTC_OK; }
     if (!strcmp(name, "lanes")) { // part-waves traced side by side (ptc_ctx::lanes)
         if (value < 0 || value > PTC_MAX_LANES) { CTX_FAIL(ctx, PTC_ERR_INVALID, "lanes must be in [0, %d] (0: chosen per wave)", PTC_MAX_LANES); }
-        ctx->lanes = (int)value; return PTC_OK;
+        ctx->options.lanes = (int)value; return PTC_OK;
     }
-    if (!strcmp(name, "count_traversal")) { ctx->countTraversal = value != 0; return PTC_OK; }
-    if (!strcmp(name, "volume_megakernel")) { ctx->volumeMegakernel = value != 0; return PTC_OK; }
+    if (!strcmp(name, "count_traversal")) { ctx->options.countTraversal = value != 0; return PTC_OK; }
+    if (!strcmp(name, "volume_megakernel")) { ctx->options.volumeMegakernel = value != 0; return PTC_OK; }
     if (!strcmp(name, "framebuffer_moments")) { // takes effect for the moments at the next ptc_framebuffer_clear
-        ctx->momentsOption = value != 0;
-        if (!ctx->momentsOption && !ctx->adaptive.on) { ctx->momentsComplete = false; } // an adaptive render's moments stay complete
+        ctx->options.framebufferMoments = value != 0;
+        if (!ctx->options.framebufferMoments && !ctx->adaptive.on) { ctx->momentsComplete = false; } // an adaptive render's moments stay complete
         return PTC_OK;
     }
     if (!strcmp(name, "bvh_builder")) { // before ptc_commit; 1 = device (default), 0 = host binned SAH
         if (ctx->committed) { CTX_FAIL(ctx, PTC_ERR_STATE, "bvh_builder must be set before ptc_commit"); }
         if (value != 0 && value != 1) { CTX_FAIL(ctx, PTC_ERR_INVALID, "bvh_builder must be 0 (host) or 1 (device)"); }
-        ctx->bvhBuilder = (int)value; return PTC_OK;
+        ctx->options.bvhBuilder = (int)value; return PTC_OK;
     }
     CTX_FAIL(ctx, PTC_ERR_INVALID, "unknown option %s", name);
-}
-
-// host copy of the device-resident BVH for the scalar traversal below
-static int fetchHostBvh(ptc_ctx *ctx)
-{
-    if (ctx->hostBvhFetched) { return PTC_OK; }
-    cudaSetDevice(ctx->device);
-    ctx->bvh.nodes.resize(ctx->bvhNodeCount); ctx->bvh.triangles.resize(ctx->bvhTriangleCount);
-    if (ctx->bvhNodeCount) {
-        CUDA_TRY(ctx, cudaMemcpy(ctx->bvh.nodes.data(), ctx->scene.bvh.nodes, (size_t)ctx->bvhNodeCount * sizeof(WideNode), cudaMemcpyDeviceToHost));
-        CUDA_TRY(ctx, cudaMemcpy(ctx->bvh.triangles.data(), ctx->scene.bvh.triangles, (size_t)ctx->bvhTriangleCount * sizeof(LeafTriangle), cudaMemcpyDeviceToHost));
-    }
-    ctx->hostBvhFetched = true;
-    return PTC_OK;
 }
 
 int ptc_count_traversal(ptc_ctx *ctx, const ptc_ray *rays, uint32_t n, uint64_t *inner, uint64_t *tris)
 {
     NEED_COMMIT(ctx);
-    { const int rc = fetchHostBvh(ctx); if (rc) { return rc; } }
+    if (!ctx->hostBvh) { // host copy of the device-resident BVH for the scalar traversal
+        cudaSetDevice(ctx->device);
+        const Committed &sc = ctx->scene;
+        WideBVH bvh;
+        bvh.nodes.resize(sc.view.bvh.nNodes); bvh.triangles.resize(sc.bvhTriangles); bvh.placements = sc.placements;
+        if (sc.view.bvh.nNodes) {
+            CUDA_TRY(ctx, cudaMemcpy(bvh.nodes.data(), sc.view.bvh.nodes, bvh.nodes.size() * sizeof(WideNode), cudaMemcpyDeviceToHost));
+            CUDA_TRY(ctx, cudaMemcpy(bvh.triangles.data(), sc.view.bvh.triangles, bvh.triangles.size() * sizeof(LeafTriangle), cudaMemcpyDeviceToHost));
+        }
+        ctx->hostBvh = std::move(bvh);
+    }
     TraversalCounts c;
-    for (uint32_t i = 0; i < n; i++) { traverseReference(ctx->bvh, rays[i].origin, rays[i].direction, PTC_TNEAR, PTC_TFAR, false, nullptr, nullptr, &c); }
+    for (uint32_t i = 0; i < n; i++) { traverseReference(*ctx->hostBvh, rays[i].origin, rays[i].direction, PTC_TNEAR, PTC_TFAR, false, nullptr, nullptr, &c); }
     if (inner) { *inner = c.innerVisits; }
     if (tris) { *tris = c.triangleTests; }
     return PTC_OK;
